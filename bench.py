@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --steps K --warmup W    # the reference's CPU path
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   # + what the last step returned
 
 A "step" is one complete Lloyd fit (BASELINE.json configs[1]: a 10-day 2048x2048 height-map
 stack per GPU, ~41.9 M pixels, k = 16, 20 iterations, tol = 0) over points already resident
@@ -12,6 +13,9 @@ with pinned HOST rasters in and host labels / centroids / fused cloud out.  One 
 printed by rank 0.  Sub-records of `roofline` say what the numbers are made of: the phases of a
 fit, the share of group-iterations settled without reading a point, the streaming path with
 settling disabled, and a cloud on which neither settling nor pruning can help (brute force).
+With `--dump-outputs DIR`, rank 0 writes what its last timed fit and its last end-to-end call
+returned as `DIR/<name>.npy` (float32 / float64, per-point arrays at a fixed seeded sample of
+points), so that two builds can be compared output for output on identical inputs.
 """
 from __future__ import annotations
 
@@ -49,6 +53,9 @@ CONFIGS = {
 # relative tolerance of the convergence test (sklearn's tol); config 5 is the time-to-solution run
 TOL = {"c5": 1e-4}
 C3 = {"D": 20, "H": 8192, "W": 8192, "k": 64, "iters": 20, "n_buildings": 1024}
+# --dump-outputs: per-point arrays of more points than this are written at a seeded sample of this
+# many points (config 2: ~29 MB in all instead of ~1.1 GB)
+DUMP_POINTS = 1 << 20
 
 
 def workload_name(cfg, n_gpus):
@@ -232,6 +239,29 @@ def run_reference(args):
 # ---------------------------------------------------------------------------------------
 # this repo's arm
 # ---------------------------------------------------------------------------------------
+def dump_sample(n, seed):
+    """Sorted indices of the points whose per-point outputs --dump-outputs writes: every point,
+    or DUMP_POINTS of them drawn with `seed` (the same draw for the same arguments)."""
+    if n <= DUMP_POINTS:
+        return np.arange(n, dtype=np.int64)
+    return np.sort(np.random.default_rng(seed).choice(n, DUMP_POINTS, replace=False))
+
+
+def fit_outputs(prefix, labels, centroids, inertia, n_iter):
+    """What a fit returns, as the float arrays --dump-outputs writes (labels < k fit float32 exactly)."""
+    return {prefix + "labels": np.asarray(labels).astype(np.float32),
+            prefix + "centroids": np.asarray(centroids, dtype=np.float64),
+            prefix + "inertia": np.array([inertia], dtype=np.float64),
+            prefix + "n_iter": np.array([n_iter], dtype=np.float64)}
+
+
+def write_outputs(path, arrays):
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def all_ranks_equal(t, world, dist):
     """True when the byte pattern of tensor `t` (CUDA) is identical on every rank."""
     import torch
@@ -423,6 +453,13 @@ def run_mine(args):
     if world > 1:
         sig = torch.from_numpy(np.concatenate([r["centers"].reshape(-1), [float(r["n_iter"]), r["inertia"]]])).to(dev)
         cross = all_ranks_equal(sig, world, dist)
+    # what the last timed fit returned, taken before later fits overwrite labels_dev
+    dumps = None
+    if args.dump_outputs and rank == 0:
+        sel = dump_sample(n_local, args.seed)
+        labels_sel = labels_dev[torch.from_numpy(sel).to(dev)].cpu().numpy()
+        dumps = {"point_index": sel.astype(np.float64),
+                 **fit_outputs("", labels_sel, r["centers"], r["inertia"], r["n_iter"])}
 
     # ---- the phases of a fit and the dominant kernel, timed alone with CUDA events ------------
     eng.profile(True)
@@ -520,6 +557,9 @@ def run_mine(args):
             its += res.n_iter
         barrier()
         wall = torch.tensor([time.perf_counter() - t0], dtype=torch.float64, device=dev)
+        if dumps is not None:
+            dumps.update(fit_outputs("e2e_", res.labels[sel], res.centroids, res.inertia, res.n_iter))
+            dumps["e2e_fused_cloud"] = res.fused_cloud[sel].astype(np.float32)
         if world > 1:
             dist.all_reduce(wall, op=dist.ReduceOp.MAX)
         e2e = {"value": n_total * its / float(wall.item()), "unit": UNIT,
@@ -631,6 +671,8 @@ def run_mine(args):
                                             "what": "c1-size stack: N-rank fit vs 1-rank fit -- centroids bitwise, "
                                                     "n_iter, labels, cloud, inertia to 1e-12"}
             line["config3"] = c3
+        if dumps is not None:
+            write_outputs(args.dump_outputs, dumps)
         print(json.dumps(line), flush=True)
     eng.close()
     if world > 1:
@@ -643,7 +685,7 @@ def run_mine(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=40)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 40; 5 with --impl reference)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="mine", choices=["mine", "reference"])
     ap.add_argument("--config", default="c2", choices=sorted(CONFIGS))
@@ -655,11 +697,19 @@ def main():
     ap.add_argument("--no-c3", action="store_true")
     ap.add_argument("--keep-caches", action="store_true",
                     help="re-use the mirror / group summaries across fits (default: rebuilt by every fit)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what rank 0's last timed fit and end-to-end call returned as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
-        if args.steps == 40:  # no --steps given: keep the default CPU run to a few minutes
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes what this repo's CUDA path returned: not with --impl reference")
+        if args.steps is None:  # keep the default CPU run to a few minutes
             args.steps = 5
         return run_reference(args)
+    if args.steps is None:
+        args.steps = 40
     if args.warmup < 3:
         args.warmup = 3  # timing rule: at least three warm-up steps
     return run_mine(args)

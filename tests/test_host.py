@@ -4,6 +4,9 @@ import ctypes
 import importlib
 import os
 import re
+import subprocess
+import sys
+import textwrap
 
 import numpy as np
 import pytest
@@ -88,18 +91,31 @@ def test_library_is_sm100a_only(built):
     assert archs == {"100a"}, archs
 
 
-def test_create_fails_loudly_without_gpu(built):
-    import torch
+def run_without_gpu(src):
+    """Runs `src` in a fresh interpreter that sees no CUDA device, so that what the package does
+    without a GPU is checked on machines that have one, too."""
+    src = f"import sys\nsys.path.insert(0, {ROOT!r})\n" + textwrap.dedent(src)
+    res = subprocess.run([sys.executable, "-c", src], cwd=ROOT, capture_output=True, text=True, timeout=600,
+                         env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert res.returncode == 0, res.stdout + res.stderr
 
-    if torch.cuda.is_available():
-        pytest.skip("a GPU is visible")
-    pkg = importlib.import_module(PKG)
-    with pytest.raises(Exception, match="MDKM_ERR_NO_DEVICE"):
-        pkg.Engine(0)
-    # the plugin wrapper keeps the reference's error-layer convention (plugin.py:236-241)
-    layers = pkg.MultiDayFusionPlugin().run(np.zeros((1, 4, 4), dtype=np.float32))
-    assert len(layers) == 1 and layers[0][2] == "image" and layers[0][1]["name"].startswith("Error:")
-    assert layers[0][0].shape == (100, 100)
+
+def test_create_fails_loudly_without_gpu(built):
+    run_without_gpu(f"""
+        import importlib
+        import numpy as np
+        import pytest
+        import torch
+
+        assert not torch.cuda.is_available()
+        pkg = importlib.import_module({PKG!r})
+        with pytest.raises(Exception, match="MDKM_ERR_NO_DEVICE"):
+            pkg.Engine(0)
+        # the plugin wrapper keeps the reference's error-layer convention (plugin.py:236-241)
+        layers = pkg.MultiDayFusionPlugin().run(np.zeros((1, 4, 4), dtype=np.float32))
+        assert len(layers) == 1 and layers[0][2] == "image" and layers[0][1]["name"].startswith("Error:")
+        assert layers[0][0].shape == (100, 100)
+    """)
 
 
 def test_product_never_imports_oracle():
@@ -325,14 +341,15 @@ def test_output_buffers_are_validated_not_copied():
 
 
 def test_plugin_error_is_logged_like_the_reference(tmp_path, built):
-    import torch
-
-    if torch.cuda.is_available():
-        pytest.skip("a GPU is visible")
-    pkg = importlib.import_module(PKG)
     log = tmp_path / "log.txt"
-    layers = pkg.MultiDayFusionPlugin(log_path=str(log)).run(np.zeros((1, 4, 4), dtype=np.float32))
-    assert layers[0][1]["name"].startswith("Error:")
+    run_without_gpu(f"""
+        import importlib
+        import numpy as np
+
+        pkg = importlib.import_module({PKG!r})
+        layers = pkg.MultiDayFusionPlugin(log_path={str(log)!r}).run(np.zeros((1, 4, 4), dtype=np.float32))
+        assert layers[0][1]["name"].startswith("Error:")
+    """)
     txt = log.read_text()  # plugin.py:238-239: "Error: <e>\n<traceback>"
     assert txt.startswith("Error: ") and "Traceback (most recent call last)" in txt
 
