@@ -814,7 +814,23 @@ struct FinalParams {
   FrameF f;
   int k, kpad;
   int split_rows;             // 1: raster-ordered cloud (row-major runs of pixels)
+  // the end of a fit, enqueued right behind its last batch of iterations:
+  int skip_paused;            // 1: do nothing but publish the status when it says paused && !done
+  DevStatus* status_host;     // or nullptr: the last CTA copies the status here (device-visible host memory)
+  double* centroids_host;     // or nullptr: the last CTA writes the k x 3 centroids (original coordinates) here
+  double origin[3];           // Frame::origin, for centroids_host
 };
+
+// Copies the status block into device-visible host memory (one thread).  L2 reads: other CTAs
+// updated it with atomics.
+__device__ __forceinline__ void publish_status(const DevStatus* st, DevStatus* dst) {
+  static_assert(sizeof(DevStatus) % 8 == 0, "status copied in 8-byte words");
+  const unsigned long long* s = reinterpret_cast<const unsigned long long*>(st);
+  unsigned long long* d = reinterpret_cast<unsigned long long*>(dst);
+#pragma unroll 4
+  for (int i = 0; i < (int)(sizeof(DevStatus) / 8); ++i) d[i] = __ldcg(s + i);
+  __threadfence_system();
+}
 
 // ---------------------------------------------------------------------------------------
 // Assignment of one warp-group.  xc/yc/zc: centred FP32 coordinates of this lane's 4 points;
@@ -2180,17 +2196,38 @@ __global__ void __launch_bounds__(kThreads, 1) lloyd_settle_kernel(const SettleP
   }
 }
 
-// Builds the centroid table from K x 3 float64 centroids in ORIGINAL coordinates.
+// Start of a fit (one launch): the status block, cleared accumulators and counters, and the
+// centroid table from K x 3 float64 centroids in ORIGINAL coordinates.
 struct InitTableParams {
-  const double* centers;  // device, k*3
+  const double* centers;  // k*3, device or device-visible host memory
   unsigned char* table;
   DevStatus* st;
   Frame fr;
   int k, kpad;
+  DevStatus st0;                    // written to *st
+  unsigned long long* acc;          // acc_words words zeroed (or nullptr)
+  long long acc_words;
+  int* work_count;                  // two counters zeroed (or nullptr)
+  unsigned int* final_ticket;       // zeroed (lloyd_final_kernel)
+  const unsigned int* index_fault;  // or nullptr: nonzero when the raster mirror index timed out -> status done + fault
 };
 
 __global__ void __launch_bounds__(kThreads, 1) init_table_kernel(const InitTableParams u) {
   __shared__ double s_red[kThreads / 32];
+  if (threadIdx.x == 0) {
+    DevStatus s = u.st0;
+    if (u.index_fault && *u.index_fault) {
+      s.done = 1;
+      s.xchg_timeout = 2;
+    }
+    *u.st = s;
+    *u.final_ticket = 0u;
+    if (u.work_count) {
+      u.work_count[0] = 0;
+      u.work_count[1] = 0;
+    }
+  }
+  for (long long i = threadIdx.x; i < u.acc_words; i += kThreads) u.acc[i] = 0ull;
   float4* fast = reinterpret_cast<float4*>(u.table);
   double4* exact = reinterpret_cast<double4*>(u.table + exact_offset(u.kpad));
   double m_cn = 0.0, m_cx = 0.0, m_cy = 0.0, m_cz = 0.0;
@@ -2334,6 +2371,10 @@ __global__ void __launch_bounds__(kThreads, kChunks == 0 ? MDKM_FINAL_CTAS0 : 3)
   const int warp = tid >> 5;
   const uint32_t bkt_bytes = kChunks == 0 ? (uint32_t)bucket_bytes(p.k, p.kpad) : 0u;
   unsigned char* s_bkt = reinterpret_cast<unsigned char*>(s_fast + kp32);
+  if (p.skip_paused && p.st->paused && !p.st->done) {  // (grid-uniform) the host relocates and runs the tail again
+    if (blockIdx.x == 0 && tid == 0 && p.status_host) publish_status(p.st, p.status_host);
+    return;
+  }
   if (tid == 0) {
     mbar_init(&s_bar, 1);
     fence_mbar_init();
@@ -2441,9 +2482,18 @@ __global__ void __launch_bounds__(kThreads, kChunks == 0 ? MDKM_FINAL_CTAS0 : 3)
     double v = 0.0;
     for (int i = tid; i < (int)gridDim.x; i += kThreads) v += p.partials[i];
     const double tot = block_sum_fixed(v, s_red);
+    if (p.centroids_host) {
+      for (int j = tid; j < p.k; j += kThreads) {
+        const double4 c = c64[j];
+        p.centroids_host[3 * j + 0] = c.x + p.origin[0];
+        p.centroids_host[3 * j + 1] = c.y + p.origin[1];
+        p.centroids_host[3 * j + 2] = c.z + p.origin[2];
+      }
+    }
     if (tid == 0) {
       p.st->inertia = tot;
       *p.ticket = 0u;
+      if (p.status_host) publish_status(p.st, p.status_host);
     }
   }
 }

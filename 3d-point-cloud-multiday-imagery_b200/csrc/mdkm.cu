@@ -96,6 +96,7 @@ struct mdkm_handle {
   int run_H = 0;
   DevBuf<unsigned char> druns;
   DevBuf<unsigned int> gfirst;
+  DevBuf<unsigned long long> index_status;  // raster_index_kernel: ticket + fault flag, look-back words
   int opt_raster_mirror = 1;  // MDKM_OPT_RASTER_MIRROR
   int opt_cell_px = 0, opt_cell_rows = 0;  // MDKM_OPT_CELL_PX / MDKM_OPT_CELL_ROWS (0 = automatic)
   int opt_two_level = -1;                  // MDKM_OPT_TWO_LEVEL (-1 = automatic)
@@ -533,7 +534,7 @@ int build_mirror(mdkm_handle* h, int cell_px) {
 }
 
 // The same for a raster cloud that came with a run table: cell sizes and the place of every run
-// follow from the table (two kernels over the cells), the copy is a gather by destination that
+// follow from the table (one scan over the runs), the copy is a gather by destination that
 // also writes the group summaries.  No histogram pass over the points, no atomics.
 int build_mirror_raster(mdkm_handle* h, int cell_px) {
   const long long cap = round_up(std::max<long long>(h->n, 1), kGroup);
@@ -561,13 +562,11 @@ int build_mirror_raster(mdkm_handle* h, int cell_px) {
   g.gy = (g.yext + g.rpc - 1) / g.rpc;
   const long long n_cells = (long long)g.gx * g.gy;
   const long long n_entries = n_cells * g.nd * g.rpc;
-  if (n_cells >= (1ll << 31) || n_entries >= (1ll << 32)) return fail(h, MDKM_ERR_INVALID, "raster too large for the run list");
-  const int n_tiles = (int)((n_cells + kScanTile - 1) / kScanTile);
-  OK(ensure(h, h->cell_counts, (size_t)n_tiles * kScanTile));
-  OK(ensure(h, h->cell_offsets, (size_t)n_cells + 2));
+  if (n_cells >= (1ll << 31) || n_entries + kIndexTile >= (1ll << 32)) return fail(h, MDKM_ERR_INVALID, "raster too large for the run list");
+  const long long n_tiles = (n_entries + kIndexTile - 1) / kIndexTile;
   OK(ensure(h, h->druns, ((size_t)n_entries + 1) * sizeof(uint2)));
   OK(ensure(h, h->gfirst, (size_t)n_groups));
-  OK(ensure(h, h->partials, (size_t)std::max(n_tiles, h->sm_count * 8) * 8 + 16));
+  OK(ensure(h, h->index_status, (size_t)n_tiles + 1));  // ticket + fault flag, then the look-back words
   if (h->n == 0) {
     CU(cudaMemsetAsync(h->tpts.p, 0, kBlockFloats * 4, h->stream));
     group_summary_kernel<<<1, kThreads, 0, h->stream>>>(h->tpts.p, h->n, h->ff, reinterpret_cast<GroupSummary*>(h->gsum.p));
@@ -575,18 +574,27 @@ int build_mirror_raster(mdkm_handle* h, int cell_px) {
     CU(cudaGetLastError());
     return MDKM_OK;
   }
-  const int cgrid = grid_for(h, (n_cells + 7) / 8, resident_per_sm(h, raster_runs_kernel));  // one warp per cell
-  raster_cell_count_kernel<<<grid_for(h, (n_cells + kThreads - 1) / kThreads, resident_per_sm(h, raster_cell_count_kernel)), kThreads, 0,
-                             h->stream>>>(g, h->cell_counts.p);  // one thread per cell
-  long long* tile_sums = reinterpret_cast<long long*>(h->partials.p);
-  mirror_tile_sums_kernel<<<n_tiles, 1024, 0, h->stream>>>(h->cell_counts.p, n_cells, tile_sums);
-  mirror_scan_kernel<<<n_tiles, 1024, 0, h->stream>>>(h->cell_counts.p, n_cells, h->cell_offsets.p, tile_sums);
-  raster_runs_kernel<<<cgrid, kThreads, 0, h->stream>>>(g, h->cell_offsets.p, h->n, reinterpret_cast<uint2*>(h->druns.p),
-                                                        h->gfirst.p);
-  raster_gather_kernel<<<grid_for(h, (n_groups + 7) / 8, resident_per_sm(h, raster_gather_kernel)), kThreads, 0, h->stream>>>(
-      h->pts.p, h->n, reinterpret_cast<const uint2*>(h->druns.p), n_entries, h->gfirst.p, h->ff, h->tpts.p,
-      reinterpret_cast<float4*>(h->gsum.p));
-  h->launches += 5;
+  CU(cudaMemsetAsync(h->index_status.p, 0, ((size_t)n_tiles + 1) * 8, h->stream));
+  raster_index_kernel<<<(unsigned int)n_tiles, kThreads, 0, h->stream>>>(
+      g, h->n, (unsigned int)n_entries, h->index_status.p + 1, reinterpret_cast<unsigned int*>(h->index_status.p),
+      reinterpret_cast<uint2*>(h->druns.p), h->gfirst.p);
+  CU(cudaGetLastError());
+  // the gather is set up while the index kernel drains (it waits for the whole grid before it reads)
+  const uint2* druns = reinterpret_cast<const uint2*>(h->druns.p);
+  const unsigned int* gfirst = h->gfirst.p;
+  float4* gsum = reinterpret_cast<float4*>(h->gsum.p);
+  void* args[] = {&h->pts.p, &h->n, &druns, const_cast<long long*>(&n_entries), &gfirst, &h->ff, &h->tpts.p, &gsum};
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = dim3(grid_for(h, (n_groups + 7) / 8, resident_per_sm(h, raster_gather_kernel)));
+  cfg.blockDim = dim3(kThreads);
+  cfg.stream = h->stream;
+  cudaLaunchAttribute attr;
+  attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr.val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = &attr;
+  cfg.numAttrs = h->opt_pdl ? 1 : 0;
+  CU(cudaLaunchKernelExC(&cfg, reinterpret_cast<const void*>(raster_gather_kernel), args));
+  h->launches += 2;
   CU(cudaGetLastError());
   return MDKM_OK;
 }
@@ -788,19 +796,39 @@ int launch_settle(mdkm_handle* h, const KmBuffers& kb) {
   return MDKM_OK;
 }
 
-int upload_table(mdkm_handle* h, const KmBuffers& kb, const double* centers_host) {
-  CU(cudaMemcpyAsync(h->dscratch.p, centers_host, (size_t)kb.k * 3 * sizeof(double), cudaMemcpyHostToDevice,
-                     h->stream));
+// Start of a fit / step / prediction in one launch: the status block `st0`, the first `acc_slots`
+// accumulator slots and the work counters cleared, the centroid table built from `centers_host`
+// (staged in the device-visible host buffer: no pageable copy on the stream).
+int fit_head(mdkm_handle* h, const KmBuffers& kb, const DevStatus& st0, const double* centers_host, int acc_slots) {
+  const size_t bytes = (size_t)kb.k * 3 * sizeof(double);
+  const size_t off = (h->mapped_used + 15) & ~(size_t)15;
+  if (off + bytes > kMappedBytes) return fail(h, MDKM_ERR_INVALID, "small result buffer exhausted");
+  memcpy(h->mapped + off, centers_host, bytes);  // (free: sync_small waited for every earlier reader)
+  h->mapped_used = off + bytes;
   InitTableParams ip{};
-  ip.centers = h->dscratch.p;
+  ip.centers = reinterpret_cast<const double*>(h->mapped + off);
   ip.table = h->table.p;
   ip.st = h->d_status;
   ip.fr = h->fr;
   ip.k = kb.k; ip.kpad = kb.kpad;
+  ip.st0 = st0;
+  ip.acc = h->acc.p;
+  ip.acc_words = (long long)acc_slots * (kb.kpad * 4 + 8);
+  ip.work_count = acc_slots ? h->worklist.p + kb.n_groups : nullptr;
+  ip.final_ticket = h->uscratch.p;
+  ip.index_fault = h->index_status.p ? reinterpret_cast<const unsigned int*>(h->index_status.p) + 1 : nullptr;
   init_table_kernel<<<1, kThreads, 0, h->stream>>>(ip);
   ++h->launches;
   CU(cudaGetLastError());
   return MDKM_OK;
+}
+
+// The raster mirror index of this cloud timed out in its look-back (fit_head turned that into a
+// finished run with status xchg_timeout = 2): report it; the next call rebuilds the mirror.
+int index_fault(mdkm_handle* h) {
+  h->summary_ok = false;
+  CU(cudaMemsetAsync(h->index_status.p, 0, 8, h->stream));
+  return fail(h, MDKM_ERR_CUDA, "raster mirror index: a tile's look-back timed out");
 }
 
 // Profiling spans: prof_begin records an event on the compute stream and returns the span's
@@ -834,7 +862,8 @@ int collect_profile(mdkm_handle* h) {
   return MDKM_OK;
 }
 
-int run_final(mdkm_handle* h, const KmBuffers& kb, int* labels_dev);
+int run_final(mdkm_handle* h, const KmBuffers& kb, int* labels_dev, bool skip_paused = false,
+              double* centroids_host = nullptr, DevStatus* status_host = nullptr);
 
 // Empty-cluster relocation (sklearn/_k_means_common.pyx:167-211), sequenced from the host
 // while the Lloyd loop is paused.  All arithmetic on the device (extras.cuh).
@@ -877,8 +906,9 @@ int relocate_empty(mdkm_handle* h, const KmBuffers& kb, int n_empty) {
   return MDKM_OK;
 }
 
-int run_final(mdkm_handle* h, const KmBuffers& kb, int* labels_dev) {
-  CU(cudaMemsetAsync(h->uscratch.p, 0, 4, h->stream));
+// (the ticket is zero: fit_head clears it, every final pass leaves it so)
+int run_final(mdkm_handle* h, const KmBuffers& kb, int* labels_dev, bool skip_paused, double* centroids_host,
+              DevStatus* status_host) {
   FinalParams fp{};
   fp.pts = h->pts.p; fp.n = h->n;
   fp.labels_out = labels_dev;
@@ -889,6 +919,10 @@ int run_final(mdkm_handle* h, const KmBuffers& kb, int* labels_dev) {
   fp.f = h->ff;
   fp.k = kb.k; fp.kpad = kb.kpad;
   fp.split_rows = h->raster_w > 0 ? 1 : 0;
+  fp.skip_paused = skip_paused ? 1 : 0;
+  fp.status_host = status_host;
+  fp.centroids_host = centroids_host;
+  for (int d = 0; d < 3; ++d) fp.origin[d] = h->fr.origin[d];
   kb.final_fn<<<kb.final_grid, kThreads, kb.final_smem, h->stream>>>(fp);
   ++h->launches;
   CU(cudaGetLastError());
@@ -959,7 +993,7 @@ void mdkm_destroy(mdkm_handle* h) {
   release(h->labels); release(h->table); release(h->acc); release(h->labels32);
   release(h->dscratch); release(h->partials); release(h->uscratch); release(h->reloc);
   release(h->gsum); release(h->ssum); release(h->glabel); release(h->worklist);
-  release(h->tpts); release(h->cell_counts); release(h->cell_offsets);
+  release(h->tpts); release(h->cell_counts); release(h->cell_offsets); release(h->index_status);
   release(h->run_src); release(h->druns); release(h->gfirst);
   release(h->tile_status); release(h->chunk_offsets); release(h->staging); release(h->planes);
   release(h->d_seg_off); release(h->sel_hist); release(h->sel_targets);
@@ -1521,13 +1555,9 @@ int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol
   st0.first = 1;
   st0.tol = tol_scaled;
   st0.epoch = h->epoch_base;
-  h->h_status[0] = st0;
-  CU(cudaMemcpyAsync(h->d_status, &h->h_status[0], sizeof(DevStatus), cudaMemcpyHostToDevice, h->stream));
   const size_t acc_slot = (size_t)kb.kpad * 4 + 8;
-  CU(cudaMemsetAsync(h->acc.p, 0, 3 * acc_slot * 8, h->stream));
-  CU(cudaMemsetAsync(h->worklist.p + kb.n_groups, 0, 8, h->stream));
   h->step_seq = 0;
-  OK(upload_table(h, kb, init));
+  OK(fit_head(h, kb, st0, init, /*acc_slots=*/3));
 
   // the host-sequenced rare path (empty cluster): everything behind the pause has left early;
   // relocate on the device from the parked global sums, finish the paused iteration
@@ -1545,9 +1575,12 @@ int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol
   };
 
   // Lloyd loop: batches of iterations are enqueued back to back; the host only looks at the
-  // device status between batches, one batch behind the GPU (no per-iteration sync).
+  // device status between batches, one batch behind the GPU (no per-iteration sync).  Once the last
+  // batch is enqueued the end of the fit goes right behind it, without waiting: a pause or an early
+  // exit makes every later kernel return at once, the final pass does nothing on a pause, and the
+  // host, after its one synchronisation, relocates and runs the end again.
   int enq = 0;  // iterations enqueued that can still complete
-  for (;;) {  // (one pass, unless the very last update finds an empty cluster)
+  for (;;) {  // (one pass, unless an update finds an empty cluster in the last batch)
     int inflight = 0, head = 0, tail = 0;
     while (true) {
       while (inflight < 2 && enq < max_iter) {
@@ -1565,19 +1598,14 @@ int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol
           }
         }
         prof_end(h, span);
+        enq += nb;
+        if (enq >= max_iter) break;  // (the end of the fit publishes the status of the last batch)
         OK(small_d2h(h, &h->h_status[tail], h->d_status, sizeof(DevStatus), /*dst_is_pinned=*/true));
         CU(cudaEventRecord(h->batch_ev[tail], h->stream));
         tail ^= 1;
         ++inflight;
-        enq += nb;
       }
-      if (inflight == 0) break;
-      if (inflight == 2 && enq >= max_iter) {
-        // nothing more to enqueue: the newer batch's status supersedes the older one (a pause or
-        // an early exit makes every later kernel return at once), so wait only for that
-        head ^= 1;
-        --inflight;
-      }
+      if (enq >= max_iter) break;
       CU(cudaEventSynchronize(h->batch_ev[head]));
       const DevStatus s = h->h_status[head];
       head ^= 1;
@@ -1606,28 +1634,41 @@ int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol
         labels_dev = h->labels32.p;
       }
     }
+    // one rank: the final kernel's last CTA also writes the centroids and the status to the host;
+    // several: the inertia is summed over the ranks first
+    const bool one_rank = h->n_ranks == 1;
+    double* centroids_host = nullptr;
+    if (one_rank && centroids_out) {
+      const size_t bytes = (size_t)k * 3 * sizeof(double);
+      const size_t off = (h->mapped_used + 15) & ~(size_t)15;
+      if (off + bytes > kMappedBytes) return fail(h, MDKM_ERR_INVALID, "small result buffer exhausted");
+      h->mapped_used = off + bytes;
+      h->small_pending.push_back({centroids_out, off, bytes});
+      centroids_host = reinterpret_cast<double*>(h->mapped + off);
+    }
     // labels in the reference's point order: always recomputed from the final centroids (the
     // stored ones follow the mirror's order).  After a strict exit the table equals the one the
     // last E-step used -- the sums are integers -- so this reproduces that step's labels exactly.
     {
       const int span = prof_begin(h, MDKM_PHASE_FINAL, h->n);
-      OK(run_final(h, kb, labels_dev));
+      OK(run_final(h, kb, labels_dev, /*skip_paused=*/true, centroids_host, one_rank ? &h->h_status[0] : nullptr));
       prof_end(h, span);
     }
-    OK(ensure(h, h->dscratch, (size_t)k * 3 + 16));
-    read_table_kernel<<<(k + 255) / 256, 256, 0, h->stream>>>(h->table.p, k, kb.kpad, h->fr, h->dscratch.p);
-    ++h->launches;
-    CU(cudaGetLastError());
-    if (h->n_ranks > 1) OK(allreduce(h, &h->d_status->inertia, 1, kNcclFloat64, kNcclSum));
-    if (centroids_out) OK(small_d2h(h, centroids_out, h->dscratch.p, (size_t)k * 3 * sizeof(double)));
-    OK(small_d2h(h, &h->h_status[0], h->d_status, sizeof(DevStatus), /*dst_is_pinned=*/true));
+    if (!one_rank) {
+      OK(ensure(h, h->dscratch, (size_t)k * 3 + 16));
+      read_table_kernel<<<(k + 255) / 256, 256, 0, h->stream>>>(h->table.p, k, kb.kpad, h->fr, h->dscratch.p);
+      ++h->launches;
+      CU(cudaGetLastError());
+      OK(allreduce(h, &h->d_status->inertia, 1, kNcclFloat64, kNcclSum));
+      if (centroids_out) OK(small_d2h(h, centroids_out, h->dscratch.p, (size_t)k * 3 * sizeof(double)));
+      OK(small_d2h(h, &h->h_status[0], h->d_status, sizeof(DevStatus), /*dst_is_pinned=*/true));
+    }
     if (labels_out && labels_mem != MDKM_MEM_DEVICE && h->n > 0)
       CU(cudaMemcpyAsync(labels_out, labels_dev, (size_t)h->n * 4, cudaMemcpyDeviceToHost, h->stream));
     OK(sync_small(h));
     if (h->h_status[0].paused && !h->h_status[0].done && !h->h_status[0].xchg_timeout) {
-      // the settle kernel found an empty cluster in the very last update: relocate, go on
+      // an update of the last batch, or the settle kernel, found an empty cluster: relocate, go on
       const DevStatus s = h->h_status[0];
-      CU(cudaStreamSynchronize(h->stream));
       OK(relocate_and_resume(s, enq));
       continue;
     }
@@ -1643,6 +1684,7 @@ int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol
           (fin.t_classify_done - fin.t_start) * 1e-3, (double)fin.t_update_done * 1e-3 / std::max(1, kb.step_grid),
           (fin.t_last_done - fin.t_start) * 1e-3);
 #endif
+  if (fin.xchg_timeout == 2) return index_fault(h);
   if (fin.xchg_timeout) return fail(h, MDKM_ERR_NCCL, "a kernel-side wait timed out (peer exchange of the partial sums: a rank is missing; or the grid barrier)");
   if (n_iter_out) *n_iter_out = fin.iter;
   if (inertia_out) *inertia_out = fin.inertia;
@@ -1681,11 +1723,7 @@ int mdkm_lloyd_step(mdkm_handle* h, int k, const double* centroids, int32_t* lab
   st0.k = k;
   st0.first = 1;
   st0.epoch = h->epoch_base;
-  h->h_status[0] = st0;
-  CU(cudaMemcpyAsync(h->d_status, &h->h_status[0], sizeof(DevStatus), cudaMemcpyHostToDevice, h->stream));
-  CU(cudaMemsetAsync(h->acc.p, 0, ((size_t)kb.kpad * 4 + 8) * 8, h->stream));
-  CU(cudaMemsetAsync(h->worklist.p + kb.n_groups, 0, 8, h->stream));
-  OK(upload_table(h, kb, centroids));
+  OK(fit_head(h, kb, st0, centroids, /*acc_slots=*/1));
   OK(launch_step(h, kb, 1));
   OK(allreduce(h, h->acc.p, (size_t)kb.kpad * 4 + 8, kNcclUint64, kNcclSum));
   OK(ensure(h, h->dscratch, (size_t)k * 4 + 16));
@@ -1711,6 +1749,7 @@ int mdkm_lloyd_step(mdkm_handle* h, int k, const double* centroids, int32_t* lab
   h->stat_refined = (long long)h->h_status[0].n_refined;
   h->stat_reloc = 0;
   OK(collect_profile(h));
+  if (h->h_status[0].xchg_timeout == 2) return index_fault(h);
   if (h->h_status[0].xchg_timeout) return fail(h, MDKM_ERR_CUDA, "the step kernel's grid barrier timed out");
   return MDKM_OK;
 }
@@ -1727,9 +1766,7 @@ int mdkm_predict(mdkm_handle* h, int k, const double* centroids, int32_t* labels
   st0.k = k;
   st0.first = 1;
   st0.epoch = h->epoch_base;
-  h->h_status[0] = st0;
-  CU(cudaMemcpyAsync(h->d_status, &h->h_status[0], sizeof(DevStatus), cudaMemcpyHostToDevice, h->stream));
-  OK(upload_table(h, kb, centroids));
+  OK(fit_head(h, kb, st0, centroids, /*acc_slots=*/0));
   int* labels_dev = nullptr;
   if (labels_out) {
     labels_dev = labels_out;
@@ -1744,6 +1781,7 @@ int mdkm_predict(mdkm_handle* h, int k, const double* centroids, int32_t* labels
   if (labels_out && labels_mem != MDKM_MEM_DEVICE && h->n > 0)
     CU(cudaMemcpyAsync(labels_out, labels_dev, (size_t)h->n * 4, cudaMemcpyDeviceToHost, h->stream));
   OK(sync_small(h));
+  if (h->h_status[0].xchg_timeout == 2) return index_fault(h);
   if (inertia_out) *inertia_out = h->h_status[0].inertia;
   h->stat_refined = (long long)h->h_status[0].n_refined;
   h->stat_reloc = 0;

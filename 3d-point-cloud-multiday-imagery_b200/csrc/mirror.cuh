@@ -231,8 +231,8 @@ __global__ void __launch_bounds__(kThreads) mirror_scatter_kernel(const float* p
 // (UnprojParams::run_src): for every 8 pixels of the range, how many points the pixels before
 // them produced.  The points of an 8- or 16-pixel run of one row are consecutive in the cloud,
 // the table says where they start and how many there are -- so the size of every cell, and the
-// place of every run inside its cell, follow from the table alone (two small kernels over the
-// cells, nothing per point), and the copy itself is a GATHER BY DESTINATION: one warp per group
+// place of every run inside its cell, follow from the table alone (one scan over the runs,
+// nothing per point), and the copy itself is a GATHER BY DESTINATION: one warp per group
 // of 128 mirror points looks up the handful of runs that make up the group, fetches them
 // (64-byte pieces of the cloud), writes the 1536-byte block in one piece and, having the whole
 // group in registers, also emits the group's summary (box + fixed-point sums) -- what used to
@@ -280,60 +280,93 @@ __device__ __forceinline__ unsigned int raster_run(const RasterGeom& g, int cxi,
   return __ldg(g.run_src + j1) - src;
 }
 
-// points per cell.  One THREAD per cell, consecutive threads on consecutive cells of a row of cells:
-// the run-table entries a warp asks for in one step are neighbours (coalesced 8-byte strides), a
-// quarter of the sectors the one-warp-per-cell form touched (lanes over the (day, row) runs: one
-// sector per lane).
-__global__ void __launch_bounds__(kThreads) raster_cell_count_kernel(const RasterGeom g, unsigned int* counts) {
-  const int n_cells = g.gx * g.gy, per_cell = g.nd * g.rpc;
-  for (int c = blockIdx.x * kThreads + threadIdx.x; c < n_cells; c += gridDim.x * kThreads) {
-    const int cyi = c / g.gx, cxi = c - cyi * g.gx;
-    unsigned int tot = 0;
-    int dd = 0, ry = 0;
-#pragma unroll 4
-    for (int e = 0; e < per_cell; ++e) {
-      unsigned int src;
-      tot += raster_run(g, cxi, cyi, dd, ry, src);
-      if (++ry == g.rpc) { ry = 0; ++dd; }
-    }
-    counts[raster_cell_index(g, cxi, cyi)] = tot;
-  }
-}
+// The run list in ONE pass over the run table.  Entries in destination order (cell, day, row):
+// entry E = (first mirror slot, first cloud index); an entry's length is the next entry's slot
+// minus its own (entry n_entries closes the list).  gfirst[g] = the entry that holds mirror slot
+// 128 g.  The slot of an entry is the number of points of all entries before it -- cells are
+// consecutive in the mirror -- so the list is an exclusive scan over the entries: a CTA takes a
+// tile of kIndexTile consecutive entries by ticket, reads its runs (kIndexItems per thread, all
+// loads in flight together), publishes the tile's total and obtains the points of all earlier
+// tiles by a decoupled look-back (ptx.cuh).  No per-cell count array, no separate scan launch.
+constexpr int kIndexItems = 8;
+constexpr int kIndexTile = kThreads * kIndexItems;
 
-// The runs in destination order: entry (cell, day, row) = (first mirror slot, first cloud index);
-// an entry's length is the next entry's slot minus its own (entry n_entries closes the list).
-// gfirst[g] = the entry that holds mirror slot 128 g.  One warp per cell, as above.
-__global__ void __launch_bounds__(kThreads) raster_runs_kernel(const RasterGeom g, const long long* cell_offsets,
-                                                               long long n, uint2* druns, unsigned int* gfirst) {
-  const int n_cells = g.gx * g.gy, per_cell = g.nd * g.rpc, lane = threadIdx.x & 31;
-  const int stride = gridDim.x * (kThreads / 32);
-  for (int c = blockIdx.x * (kThreads / 32) + (threadIdx.x >> 5); c < n_cells; c += stride) {
-    const int cyi = c / g.gx, cxi = c - cyi * g.gx;
-    const int lin = raster_cell_index(g, cxi, cyi);
-    unsigned int carry = (unsigned int)cell_offsets[lin];
-    uint2* out = druns + (size_t)lin * per_cell;
-    const float inv_rpc = 1.0f / (float)g.rpc;
-    for (int e0 = 0; e0 < per_cell; e0 += 32) {  // warp-uniform trip count
-      const int e = e0 + lane;
-      unsigned int src = 0u;
-      const int dd = per_cell <= 4096 ? (int)(((float)e + 0.5f) * inv_rpc) : e / g.rpc;  // (checked exact for e < 4096)
-      const unsigned int cnt = e < per_cell ? raster_run(g, cxi, cyi, dd, e - dd * g.rpc, src) : 0u;
-      unsigned int incl = cnt;
+// status: [n_tiles] look-back words; ticket[0] = tile counter, ticket[1] = fault flag (look-back
+// timed out); all zero before the launch.  n_entries + kIndexTile < 2^32.
+__global__ void __launch_bounds__(kThreads) raster_index_kernel(const RasterGeom g, long long n, unsigned int n_entries,
+                                                                unsigned long long* status, unsigned int* ticket,
+                                                                uint2* druns, unsigned int* gfirst) {
+  __shared__ unsigned int s_tile;
+  __shared__ unsigned int s_warp[kThreads / 32];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  if (tid == 0) s_tile = atomicAdd(ticket, 1u);
+  __syncthreads();
+  const unsigned int t = s_tile;
+  // the gather behind this kernel may be set up (it waits for the whole grid before it reads)
+  grid_launch_dependents();
+  const unsigned int per_cell = (unsigned int)(g.nd * g.rpc), rpc = (unsigned int)g.rpc, gx = (unsigned int)g.gx;
+  const unsigned int e0 = t * kIndexTile + tid * kIndexItems;
+  unsigned int cnt[kIndexItems], src[kIndexItems];
+  unsigned int tot = 0;
 #pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const unsigned int v = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= o) incl += v;
-      }
-      const unsigned int dst = carry + incl - cnt;
-      if (e < per_cell) out[e] = make_uint2(dst, src);
-      if (cnt) {  // a run is shorter than a group: it holds at most one group start
-        const unsigned long long gs = ((unsigned long long)dst + (kGroup - 1)) / kGroup;
-        if (gs * kGroup < (unsigned long long)dst + cnt) gfirst[gs] = (unsigned int)((size_t)lin * per_cell + e);
-      }
-      carry += __shfl_sync(0xffffffffu, incl, 31);
+  for (int i = 0; i < kIndexItems; ++i) {
+    const unsigned int E = e0 + i;
+    cnt[i] = 0u;
+    src[i] = 0u;
+    if (E < n_entries) {
+      const unsigned int lin = E / per_cell, e = E - lin * per_cell;
+      const unsigned int dd = e / rpc, ry = e - dd * rpc;
+      const unsigned int cyi = lin / gx, pos = lin - cyi * gx;
+      const unsigned int cxi = (cyi & 1u) ? gx - 1u - pos : pos;  // serpentine, as raster_cell_index
+      cnt[i] = raster_run(g, (int)cxi, (int)cyi, (int)dd, (int)ry, src[i]);
     }
-    if (c == 0 && lane == 0) druns[(size_t)n_cells * per_cell] = make_uint2((unsigned int)n, 0u);
+    tot += cnt[i];
   }
+  unsigned int incl = tot;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const unsigned int v = __shfl_up_sync(0xffffffffu, incl, o);
+    if (lane >= o) incl += v;
+  }
+  if (lane == 31) s_warp[warp] = incl;
+  __syncthreads();
+  if (warp == 0) {
+    const unsigned int w = lane < kThreads / 32 ? s_warp[lane] : 0u;
+    unsigned int ws = w;
+#pragma unroll
+    for (int o = 1; o < kThreads / 32; o <<= 1) {
+      const unsigned int v = __shfl_up_sync(0xffffffffu, ws, o);
+      if (lane >= o) ws += v;
+    }
+    const unsigned int agg = __shfl_sync(0xffffffffu, ws, kThreads / 32 - 1);
+    if (t > 0 && lane == 0) st_status(status + t, kStAggregate | agg);
+    const unsigned int base = (unsigned int)tile_lookback(status, t, agg, lane, ticket + 1);
+    __syncwarp();
+    if (lane < kThreads / 32) s_warp[lane] = base + ws - w;  // points before the warp's first entry
+  }
+  __syncthreads();
+  unsigned int dst = s_warp[warp] + incl - tot;
+  uint2 out[kIndexItems];
+#pragma unroll
+  for (int i = 0; i < kIndexItems; ++i) {
+    out[i] = make_uint2(dst, src[i]);
+    if (cnt[i]) {  // a run is shorter than a group: it holds at most one group start
+      const unsigned long long gs = ((unsigned long long)dst + (kGroup - 1)) / kGroup;
+      if (gs * kGroup < (unsigned long long)dst + cnt[i]) gfirst[gs] = e0 + i;
+    }
+    dst += cnt[i];
+  }
+  if (e0 + kIndexItems <= n_entries) {
+    uint4* o4 = reinterpret_cast<uint4*>(druns + e0);  // 64-byte aligned
+#pragma unroll
+    for (int i = 0; i < kIndexItems / 2; ++i)
+      o4[i] = make_uint4(out[2 * i].x, out[2 * i].y, out[2 * i + 1].x, out[2 * i + 1].y);
+  } else {
+#pragma unroll
+    for (int i = 0; i < kIndexItems; ++i)
+      if (e0 + i < n_entries) druns[e0 + i] = out[i];
+  }
+  if (t == 0 && tid == 0) druns[n_entries] = make_uint2((unsigned int)n, 0u);
 }
 
 // One warp per group of 128 mirror points: resolve the group's slots to cloud indices through
@@ -344,6 +377,9 @@ __global__ void __launch_bounds__(kThreads, MDKM_GATHER_CTAS) raster_gather_kern
                                                                  const uint2* __restrict__ druns, long long n_entries,
                                                                  const unsigned int* __restrict__ gfirst, FrameF f,
                                                                  float* __restrict__ tpts, float4* __restrict__ summaries) {
+  // launched behind raster_index_kernel with programmatic stream serialisation: nothing of its
+  // output is read before the whole index grid has finished
+  grid_dependency_wait();
   const int lane = threadIdx.x & 31;
   const long long n_groups = (n + kGroup - 1) / kGroup;
   const long long stride = (long long)gridDim.x * (kThreads / 32);

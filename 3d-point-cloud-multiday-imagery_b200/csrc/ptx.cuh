@@ -162,6 +162,59 @@ __device__ __forceinline__ uint2 ld_relaxed_sys_v2u32(const void* p) {
   return v;
 }
 
+// Decoupled look-back (single-pass exclusive scan over tiles that a ticket counter hands out in
+// order, so every predecessor of a running tile is itself running or done).  Per-tile status
+// word: flag in the two top bits, count below.
+constexpr unsigned long long kStAggregate = 1ull << 62;  // value = items of this tile
+constexpr unsigned long long kStPrefix = 2ull << 62;     // value = items up to and including this tile
+constexpr unsigned long long kStValue = (1ull << 62) - 1ull;
+
+__device__ __forceinline__ unsigned long long ld_status(const unsigned long long* p) {
+  unsigned long long v;
+  asm volatile("ld.relaxed.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
+  return v;
+}
+__device__ __forceinline__ void st_status(unsigned long long* p, unsigned long long v) {
+  asm volatile("st.relaxed.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
+}
+
+// Items of all tiles before tile t (warp-collective; the tile's own aggregate has been published
+// by the caller, except for tile 0).  Also publishes tile t's prefix.  Sums of up to 32 tiles must
+// fit 32 bits.  Flag and value share one 64-bit status word, so no fence is
+// involved: a word is either not there yet, an aggregate or a prefix.
+__device__ __forceinline__ unsigned long long tile_lookback(unsigned long long* status, long long t, unsigned int agg,
+                                                            int lane, unsigned int* fault) {
+  unsigned long long excl = 0ull;
+  const long long t0 = clock64();
+  for (long long j = t - 1;; j -= 32) {
+    const long long jj = j - lane;
+    unsigned long long s;
+    unsigned int first_pre, invalid;
+    do {
+      // bounded wait (about 4 s): every predecessor holds an earlier ticket, so it is running or done
+      // and this never triggers; if it ever did, a flagged failure beats a hung GPU
+      if (clock64() - t0 > (8ll << 30)) {
+        if (lane == 0) atomicExch(fault, 1u);
+        return 0ull;
+      }
+      s = jj >= 0 ? ld_status(status + jj) : kStPrefix;  // before tile 0: a prefix of zero items
+      const unsigned int flag = (unsigned int)(s >> 62);
+      const unsigned int pre = __ballot_sync(0xffffffffu, flag == 2u);
+      first_pre = pre ? (unsigned int)__ffs(pre) - 1u : 32u;
+      // every tile between t and the nearest prefix must have published its aggregate
+      const unsigned int need = first_pre < 32u ? ((2u << first_pre) - 1u) : 0xffffffffu;
+      invalid = __ballot_sync(0xffffffffu, flag == 0u) & need;
+    } while (invalid);
+    excl += __reduce_add_sync(0xffffffffu, (unsigned int)lane < first_pre ? (unsigned int)(s & kStValue) : 0u);
+    if (first_pre < 32u) {
+      excl += __shfl_sync(0xffffffffu, s, first_pre) & kStValue;
+      break;
+    }
+  }
+  if (lane == 0) st_status(status + t, kStPrefix | (excl + agg));
+  return excl;
+}
+
 // warp-wide float min / max in one instruction (sm_100a: CREDUX.MIN/MAX.F32)
 __device__ __forceinline__ float redux_min_f32(float v) {
   float r;

@@ -31,11 +31,6 @@ constexpr int kChunk = 4096;
 #define MDKM_UNPROJ_CTAS 2
 #endif
 constexpr int kTile = MDKM_TILE;  // pixels per warp tile of the fused pass
-// per-tile status word of the decoupled look-back: flag in the two top bits, count below
-constexpr unsigned long long kStAggregate = 1ull << 62;  // value = valid pixels of this tile
-constexpr unsigned long long kStPrefix = 2ull << 62;     // value = valid pixels up to and including this tile
-constexpr unsigned long long kStValue = (1ull << 62) - 1ull;
-
 struct UnprojParams {
   const void* hm;         // points at pixel pix_begin
   const uint8_t* mask;    // idem, or nullptr
@@ -86,54 +81,6 @@ __device__ __forceinline__ unsigned int f2ord(float f) {
   const unsigned int b = __float_as_uint(f);
   return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
 }
-__device__ __forceinline__ unsigned long long ld_status(const unsigned long long* p) {
-  unsigned long long v;
-  asm volatile("ld.relaxed.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ void st_status(unsigned long long* p, unsigned long long v) {
-  asm volatile("st.relaxed.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-}
-
-// Points of all super-tiles before super-tile t (warp-collective; the super-tile's own aggregate has
-// been published by the caller).  Flag and value share one 64-bit status word, so no fence is
-// involved: a word is either not there yet, an aggregate or a prefix.
-__device__ __forceinline__ unsigned long long tile_lookback(unsigned long long* status, long long t, unsigned int agg,
-                                                            int lane, unsigned int* fault) {
-#ifdef MDKM_NO_LOOKBACK  // timing experiment only (wrong offsets): the pass without its look-back
-  return (unsigned long long)t * ((kThreads / 32) * kTile);
-#endif
-  unsigned long long excl = 0ull;
-  const long long t0 = clock64();
-  for (long long j = t - 1;; j -= 32) {
-    const long long jj = j - lane;
-    unsigned long long s;
-    unsigned int first_pre, invalid;
-    do {
-      // bounded wait (about 4 s): every predecessor holds an earlier ticket, so it is running or done
-      // and this never triggers; if it ever did, a flagged failure beats a hung GPU
-      if (clock64() - t0 > (8ll << 30)) {
-        if (lane == 0) atomicExch(fault, 1u);
-        return 0ull;
-      }
-      s = jj >= 0 ? ld_status(status + jj) : kStPrefix;  // before tile 0: a prefix of zero points
-      const unsigned int flag = (unsigned int)(s >> 62);
-      const unsigned int pre = __ballot_sync(0xffffffffu, flag == 2u);
-      first_pre = pre ? (unsigned int)__ffs(pre) - 1u : 32u;
-      // every tile between t and the nearest prefix must have published its aggregate
-      const unsigned int need = first_pre < 32u ? ((2u << first_pre) - 1u) : 0xffffffffu;
-      invalid = __ballot_sync(0xffffffffu, flag == 0u) & need;
-    } while (invalid);
-    excl += __reduce_add_sync(0xffffffffu, (unsigned int)lane < first_pre ? (unsigned int)(s & kStValue) : 0u);
-    if (first_pre < 32u) {
-      excl += __shfl_sync(0xffffffffu, s, first_pre) & kStValue;
-      break;
-    }
-  }
-  if (lane == 0) st_status(status + t, kStPrefix | (excl + agg));
-  return excl;
-}
-
 // plugin.py:171: height_rel = dot(P - center, normal), in a fixed evaluation order
 __device__ __forceinline__ float plane_height(const double* __restrict__ pl, unsigned int col, unsigned int row, float z) {
   double v = __dmul_rn((double)z - pl[2], pl[5]);
@@ -283,7 +230,11 @@ __global__ void __launch_bounds__(kThreads, MDKM_UNPROJ_CTAS) unproject_fused_ke
         if (lane == 0) st_status(p.status + sup_n, kStAggregate | agg_n);
       }
       const unsigned int agg = __reduce_add_sync(0xffffffffu, lane < kWarps ? s_cnt[par][lane] : 0u);
+#ifdef MDKM_NO_LOOKBACK  // timing experiment only (wrong offsets): the pass without its look-back
+      const unsigned long long base = (unsigned long long)sup * ((kThreads / 32) * kTile);
+#else
       const unsigned long long base = tile_lookback(p.status, sup, agg, lane, p.ticket + 1);
+#endif
       if (lane == 0) s_base = base;
     }
     __syncthreads();

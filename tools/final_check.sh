@@ -22,7 +22,7 @@ timeout 300 ncu --set full --clock-control none --cache-control none --import-so
   -o $out/prof_step_$tag python bench.py $args > $out/ncu2_$tag.log 2>&1
 # the once-per-cloud kernels and the final pass
 timeout 300 ncu --set full --clock-control none --import-source on \
-  -k regex:"raster_gather|unproject_fused|lloyd_final|raster_runs|raster_cell_count" -s 10 -c 5 -f \
+  -k regex:"raster_gather|unproject_fused|lloyd_final|raster_index" -s 10 -c 5 -f \
   -o $out/prof_build_$tag python bench.py $args > $out/ncu3_$tag.log 2>&1
 # many centroids (config 4, k = 1024): FMA pipe and issue rates of the step kernel
 args4="--no-e2e --no-cpu --no-stream-all --no-bruteforce --config c4 --steps 3 --warmup 3"
