@@ -46,6 +46,9 @@ class FusionResult:
     n_relocations: int = 0
     height_norm: Optional[np.ndarray] = None  # plugin.py:184-188 'height' property, if requested
     extra: Dict[str, Any] = field(default_factory=dict)
+    # labels on the pixel grid (return_cluster_map=True): label + 1 where a pixel produced a point,
+    # 0 elsewhere; uint8 (k <= 255) or uint16, [D,H,W] -- or this rank's flat pixel range
+    cluster_map: Optional[np.ndarray] = None
 
     # scikit-learn style aliases
     @property
@@ -114,11 +117,19 @@ def _random_seeds(rs, n: int, k: int) -> np.ndarray:
     return choice_uniform_without_replacement(rs, n, k)
 
 
+def cluster_map_dtype(n_clusters: int):
+    """Element type of a cluster map for ``n_clusters`` labels (0 is the background)."""
+    return np.uint8 if int(n_clusters) <= 255 else np.uint16
+
+
 def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_state, want_labels=True,
-                labels_out=None, gather_mappings=None):
+                labels_out=None, gather_mappings=None, cluster_map_out=None):
     """KMeans.fit driver (sklearn/_kmeans.py:1436-1563): init, n_init restarts, best inertia.
 
     ``labels_out``: optional int32 array that receives this rank's labels of the best run.
+    ``cluster_map_out``: optional uint8 / uint16 array that receives the best run's cluster map
+    (``Engine.fit``).  With restarts every run writes its map into a device scratch tensor; the
+    best one is kept by swapping and copied out once at the end.
     ``gather_mappings``: with a multi-rank engine, the collective that lets the ranks agree on
     sklearn's "same clustering up to a permutation" test (see ``_is_same_clustering``); when it is
     missing the test is skipped on multi-rank engines (the inertia comparison alone decides)."""
@@ -145,6 +156,14 @@ def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_
         gather_mappings = torch_gather_mappings(eng)  # None unless torch.distributed spans the ranks
     single = int(n_init) == 1
     best = None
+    run_map = best_map = None
+    if cluster_map_out is not None and not single:
+        import torch
+
+        # (a copy of the best map per improvement would cost a device->host transfer each time)
+        tdt = torch.uint8 if np.dtype(cluster_map_dtype(k)) == np.uint8 else torch.uint16
+        run_map = torch.empty(eng.raster_range[4], dtype=tdt, device=f"cuda:{eng.device}")
+        best_map = torch.empty_like(run_map)
     for _ in range(int(n_init)):
         if init_is_array:
             centers0 = init_arr
@@ -153,7 +172,8 @@ def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_
         else:
             centers0, _ = eng.kmeans_plusplus(k, rs)
         r = eng.fit(centers0, max_iter=max_iter, tol=tol, want_labels=want_labels,
-                    labels_out=labels_out if (single and want_labels) else None)
+                    labels_out=labels_out if (single and want_labels) else None,
+                    cluster_map_out=cluster_map_out if single else run_map)
         # sklearn/_kmeans.py:1534-1541: a run replaces the best one when its inertia is lower AND it
         # is not the same clustering up to a permutation.  The inertia is global, so every rank
         # takes the same branch and the (collective) permutation test pairs up.
@@ -165,17 +185,36 @@ def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_
             best = r
             if not single and r["labels"] is not None:
                 best = dict(r, labels=r["labels"].copy())  # result buffers are reused by the next run
+            if run_map is not None:
+                run_map, best_map = best_map, run_map
     if labels_out is not None and want_labels and not single:
         labels_out[...] = best["labels"]
         best = dict(best, labels=labels_out)
+    if best_map is not None:
+        _copy_map_out(best_map, cluster_map_out)
     return best
+
+
+def _copy_map_out(src, out):
+    """Device map ``src`` (flat torch tensor) -> the caller's ``out`` (numpy array or torch tensor).
+    16-bit maps are moved as int16: the bits are the same and every torch build copies int16."""
+    import torch
+
+    wide = src.dtype == torch.uint16
+    s = src.view(torch.int16) if wide else src
+    if type(out).__module__.startswith("torch"):
+        o = out.view(torch.int16) if wide else out
+        o.view(-1).copy_(s)
+    else:
+        host = s.cpu().numpy()
+        out.reshape(-1)[...] = host.view(np.uint16) if wide else host
 
 
 def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k-means++", n_init=1,
                          max_iter=300, tol=1e-4, random_state=None, max_abs_height=MAX_ABS_HEIGHT,
                          detrend=False, disparity_scale=None, ground_level=False, return_cloud=True,
                          device=0, devices=None, engine=None, stack_shape=None,
-                         pix_begin=0, raster_layout=None) -> FusionResult:
+                         pix_begin=0, raster_layout=None, return_cluster_map=False) -> FusionResult:
     """Unproject a multi-day height-map stack into one XYZ cloud and cluster it (Lloyd).
 
     height_maps : float32 ``[D,H,W]`` (NaN = nodata), numpy or torch (CPU or CUDA); or int16
@@ -198,6 +237,11 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
         assembled in the reference's point order -- bit-identical to one device.  This is how the
         in-process caller of the reference (a napari worker thread, widget.py:116-147) gets more
         than one GPU without ``torchrun``.
+    return_cluster_map : also return ``cluster_map``, the labels on the input pixel grid (a
+        napari Labels layer): ``label + 1`` at each pixel that produced a point, 0 at the others;
+        uint8 for ``n_clusters <= 255``, else uint16.  ``[D,H,W]`` for a whole stack; this rank's
+        flat ``[pix_count]`` slice for a pre-sharded call (``stack_shape`` / ``pix_begin``), as
+        ``labels`` is this rank's shard.  The map is written on the GPU by the final labelling pass.
     Returns a FusionResult; ``fused_cloud`` is float32 ``[N,3]`` in napari (z,y,x) order.
     """
     from .group import DeviceGroup
@@ -209,7 +253,7 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
                               devices=devices, n_clusters=n_clusters, init=init, n_init=n_init, max_iter=max_iter,
                               tol=tol, random_state=random_state, max_abs_height=max_abs_height, detrend=detrend,
                               disparity_scale=disparity_scale, ground_level=ground_level, return_cloud=return_cloud,
-                              raster_layout=raster_layout)
+                              raster_layout=raster_layout, return_cluster_map=return_cluster_map)
     own = engine is None
     eng = engine or Engine(device)
     try:
@@ -230,20 +274,24 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
         # otherwise its device->host copy is issued now and overlaps the Lloyd loop
         if return_cloud and cloud is None:
             cloud = eng.get_cloud(napari_order=True, wait=False)
+        cmap = None
+        if return_cluster_map:
+            D, H, W, _, count = eng.raster_range
+            cmap = np.empty((D, H, W) if stack_shape is None else (count,), dtype=cluster_map_dtype(n_clusters))
         r = _run_kmeans(eng, n_clusters=n_clusters, init=init, n_init=n_init, max_iter=max_iter,
-                        tol=tol, random_state=random_state)
+                        tol=tol, random_state=random_state, cluster_map_out=cmap)
         eng.wait()
         return FusionResult(labels=r["labels"], centroids=r["centers"], fused_cloud=cloud,
                             n_iter=r["n_iter"], inertia=r["inertia"], n_points=n,
                             n_refined=r["n_refined"], n_relocations=r["n_relocations"],
-                            height_norm=hn, extra=extra)
+                            height_norm=hn, extra=extra, cluster_map=cmap)
     finally:
         if own:
             eng.close()
 
 
 def _fuse_on_group(height_maps, valid_masks, *, group, devices, n_clusters, init, n_init, max_iter, tol,
-                   random_state, **unproject_kw) -> FusionResult:
+                   random_state, return_cluster_map=False, **unproject_kw) -> FusionResult:
     """``fuse_multiday_kmeans`` on several devices of this process (``group.DeviceGroup``)."""
     import threading
 
@@ -268,16 +316,20 @@ def _fuse_on_group(height_maps, valid_masks, *, group, devices, n_clusters, init
                 return [g[0] for g in got], [g[1] for g in got]
             return gather
 
-        def run(eng, labels_out):
+        def run(eng, labels_out, cluster_map_out=None):
             r = eng.rank
             return _run_kmeans(eng, n_clusters=n_clusters, init=init, n_init=n_init, max_iter=max_iter, tol=tol,
                                random_state=states[r], labels_out=labels_out,
-                               gather_mappings=gather_for(r) if grp.world > 1 else None)
+                               gather_mappings=gather_for(r) if grp.world > 1 else None,
+                               cluster_map_out=cluster_map_out)
 
-        res, labels, cloud, hn, extra = grp.fuse(height_maps, valid_masks, run_kmeans=run, **unproject_kw)
+        res, labels, cloud, hn, extra = grp.fuse(
+            height_maps, valid_masks, run_kmeans=run,
+            cluster_map_dtype=cluster_map_dtype(n_clusters) if return_cluster_map else None, **unproject_kw)
         return FusionResult(labels=labels, centroids=res["centers"], fused_cloud=cloud, n_iter=res["n_iter"],
                             inertia=res["inertia"], n_points=int(labels.shape[0]), n_refined=res["n_refined"],
-                            n_relocations=res["n_relocations"], height_norm=hn, extra=extra)
+                            n_relocations=res["n_relocations"], height_norm=hn, extra=extra,
+                            cluster_map=extra.pop("cluster_map", None))
     finally:
         if own:
             grp.close()
@@ -317,7 +369,8 @@ def to_layers(result: FusionResult, prefix: str = "Multi-day") -> List[Layer]:
     """napari layers for a FusionResult, mirroring plugin.py:220-233.
 
     One Points layer with the fused cloud coloured by cluster (or by the reference's
-    'height' property when it was computed) and one with the K centroids.
+    'height' property when it was computed) and one with the K centroids; when the result has a
+    ``cluster_map``, a third, Labels layer with it (0 = no point at that pixel).
     """
     if result.fused_cloud is None:
         raise ValueError("result has no fused_cloud (return_cloud=False)")
@@ -347,6 +400,8 @@ def to_layers(result: FusionResult, prefix: str = "Multi-day") -> List[Layer]:
          "face_colormap": "turbo", "symbol": "cross"},
         "points",
     ))
+    if result.cluster_map is not None:
+        layers.append((result.cluster_map, {"name": f"{prefix} Cluster Map", "opacity": 0.7}, "labels"))
     return layers
 
 

@@ -819,7 +819,40 @@ struct FinalParams {
   DevStatus* status_host;     // or nullptr: the last CTA copies the status here (device-visible host memory)
   double* centroids_host;     // or nullptr: the last CTA writes the k x 3 centroids (original coordinates) here
   double origin[3];           // Frame::origin, for centroids_host
+  // cluster map (lloyd_final_kernel<kChunks, true>): label + 1 at the pixel of every point, local
+  // pixel (day - map_day0) * map_HW + y * map_W + x - (map_pix_begin - map_day0 * map_HW)
+  void* map_out;              // uint8 / uint16 per pixel of the range of the last unprojection
+  int map_elem;               // 1 or 2 bytes
+  int map_W;
+  long long map_pix_begin;    // global index of the range's first pixel
+  long long map_HW;
+  long long map_day0;         // day of map_pix_begin
+  const long long* map_seg;   // [map_nseg + 1] point offsets of the days of the range (device)
+  int map_nseg;
 };
+
+// Day of this lane's points in the cluster map: segment `day` holds the points before `next`,
+// and its pixel (0, 0) is element `base` of the map.  A warp walks its groups in point order, so
+// the cursor only moves forward.
+struct MapCursor {
+  int day;
+  long long next;
+  long long base;
+};
+
+// the cursor of point i: the last segment that starts at or before i (empty days are skipped)
+__device__ __forceinline__ MapCursor map_cursor(const FinalParams& p, long long i) {
+  int lo = 0, hi = p.map_nseg;
+  while (hi - lo > 1) {
+    const int mid = (lo + hi) >> 1;
+    if (__ldg(p.map_seg + mid) <= i) lo = mid; else hi = mid;
+  }
+  return MapCursor{lo, __ldg(p.map_seg + lo + 1), (long long)lo * p.map_HW - (p.map_pix_begin - p.map_day0 * p.map_HW)};
+}
+
+// exact pixel coordinate (an integer in [0, 2^23), mdkm_bind_cluster_map checks H and W) -> int,
+// with one FADD instead of a float-to-int conversion
+__device__ __forceinline__ int pixel_index(float v) { return __float_as_int(v + 8388608.0f) - 0x4B000000; }
 
 // Copies the status block into device-visible host memory (one thread).  L2 reads: other CTAs
 // updated it with atomics.
@@ -2327,10 +2360,28 @@ __device__ __forceinline__ void assign_split_group(const float (&xo)[4], const f
   }
 }
 
-// labels and FP64 inertia (direct form) of this lane's four points of a group
+// labels and FP64 inertia (direct form) of this lane's four points of a group; with kMap also
+// label + 1 at each point's pixel of the cluster map (x and y are exact pixel coordinates)
+template <bool kMap>
 __device__ __forceinline__ void final_emit(const FinalParams& p, const double4* __restrict__ c64, const FrameF& f,
                                            long long i0, const float (&xo)[4], const float (&yo)[4],
-                                           const float (&zo)[4], const int (&lab)[4], double& inert) {
+                                           const float (&zo)[4], const int (&lab)[4], double& inert,
+                                           MapCursor& mc) {
+  if (kMap) {
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      const long long i = i0 + e;
+      if (i < p.n) {
+        while (i >= mc.next) {
+          mc.next = __ldg(p.map_seg + ++mc.day + 1);
+          mc.base += p.map_HW;
+        }
+        const long long pix = mc.base + (long long)pixel_index(yo[e]) * p.map_W + pixel_index(xo[e]);
+        if (p.map_elem == 1) static_cast<unsigned char*>(p.map_out)[pix] = (unsigned char)(lab[e] + 1);
+        else static_cast<unsigned short*>(p.map_out)[pix] = (unsigned short)(lab[e] + 1);
+      }
+    }
+  }
 #pragma unroll
   for (int e = 0; e < 4; ++e) {
     if (i0 + e < p.n) {
@@ -2354,9 +2405,10 @@ __device__ __forceinline__ void final_emit(const FinalParams& p, const double4* 
 
 // ---------------------------------------------------------------------------------------
 // Final pass over the resident cloud (reference point order): E-step with the final centroids
-// -> int32 labels, and the inertia in FP64 (direct form, fixed-order reduction).
+// -> int32 labels, and the inertia in FP64 (direct form, fixed-order reduction).  kMap: the
+// labels also go to the cluster map (FinalParams::map_out, cleared by the host beforehand).
 // ---------------------------------------------------------------------------------------
-template <int kChunks>
+template <int kChunks, bool kMap>
 __global__ void __launch_bounds__(kThreads, kChunks == 0 ? MDKM_FINAL_CTAS0 : 3) lloyd_final_kernel(const FinalParams p) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const int kp32 = kChunks > 0 ? kChunks * 32 : ((p.kpad + 31) & ~31);
@@ -2404,6 +2456,8 @@ __global__ void __launch_bounds__(kThreads, kChunks == 0 ? MDKM_FINAL_CTAS0 : 3)
   const long long per_warp = (n_groups + n_warps - 1) / n_warps;
   const long long g_first = ((long long)blockIdx.x * (kThreads / 32) + warp) * per_warp;
   const long long g_last = min(n_groups, g_first + per_warp);
+  MapCursor mc{0, 0, 0};
+  if (kMap && g_first < g_last) mc = map_cursor(p, g_first * kGroup + lane * 4);
   // few centroids: the next group's block is requested before this one is worked on (one group
   // of look-ahead in registers) -- a warp walks its run serially, so without it every group pays
   // a DRAM round trip.  With many centroids the pass is bound by the candidate walk instead and
@@ -2440,10 +2494,11 @@ __global__ void __launch_bounds__(kThreads, kChunks == 0 ? MDKM_FINAL_CTAS0 : 3)
                                     s_cand + warp * kCandCap, lane, lab, n_ref);
     if (ncand < 0) assign_group<kChunks>(xc, yc, zc, xo, yo, zo, f, s_fast, c64, p.k, kp32, thresh, lane, lab, n_ref);
     hint = __shfl_sync(0xffffffffu, lab[0], 0);
-    final_emit(p, c64, f, i0, xo, yo, zo, lab, inert);
+    final_emit<kMap>(p, c64, f, i0, xo, yo, zo, lab, inert, mc);
   }
   // second loop: the groups that run over the end of a raster row (one in W/128), two halves each
   if (p.split_rows) {
+    if (kMap && g_first < g_last) mc = map_cursor(p, g_first * kGroup + lane * 4);  // (walks the run again)
     for (long long gb = g_first; gb < g_last; gb += 32) {
       bool sp = false;
       if (gb + lane < g_last) {
@@ -2460,7 +2515,7 @@ __global__ void __launch_bounds__(kThreads, kChunks == 0 ? MDKM_FINAL_CTAS0 : 3)
         int lab[4] = {0, 0, 0, 0};
         assign_split_group<kChunks>(xo, yo, zo, f, s_fast, c64, bkt_bytes ? s_bkt : nullptr, p.k, kp32, thresh,
                                     s_cand + warp * kCandCap, lane, lab, n_ref);
-        final_emit(p, c64, f, g * kGroup + lane * 4, xo, yo, zo, lab, inert);
+        final_emit<kMap>(p, c64, f, g * kGroup + lane * 4, xo, yo, zo, lab, inert, mc);
       }
     }
   }

@@ -151,6 +151,13 @@ struct mdkm_handle {
   float* bound_cloud_out = nullptr;  // mdkm_bind_cloud_output
   long long bound_cloud_cap = 0;
   int bound_cloud_napari = 1;
+  // cluster map (mdkm_bind_cluster_map) over the pixel range of the last mdkm_unproject
+  long long raster_pix_begin = 0, raster_pix_count = 0;
+  int raster_H = 0;                  // (the width is raster_w)
+  void* bound_map = nullptr;
+  int bound_map_elem = 0, bound_map_mem = MDKM_MEM_HOST;
+  DevBuf<unsigned char> map_stage;   // host outputs are written here, then copied
+  DevBuf<long long> map_seg;         // the days' point offsets (d_seg_off may hold merged segments)
 
   // communicator
   ncclComm_t comm = nullptr;
@@ -455,10 +462,15 @@ int step_occupancy(mdkm_handle* h, StepKernel fn, size_t smem, int* occ) {
 }
 
 typedef void (*FinalKernel)(const FinalParams);
-FinalKernel pick_final_kernel(int kpad) {
-  if (kpad <= 32) return lloyd_final_kernel<1>;
-  if (kpad <= 64) return lloyd_final_kernel<2>;
-  return lloyd_final_kernel<0>;
+FinalKernel pick_final_kernel(int kpad, bool map = false) {
+  if (map) {
+    if (kpad <= 32) return lloyd_final_kernel<1, true>;
+    if (kpad <= 64) return lloyd_final_kernel<2, true>;
+    return lloyd_final_kernel<0, true>;
+  }
+  if (kpad <= 32) return lloyd_final_kernel<1, false>;
+  if (kpad <= 64) return lloyd_final_kernel<2, false>;
+  return lloyd_final_kernel<0, false>;
 }
 
 struct KmBuffers {
@@ -862,8 +874,48 @@ int collect_profile(mdkm_handle* h) {
   return MDKM_OK;
 }
 
+// A cluster map taken by one fit / predict: written at `dev` by the final pass, then copied to
+// `host` unless that is null (device output).
+struct MapOut {
+  void* dev = nullptr;
+  void* host = nullptr;
+  int elem = 0;
+  size_t bytes = 0;
+};
+
 int run_final(mdkm_handle* h, const KmBuffers& kb, int* labels_dev, bool skip_paused = false,
-              double* centroids_host = nullptr, DevStatus* status_host = nullptr);
+              double* centroids_host = nullptr, DevStatus* status_host = nullptr, const MapOut* map = nullptr);
+
+// Consumes the binding of mdkm_bind_cluster_map (whatever happens) for a call with k clusters:
+// checks that k fits the element type, stages host outputs, uploads the days' point offsets.
+int take_cluster_map(mdkm_handle* h, int k, MapOut& m) {
+  void* out = h->bound_map;
+  const int elem = h->bound_map_elem, mem = h->bound_map_mem;
+  h->bound_map = nullptr;
+  if (!out) return MDKM_OK;
+  if (k > (elem == 1 ? 255 : 65535))
+    return fail(h, MDKM_ERR_INVALID, "k=%d labels do not fit a cluster map of %d-byte elements", k, elem);
+  CU(cudaSetDevice(h->device));
+  m.elem = elem;
+  m.bytes = (size_t)h->raster_pix_count * elem;
+  if (mem == MDKM_MEM_DEVICE) {
+    m.dev = out;
+  } else {
+    OK(ensure(h, h->map_stage, std::max<size_t>(m.bytes, 1)));
+    m.dev = h->map_stage.p;
+    m.host = out;
+  }
+  const size_t n_off = h->seg_off.size();
+  OK(ensure(h, h->map_seg, n_off));
+  CU(cudaMemcpyAsync(h->map_seg.p, h->seg_off.data(), n_off * 8, cudaMemcpyHostToDevice, h->stream));
+  return MDKM_OK;
+}
+
+// The map's device->host copy (host outputs), on the compute stream behind the final pass.
+int copy_cluster_map(mdkm_handle* h, const MapOut& m) {
+  if (m.host && m.bytes) CU(cudaMemcpyAsync(m.host, m.dev, m.bytes, cudaMemcpyDeviceToHost, h->stream));
+  return MDKM_OK;
+}
 
 // Empty-cluster relocation (sklearn/_k_means_common.pyx:167-211), sequenced from the host
 // while the Lloyd loop is paused.  All arithmetic on the device (extras.cuh).
@@ -908,8 +960,23 @@ int relocate_empty(mdkm_handle* h, const KmBuffers& kb, int n_empty) {
 
 // (the ticket is zero: fit_head clears it, every final pass leaves it so)
 int run_final(mdkm_handle* h, const KmBuffers& kb, int* labels_dev, bool skip_paused, double* centroids_host,
-              DevStatus* status_host) {
+              DevStatus* status_host, const MapOut* map) {
   FinalParams fp{};
+  FinalKernel fn = kb.final_fn;
+  if (map && map->dev) {
+    // pixels without a point stay 0 (napari's background label)
+    if (map->bytes) CU(cudaMemsetAsync(map->dev, 0, map->bytes, h->stream));
+    fn = pick_final_kernel(kb.kpad, /*map=*/true);
+    CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kb.final_smem));
+    fp.map_out = map->dev;
+    fp.map_elem = map->elem;
+    fp.map_W = h->raster_w;
+    fp.map_pix_begin = h->raster_pix_begin;
+    fp.map_HW = (long long)h->raster_H * h->raster_w;
+    fp.map_day0 = h->raster_pix_begin / fp.map_HW;
+    fp.map_seg = h->map_seg.p;
+    fp.map_nseg = (int)h->seg_off.size() - 1;
+  }
   fp.pts = h->pts.p; fp.n = h->n;
   fp.labels_out = labels_dev;
   fp.table = h->table.p;
@@ -923,7 +990,7 @@ int run_final(mdkm_handle* h, const KmBuffers& kb, int* labels_dev, bool skip_pa
   fp.status_host = status_host;
   fp.centroids_host = centroids_host;
   for (int d = 0; d < 3; ++d) fp.origin[d] = h->fr.origin[d];
-  kb.final_fn<<<kb.final_grid, kThreads, kb.final_smem, h->stream>>>(fp);
+  fn<<<kb.final_grid, kThreads, kb.final_smem, h->stream>>>(fp);
   ++h->launches;
   CU(cudaGetLastError());
   return MDKM_OK;
@@ -997,6 +1064,7 @@ void mdkm_destroy(mdkm_handle* h) {
   release(h->run_src); release(h->druns); release(h->gfirst);
   release(h->tile_status); release(h->chunk_offsets); release(h->staging); release(h->planes);
   release(h->d_seg_off); release(h->sel_hist); release(h->sel_targets);
+  release(h->map_stage); release(h->map_seg);
   release(h->kpp_closest); release(h->kpp_cell); release(h->kpp_blk); release(h->kpp_prefix);
   release(h->kpp_partials); release(h->kpp_rand); release(h->kpp_state);
   if (h->d_status) cudaFree(h->d_status);
@@ -1197,6 +1265,7 @@ int mdkm_set_points(mdkm_handle* h, const float* xyz, int64_t n, int layout, int
   h->seg_off.assign({0, (long long)n});
   h->seg_whole = true;
   h->raster_w = 0;
+  h->bound_map = nullptr;
   h->runs_ok = false;
   h->have_points = true;
   h->frame_ok = false;
@@ -1245,6 +1314,24 @@ int mdkm_bind_cloud_output(mdkm_handle* h, float* out_host, int64_t capacity_poi
   return MDKM_OK;
 }
 
+int mdkm_bind_cluster_map(mdkm_handle* h, void* out, int elem_bytes, int64_t capacity_pixels, int mem) {
+  if (!h) return MDKM_ERR_INVALID;
+  h->bound_map = nullptr;
+  if (!out) return MDKM_OK;
+  if (!h->have_points || h->raster_w <= 0)
+    return fail(h, MDKM_ERR_STATE, "a cluster map needs a resident cloud from mdkm_unproject");
+  if (elem_bytes != 1 && elem_bytes != 2) return fail(h, MDKM_ERR_INVALID, "elem_bytes must be 1 or 2");
+  if (h->raster_w >= (1 << 23) || h->raster_H >= (1 << 23))  // (the final pass converts x, y with an FADD)
+    return fail(h, MDKM_ERR_INVALID, "cluster maps need rasters narrower and shorter than 2^23 pixels");
+  if (capacity_pixels < h->raster_pix_count)
+    return fail(h, MDKM_ERR_INVALID, "cluster map holds %lld pixels, the range has %lld", (long long)capacity_pixels,
+                h->raster_pix_count);
+  h->bound_map = out;
+  h->bound_map_elem = elem_bytes;
+  h->bound_map_mem = mem;
+  return MDKM_OK;
+}
+
 // Unprojection as a pipeline of slabs: the host->device copy of slab s+1 (copy stream) overlaps
 // the kernels of slab s (compute stream) and, when a cloud output is bound, the device->host
 // copy of the points slab s-1 produced (result stream).  PCIe is full duplex, so the two copy
@@ -1258,6 +1345,7 @@ int mdkm_unproject(mdkm_handle* h, const void* hm, int hm_dtype, float hm_scale,
   const int cloud_napari = h->bound_cloud_napari;
   h->bound_cloud_out = nullptr;
   h->bound_cloud_cap = 0;
+  h->bound_map = nullptr;  // (a cluster map describes the range it was bound for)
   if (D < 0 || H <= 0 || W <= 0 || pix_begin < 0 || pix_count < 0 ||
       pix_begin + pix_count > (int64_t)D * H * W || (pix_count > 0 && !hm))
     return fail(h, MDKM_ERR_INVALID, "bad stack geometry");
@@ -1469,6 +1557,9 @@ int mdkm_unproject(mdkm_handle* h, const void* hm, int hm_dtype, float hm_scale,
   }
   h->n = n_out;
   h->raster_w = W;
+  h->raster_H = H;
+  h->raster_pix_begin = pix_begin;
+  h->raster_pix_count = pix_count;
   if (want_runs) {
     const unsigned int n32 = (unsigned int)n_out;  // closes the table
     CU(cudaMemcpyAsync(h->run_src.p + pix_count / 8, &n32, 4, cudaMemcpyHostToDevice, h->stream));
@@ -1533,6 +1624,8 @@ int mdkm_wait(mdkm_handle* h) {
 int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol, int32_t* labels_out,
              int labels_mem, double* centroids_out, int* n_iter_out, double* inertia_out) {
   if (!h) return MDKM_ERR_INVALID;
+  MapOut map;
+  OK(take_cluster_map(h, k, map));
   if (!init) return fail(h, MDKM_ERR_INVALID, "init centroids required");
   if (max_iter < 1) return fail(h, MDKM_ERR_INVALID, "max_iter must be >= 1");
   if (tol < 0) return fail(h, MDKM_ERR_INVALID, "tol must be >= 0");
@@ -1651,7 +1744,9 @@ int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol
     // last E-step used -- the sums are integers -- so this reproduces that step's labels exactly.
     {
       const int span = prof_begin(h, MDKM_PHASE_FINAL, h->n);
-      OK(run_final(h, kb, labels_dev, /*skip_paused=*/true, centroids_host, one_rank ? &h->h_status[0] : nullptr));
+      // (a pause leaves the map alone: the pass after the relocation writes it)
+      OK(run_final(h, kb, labels_dev, /*skip_paused=*/true, centroids_host, one_rank ? &h->h_status[0] : nullptr,
+                   &map));
       prof_end(h, span);
     }
     if (!one_rank) {
@@ -1665,6 +1760,7 @@ int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol
     }
     if (labels_out && labels_mem != MDKM_MEM_DEVICE && h->n > 0)
       CU(cudaMemcpyAsync(labels_out, labels_dev, (size_t)h->n * 4, cudaMemcpyDeviceToHost, h->stream));
+    OK(copy_cluster_map(h, map));
     OK(sync_small(h));
     if (h->h_status[0].paused && !h->h_status[0].done && !h->h_status[0].xchg_timeout) {
       // an update of the last batch, or the settle kernel, found an empty cluster: relocate, go on
@@ -1757,6 +1853,8 @@ int mdkm_lloyd_step(mdkm_handle* h, int k, const double* centroids, int32_t* lab
 int mdkm_predict(mdkm_handle* h, int k, const double* centroids, int32_t* labels_out, int labels_mem,
                  double* inertia_out) {
   if (!h) return MDKM_ERR_INVALID;
+  MapOut map;
+  OK(take_cluster_map(h, k, map));
   if (!centroids) return fail(h, MDKM_ERR_INVALID, "centroids required");
   CU(cudaSetDevice(h->device));
   KmBuffers kb{};
@@ -1775,11 +1873,12 @@ int mdkm_predict(mdkm_handle* h, int k, const double* centroids, int32_t* labels
       labels_dev = h->labels32.p;
     }
   }
-  OK(run_final(h, kb, labels_dev));
+  OK(run_final(h, kb, labels_dev, false, nullptr, nullptr, &map));
   if (h->n_ranks > 1) OK(allreduce(h, &h->d_status->inertia, 1, kNcclFloat64, kNcclSum));
   OK(small_d2h(h, &h->h_status[0], h->d_status, sizeof(DevStatus), /*dst_is_pinned=*/true));
   if (labels_out && labels_mem != MDKM_MEM_DEVICE && h->n > 0)
     CU(cudaMemcpyAsync(labels_out, labels_dev, (size_t)h->n * 4, cudaMemcpyDeviceToHost, h->stream));
+  OK(copy_cluster_map(h, map));
   OK(sync_small(h));
   if (h->h_status[0].xchg_timeout == 2) return index_fault(h);
   if (inertia_out) *inertia_out = h->h_status[0].inertia;

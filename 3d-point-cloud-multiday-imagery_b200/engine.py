@@ -44,14 +44,17 @@ def _as_buffer(a, dtype=None):
 def _as_out_buffer(a, dtype, n_elems, what):
     """-> (pointer:int, mem_kind) of a caller-supplied OUTPUT array.  The library writes through
     the raw pointer, so anything that would make numpy / torch hand over a temporary copy (wrong
-    dtype, non-contiguous view) is rejected instead of silently losing the result."""
-    dt = np.dtype(dtype)
+    dtype, non-contiguous view) is rejected instead of silently losing the result.  ``dtype``: one
+    dtype, or a tuple of the dtypes the output may have."""
+    dts = tuple(np.dtype(d) for d in (dtype if isinstance(dtype, tuple) else (dtype,)))
+    names = " or ".join(d.name for d in dts)
     if _is_torch(a):
         import torch
 
-        want = {np.dtype(np.float32): torch.float32, np.dtype(np.int32): torch.int32}[dt]
-        if a.dtype != want:
-            raise ValueError(f"{what} must be {dt.name}, got {a.dtype}")
+        tmap = {np.dtype(np.float32): torch.float32, np.dtype(np.int32): torch.int32,
+                np.dtype(np.uint8): torch.uint8, np.dtype(np.uint16): torch.uint16}
+        if a.dtype not in [tmap[d] for d in dts]:
+            raise ValueError(f"{what} must be {names}, got {a.dtype}")
         if not a.is_contiguous():
             raise ValueError(f"{what} must be contiguous")
         if a.numel() != n_elems:
@@ -59,8 +62,8 @@ def _as_out_buffer(a, dtype, n_elems, what):
         return a.data_ptr(), (C.MEM_DEVICE if a.is_cuda else C.MEM_HOST)
     if not isinstance(a, np.ndarray):
         raise ValueError(f"{what} must be a numpy array or a torch tensor")
-    if a.dtype != dt:
-        raise ValueError(f"{what} must be {dt.name}, got {a.dtype}")
+    if a.dtype not in dts:
+        raise ValueError(f"{what} must be {names}, got {a.dtype}")
     if not a.flags["C_CONTIGUOUS"]:
         raise ValueError(f"{what} must be C-contiguous")
     if not a.flags["WRITEABLE"]:
@@ -94,6 +97,7 @@ class Engine:
         self.p2p = False
         self._stream_ptr = int(self._lib.mdkm_get_stream(self._h) or 0)
         self._ext_stream = None
+        self._raster = None  # (D, H, W, pix_begin, pix_count) of the last unproject
 
     # -- ordering against torch's streams ----------------------------------------------------
     # The handle enqueues on its own stream.  A CUDA tensor handed to it may still be being
@@ -283,6 +287,7 @@ class Engine:
             int(D), int(H), int(W), int(pix_begin), int(count), float(max_abs_height),
             1 if detrend else 0, mem, byref(n)))
         del keep, keep_m
+        self._raster = (int(D), int(H), int(W), int(pix_begin), int(count))
         if stream_cloud is not None:
             return int(n.value), cloud_buf[: int(n.value)]
         return int(n.value)
@@ -302,6 +307,7 @@ class Engine:
             lay = C.POINTS_SOA
         if mem == C.MEM_DEVICE:
             self._after_torch(keep)
+        self._raster = None
         self._check(self._lib.mdkm_set_points(self._h, c_void_p(ptr), int(n), lay, mem))
         del keep
         return int(n)
@@ -348,6 +354,23 @@ class Engine:
         self._check(self._lib.mdkm_wait(self._h))
 
     @property
+    def raster_range(self):
+        """``(D, H, W, pix_begin, pix_count)`` of the last ``unproject``, or None when the resident
+        cloud came from ``set_points`` (or there is none)."""
+        return self._raster
+
+    def _bind_cluster_map(self, out):
+        """Bind ``out`` (uint8 / uint16, one element per pixel of the last unprojected range) as the
+        cluster map of the next fit / predict.  -> its memory kind."""
+        n_pix = self._raster[4] if self._raster is not None else (out.numel() if _is_torch(out) else np.size(out))
+        ptr, mem = _as_out_buffer(out, (np.uint8, np.uint16), n_pix, "cluster_map_out")
+        elem = out.element_size() if _is_torch(out) else out.itemsize
+        self._check(self._lib.mdkm_bind_cluster_map(self._h, c_void_p(ptr), int(elem), int(n_pix), mem))
+        if mem == C.MEM_DEVICE:
+            self._after_torch(out)  # earlier work on torch's stream may still use the buffer
+        return mem
+
+    @property
     def segment_offsets(self) -> np.ndarray:
         """Point offsets of the cloud's segments (one per day), int64 ``[n_segments + 1]``."""
         ns = int(self._lib.mdkm_num_segments(self._h))
@@ -370,8 +393,13 @@ class Engine:
         return lo[:ns], hi[:ns], hn
 
     # -- k-means -------------------------------------------------------------------------
-    def fit(self, init, max_iter=300, tol=1e-4, want_labels=True, labels_out=None):
-        """One Lloyd run from explicit centroids.  Returns dict(labels, centers, n_iter, inertia, ...)."""
+    def fit(self, init, max_iter=300, tol=1e-4, want_labels=True, labels_out=None, cluster_map_out=None):
+        """One Lloyd run from explicit centroids.  Returns dict(labels, centers, n_iter, inertia, ...).
+
+        ``cluster_map_out``: optional uint8 (k <= 255) or uint16 array / tensor, host or CUDA, with
+        one element per pixel of the last ``unproject``'s range; it receives the labels on the
+        pixel grid (label + 1 where a pixel produced a point, 0 elsewhere), written by the final
+        pass.  A CUDA output is ordered against torch's current stream like ``labels_out``."""
         init = np.ascontiguousarray(init, dtype=np.float64)
         if init.ndim != 2 or init.shape[1] != 3:
             raise ValueError("init must be [K,3]")
@@ -389,11 +417,12 @@ class Engine:
         centers = np.empty((k, 3), dtype=np.float64)
         n_iter = c_int(0)
         inertia = c_double(0.0)
+        map_mem = self._bind_cluster_map(cluster_map_out) if cluster_map_out is not None else None
         self._check(self._lib.mdkm_fit(
             self._h, int(k), init.ctypes.data_as(POINTER(c_double)), int(max_iter), float(tol),
             c_void_p(lab_ptr) if lab_ptr else None, lab_mem,
             centers.ctypes.data_as(POINTER(c_double)), byref(n_iter), byref(inertia)))
-        if lab_mem == C.MEM_DEVICE:
+        if lab_mem == C.MEM_DEVICE or map_mem == C.MEM_DEVICE:
             self._before_torch()
         nref, nrel, tols = c_int64(0), c_int64(0), c_double(0)
         self._lib.mdkm_fit_stats(self._h, byref(nref), byref(nrel), byref(tols))
@@ -422,16 +451,20 @@ class Engine:
         self._lib.mdkm_fit_stats(self._h, byref(nref), None, None)
         return labels, sums, counts, int(nref.value)
 
-    def predict(self, centroids, want_labels=True):
-        """E-step only (KMeans.predict): returns (labels int32[N] or None, inertia)."""
+    def predict(self, centroids, want_labels=True, cluster_map_out=None):
+        """E-step only (KMeans.predict): returns (labels int32[N] or None, inertia).
+        ``cluster_map_out``: as in ``fit``."""
         c = np.ascontiguousarray(centroids, dtype=np.float64)
         if c.ndim != 2 or c.shape[1] != 3:
             raise ValueError("centroids must be [K,3]")
         labels = self._result_buffer("labels", (self.n_points,), np.int32) if want_labels else None
         inertia = c_double(0.0)
+        map_mem = self._bind_cluster_map(cluster_map_out) if cluster_map_out is not None else None
         self._check(self._lib.mdkm_predict(
             self._h, int(c.shape[0]), c.ctypes.data_as(POINTER(c_double)),
             c_void_p(labels.ctypes.data) if labels is not None else None, C.MEM_HOST, byref(inertia)))
+        if map_mem == C.MEM_DEVICE:
+            self._before_torch()
         return labels, float(inertia.value)
 
     def kmeans_plusplus(self, n_clusters: int, random_state):

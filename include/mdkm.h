@@ -138,6 +138,21 @@ int mdkm_unproject(mdkm_handle* h, const void* hm, int hm_dtype, float hm_scale,
 int mdkm_bind_cloud_output(mdkm_handle* h, float* out_host, int64_t capacity_points,
                            int napari_order);
 
+/* Optional: have the NEXT mdkm_fit or mdkm_predict on this handle also write its labels as a
+ * cluster map over the pixel range [pix_begin, pix_begin + pix_count) of the last
+ * mdkm_unproject: a pixel that produced a point holds that point's label + 1, every other
+ * pixel 0 (napari's background label).  The map encodes exactly the labels the call returns.
+ * elem_bytes: 1 (uint8, k <= 255) or 2 (uint16); out holds capacity_pixels >= pix_count
+ * elements, in host or device memory per `mem` (device outputs are written in place on the
+ * handle's stream).  The map is written by the final labelling pass itself, without a second
+ * pass over the cloud.  out == NULL clears the binding.  The binding is consumed by that one
+ * call, and dropped by mdkm_unproject / mdkm_set_points.  Errors: MDKM_ERR_STATE when the
+ * resident cloud came from mdkm_set_points (it has no raster); MDKM_ERR_INVALID for a bad
+ * elem_bytes or a capacity that is too small here, and from the mdkm_fit / mdkm_predict, before
+ * any work is enqueued, when k labels do not fit elem_bytes. */
+int mdkm_bind_cluster_map(mdkm_handle* h, void* out, int elem_bytes, int64_t capacity_pixels,
+                          int mem);
+
 /* Load an already unprojected cloud (this rank's shard).  Replaces the `X` argument of the
  * reference's KMeans(...).fit_predict(X) call (members/jasraj/land_use_classification/
  * core.py:227-228) for d = 3. */
