@@ -396,6 +396,21 @@ int compute_frame(mdkm_handle* h, bool minmax_ready = false) {
     double half = 0.5 * (hi - lo);
     double o = (fabs(mid) > 0.25 * half) ? nearbyint(mid) : 0.0;
     o = (double)(float)o;
+    // A cloud narrower than a unit and away from an integer (extent 1e-3 around 0.5): the integer
+    // origin would leave a half-range of up to 0.5 and a quantum set by it instead of by the
+    // extent.  Then the origin is a multiple of the largest power of two not above the half-range
+    // (half-range below 1.5x the cloud's), provided x - o stays exact in FP32: that step is no
+    // finer than the ulp of the largest |x| (x - o is a multiple of the ulp of x) and every |x|
+    // exceeds the new half-range (so x - o needs no more bits than x).
+    if (half > 0.0 && fabs(mid - o) > half) {
+      const double step = ldexp(1.0, ilogb(half));
+      const double o2 = nearbyint(mid / step) * step;
+      const double hr2 = std::max(fabs(lo - o2), fabs(hi - o2));
+      const double amin = lo > 0.0 ? lo : (hi < 0.0 ? -hi : 0.0);
+      const double amax = std::max(fabs(lo), fabs(hi));
+      const double ulp_max = ldexp(1.0, ilogb(amax) - 23);
+      if (hr2 < amin && step >= ulp_max && (double)(float)o2 == o2) o = o2;
+    }
     double hr = std::max(fabs(lo - o), fabs(hi - o));
     hr = hr * (1.0 + 1e-6) + 1e-30;  // FP32 rounding of x - o
     int e = (int)floor(log2((double)((1 << kQuantBits) - 2) / hr));
@@ -608,6 +623,15 @@ int build_mirror_raster(mdkm_handle* h, int cell_px) {
   CU(cudaLaunchKernelExC(&cfg, reinterpret_cast<const void*>(raster_gather_kernel), args));
   h->launches += 2;
   CU(cudaGetLastError());
+  return MDKM_OK;
+}
+
+// The k x 3 centroids a caller hands in: a NaN or an infinity would go straight into the tables
+// (scikit-learn rejects such an init; the points get the same check in compute_frame).
+int check_centroids(mdkm_handle* h, int k, const double* c, const char* what) {
+  if (k < 1 || k > kMaxK) return fail(h, MDKM_ERR_INVALID, "k must be in [1, %d]", kMaxK);
+  for (long long i = 0; i < 3ll * k; ++i)
+    if (!isfinite(c[i])) return fail(h, MDKM_ERR_INVALID, "%s row %lld has a non-finite coordinate", what, i / 3);
   return MDKM_OK;
 }
 
@@ -1627,6 +1651,7 @@ int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol
   MapOut map;
   OK(take_cluster_map(h, k, map));
   if (!init) return fail(h, MDKM_ERR_INVALID, "init centroids required");
+  OK(check_centroids(h, k, init, "init"));
   if (max_iter < 1) return fail(h, MDKM_ERR_INVALID, "max_iter must be >= 1");
   if (tol < 0) return fail(h, MDKM_ERR_INVALID, "tol must be >= 0");
   CU(cudaSetDevice(h->device));
@@ -1811,6 +1836,7 @@ int mdkm_lloyd_step(mdkm_handle* h, int k, const double* centroids, int32_t* lab
                     double* sums_out, int64_t* counts_out) {
   if (!h) return MDKM_ERR_INVALID;
   if (!centroids) return fail(h, MDKM_ERR_INVALID, "centroids required");
+  OK(check_centroids(h, k, centroids, "centroids"));
   CU(cudaSetDevice(h->device));
   KmBuffers kb{};
   OK(prepare_kmeans(h, k, kb));
@@ -1856,6 +1882,7 @@ int mdkm_predict(mdkm_handle* h, int k, const double* centroids, int32_t* labels
   MapOut map;
   OK(take_cluster_map(h, k, map));
   if (!centroids) return fail(h, MDKM_ERR_INVALID, "centroids required");
+  OK(check_centroids(h, k, centroids, "centroids"));
   CU(cudaSetDevice(h->device));
   KmBuffers kb{};
   OK(prepare_kmeans(h, k, kb));

@@ -201,6 +201,7 @@ int mdkm_ground_level(mdkm_handle* h, float* height_norm_out, int mem, double* h
  * algorithm="lloyd", max_iter, tol).fit(X) as the reference calls it (core.py:227-228;
  * algorithm in sklearn/cluster/_kmeans.py:630-758, 1436-1563 and _k_means_lloyd.pyx).
  * init: k x 3 float64, row-major, same coordinates as the points.
+ * A NaN or infinite coordinate in init, or in the centroids of mdkm_lloyd_step / mdkm_predict, gives MDKM_ERR_INVALID.
  * labels_out: int32[n_local] (may be NULL); centroids_out: float64[k*3]; n_iter_out,
  * inertia_out as scikit-learn's n_iter_ / inertia_.  With a communicator the point set is
  * the union of all ranks' shards and every rank gets the same centroids / n_iter /
