@@ -57,6 +57,7 @@ SIGNATURES = {
                                c_int64, c_int64, c_float, c_int, c_int, POINTER(c_int64)]),
     "mdkm_bind_cloud_output": (c_int, [c_void_p, c_void_p, c_int64, c_int]),
     "mdkm_bind_cluster_map": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int]),
+    "mdkm_bind_day_stats": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int]),
     "mdkm_set_points": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_int]),
     "mdkm_num_points": (c_int64, [c_void_p]),
     "mdkm_num_points_global": (c_int64, [c_void_p]),

@@ -49,6 +49,11 @@ class FusionResult:
     # labels on the pixel grid (return_cluster_map=True): label + 1 where a pixel produced a point,
     # 0 elsewhere; uint8 (k <= 255) or uint16, [D,H,W] -- or this rank's flat pixel range
     cluster_map: Optional[np.ndarray] = None
+    # per-day composition (return_day_stats=True), rows = global days of the stack: points of day d
+    # with label j (int64 [D,K]) and their mean (x, y, z) in the clustered frame (float64 [D,K,3],
+    # NaN where the count is 0); summed over all ranks
+    day_counts: Optional[np.ndarray] = None
+    day_means: Optional[np.ndarray] = None
 
     # scikit-learn style aliases
     @property
@@ -123,13 +128,15 @@ def cluster_map_dtype(n_clusters: int):
 
 
 def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_state, want_labels=True,
-                labels_out=None, gather_mappings=None, cluster_map_out=None):
+                labels_out=None, gather_mappings=None, cluster_map_out=None, day_stats=False):
     """KMeans.fit driver (sklearn/_kmeans.py:1436-1563): init, n_init restarts, best inertia.
 
     ``labels_out``: optional int32 array that receives this rank's labels of the best run.
     ``cluster_map_out``: optional uint8 / uint16 array that receives the best run's cluster map
     (``Engine.fit``).  With restarts every run writes its map into a device scratch tensor; the
     best one is kept by swapping and copied out once at the end.
+    ``day_stats``: the result also has ``day_counts`` / ``day_means`` (``Engine.fit``) -- every run
+    returns fresh arrays, so the best run's stay with it.
     ``gather_mappings``: with a multi-rank engine, the collective that lets the ranks agree on
     sklearn's "same clustering up to a permutation" test (see ``_is_same_clustering``); when it is
     missing the test is skipped on multi-rank engines (the inertia comparison alone decides)."""
@@ -173,7 +180,7 @@ def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_
             centers0, _ = eng.kmeans_plusplus(k, rs)
         r = eng.fit(centers0, max_iter=max_iter, tol=tol, want_labels=want_labels,
                     labels_out=labels_out if (single and want_labels) else None,
-                    cluster_map_out=cluster_map_out if single else run_map)
+                    cluster_map_out=cluster_map_out if single else run_map, day_stats=day_stats)
         # sklearn/_kmeans.py:1534-1541: a run replaces the best one when its inertia is lower AND it
         # is not the same clustering up to a permutation.  The inertia is global, so every rank
         # takes the same branch and the (collective) permutation test pairs up.
@@ -214,7 +221,8 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
                          max_iter=300, tol=1e-4, random_state=None, max_abs_height=MAX_ABS_HEIGHT,
                          detrend=False, disparity_scale=None, ground_level=False, return_cloud=True,
                          device=0, devices=None, engine=None, stack_shape=None,
-                         pix_begin=0, raster_layout=None, return_cluster_map=False) -> FusionResult:
+                         pix_begin=0, raster_layout=None, return_cluster_map=False,
+                         return_day_stats=False) -> FusionResult:
     """Unproject a multi-day height-map stack into one XYZ cloud and cluster it (Lloyd).
 
     height_maps : float32 ``[D,H,W]`` (NaN = nodata), numpy or torch (CPU or CUDA); or int16
@@ -242,6 +250,12 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
         uint8 for ``n_clusters <= 255``, else uint16.  ``[D,H,W]`` for a whole stack; this rank's
         flat ``[pix_count]`` slice for a pre-sharded call (``stack_shape`` / ``pix_begin``), as
         ``labels`` is this rank's shard.  The map is written on the GPU by the final labelling pass.
+    return_day_stats : also return ``day_counts`` (int64 ``[D,K]``: points of day d with label j) and
+        ``day_means`` (float64 ``[D,K,3]``: their mean (x, y, z) in the clustered coordinates, like
+        ``centroids``; NaN where the count is 0).  Rows are the global days of the stack, also for a
+        pre-sharded call, and the numbers are summed over all ranks.  They come from integer sums on
+        the fixed-point frame accumulated by the final labelling pass, so they are bitwise the same
+        for any number of GPUs.
     Returns a FusionResult; ``fused_cloud`` is float32 ``[N,3]`` in napari (z,y,x) order.
     """
     from .group import DeviceGroup
@@ -253,7 +267,8 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
                               devices=devices, n_clusters=n_clusters, init=init, n_init=n_init, max_iter=max_iter,
                               tol=tol, random_state=random_state, max_abs_height=max_abs_height, detrend=detrend,
                               disparity_scale=disparity_scale, ground_level=ground_level, return_cloud=return_cloud,
-                              raster_layout=raster_layout, return_cluster_map=return_cluster_map)
+                              raster_layout=raster_layout, return_cluster_map=return_cluster_map,
+                              return_day_stats=return_day_stats)
     own = engine is None
     eng = engine or Engine(device)
     try:
@@ -279,19 +294,20 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
             D, H, W, _, count = eng.raster_range
             cmap = np.empty((D, H, W) if stack_shape is None else (count,), dtype=cluster_map_dtype(n_clusters))
         r = _run_kmeans(eng, n_clusters=n_clusters, init=init, n_init=n_init, max_iter=max_iter,
-                        tol=tol, random_state=random_state, cluster_map_out=cmap)
+                        tol=tol, random_state=random_state, cluster_map_out=cmap, day_stats=return_day_stats)
         eng.wait()
         return FusionResult(labels=r["labels"], centroids=r["centers"], fused_cloud=cloud,
                             n_iter=r["n_iter"], inertia=r["inertia"], n_points=n,
                             n_refined=r["n_refined"], n_relocations=r["n_relocations"],
-                            height_norm=hn, extra=extra, cluster_map=cmap)
+                            height_norm=hn, extra=extra, cluster_map=cmap,
+                            day_counts=r.get("day_counts"), day_means=r.get("day_means"))
     finally:
         if own:
             eng.close()
 
 
 def _fuse_on_group(height_maps, valid_masks, *, group, devices, n_clusters, init, n_init, max_iter, tol,
-                   random_state, return_cluster_map=False, **unproject_kw) -> FusionResult:
+                   random_state, return_cluster_map=False, return_day_stats=False, **unproject_kw) -> FusionResult:
     """``fuse_multiday_kmeans`` on several devices of this process (``group.DeviceGroup``)."""
     import threading
 
@@ -321,7 +337,7 @@ def _fuse_on_group(height_maps, valid_masks, *, group, devices, n_clusters, init
             return _run_kmeans(eng, n_clusters=n_clusters, init=init, n_init=n_init, max_iter=max_iter, tol=tol,
                                random_state=states[r], labels_out=labels_out,
                                gather_mappings=gather_for(r) if grp.world > 1 else None,
-                               cluster_map_out=cluster_map_out)
+                               cluster_map_out=cluster_map_out, day_stats=return_day_stats)
 
         res, labels, cloud, hn, extra = grp.fuse(
             height_maps, valid_masks, run_kmeans=run,
@@ -329,7 +345,8 @@ def _fuse_on_group(height_maps, valid_masks, *, group, devices, n_clusters, init
         return FusionResult(labels=labels, centroids=res["centers"], fused_cloud=cloud, n_iter=res["n_iter"],
                             inertia=res["inertia"], n_points=int(labels.shape[0]), n_refined=res["n_refined"],
                             n_relocations=res["n_relocations"], height_norm=hn, extra=extra,
-                            cluster_map=extra.pop("cluster_map", None))
+                            cluster_map=extra.pop("cluster_map", None),
+                            day_counts=res.get("day_counts"), day_means=res.get("day_means"))
     finally:
         if own:
             grp.close()

@@ -827,8 +827,15 @@ struct FinalParams {
   long long map_pix_begin;    // global index of the range's first pixel
   long long map_HW;
   long long map_day0;         // day of map_pix_begin
-  const long long* map_seg;   // [map_nseg + 1] point offsets of the days of the range (device)
-  int map_nseg;
+  const long long* map_seg;   // [map_nseg + 1] point offsets of the days of the range (device; also
+  int map_nseg;               // read by the statistics below)
+  // per-(day, cluster) statistics (lloyd_final_kernel<kChunks, kMap, true>): every point adds
+  // (qx, qy, qz, 1) to the four int64 words of slot (stats_day0 + day) * k + label
+  unsigned long long* stats_acc;  // [slots * 4], cleared by the host
+  long long stats_day0;           // global day of segment 0 of the cloud
+  int stats_slots;                // days of the stack * k
+  int stats_smem_off;             // > 0: per-warp copies of the slots at this byte offset of the dynamic shared
+                                  // memory, flushed once per CTA at the end; 0: points go to stats_acc directly
 };
 
 // Day of this lane's points in the cluster map: segment `day` holds the points before `next`,
@@ -2317,6 +2324,22 @@ __global__ void read_sums_kernel(const unsigned long long* acc, int k, Frame fr,
   }
 }
 
+// Per-(day, cluster) slots of the final pass -> counts and means (original frame).  The exact
+// coordinate sum is rebuilt first and divided once: exact whenever it fits 53 bits, so the mean
+// is then the correctly rounded mean of the grid points.  Explicit roundings: no FMA contraction.
+__global__ void day_stats_kernel(const unsigned long long* acc, long long slots, Frame fr, long long* counts_out,
+                                 double* means_out) {
+  for (long long j = blockIdx.x * (long long)blockDim.x + threadIdx.x; j < slots; j += (long long)gridDim.x * blockDim.x) {
+    const long long cnt = (long long)acc[j * 4 + 3];
+    counts_out[j] = cnt;
+    for (int d = 0; d < 3; ++d) {
+      const double sum = __dadd_rn(__ddiv_rn((double)(long long)acc[j * 4 + d], fr.scale[d]),
+                                   __dmul_rn((double)cnt, fr.origin[d]));
+      means_out[3 * j + d] = cnt ? __ddiv_rn(sum, (double)cnt) : __longlong_as_double(0x7ff8000000000000ll);
+    }
+  }
+}
+
 // ---------------------------------------------------------------------------------------
 // In raster order a group is a strip of one row -- except the one that runs over the end of a
 // row (one in W/128): its box spans the whole width of the frame, every cluster along the row
@@ -2360,27 +2383,80 @@ __device__ __forceinline__ void assign_split_group(const float (&xo)[4], const f
   }
 }
 
+// Adds this lane's points to their (day, cluster) slots; key[e] < 0 for a point past the end.
+// Warp-synchronous.  Lanes with equal keys are summed first (__match_any_sync, one key per lane
+// and round, so at most four rounds): consecutive points mostly share a raster row and a
+// cluster, and a group of one key costs one slot update.  32-bit partial sums: a round sums at
+// most 128 points of |q| < 2^22.  kPrivate: `acc` is this warp's own copy of the slots (shared
+// memory), updated without atomics -- the keys of one round are distinct, and __syncwarp orders
+// the rounds; otherwise the global slots, with 64-bit atomic adds.
+template <bool kPrivate>
+__device__ __forceinline__ void stats_add(unsigned long long* acc, const int (&key)[4], const int (&qx)[4],
+                                          const int (&qy)[4], const int (&qz)[4], int lane) {
+  unsigned int rem = (key[0] >= 0 ? 1u : 0u) | (key[1] >= 0 ? 2u : 0u) | (key[2] >= 0 ? 4u : 0u) |
+                     (key[3] >= 0 ? 8u : 0u);
+  while (__any_sync(0xffffffffu, rem != 0)) {
+    const int mine = (rem & 1u) ? key[0] : ((rem & 2u) ? key[1] : ((rem & 4u) ? key[2] : ((rem & 8u) ? key[3] : -1)));
+    int sx = 0, sy = 0, sz = 0, sc = 0;
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      const bool hit = ((rem >> e) & 1u) && key[e] == mine;
+      sx += hit ? qx[e] : 0;
+      sy += hit ? qy[e] : 0;
+      sz += hit ? qz[e] : 0;
+      sc += hit ? 1 : 0;
+      rem &= hit ? ~(1u << e) : ~0u;
+    }
+    const unsigned int peers = __match_any_sync(0xffffffffu, mine);
+    sx = __reduce_add_sync(peers, sx);
+    sy = __reduce_add_sync(peers, sy);
+    sz = __reduce_add_sync(peers, sz);
+    sc = __reduce_add_sync(peers, sc);
+    if (mine >= 0 && lane == __ffs(peers) - 1) acc_add<kPrivate>(acc, mine, sx, sy, sz, (unsigned int)sc);
+    if (kPrivate) __syncwarp();
+  }
+}
+
 // labels and FP64 inertia (direct form) of this lane's four points of a group; with kMap also
-// label + 1 at each point's pixel of the cluster map (x and y are exact pixel coordinates)
-template <bool kMap>
+// label + 1 at each point's pixel of the cluster map (x and y are exact pixel coordinates); with
+// kStats also the point's fixed-point coordinates into its (day, label) slot.  Warp-synchronous
+// with kStats.
+template <bool kMap, bool kStats>
 __device__ __forceinline__ void final_emit(const FinalParams& p, const double4* __restrict__ c64, const FrameF& f,
                                            long long i0, const float (&xo)[4], const float (&yo)[4],
                                            const float (&zo)[4], const int (&lab)[4], double& inert,
-                                           MapCursor& mc) {
-  if (kMap) {
+                                           MapCursor& mc, unsigned long long* s_stats, int lane) {
+  int day[4] = {-1, -1, -1, -1};
+  if (kMap || kStats) {
 #pragma unroll
     for (int e = 0; e < 4; ++e) {
       const long long i = i0 + e;
       if (i < p.n) {
         while (i >= mc.next) {
           mc.next = __ldg(p.map_seg + ++mc.day + 1);
-          mc.base += p.map_HW;
+          if (kMap) mc.base += p.map_HW;
         }
-        const long long pix = mc.base + (long long)pixel_index(yo[e]) * p.map_W + pixel_index(xo[e]);
-        if (p.map_elem == 1) static_cast<unsigned char*>(p.map_out)[pix] = (unsigned char)(lab[e] + 1);
-        else static_cast<unsigned short*>(p.map_out)[pix] = (unsigned short)(lab[e] + 1);
+        if (kStats) day[e] = mc.day;
+        if (kMap) {
+          const long long pix = mc.base + (long long)pixel_index(yo[e]) * p.map_W + pixel_index(xo[e]);
+          if (p.map_elem == 1) static_cast<unsigned char*>(p.map_out)[pix] = (unsigned char)(lab[e] + 1);
+          else static_cast<unsigned short*>(p.map_out)[pix] = (unsigned short)(lab[e] + 1);
+        }
       }
     }
+  }
+  if (kStats) {
+    // q = rint(x' * scale) exactly as the Lloyd step's sums take it (lloyd_step_kernel)
+    int key[4], qx[4], qy[4], qz[4];
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      key[e] = day[e] >= 0 ? (int)(p.stats_day0 + day[e]) * p.k + lab[e] : -1;
+      qx[e] = (int)(__float_as_uint(fmaf(xo[e] - f.ox, f.sx, kMagic)) - kMagicBits);
+      qy[e] = (int)(__float_as_uint(fmaf(yo[e] - f.oy, f.sy, kMagic)) - kMagicBits);
+      qz[e] = (int)(__float_as_uint(fmaf(zo[e] - f.oz, f.sz, kMagic)) - kMagicBits);
+    }
+    if (s_stats) stats_add<true>(s_stats, key, qx, qy, qz, lane);
+    else stats_add<false>(p.stats_acc, key, qx, qy, qz, lane);
   }
 #pragma unroll
   for (int e = 0; e < 4; ++e) {
@@ -2407,8 +2483,10 @@ __device__ __forceinline__ void final_emit(const FinalParams& p, const double4* 
 // Final pass over the resident cloud (reference point order): E-step with the final centroids
 // -> int32 labels, and the inertia in FP64 (direct form, fixed-order reduction).  kMap: the
 // labels also go to the cluster map (FinalParams::map_out, cleared by the host beforehand).
+// kStats: per-(day, cluster) counts and fixed-point coordinate sums (FinalParams::stats_acc,
+// cleared by the host beforehand); integers, so the same for any grid or point order.
 // ---------------------------------------------------------------------------------------
-template <int kChunks, bool kMap>
+template <int kChunks, bool kMap, bool kStats>
 __global__ void __launch_bounds__(kThreads, kChunks == 0 ? MDKM_FINAL_CTAS0 : 3) lloyd_final_kernel(const FinalParams p) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const int kp32 = kChunks > 0 ? kChunks * 32 : ((p.kpad + 31) & ~31);
@@ -2435,6 +2513,12 @@ __global__ void __launch_bounds__(kThreads, kChunks == 0 ? MDKM_FINAL_CTAS0 : 3)
   for (int i = p.kpad + tid; i < kp32; i += kThreads) {
     s_fast[i] = make_float4(0.f, 0.f, 0.f, __int_as_float(0x7f800000));
   }
+  unsigned long long* s_stats = nullptr;  // this warp's slots
+  if (kStats && p.stats_smem_off) {
+    unsigned long long* s_all = reinterpret_cast<unsigned long long*>(smem_raw + p.stats_smem_off);
+    for (int i = tid; i < (kThreads / 32) * p.stats_slots * 4; i += kThreads) s_all[i] = 0ull;
+    s_stats = s_all + (size_t)warp * p.stats_slots * 4;
+  }
   __syncthreads();
   if (tid == 0) {
     mbar_expect_tx(&s_bar, (uint32_t)p.kpad * 16u + bkt_bytes);
@@ -2457,7 +2541,7 @@ __global__ void __launch_bounds__(kThreads, kChunks == 0 ? MDKM_FINAL_CTAS0 : 3)
   const long long g_first = ((long long)blockIdx.x * (kThreads / 32) + warp) * per_warp;
   const long long g_last = min(n_groups, g_first + per_warp);
   MapCursor mc{0, 0, 0};
-  if (kMap && g_first < g_last) mc = map_cursor(p, g_first * kGroup + lane * 4);
+  if ((kMap || kStats) && g_first < g_last) mc = map_cursor(p, g_first * kGroup + lane * 4);
   // few centroids: the next group's block is requested before this one is worked on (one group
   // of look-ahead in registers) -- a warp walks its run serially, so without it every group pays
   // a DRAM round trip.  With many centroids the pass is bound by the candidate walk instead and
@@ -2494,11 +2578,11 @@ __global__ void __launch_bounds__(kThreads, kChunks == 0 ? MDKM_FINAL_CTAS0 : 3)
                                     s_cand + warp * kCandCap, lane, lab, n_ref);
     if (ncand < 0) assign_group<kChunks>(xc, yc, zc, xo, yo, zo, f, s_fast, c64, p.k, kp32, thresh, lane, lab, n_ref);
     hint = __shfl_sync(0xffffffffu, lab[0], 0);
-    final_emit<kMap>(p, c64, f, i0, xo, yo, zo, lab, inert, mc);
+    final_emit<kMap, kStats>(p, c64, f, i0, xo, yo, zo, lab, inert, mc, s_stats, lane);
   }
   // second loop: the groups that run over the end of a raster row (one in W/128), two halves each
   if (p.split_rows) {
-    if (kMap && g_first < g_last) mc = map_cursor(p, g_first * kGroup + lane * 4);  // (walks the run again)
+    if ((kMap || kStats) && g_first < g_last) mc = map_cursor(p, g_first * kGroup + lane * 4);  // (walks the run again)
     for (long long gb = g_first; gb < g_last; gb += 32) {
       bool sp = false;
       if (gb + lane < g_last) {
@@ -2515,7 +2599,7 @@ __global__ void __launch_bounds__(kThreads, kChunks == 0 ? MDKM_FINAL_CTAS0 : 3)
         int lab[4] = {0, 0, 0, 0};
         assign_split_group<kChunks>(xo, yo, zo, f, s_fast, c64, bkt_bytes ? s_bkt : nullptr, p.k, kp32, thresh,
                                     s_cand + warp * kCandCap, lane, lab, n_ref);
-        final_emit<kMap>(p, c64, f, g * kGroup + lane * 4, xo, yo, zo, lab, inert, mc);
+        final_emit<kMap, kStats>(p, c64, f, g * kGroup + lane * 4, xo, yo, zo, lab, inert, mc, s_stats, lane);
       }
     }
   }
@@ -2523,6 +2607,15 @@ __global__ void __launch_bounds__(kThreads, kChunks == 0 ? MDKM_FINAL_CTAS0 : 3)
   n_ref = __reduce_add_sync(0xffffffffu, n_ref);
   if (lane == 0 && n_ref) atomicAdd(&s_refined, n_ref);
   __syncthreads();
+  if (s_stats) {  // (block_sum_fixed synchronised the CTA: every point is in the warps' slots)
+    const unsigned long long* s_all = reinterpret_cast<const unsigned long long*>(smem_raw + p.stats_smem_off);
+    const int words = p.stats_slots * 4;
+    for (int i = tid; i < words; i += kThreads) {
+      unsigned long long v = 0ull;
+      for (int w = 0; w < kThreads / 32; ++w) v += s_all[w * words + i];
+      if (v) atomicAdd(&p.stats_acc[i], v);
+    }
+  }
   if (tid == 0) {
     p.partials[blockIdx.x] = bsum;
     if (s_refined) atomicAdd(&p.st->n_refined, (unsigned long long)s_refined);

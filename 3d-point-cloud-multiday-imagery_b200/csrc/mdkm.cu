@@ -158,6 +158,16 @@ struct mdkm_handle {
   int bound_map_elem = 0, bound_map_mem = MDKM_MEM_HOST;
   DevBuf<unsigned char> map_stage;   // host outputs are written here, then copied
   DevBuf<long long> map_seg;         // the days' point offsets (d_seg_off may hold merged segments)
+  // per-(day, cluster) statistics (mdkm_bind_day_stats) of the next fit / predict
+  int stack_days = 0;                // days of the stack of the last mdkm_unproject (1 after mdkm_set_points)
+  long long day0 = 0;                // global day of the resident cloud's first segment
+  int64_t* bound_counts = nullptr;
+  double* bound_means = nullptr;
+  int bound_stats_kcap = 0;
+  DevBuf<unsigned long long> stats_acc;  // [days * k * 4] (qx, qy, qz, count) per slot
+  DevBuf<unsigned char> stats_dev;       // counts, then means, converted on the device
+  unsigned char* stats_host = nullptr;   // pinned: their copy, handed to the caller after the sync
+  size_t stats_host_cap = 0;
 
   // communicator
   ncclComm_t comm = nullptr;
@@ -477,15 +487,15 @@ int step_occupancy(mdkm_handle* h, StepKernel fn, size_t smem, int* occ) {
 }
 
 typedef void (*FinalKernel)(const FinalParams);
-FinalKernel pick_final_kernel(int kpad, bool map = false) {
-  if (map) {
-    if (kpad <= 32) return lloyd_final_kernel<1, true>;
-    if (kpad <= 64) return lloyd_final_kernel<2, true>;
-    return lloyd_final_kernel<0, true>;
-  }
-  if (kpad <= 32) return lloyd_final_kernel<1, false>;
-  if (kpad <= 64) return lloyd_final_kernel<2, false>;
-  return lloyd_final_kernel<0, false>;
+template <bool kMap, bool kStats>
+FinalKernel pick_final_chunks(int kpad) {
+  if (kpad <= 32) return lloyd_final_kernel<1, kMap, kStats>;
+  if (kpad <= 64) return lloyd_final_kernel<2, kMap, kStats>;
+  return lloyd_final_kernel<0, kMap, kStats>;
+}
+FinalKernel pick_final_kernel(int kpad, bool map = false, bool stats = false) {
+  if (stats) return map ? pick_final_chunks<true, true>(kpad) : pick_final_chunks<false, true>(kpad);
+  return map ? pick_final_chunks<true, false>(kpad) : pick_final_chunks<false, false>(kpad);
 }
 
 struct KmBuffers {
@@ -907,8 +917,26 @@ struct MapOut {
   size_t bytes = 0;
 };
 
+// Per-(day, cluster) statistics taken by one fit / predict (mdkm_bind_day_stats): accumulated by
+// the final pass, summed over the ranks, converted on the device and copied to the pinned
+// stage; `counts` / `means` receive them after the call's synchronisation.
+struct StatsOut {
+  long long slots = 0;  // days * k
+  int64_t* counts = nullptr;
+  double* means = nullptr;
+};
+
 int run_final(mdkm_handle* h, const KmBuffers& kb, int* labels_dev, bool skip_paused = false,
-              double* centroids_host = nullptr, DevStatus* status_host = nullptr, const MapOut* map = nullptr);
+              double* centroids_host = nullptr, DevStatus* status_host = nullptr, const MapOut* map = nullptr,
+              const StatsOut* stats = nullptr);
+
+// the days' point offsets on the device, for the day cursor of the final pass
+int upload_day_offsets(mdkm_handle* h) {
+  const size_t n_off = h->seg_off.size();
+  OK(ensure(h, h->map_seg, n_off));
+  CU(cudaMemcpyAsync(h->map_seg.p, h->seg_off.data(), n_off * 8, cudaMemcpyHostToDevice, h->stream));
+  return MDKM_OK;
+}
 
 // Consumes the binding of mdkm_bind_cluster_map (whatever happens) for a call with k clusters:
 // checks that k fits the element type, stages host outputs, uploads the days' point offsets.
@@ -929,10 +957,60 @@ int take_cluster_map(mdkm_handle* h, int k, MapOut& m) {
     m.dev = h->map_stage.p;
     m.host = out;
   }
-  const size_t n_off = h->seg_off.size();
-  OK(ensure(h, h->map_seg, n_off));
-  CU(cudaMemcpyAsync(h->map_seg.p, h->seg_off.data(), n_off * 8, cudaMemcpyHostToDevice, h->stream));
+  return upload_day_offsets(h);
+}
+
+// Consumes the binding of mdkm_bind_day_stats (whatever happens) for a call with k clusters:
+// checks k against the bound capacity, sizes the accumulators, uploads the days' point offsets.
+int take_day_stats(mdkm_handle* h, int k, StatsOut& s) {
+  int64_t* counts = h->bound_counts;
+  double* means = h->bound_means;
+  const int kcap = h->bound_stats_kcap;
+  h->bound_counts = nullptr;
+  h->bound_means = nullptr;
+  if (!counts) return MDKM_OK;
+  if (k > kcap) return fail(h, MDKM_ERR_INVALID, "k=%d exceeds the k_capacity %d of the bound day statistics", k, kcap);
+  if (k < 1 || k > kMaxK) return MDKM_OK;  // (rejected with the call's own message)
+  CU(cudaSetDevice(h->device));
+  s.slots = (long long)h->stack_days * k;
+  s.counts = counts;
+  s.means = means;
+  OK(ensure(h, h->stats_acc, (size_t)s.slots * 4));
+  OK(ensure(h, h->stats_dev, (size_t)s.slots * 32));
+  if (h->stats_host_cap < (size_t)s.slots * 32) {
+    if (h->stats_host) {
+      CU(cudaStreamSynchronize(h->stream));
+      CU(cudaFreeHost(h->stats_host));
+      h->stats_host = nullptr;
+      h->stats_host_cap = 0;
+    }
+    CU(cudaMallocHost(&h->stats_host, (size_t)s.slots * 32));
+    h->stats_host_cap = (size_t)s.slots * 32;
+  }
+  return upload_day_offsets(h);
+}
+
+// Behind the final pass, on the stream: the sums over the ranks, counts and means, their copy
+// to the pinned stage.  (A final pass that returned early for a relocation leaves zeros; the
+// pass after the relocation runs this again.)
+int reduce_day_stats(mdkm_handle* h, const StatsOut& s) {
+  if (!s.counts) return MDKM_OK;
+  OK(allreduce(h, h->stats_acc.p, (size_t)s.slots * 4, kNcclInt64, kNcclSum));
+  long long* d_counts = reinterpret_cast<long long*>(h->stats_dev.p);
+  double* d_means = reinterpret_cast<double*>(h->stats_dev.p + (size_t)s.slots * 8);
+  day_stats_kernel<<<grid_for(h, (s.slots + kThreads - 1) / kThreads, 4), kThreads, 0, h->stream>>>(
+      h->stats_acc.p, s.slots, h->fr, d_counts, d_means);
+  ++h->launches;
+  CU(cudaGetLastError());
+  CU(cudaMemcpyAsync(h->stats_host, h->stats_dev.p, (size_t)s.slots * 32, cudaMemcpyDeviceToHost, h->stream));
   return MDKM_OK;
+}
+
+// After the call's synchronisation: the pinned stage -> the caller's arrays.
+void deliver_day_stats(mdkm_handle* h, const StatsOut& s) {
+  if (!s.counts) return;
+  memcpy(s.counts, h->stats_host, (size_t)s.slots * 8);
+  memcpy(s.means, h->stats_host + (size_t)s.slots * 8, (size_t)s.slots * 24);
 }
 
 // The map's device->host copy (host outputs), on the compute stream behind the final pass.
@@ -984,23 +1062,46 @@ int relocate_empty(mdkm_handle* h, const KmBuffers& kb, int n_empty) {
 
 // (the ticket is zero: fit_head clears it, every final pass leaves it so)
 int run_final(mdkm_handle* h, const KmBuffers& kb, int* labels_dev, bool skip_paused, double* centroids_host,
-              DevStatus* status_host, const MapOut* map) {
+              DevStatus* status_host, const MapOut* map, const StatsOut* stats) {
   FinalParams fp{};
   FinalKernel fn = kb.final_fn;
-  if (map && map->dev) {
+  size_t smem = kb.final_smem;
+  const bool want_map = map && map->dev, want_stats = stats && stats->counts;
+  if (want_map) {
     // pixels without a point stay 0 (napari's background label)
     if (map->bytes) CU(cudaMemsetAsync(map->dev, 0, map->bytes, h->stream));
-    fn = pick_final_kernel(kb.kpad, /*map=*/true);
-    CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kb.final_smem));
     fp.map_out = map->dev;
     fp.map_elem = map->elem;
     fp.map_W = h->raster_w;
     fp.map_pix_begin = h->raster_pix_begin;
     fp.map_HW = (long long)h->raster_H * h->raster_w;
     fp.map_day0 = h->raster_pix_begin / fp.map_HW;
+  }
+  if (want_map || want_stats) {
+    fn = pick_final_kernel(kb.kpad, want_map, want_stats);
     fp.map_seg = h->map_seg.p;
     fp.map_nseg = (int)h->seg_off.size() - 1;
   }
+  if (want_stats) {
+    CU(cudaMemsetAsync(h->stats_acc.p, 0, (size_t)stats->slots * 32, h->stream));
+    fp.stats_acc = h->stats_acc.p;
+    fp.stats_day0 = h->day0;
+    fp.stats_slots = (int)stats->slots;
+    // a copy of the slots per warp in shared memory when they fit without costing a resident CTA;
+    // otherwise straight to the global slots (many days x many clusters)
+    const size_t with_slots = kb.final_smem + (size_t)(kThreads / 32) * stats->slots * 32;
+    int optin = 0, occ = 0;
+    CU(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
+    if (with_slots <= (size_t)optin) {
+      CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)with_slots));
+      CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, kThreads, with_slots));
+    }
+    if (occ >= h->occ_final) {
+      smem = with_slots;
+      fp.stats_smem_off = (int)kb.final_smem;
+    }
+  }
+  if (fn != kb.final_fn) CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   fp.pts = h->pts.p; fp.n = h->n;
   fp.labels_out = labels_dev;
   fp.table = h->table.p;
@@ -1014,7 +1115,7 @@ int run_final(mdkm_handle* h, const KmBuffers& kb, int* labels_dev, bool skip_pa
   fp.status_host = status_host;
   fp.centroids_host = centroids_host;
   for (int d = 0; d < 3; ++d) fp.origin[d] = h->fr.origin[d];
-  fn<<<kb.final_grid, kThreads, kb.final_smem, h->stream>>>(fp);
+  fn<<<kb.final_grid, kThreads, smem, h->stream>>>(fp);
   ++h->launches;
   CU(cudaGetLastError());
   return MDKM_OK;
@@ -1088,7 +1189,8 @@ void mdkm_destroy(mdkm_handle* h) {
   release(h->run_src); release(h->druns); release(h->gfirst);
   release(h->tile_status); release(h->chunk_offsets); release(h->staging); release(h->planes);
   release(h->d_seg_off); release(h->sel_hist); release(h->sel_targets);
-  release(h->map_stage); release(h->map_seg);
+  release(h->map_stage); release(h->map_seg); release(h->stats_acc); release(h->stats_dev);
+  if (h->stats_host) cudaFreeHost(h->stats_host);
   release(h->kpp_closest); release(h->kpp_cell); release(h->kpp_blk); release(h->kpp_prefix);
   release(h->kpp_partials); release(h->kpp_rand); release(h->kpp_state);
   if (h->d_status) cudaFree(h->d_status);
@@ -1290,6 +1392,9 @@ int mdkm_set_points(mdkm_handle* h, const float* xyz, int64_t n, int layout, int
   h->seg_whole = true;
   h->raster_w = 0;
   h->bound_map = nullptr;
+  h->bound_counts = nullptr;
+  h->stack_days = 1;
+  h->day0 = 0;
   h->runs_ok = false;
   h->have_points = true;
   h->frame_ok = false;
@@ -1356,6 +1461,23 @@ int mdkm_bind_cluster_map(mdkm_handle* h, void* out, int elem_bytes, int64_t cap
   return MDKM_OK;
 }
 
+int mdkm_bind_day_stats(mdkm_handle* h, int64_t* counts_out, double* means_out, int n_days, int k_capacity) {
+  if (!h) return MDKM_ERR_INVALID;
+  h->bound_counts = nullptr;
+  h->bound_means = nullptr;
+  if (!counts_out) return MDKM_OK;
+  if (!h->have_points) return fail(h, MDKM_ERR_STATE, "day statistics need a resident cloud");
+  if (!means_out) return fail(h, MDKM_ERR_INVALID, "day statistics need a means array");
+  if (n_days != h->stack_days)
+    return fail(h, MDKM_ERR_INVALID, "n_days=%d, the resident cloud's stack has %d days", n_days, h->stack_days);
+  if (k_capacity < 1 || (long long)n_days * k_capacity >= (1ll << 29))  // (slot indices are int32 on the device)
+    return fail(h, MDKM_ERR_INVALID, "k_capacity must be >= 1 and n_days * k_capacity < 2^29");
+  h->bound_counts = counts_out;
+  h->bound_means = means_out;
+  h->bound_stats_kcap = k_capacity;
+  return MDKM_OK;
+}
+
 // Unprojection as a pipeline of slabs: the host->device copy of slab s+1 (copy stream) overlaps
 // the kernels of slab s (compute stream) and, when a cloud output is bound, the device->host
 // copy of the points slab s-1 produced (result stream).  PCIe is full duplex, so the two copy
@@ -1370,6 +1492,7 @@ int mdkm_unproject(mdkm_handle* h, const void* hm, int hm_dtype, float hm_scale,
   h->bound_cloud_out = nullptr;
   h->bound_cloud_cap = 0;
   h->bound_map = nullptr;  // (a cluster map describes the range it was bound for)
+  h->bound_counts = nullptr;  // (and day statistics the stack)
   if (D < 0 || H <= 0 || W <= 0 || pix_begin < 0 || pix_count < 0 ||
       pix_begin + pix_count > (int64_t)D * H * W || (pix_count > 0 && !hm))
     return fail(h, MDKM_ERR_INVALID, "bad stack geometry");
@@ -1584,6 +1707,8 @@ int mdkm_unproject(mdkm_handle* h, const void* hm, int hm_dtype, float hm_scale,
   h->raster_H = H;
   h->raster_pix_begin = pix_begin;
   h->raster_pix_count = pix_count;
+  h->stack_days = D;
+  h->day0 = pix_begin / ((long long)H * W);
   if (want_runs) {
     const unsigned int n32 = (unsigned int)n_out;  // closes the table
     CU(cudaMemcpyAsync(h->run_src.p + pix_count / 8, &n32, 4, cudaMemcpyHostToDevice, h->stream));
@@ -1649,7 +1774,10 @@ int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol
              int labels_mem, double* centroids_out, int* n_iter_out, double* inertia_out) {
   if (!h) return MDKM_ERR_INVALID;
   MapOut map;
-  OK(take_cluster_map(h, k, map));
+  StatsOut stats;
+  const int map_rc = take_cluster_map(h, k, map);
+  OK(take_day_stats(h, k, stats));
+  OK(map_rc);
   if (!init) return fail(h, MDKM_ERR_INVALID, "init centroids required");
   OK(check_centroids(h, k, init, "init"));
   if (max_iter < 1) return fail(h, MDKM_ERR_INVALID, "max_iter must be >= 1");
@@ -1771,9 +1899,10 @@ int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol
       const int span = prof_begin(h, MDKM_PHASE_FINAL, h->n);
       // (a pause leaves the map alone: the pass after the relocation writes it)
       OK(run_final(h, kb, labels_dev, /*skip_paused=*/true, centroids_host, one_rank ? &h->h_status[0] : nullptr,
-                   &map));
+                   &map, &stats));
       prof_end(h, span);
     }
+    OK(reduce_day_stats(h, stats));
     if (!one_rank) {
       OK(ensure(h, h->dscratch, (size_t)k * 3 + 16));
       read_table_kernel<<<(k + 255) / 256, 256, 0, h->stream>>>(h->table.p, k, kb.kpad, h->fr, h->dscratch.p);
@@ -1807,6 +1936,7 @@ int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol
 #endif
   if (fin.xchg_timeout == 2) return index_fault(h);
   if (fin.xchg_timeout) return fail(h, MDKM_ERR_NCCL, "a kernel-side wait timed out (peer exchange of the partial sums: a rank is missing; or the grid barrier)");
+  deliver_day_stats(h, stats);
   if (n_iter_out) *n_iter_out = fin.iter;
   if (inertia_out) *inertia_out = fin.inertia;
   h->stat_refined = (long long)fin.n_refined;
@@ -1880,7 +2010,10 @@ int mdkm_predict(mdkm_handle* h, int k, const double* centroids, int32_t* labels
                  double* inertia_out) {
   if (!h) return MDKM_ERR_INVALID;
   MapOut map;
-  OK(take_cluster_map(h, k, map));
+  StatsOut stats;
+  const int map_rc = take_cluster_map(h, k, map);
+  OK(take_day_stats(h, k, stats));
+  OK(map_rc);
   if (!centroids) return fail(h, MDKM_ERR_INVALID, "centroids required");
   OK(check_centroids(h, k, centroids, "centroids"));
   CU(cudaSetDevice(h->device));
@@ -1900,14 +2033,16 @@ int mdkm_predict(mdkm_handle* h, int k, const double* centroids, int32_t* labels
       labels_dev = h->labels32.p;
     }
   }
-  OK(run_final(h, kb, labels_dev, false, nullptr, nullptr, &map));
+  OK(run_final(h, kb, labels_dev, false, nullptr, nullptr, &map, &stats));
   if (h->n_ranks > 1) OK(allreduce(h, &h->d_status->inertia, 1, kNcclFloat64, kNcclSum));
+  OK(reduce_day_stats(h, stats));
   OK(small_d2h(h, &h->h_status[0], h->d_status, sizeof(DevStatus), /*dst_is_pinned=*/true));
   if (labels_out && labels_mem != MDKM_MEM_DEVICE && h->n > 0)
     CU(cudaMemcpyAsync(labels_out, labels_dev, (size_t)h->n * 4, cudaMemcpyDeviceToHost, h->stream));
   OK(copy_cluster_map(h, map));
   OK(sync_small(h));
   if (h->h_status[0].xchg_timeout == 2) return index_fault(h);
+  deliver_day_stats(h, stats);
   if (inertia_out) *inertia_out = h->h_status[0].inertia;
   h->stat_refined = (long long)h->h_status[0].n_refined;
   h->stat_reloc = 0;

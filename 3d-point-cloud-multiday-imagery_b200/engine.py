@@ -371,6 +371,22 @@ class Engine:
         return mem
 
     @property
+    def n_days(self) -> int:
+        """Days of the stack of the last ``unproject`` (its ``stack_shape``), 1 after ``set_points``:
+        the rows of ``day_counts`` / ``day_means``."""
+        return self._raster[0] if self._raster is not None else 1
+
+    def _bind_day_stats(self, k):
+        """Bind fresh ``day_counts`` int64 ``[D,k]`` / ``day_means`` float64 ``[D,k,3]`` arrays to the
+        next fit / predict.  -> (counts, means)."""
+        d = self.n_days
+        counts = np.empty((d, k), dtype=np.int64)
+        means = np.empty((d, k, 3), dtype=np.float64)
+        self._check(self._lib.mdkm_bind_day_stats(self._h, c_void_p(counts.ctypes.data), c_void_p(means.ctypes.data),
+                                                  int(d), int(k)))
+        return counts, means
+
+    @property
     def segment_offsets(self) -> np.ndarray:
         """Point offsets of the cloud's segments (one per day), int64 ``[n_segments + 1]``."""
         ns = int(self._lib.mdkm_num_segments(self._h))
@@ -393,13 +409,19 @@ class Engine:
         return lo[:ns], hi[:ns], hn
 
     # -- k-means -------------------------------------------------------------------------
-    def fit(self, init, max_iter=300, tol=1e-4, want_labels=True, labels_out=None, cluster_map_out=None):
+    def fit(self, init, max_iter=300, tol=1e-4, want_labels=True, labels_out=None, cluster_map_out=None,
+            day_stats=False):
         """One Lloyd run from explicit centroids.  Returns dict(labels, centers, n_iter, inertia, ...).
 
         ``cluster_map_out``: optional uint8 (k <= 255) or uint16 array / tensor, host or CUDA, with
         one element per pixel of the last ``unproject``'s range; it receives the labels on the
         pixel grid (label + 1 where a pixel produced a point, 0 elsewhere), written by the final
-        pass.  A CUDA output is ordered against torch's current stream like ``labels_out``."""
+        pass.  A CUDA output is ordered against torch's current stream like ``labels_out``.
+
+        ``day_stats=True``: the result also has ``day_counts`` (int64 ``[D,k]``, points of day d with
+        label j) and ``day_means`` (float64 ``[D,k,3]``, their mean (x, y, z) in the clustered frame,
+        NaN where the count is 0), accumulated by the final pass; D is ``n_days`` (global days of the
+        stack), and with several ranks both are summed over all of them."""
         init = np.ascontiguousarray(init, dtype=np.float64)
         if init.ndim != 2 or init.shape[1] != 3:
             raise ValueError("init must be [K,3]")
@@ -418,6 +440,7 @@ class Engine:
         n_iter = c_int(0)
         inertia = c_double(0.0)
         map_mem = self._bind_cluster_map(cluster_map_out) if cluster_map_out is not None else None
+        stats = self._bind_day_stats(k) if day_stats else None
         self._check(self._lib.mdkm_fit(
             self._h, int(k), init.ctypes.data_as(POINTER(c_double)), int(max_iter), float(tol),
             c_void_p(lab_ptr) if lab_ptr else None, lab_mem,
@@ -428,12 +451,15 @@ class Engine:
         self._lib.mdkm_fit_stats(self._h, byref(nref), byref(nrel), byref(tols))
         work, groups = c_int64(0), c_int64(0)
         self._lib.mdkm_fit_worklist(self._h, byref(work), byref(groups))
-        return {
+        out = {
             "labels": labels, "centers": centers, "n_iter": int(n_iter.value),
             "inertia": float(inertia.value), "n_refined": int(nref.value),
             "n_relocations": int(nrel.value), "tol_scaled": float(tols.value),
             "worklist_groups": int(work.value), "groups": int(groups.value),
         }
+        if stats is not None:
+            out["day_counts"], out["day_means"] = stats
+        return out
 
     def lloyd_step(self, centroids, want_labels=True):
         """Single E-step + sums (test hook).  Returns (labels, sums[K,3], counts[K], n_refined)."""
@@ -451,20 +477,24 @@ class Engine:
         self._lib.mdkm_fit_stats(self._h, byref(nref), None, None)
         return labels, sums, counts, int(nref.value)
 
-    def predict(self, centroids, want_labels=True, cluster_map_out=None):
+    def predict(self, centroids, want_labels=True, cluster_map_out=None, day_stats=False):
         """E-step only (KMeans.predict): returns (labels int32[N] or None, inertia).
-        ``cluster_map_out``: as in ``fit``."""
+        ``cluster_map_out``: as in ``fit``.  ``day_stats=True``: returns
+        (labels, inertia, day_counts, day_means) instead, as in ``fit``."""
         c = np.ascontiguousarray(centroids, dtype=np.float64)
         if c.ndim != 2 or c.shape[1] != 3:
             raise ValueError("centroids must be [K,3]")
         labels = self._result_buffer("labels", (self.n_points,), np.int32) if want_labels else None
         inertia = c_double(0.0)
         map_mem = self._bind_cluster_map(cluster_map_out) if cluster_map_out is not None else None
+        stats = self._bind_day_stats(c.shape[0]) if day_stats else None
         self._check(self._lib.mdkm_predict(
             self._h, int(c.shape[0]), c.ctypes.data_as(POINTER(c_double)),
             c_void_p(labels.ctypes.data) if labels is not None else None, C.MEM_HOST, byref(inertia)))
         if map_mem == C.MEM_DEVICE:
             self._before_torch()
+        if stats is not None:
+            return labels, float(inertia.value), stats[0], stats[1]
         return labels, float(inertia.value)
 
     def kmeans_plusplus(self, n_clusters: int, random_state):

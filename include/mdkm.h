@@ -153,6 +153,30 @@ int mdkm_bind_cloud_output(mdkm_handle* h, float* out_host, int64_t capacity_poi
 int mdkm_bind_cluster_map(mdkm_handle* h, void* out, int elem_bytes, int64_t capacity_pixels,
                           int mem);
 
+/* Optional: have the NEXT mdkm_fit or mdkm_predict on this handle also return the composition
+ * of every day by cluster.  counts_out (int64) receives n_days * k counts, means_out (float64)
+ * n_days * k * 3 coordinates, both row-major [day][cluster] with the k of that call; both are
+ * host memory holding at least n_days * k_capacity rows.  counts_out[d*k + j] is the number of
+ * points of day d whose returned label is j; means_out[(d*k + j)*3 + c] is the mean of their
+ * coordinate c (x, y, z) in the frame that was clustered (after detrending / ground levelling,
+ * like the centroids), NaN where the count is 0.  Rows are the global days of the stack:
+ * n_days is the D of the last mdkm_unproject (1 after mdkm_set_points), and with several ranks
+ * every rank receives the sums over all ranks.
+ * Where the numbers come from: the final labelling pass adds every point's fixed-point
+ * coordinates (the integers the Lloyd sums use) into an int64 slot per (day, cluster); the
+ * ranks' slots are summed with one all-reduce, and each mean is (sum_q / scale + count *
+ * origin) / count in float64.  The integer sums do not depend on the point order, the number of
+ * ranks or the schedule, so the results are bitwise reproducible; a mean is within half a grid
+ * step of the exact mean, and is the correctly rounded exact mean when the points lie on the
+ * grid.  Asking for them changes no other result of the call.
+ * counts_out == NULL clears the binding.  The binding is consumed by that one call, and dropped
+ * by mdkm_unproject / mdkm_set_points.  Errors: MDKM_ERR_STATE when no points are resident;
+ * MDKM_ERR_INVALID when n_days is not the stack's day count, means_out is NULL or k_capacity < 1
+ * (n_days * k_capacity < 2^29), and from the mdkm_fit / mdkm_predict, before any work is
+ * enqueued, when its k exceeds k_capacity. */
+int mdkm_bind_day_stats(mdkm_handle* h, int64_t* counts_out, double* means_out, int n_days,
+                        int k_capacity);
+
 /* Load an already unprojected cloud (this rank's shard).  Replaces the `X` argument of the
  * reference's KMeans(...).fit_predict(X) call (members/jasraj/land_use_classification/
  * core.py:227-228) for d = 3. */
