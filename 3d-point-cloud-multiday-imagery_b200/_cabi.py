@@ -58,6 +58,7 @@ SIGNATURES = {
     "mdkm_bind_cloud_output": (c_int, [c_void_p, c_void_p, c_int64, c_int]),
     "mdkm_bind_cluster_map": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int]),
     "mdkm_bind_day_stats": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int]),
+    "mdkm_bind_day_transitions": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int]),
     "mdkm_set_points": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_int]),
     "mdkm_num_points": (c_int64, [c_void_p]),
     "mdkm_num_points_global": (c_int64, [c_void_p]),

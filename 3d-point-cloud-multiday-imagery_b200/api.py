@@ -54,6 +54,11 @@ class FusionResult:
     # NaN where the count is 0); summed over all ranks
     day_counts: Optional[np.ndarray] = None
     day_means: Optional[np.ndarray] = None
+    # from-to counts of day pairs (return_transitions): transitions[p, s, t] = pixels with state s on
+    # day a and t on day b of transition_pairs[p] = (a, b), state = label + 1 or 0 (no point);
+    # int64 [P,K+1,K+1] and int64 [P,2], over the whole stack on every rank
+    transitions: Optional[np.ndarray] = None
+    transition_pairs: Optional[np.ndarray] = None
 
     # scikit-learn style aliases
     @property
@@ -127,8 +132,44 @@ def cluster_map_dtype(n_clusters: int):
     return np.uint8 if int(n_clusters) <= 255 else np.uint16
 
 
+def transition_pairs(spec, n_days: int) -> np.ndarray:
+    """The day pairs ``return_transitions`` asks for, as int64 ``[P,2]``: ``True`` -> the
+    consecutive pairs ``(d, d+1)``; a sequence of ``(a, b)`` -> those pairs in that order (they
+    may skip days, run backwards, repeat, or have ``a == b``).  Raises ``ValueError`` for a day
+    outside ``[0, n_days)`` or when there is no pair."""
+    if isinstance(spec, (bool, np.bool_)):
+        if not spec:
+            raise ValueError("return_transitions=False asks for no pairs")
+        d = np.arange(max(int(n_days) - 1, 0), dtype=np.int64)
+        pairs = np.stack([d, d + 1], axis=1)
+    else:
+        pairs = np.asarray(spec)
+        if pairs.size == 0:
+            pairs = pairs.reshape(0, 2)
+        if pairs.ndim != 2 or pairs.shape[1] != 2 or not (np.issubdtype(pairs.dtype, np.integer)):
+            raise ValueError("return_transitions must be True or a sequence of (day_a, day_b) integer pairs")
+        pairs = pairs.astype(np.int64)
+    if pairs.shape[0] == 0:
+        raise ValueError(f"no day pair to count transitions of (the stack has {n_days} day(s))")
+    bad = (pairs < 0) | (pairs >= n_days)
+    if bad.any():
+        p = int(np.argmax(bad.any(axis=1)))
+        raise ValueError(f"transition pair {p} = {tuple(int(v) for v in pairs[p])}: days must be in [0, {n_days})")
+    return pairs
+
+
+def _stack_days(height_maps, stack_shape, raster_layout) -> int:
+    """D of the stack ``fuse_multiday_kmeans`` is given (before anything reaches the GPU)."""
+    if stack_shape is not None:
+        return int(stack_shape[0])
+    shp = tuple(height_maps.shape)
+    if raster_layout == "gtiff3":
+        shp = shp[:-1]
+    return 1 if len(shp) == 2 else int(shp[0])
+
+
 def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_state, want_labels=True,
-                labels_out=None, gather_mappings=None, cluster_map_out=None, day_stats=False):
+                labels_out=None, gather_mappings=None, cluster_map_out=None, day_stats=False, transitions=None):
     """KMeans.fit driver (sklearn/_kmeans.py:1436-1563): init, n_init restarts, best inertia.
 
     ``labels_out``: optional int32 array that receives this rank's labels of the best run.
@@ -137,6 +178,8 @@ def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_
     best one is kept by swapping and copied out once at the end.
     ``day_stats``: the result also has ``day_counts`` / ``day_means`` (``Engine.fit``) -- every run
     returns fresh arrays, so the best run's stay with it.
+    ``transitions``: day pairs ``[P,2]``; the result also has ``transitions`` (``Engine.fit``), the
+    best run's, as with ``day_stats``.
     ``gather_mappings``: with a multi-rank engine, the collective that lets the ranks agree on
     sklearn's "same clustering up to a permutation" test (see ``_is_same_clustering``); when it is
     missing the test is skipped on multi-rank engines (the inertia comparison alone decides)."""
@@ -180,7 +223,8 @@ def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_
             centers0, _ = eng.kmeans_plusplus(k, rs)
         r = eng.fit(centers0, max_iter=max_iter, tol=tol, want_labels=want_labels,
                     labels_out=labels_out if (single and want_labels) else None,
-                    cluster_map_out=cluster_map_out if single else run_map, day_stats=day_stats)
+                    cluster_map_out=cluster_map_out if single else run_map, day_stats=day_stats,
+                    transitions=transitions)
         # sklearn/_kmeans.py:1534-1541: a run replaces the best one when its inertia is lower AND it
         # is not the same clustering up to a permutation.  The inertia is global, so every rank
         # takes the same branch and the (collective) permutation test pairs up.
@@ -222,7 +266,7 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
                          detrend=False, disparity_scale=None, ground_level=False, return_cloud=True,
                          device=0, devices=None, engine=None, stack_shape=None,
                          pix_begin=0, raster_layout=None, return_cluster_map=False,
-                         return_day_stats=False) -> FusionResult:
+                         return_day_stats=False, return_transitions=False) -> FusionResult:
     """Unproject a multi-day height-map stack into one XYZ cloud and cluster it (Lloyd).
 
     height_maps : float32 ``[D,H,W]`` (NaN = nodata), numpy or torch (CPU or CUDA); or int16
@@ -256,10 +300,22 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
         pre-sharded call, and the numbers are summed over all ranks.  They come from integer sums on
         the fixed-point frame accumulated by the final labelling pass, so they are bitwise the same
         for any number of GPUs.
+    return_transitions : ``True`` (the consecutive pairs ``(d, d+1)``) or a sequence of day pairs
+        ``(a, b)``: also return ``transitions``, int64 ``[P,K+1,K+1]``, the from-to matrix of every
+        pair -- ``transitions[p, s, t]`` is the number of pixels with state s on day a and t on day
+        b, where a pixel's state is ``label + 1`` when it produced a point that day and 0 when it
+        did not (row 0 / column 0: pixels that gained / lost their point) -- and
+        ``transition_pairs`` (int64 ``[P,2]``).  Binned on the GPU from the cluster map the final
+        labelling pass writes (the map itself need not be returned).  A pre-sharded call needs
+        ranks that together hold the whole stack; every rank receives the global counts.
+        Out-of-range days raise ``ValueError`` before any GPU work.
     Returns a FusionResult; ``fused_cloud`` is float32 ``[N,3]`` in napari (z,y,x) order.
     """
     from .group import DeviceGroup
 
+    pairs = None
+    if return_transitions is not None and not (isinstance(return_transitions, (bool, np.bool_)) and not return_transitions):
+        pairs = transition_pairs(return_transitions, _stack_days(height_maps, stack_shape, raster_layout))
     if devices is not None or isinstance(engine, DeviceGroup):
         if stack_shape is not None or pix_begin:
             raise ValueError("stack_shape / pix_begin describe a pre-sharded stack; a device group shards by itself")
@@ -268,7 +324,7 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
                               tol=tol, random_state=random_state, max_abs_height=max_abs_height, detrend=detrend,
                               disparity_scale=disparity_scale, ground_level=ground_level, return_cloud=return_cloud,
                               raster_layout=raster_layout, return_cluster_map=return_cluster_map,
-                              return_day_stats=return_day_stats)
+                              return_day_stats=return_day_stats, transitions=pairs)
     own = engine is None
     eng = engine or Engine(device)
     try:
@@ -294,20 +350,23 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
             D, H, W, _, count = eng.raster_range
             cmap = np.empty((D, H, W) if stack_shape is None else (count,), dtype=cluster_map_dtype(n_clusters))
         r = _run_kmeans(eng, n_clusters=n_clusters, init=init, n_init=n_init, max_iter=max_iter,
-                        tol=tol, random_state=random_state, cluster_map_out=cmap, day_stats=return_day_stats)
+                        tol=tol, random_state=random_state, cluster_map_out=cmap, day_stats=return_day_stats,
+                        transitions=pairs)
         eng.wait()
         return FusionResult(labels=r["labels"], centroids=r["centers"], fused_cloud=cloud,
                             n_iter=r["n_iter"], inertia=r["inertia"], n_points=n,
                             n_refined=r["n_refined"], n_relocations=r["n_relocations"],
                             height_norm=hn, extra=extra, cluster_map=cmap,
-                            day_counts=r.get("day_counts"), day_means=r.get("day_means"))
+                            day_counts=r.get("day_counts"), day_means=r.get("day_means"),
+                            transitions=r.get("transitions"), transition_pairs=pairs)
     finally:
         if own:
             eng.close()
 
 
 def _fuse_on_group(height_maps, valid_masks, *, group, devices, n_clusters, init, n_init, max_iter, tol,
-                   random_state, return_cluster_map=False, return_day_stats=False, **unproject_kw) -> FusionResult:
+                   random_state, return_cluster_map=False, return_day_stats=False, transitions=None,
+                   **unproject_kw) -> FusionResult:
     """``fuse_multiday_kmeans`` on several devices of this process (``group.DeviceGroup``)."""
     import threading
 
@@ -337,7 +396,7 @@ def _fuse_on_group(height_maps, valid_masks, *, group, devices, n_clusters, init
             return _run_kmeans(eng, n_clusters=n_clusters, init=init, n_init=n_init, max_iter=max_iter, tol=tol,
                                random_state=states[r], labels_out=labels_out,
                                gather_mappings=gather_for(r) if grp.world > 1 else None,
-                               cluster_map_out=cluster_map_out, day_stats=return_day_stats)
+                               cluster_map_out=cluster_map_out, day_stats=return_day_stats, transitions=transitions)
 
         res, labels, cloud, hn, extra = grp.fuse(
             height_maps, valid_masks, run_kmeans=run,
@@ -346,7 +405,8 @@ def _fuse_on_group(height_maps, valid_masks, *, group, devices, n_clusters, init
                             inertia=res["inertia"], n_points=int(labels.shape[0]), n_refined=res["n_refined"],
                             n_relocations=res["n_relocations"], height_norm=hn, extra=extra,
                             cluster_map=extra.pop("cluster_map", None),
-                            day_counts=res.get("day_counts"), day_means=res.get("day_means"))
+                            day_counts=res.get("day_counts"), day_means=res.get("day_means"),
+                            transitions=res.get("transitions"), transition_pairs=transitions)
     finally:
         if own:
             grp.close()

@@ -23,6 +23,7 @@
 #include "mirror.cuh"
 #include "nccl_shim.h"
 #include "seeding.cuh"
+#include "transitions.cuh"
 #include "unproject.cuh"
 
 using namespace mdkm;
@@ -168,6 +169,17 @@ struct mdkm_handle {
   DevBuf<unsigned char> stats_dev;       // counts, then means, converted on the device
   unsigned char* stats_host = nullptr;   // pinned: their copy, handed to the caller after the sync
   size_t stats_host_cap = 0;
+  // day-pair transition counts (mdkm_bind_day_transitions) of the next fit / predict
+  std::vector<int> bound_pairs;          // [n_pairs][2] days, copied when bound
+  int64_t* bound_trans = nullptr;
+  int bound_trans_kcap = 0;
+  int trans_cover = -1;                  // the ranks' pixel ranges cover the stack (1) or not (0); -1: not checked
+  DevBuf<unsigned char> trans_map;       // the map the final pass writes when none is bound; the whole stack with
+                                         // several ranks
+  DevBuf<int> trans_pairs;
+  DevBuf<unsigned long long> trans_bins;  // [n_pairs][(k+1)^2]
+  unsigned char* trans_host = nullptr;    // pinned: their copy, handed to the caller after the sync
+  size_t trans_host_cap = 0;
 
   // communicator
   ncclComm_t comm = nullptr;
@@ -915,6 +927,11 @@ struct MapOut {
   void* host = nullptr;
   int elem = 0;
   size_t bytes = 0;
+  // several ranks with day transitions: `dev` is this rank's band of the whole-stack map `stack`,
+  // which the final pass clears; a device output receives the band afterwards at `dev_out`
+  unsigned char* stack = nullptr;
+  size_t stack_bytes = 0;
+  void* dev_out = nullptr;
 };
 
 // Per-(day, cluster) statistics taken by one fit / predict (mdkm_bind_day_stats): accumulated by
@@ -925,6 +942,32 @@ struct StatsOut {
   int64_t* counts = nullptr;
   double* means = nullptr;
 };
+
+// Day-pair transition counts taken by one fit / predict (mdkm_bind_day_transitions): binned from
+// the cluster map behind the final pass, summed over the ranks and copied to the pinned stage;
+// `out` receives them after the call's synchronisation.
+struct TransOut {
+  int64_t* out = nullptr;
+  int n_pairs = 0;
+  int k1 = 0;                          // states: k + 1
+  const unsigned char* map = nullptr;  // the whole stack's map (device)
+  int elem = 1;
+  bool reduce_map = false;             // several ranks: the bands of `map` are summed over the ranks first
+};
+
+// page-locked host buffer of at least `bytes` (the stages of results handed over after a sync)
+int ensure_pinned(mdkm_handle* h, unsigned char*& p, size_t& cap, size_t bytes) {
+  if (cap >= bytes && p) return MDKM_OK;
+  if (p) {
+    CU(cudaStreamSynchronize(h->stream));
+    CU(cudaFreeHost(p));
+    p = nullptr;
+    cap = 0;
+  }
+  CU(cudaMallocHost(&p, std::max<size_t>(bytes, 1)));
+  cap = std::max<size_t>(bytes, 1);
+  return MDKM_OK;
+}
 
 int run_final(mdkm_handle* h, const KmBuffers& kb, int* labels_dev, bool skip_paused = false,
               double* centroids_host = nullptr, DevStatus* status_host = nullptr, const MapOut* map = nullptr,
@@ -977,17 +1020,143 @@ int take_day_stats(mdkm_handle* h, int k, StatsOut& s) {
   s.means = means;
   OK(ensure(h, h->stats_acc, (size_t)s.slots * 4));
   OK(ensure(h, h->stats_dev, (size_t)s.slots * 32));
-  if (h->stats_host_cap < (size_t)s.slots * 32) {
-    if (h->stats_host) {
-      CU(cudaStreamSynchronize(h->stream));
-      CU(cudaFreeHost(h->stats_host));
-      h->stats_host = nullptr;
-      h->stats_host_cap = 0;
-    }
-    CU(cudaMallocHost(&h->stats_host, (size_t)s.slots * 32));
-    h->stats_host_cap = (size_t)s.slots * 32;
-  }
+  OK(ensure_pinned(h, h->stats_host, h->stats_host_cap, (size_t)s.slots * 32));
   return upload_day_offsets(h);
+}
+
+// Takes the binding of mdkm_bind_day_transitions (`out`, already consumed) for a call with k
+// clusters and its cluster map `m`: checks k against the bound capacity and, once per cloud, that
+// the ranks' pixel ranges cover the stack (one all-reduce); sizes the bins, uploads the pairs.
+// The map the pairs are binned from is the bound one (one rank) or one the final pass writes for
+// them: an internal map of the range when none is bound, and with several ranks a whole-stack
+// map of which every rank writes its band (a bound output then receives that band).
+int take_transitions(mdkm_handle* h, int k, int64_t* out, MapOut& m, TransOut& t) {
+  if (!out) return MDKM_OK;
+  const int kcap = h->bound_trans_kcap;
+  if (k > kcap) return fail(h, MDKM_ERR_INVALID, "k=%d exceeds the k_capacity %d of the bound day transitions", k, kcap);
+  if (k < 1 || k > kMaxK) return MDKM_OK;  // (rejected with the call's own message)
+  CU(cudaSetDevice(h->device));
+  const long long HW = (long long)h->raster_H * h->raster_w, stack_px = (long long)h->stack_days * HW;
+  if (h->trans_cover < 0) {
+    long long px = h->raster_pix_count;
+    if (h->n_ranks > 1) {
+      OK(ensure(h, h->dscratch, 64));
+      long long* d = reinterpret_cast<long long*>(h->dscratch.p);
+      CU(cudaMemcpyAsync(d, &px, 8, cudaMemcpyHostToDevice, h->stream));
+      OK(allreduce(h, d, 1, kNcclInt64, kNcclSum));
+      OK(small_d2h(h, &px, d, 8));
+      OK(sync_small(h));
+    }
+    h->trans_cover = px == stack_px ? 1 : 0;
+  }
+  if (!h->trans_cover)
+    return fail(h, MDKM_ERR_STATE, "day transitions need the pixel ranges of the ranks to cover the whole stack");
+  t.out = out;
+  t.n_pairs = (int)(h->bound_pairs.size() / 2);
+  t.k1 = k + 1;
+  const size_t words = (size_t)t.n_pairs * t.k1 * t.k1;
+  OK(ensure(h, h->trans_bins, words));
+  OK(ensure(h, h->trans_pairs, h->bound_pairs.size()));
+  CU(cudaMemcpyAsync(h->trans_pairs.p, h->bound_pairs.data(), h->bound_pairs.size() * 4, cudaMemcpyHostToDevice,
+                     h->stream));
+  OK(ensure_pinned(h, h->trans_host, h->trans_host_cap, words * 8));
+  if (h->n_ranks == 1) {
+    if (!m.dev) {
+      m.elem = k <= 255 ? 1 : 2;
+      m.bytes = (size_t)h->raster_pix_count * m.elem;
+      OK(ensure(h, h->trans_map, std::max<size_t>(m.bytes, 1)));
+      m.dev = h->trans_map.p;
+      OK(upload_day_offsets(h));
+    }
+    t.map = static_cast<const unsigned char*>(m.dev);
+    t.elem = m.elem;
+    return MDKM_OK;
+  }
+  const int elem = m.dev ? m.elem : (k <= 255 ? 1 : 2);
+  const size_t stack_bytes = (size_t)stack_px * elem;
+  OK(ensure(h, h->trans_map, std::max<size_t>(stack_bytes, 1)));
+  if (m.dev && !m.host) m.dev_out = m.dev;
+  if (!m.dev) OK(upload_day_offsets(h));
+  m.dev = h->trans_map.p + (size_t)h->raster_pix_begin * elem;
+  m.elem = elem;
+  m.bytes = (size_t)h->raster_pix_count * elem;
+  m.stack = h->trans_map.p;
+  m.stack_bytes = stack_bytes;
+  t.map = h->trans_map.p;
+  t.elem = elem;
+  t.reduce_map = true;
+  return MDKM_OK;
+}
+
+typedef void (*TransKernel)(const TransParams);
+template <typename T>
+TransKernel pick_trans_kernel(int mode) {
+  if (mode == kTransWarpBins) return day_transitions_kernel<T, kTransWarpBins>;
+  if (mode == kTransCtaBins) return day_transitions_kernel<T, kTransCtaBins>;
+  return day_transitions_kernel<T, kTransGlobalBins>;
+}
+
+// Behind the final pass, on the stream: with several ranks the map's bands summed over the ranks,
+// then the bins of this rank's share of the pixels of every day, their sum over the ranks, the
+// copy to the pinned stage.  (Behind a final pass that returned early for a relocation this bins
+// a map of zeros; the pass after the relocation runs it again.)
+int run_transitions(mdkm_handle* h, const TransOut& t) {
+  if (!t.out) return MDKM_OK;
+  const long long HW = (long long)h->raster_H * h->raster_w;
+  // the bands are disjoint: their byte-wise sum is their union, for 16-bit maps too
+  if (t.reduce_map)
+    OK(allreduce(h, const_cast<unsigned char*>(t.map), (size_t)h->stack_days * HW * t.elem, kNcclUint8, kNcclSum));
+  const size_t nb = (size_t)t.k1 * t.k1, words = nb * t.n_pairs;
+  CU(cudaMemsetAsync(h->trans_bins.p, 0, words * 8, h->stream));
+  TransParams tp{};
+  tp.map = t.map;
+  tp.HW = HW;
+  tp.q_begin = HW * h->rank / h->n_ranks;
+  tp.q_end = HW * (h->rank + 1) / h->n_ranks;
+  tp.pairs = h->trans_pairs.p;
+  tp.n_pairs = t.n_pairs;
+  tp.k1 = t.k1;
+  tp.bins = h->trans_bins.p;
+  // bins in shared memory when they do not cost a resident CTA (run-time occupancy query): a copy
+  // per warp, else one per CTA; otherwise straight to the global bins
+  auto pick = [&](int mode) { return t.elem == 2 ? pick_trans_kernel<unsigned short>(mode) : pick_trans_kernel<unsigned char>(mode); };
+  int base = 0, optin = 0;
+  CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&base, pick(kTransGlobalBins), kThreads, 0));
+  CU(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
+  int mode = kTransGlobalBins, occ = base;
+  size_t smem = 0;
+  for (int md = kTransWarpBins; md < kTransGlobalBins; ++md) {
+    const size_t bytes = nb * 4 * (md == kTransWarpBins ? kThreads / 32 : 1);
+    int o = 0;
+    if (bytes <= (size_t)optin) {
+      CU(cudaFuncSetAttribute(pick(md), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+      CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, pick(md), kThreads, bytes));
+    }
+    if (o >= base) {
+      mode = md;
+      occ = o;
+      smem = bytes;
+      break;
+    }
+  }
+  // one wave of resident CTAs over (pairs, chunks); shared bins count in 32 bits, so no CTA
+  // bins more than 2^30 + 30 pixels of a pair
+  const long long chunks = (tp.q_end - tp.q_begin) / kTransPx + 1;
+  const int gy = (int)std::min<long long>(t.n_pairs, 65535);
+  long long gx = std::max<long long>(1, (long long)h->sm_count * std::max(occ, 1) / gy);
+  gx = std::min(gx, (chunks + kThreads - 1) / kThreads);
+  gx = std::max(gx, chunks * kTransPx / (1ll << 30) + 1);
+  pick(mode)<<<dim3((unsigned int)gx, (unsigned int)gy), kThreads, smem, h->stream>>>(tp);
+  ++h->launches;
+  CU(cudaGetLastError());
+  OK(allreduce(h, h->trans_bins.p, words, kNcclInt64, kNcclSum));
+  CU(cudaMemcpyAsync(h->trans_host, h->trans_bins.p, words * 8, cudaMemcpyDeviceToHost, h->stream));
+  return MDKM_OK;
+}
+
+// After the call's synchronisation: the pinned stage -> the caller's counts.
+void deliver_transitions(mdkm_handle* h, const TransOut& t) {
+  if (t.out) memcpy(t.out, h->trans_host, (size_t)t.n_pairs * t.k1 * t.k1 * 8);
 }
 
 // Behind the final pass, on the stream: the sums over the ranks, counts and means, their copy
@@ -1016,6 +1185,7 @@ void deliver_day_stats(mdkm_handle* h, const StatsOut& s) {
 // The map's device->host copy (host outputs), on the compute stream behind the final pass.
 int copy_cluster_map(mdkm_handle* h, const MapOut& m) {
   if (m.host && m.bytes) CU(cudaMemcpyAsync(m.host, m.dev, m.bytes, cudaMemcpyDeviceToHost, h->stream));
+  if (m.dev_out && m.bytes) CU(cudaMemcpyAsync(m.dev_out, m.dev, m.bytes, cudaMemcpyDeviceToDevice, h->stream));
   return MDKM_OK;
 }
 
@@ -1069,7 +1239,8 @@ int run_final(mdkm_handle* h, const KmBuffers& kb, int* labels_dev, bool skip_pa
   const bool want_map = map && map->dev, want_stats = stats && stats->counts;
   if (want_map) {
     // pixels without a point stay 0 (napari's background label)
-    if (map->bytes) CU(cudaMemsetAsync(map->dev, 0, map->bytes, h->stream));
+    if (map->stack) CU(cudaMemsetAsync(map->stack, 0, map->stack_bytes, h->stream));
+    else if (map->bytes) CU(cudaMemsetAsync(map->dev, 0, map->bytes, h->stream));
     fp.map_out = map->dev;
     fp.map_elem = map->elem;
     fp.map_W = h->raster_w;
@@ -1191,6 +1362,8 @@ void mdkm_destroy(mdkm_handle* h) {
   release(h->d_seg_off); release(h->sel_hist); release(h->sel_targets);
   release(h->map_stage); release(h->map_seg); release(h->stats_acc); release(h->stats_dev);
   if (h->stats_host) cudaFreeHost(h->stats_host);
+  release(h->trans_map); release(h->trans_pairs); release(h->trans_bins);
+  if (h->trans_host) cudaFreeHost(h->trans_host);
   release(h->kpp_closest); release(h->kpp_cell); release(h->kpp_blk); release(h->kpp_prefix);
   release(h->kpp_partials); release(h->kpp_rand); release(h->kpp_state);
   if (h->d_status) cudaFree(h->d_status);
@@ -1226,6 +1399,7 @@ int mdkm_comm_init(mdkm_handle* h, int n_ranks, int rank, const unsigned char id
   h->n_ranks = n_ranks;
   h->rank = rank;
   h->frame_ok = false;
+  h->trans_cover = -1;
   close_p2p(h);
   if (n_ranks == 1) return MDKM_OK;
   if (!id) return fail(h, MDKM_ERR_INVALID, "unique id required");
@@ -1393,6 +1567,8 @@ int mdkm_set_points(mdkm_handle* h, const float* xyz, int64_t n, int layout, int
   h->raster_w = 0;
   h->bound_map = nullptr;
   h->bound_counts = nullptr;
+  h->bound_trans = nullptr;
+  h->trans_cover = -1;
   h->stack_days = 1;
   h->day0 = 0;
   h->runs_ok = false;
@@ -1461,6 +1637,26 @@ int mdkm_bind_cluster_map(mdkm_handle* h, void* out, int elem_bytes, int64_t cap
   return MDKM_OK;
 }
 
+int mdkm_bind_day_transitions(mdkm_handle* h, const int32_t* pairs, int n_pairs, int64_t* counts_out, int k_capacity) {
+  if (!h) return MDKM_ERR_INVALID;
+  h->bound_trans = nullptr;
+  if (!counts_out) return MDKM_OK;
+  if (!h->have_points || h->raster_w <= 0)
+    return fail(h, MDKM_ERR_STATE, "day transitions need a resident cloud from mdkm_unproject");
+  if (!pairs || n_pairs < 1 || k_capacity < 1 ||
+      (double)n_pairs * ((double)k_capacity + 1.0) * ((double)k_capacity + 1.0) >= 2147483648.0)
+    return fail(h, MDKM_ERR_INVALID, "day transitions need n_pairs >= 1, k_capacity >= 1 and n_pairs * (k_capacity + 1)^2 < 2^31");
+  if (h->raster_w >= (1 << 23) || h->raster_H >= (1 << 23))  // (the final pass writes the map they are binned from)
+    return fail(h, MDKM_ERR_INVALID, "day transitions need rasters narrower and shorter than 2^23 pixels");
+  for (int i = 0; i < 2 * n_pairs; ++i)
+    if (pairs[i] < 0 || pairs[i] >= h->stack_days)
+      return fail(h, MDKM_ERR_INVALID, "pair %d: day %d is not in [0, %d)", i / 2, (int)pairs[i], h->stack_days);
+  h->bound_pairs.assign(pairs, pairs + 2 * (size_t)n_pairs);
+  h->bound_trans = counts_out;
+  h->bound_trans_kcap = k_capacity;
+  return MDKM_OK;
+}
+
 int mdkm_bind_day_stats(mdkm_handle* h, int64_t* counts_out, double* means_out, int n_days, int k_capacity) {
   if (!h) return MDKM_ERR_INVALID;
   h->bound_counts = nullptr;
@@ -1493,6 +1689,8 @@ int mdkm_unproject(mdkm_handle* h, const void* hm, int hm_dtype, float hm_scale,
   h->bound_cloud_cap = 0;
   h->bound_map = nullptr;  // (a cluster map describes the range it was bound for)
   h->bound_counts = nullptr;  // (and day statistics the stack)
+  h->bound_trans = nullptr;
+  h->trans_cover = -1;
   if (D < 0 || H <= 0 || W <= 0 || pix_begin < 0 || pix_count < 0 ||
       pix_begin + pix_count > (int64_t)D * H * W || (pix_count > 0 && !hm))
     return fail(h, MDKM_ERR_INVALID, "bad stack geometry");
@@ -1775,9 +1973,13 @@ int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol
   if (!h) return MDKM_ERR_INVALID;
   MapOut map;
   StatsOut stats;
+  TransOut trans;
+  int64_t* trans_out = h->bound_trans;
+  h->bound_trans = nullptr;
   const int map_rc = take_cluster_map(h, k, map);
   OK(take_day_stats(h, k, stats));
   OK(map_rc);
+  OK(take_transitions(h, k, trans_out, map, trans));
   if (!init) return fail(h, MDKM_ERR_INVALID, "init centroids required");
   OK(check_centroids(h, k, init, "init"));
   if (max_iter < 1) return fail(h, MDKM_ERR_INVALID, "max_iter must be >= 1");
@@ -1903,6 +2105,7 @@ int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol
       prof_end(h, span);
     }
     OK(reduce_day_stats(h, stats));
+    OK(run_transitions(h, trans));
     if (!one_rank) {
       OK(ensure(h, h->dscratch, (size_t)k * 3 + 16));
       read_table_kernel<<<(k + 255) / 256, 256, 0, h->stream>>>(h->table.p, k, kb.kpad, h->fr, h->dscratch.p);
@@ -1937,6 +2140,7 @@ int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol
   if (fin.xchg_timeout == 2) return index_fault(h);
   if (fin.xchg_timeout) return fail(h, MDKM_ERR_NCCL, "a kernel-side wait timed out (peer exchange of the partial sums: a rank is missing; or the grid barrier)");
   deliver_day_stats(h, stats);
+  deliver_transitions(h, trans);
   if (n_iter_out) *n_iter_out = fin.iter;
   if (inertia_out) *inertia_out = fin.inertia;
   h->stat_refined = (long long)fin.n_refined;
@@ -2011,9 +2215,13 @@ int mdkm_predict(mdkm_handle* h, int k, const double* centroids, int32_t* labels
   if (!h) return MDKM_ERR_INVALID;
   MapOut map;
   StatsOut stats;
+  TransOut trans;
+  int64_t* trans_out = h->bound_trans;
+  h->bound_trans = nullptr;
   const int map_rc = take_cluster_map(h, k, map);
   OK(take_day_stats(h, k, stats));
   OK(map_rc);
+  OK(take_transitions(h, k, trans_out, map, trans));
   if (!centroids) return fail(h, MDKM_ERR_INVALID, "centroids required");
   OK(check_centroids(h, k, centroids, "centroids"));
   CU(cudaSetDevice(h->device));
@@ -2036,6 +2244,7 @@ int mdkm_predict(mdkm_handle* h, int k, const double* centroids, int32_t* labels
   OK(run_final(h, kb, labels_dev, false, nullptr, nullptr, &map, &stats));
   if (h->n_ranks > 1) OK(allreduce(h, &h->d_status->inertia, 1, kNcclFloat64, kNcclSum));
   OK(reduce_day_stats(h, stats));
+  OK(run_transitions(h, trans));
   OK(small_d2h(h, &h->h_status[0], h->d_status, sizeof(DevStatus), /*dst_is_pinned=*/true));
   if (labels_out && labels_mem != MDKM_MEM_DEVICE && h->n > 0)
     CU(cudaMemcpyAsync(labels_out, labels_dev, (size_t)h->n * 4, cudaMemcpyDeviceToHost, h->stream));
@@ -2043,6 +2252,7 @@ int mdkm_predict(mdkm_handle* h, int k, const double* centroids, int32_t* labels
   OK(sync_small(h));
   if (h->h_status[0].xchg_timeout == 2) return index_fault(h);
   deliver_day_stats(h, stats);
+  deliver_transitions(h, trans);
   if (inertia_out) *inertia_out = h->h_status[0].inertia;
   h->stat_refined = (long long)h->h_status[0].n_refined;
   h->stat_reloc = 0;

@@ -386,6 +386,31 @@ class Engine:
                                                   int(d), int(k)))
         return counts, means
 
+    def _bind_day_transitions(self, pairs, k):
+        """Bind the day pairs ``pairs`` (``[P,2]`` global days) and a fresh int64 ``[P,k+1,k+1]``
+        array to the next fit / predict.  -> the array."""
+        pr = np.clip(np.asarray(pairs, dtype=np.int64).reshape(-1, 2), -1, 2**31 - 1).astype(np.int32)
+        counts = np.empty((pr.shape[0], k + 1, k + 1), dtype=np.int64)
+        self._check(self._lib.mdkm_bind_day_transitions(self._h, c_void_p(pr.ctypes.data), int(pr.shape[0]),
+                                                        c_void_p(counts.ctypes.data), int(k)))
+        return counts
+
+    def _bind_outputs(self, k, cluster_map_out, day_stats, transitions):
+        """Bind the optional outputs of the next fit / predict -> (map memory kind, (counts, means),
+        transitions), each None when not asked for.  When one binding is refused none is left
+        behind: the statistics and transition arrays live only in this call, and a binding that
+        outlived them would have the next fit / predict write into freed memory."""
+        try:
+            map_mem = self._bind_cluster_map(cluster_map_out) if cluster_map_out is not None else None
+            stats = self._bind_day_stats(k) if day_stats else None
+            trans = self._bind_day_transitions(transitions, k) if transitions is not None else None
+        except BaseException:
+            self._lib.mdkm_bind_cluster_map(self._h, None, 1, 0, C.MEM_HOST)
+            self._lib.mdkm_bind_day_stats(self._h, None, None, 0, 0)
+            self._lib.mdkm_bind_day_transitions(self._h, None, 0, None, 0)
+            raise
+        return map_mem, stats, trans
+
     @property
     def segment_offsets(self) -> np.ndarray:
         """Point offsets of the cloud's segments (one per day), int64 ``[n_segments + 1]``."""
@@ -410,7 +435,7 @@ class Engine:
 
     # -- k-means -------------------------------------------------------------------------
     def fit(self, init, max_iter=300, tol=1e-4, want_labels=True, labels_out=None, cluster_map_out=None,
-            day_stats=False):
+            day_stats=False, transitions=None):
         """One Lloyd run from explicit centroids.  Returns dict(labels, centers, n_iter, inertia, ...).
 
         ``cluster_map_out``: optional uint8 (k <= 255) or uint16 array / tensor, host or CUDA, with
@@ -421,7 +446,14 @@ class Engine:
         ``day_stats=True``: the result also has ``day_counts`` (int64 ``[D,k]``, points of day d with
         label j) and ``day_means`` (float64 ``[D,k,3]``, their mean (x, y, z) in the clustered frame,
         NaN where the count is 0), accumulated by the final pass; D is ``n_days`` (global days of the
-        stack), and with several ranks both are summed over all of them."""
+        stack), and with several ranks both are summed over all of them.
+
+        ``transitions``: day pairs ``[P,2]`` (global days of the stack); the result also has
+        ``transitions``, int64 ``[P,k+1,k+1]``: ``[p,s,t]`` pixels with state s on day a and t on
+        day b of pair p, state = label + 1 where the pixel produced a point, 0 where it did not
+        (the cluster map's value).  Binned on the GPU from the map the final pass writes; needs a
+        cloud from ``unproject`` whose ranks together hold the whole stack, and with several ranks
+        every rank receives the counts of the whole stack."""
         init = np.ascontiguousarray(init, dtype=np.float64)
         if init.ndim != 2 or init.shape[1] != 3:
             raise ValueError("init must be [K,3]")
@@ -439,8 +471,7 @@ class Engine:
         centers = np.empty((k, 3), dtype=np.float64)
         n_iter = c_int(0)
         inertia = c_double(0.0)
-        map_mem = self._bind_cluster_map(cluster_map_out) if cluster_map_out is not None else None
-        stats = self._bind_day_stats(k) if day_stats else None
+        map_mem, stats, trans = self._bind_outputs(k, cluster_map_out, day_stats, transitions)
         self._check(self._lib.mdkm_fit(
             self._h, int(k), init.ctypes.data_as(POINTER(c_double)), int(max_iter), float(tol),
             c_void_p(lab_ptr) if lab_ptr else None, lab_mem,
@@ -459,6 +490,8 @@ class Engine:
         }
         if stats is not None:
             out["day_counts"], out["day_means"] = stats
+        if trans is not None:
+            out["transitions"] = trans
         return out
 
     def lloyd_step(self, centroids, want_labels=True):
@@ -477,25 +510,28 @@ class Engine:
         self._lib.mdkm_fit_stats(self._h, byref(nref), None, None)
         return labels, sums, counts, int(nref.value)
 
-    def predict(self, centroids, want_labels=True, cluster_map_out=None, day_stats=False):
+    def predict(self, centroids, want_labels=True, cluster_map_out=None, day_stats=False, transitions=None):
         """E-step only (KMeans.predict): returns (labels int32[N] or None, inertia).
         ``cluster_map_out``: as in ``fit``.  ``day_stats=True``: returns
-        (labels, inertia, day_counts, day_means) instead, as in ``fit``."""
+        (labels, inertia, day_counts, day_means) instead, as in ``fit``.  ``transitions``: day
+        pairs as in ``fit``; their counts are appended to the returned tuple."""
         c = np.ascontiguousarray(centroids, dtype=np.float64)
         if c.ndim != 2 or c.shape[1] != 3:
             raise ValueError("centroids must be [K,3]")
         labels = self._result_buffer("labels", (self.n_points,), np.int32) if want_labels else None
         inertia = c_double(0.0)
-        map_mem = self._bind_cluster_map(cluster_map_out) if cluster_map_out is not None else None
-        stats = self._bind_day_stats(c.shape[0]) if day_stats else None
+        map_mem, stats, trans = self._bind_outputs(c.shape[0], cluster_map_out, day_stats, transitions)
         self._check(self._lib.mdkm_predict(
             self._h, int(c.shape[0]), c.ctypes.data_as(POINTER(c_double)),
             c_void_p(labels.ctypes.data) if labels is not None else None, C.MEM_HOST, byref(inertia)))
         if map_mem == C.MEM_DEVICE:
             self._before_torch()
+        out = (labels, float(inertia.value))
         if stats is not None:
-            return labels, float(inertia.value), stats[0], stats[1]
-        return labels, float(inertia.value)
+            out += stats
+        if trans is not None:
+            out += (trans,)
+        return out
 
     def kmeans_plusplus(self, n_clusters: int, random_state):
         """k-means++ seeding (sklearn/_kmeans.py:180-278); RNG draws come from ``random_state``

@@ -177,6 +177,32 @@ int mdkm_bind_cluster_map(mdkm_handle* h, void* out, int elem_bytes, int64_t cap
 int mdkm_bind_day_stats(mdkm_handle* h, int64_t* counts_out, double* means_out, int n_days,
                         int k_capacity);
 
+/* Optional: have the NEXT mdkm_fit or mdkm_predict on this handle also return the from-to
+ * (transition) counts of pairs of days.  A pixel's state on a day is label + 1 when the pixel
+ * produced a point that day and 0 when it did not -- the value of the cluster map.  For pair p =
+ * (a, b), pairs[2p] = a and pairs[2p+1] = b (global days of the stack; any order, repeats and
+ * a == b allowed; copied by this call), counts_out[(p*(k+1) + s)*(k+1) + t] is the number of
+ * pixels of the H x W grid with state s on day a and t on day b, with the k of that call: row 0
+ * counts the pixels that gain their point, column 0 those that lose it.  counts_out is host
+ * memory with room for n_pairs * (k_capacity + 1)^2 counts.  With several ranks every rank
+ * receives the counts of the whole stack.
+ * Where the numbers come from: the final labelling pass writes the cluster map (the bound one,
+ * or an internal one when none is bound); a kernel bins it behind that pass.  With several ranks
+ * each rank writes its band of a zeroed whole-stack map, the bands are merged with one byte-wise
+ * all-reduce (a full-stack map on every rank), each rank bins 1/n_ranks of the pixels, and one
+ * all-reduce of the int64 counts sums them: the same bits on any number of ranks.  Asking for
+ * them changes no other result of the call.
+ * counts_out == NULL clears the binding.  The binding is consumed by that one call, and dropped
+ * by mdkm_unproject / mdkm_set_points.  Errors: MDKM_ERR_STATE when the resident cloud did not
+ * come from mdkm_unproject; MDKM_ERR_INVALID when pairs is NULL, n_pairs < 1, k_capacity < 1, a
+ * day is outside [0, D) or n_pairs * (k_capacity + 1)^2 >= 2^31; from the mdkm_fit /
+ * mdkm_predict, before any work is enqueued, MDKM_ERR_INVALID when its k exceeds k_capacity, and
+ * MDKM_ERR_STATE on every rank when the ranks' pixel ranges do not cover the whole stack (their
+ * pixel counts summed by one all-reduce, once per cloud; one handle without a communicator must
+ * hold the whole stack). */
+int mdkm_bind_day_transitions(mdkm_handle* h, const int32_t* pairs, int n_pairs, int64_t* counts_out,
+                              int k_capacity);
+
 /* Load an already unprojected cloud (this rank's shard).  Replaces the `X` argument of the
  * reference's KMeans(...).fit_predict(X) call (members/jasraj/land_use_classification/
  * core.py:227-228) for d = 3. */
