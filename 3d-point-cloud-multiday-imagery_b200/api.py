@@ -59,6 +59,14 @@ class FusionResult:
     # int64 [P,K+1,K+1] and int64 [P,2], over the whole stack on every rank
     transitions: Optional[np.ndarray] = None
     transition_pairs: Optional[np.ndarray] = None
+    # connected regions of the cluster map (return_regions): one row per region, numbered 1..R in
+    # the raster order (day, y, x) of its first pixel -- int64 [R,7] (day, cluster, pixels, y_min,
+    # x_min, y_max, x_max) and float64 [R,3] mean (x, y, z) in the clustered frame, over the whole
+    # stack on every rank; region_map (return_region_map): int32 region id per pixel, 0 where no
+    # point, [D,H,W] or this rank's flat pixel range like cluster_map
+    regions: Optional[np.ndarray] = None
+    region_means: Optional[np.ndarray] = None
+    region_map: Optional[np.ndarray] = None
 
     # scikit-learn style aliases
     @property
@@ -158,6 +166,17 @@ def transition_pairs(spec, n_days: int) -> np.ndarray:
     return pairs
 
 
+def requested_connectivity(return_regions, connectivity=4, return_region_map=False):
+    """The connectivity ``return_regions`` / ``return_region_map`` ask for: None (no regions) or
+    4 / 8.  The region map implies the regions.  Raises ``ValueError`` for a connectivity other
+    than 4 or 8."""
+    if not (return_regions or return_region_map):
+        return None
+    if isinstance(connectivity, (bool, np.bool_)) or connectivity not in (4, 8):
+        raise ValueError(f"region_connectivity must be 4 or 8, got {connectivity!r}")
+    return int(connectivity)
+
+
 def _stack_days(height_maps, stack_shape, raster_layout) -> int:
     """D of the stack ``fuse_multiday_kmeans`` is given (before anything reaches the GPU)."""
     if stack_shape is not None:
@@ -169,7 +188,8 @@ def _stack_days(height_maps, stack_shape, raster_layout) -> int:
 
 
 def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_state, want_labels=True,
-                labels_out=None, gather_mappings=None, cluster_map_out=None, day_stats=False, transitions=None):
+                labels_out=None, gather_mappings=None, cluster_map_out=None, day_stats=False, transitions=None,
+                regions=None, region_map_out=None):
     """KMeans.fit driver (sklearn/_kmeans.py:1436-1563): init, n_init restarts, best inertia.
 
     ``labels_out``: optional int32 array that receives this rank's labels of the best run.
@@ -180,6 +200,8 @@ def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_
     returns fresh arrays, so the best run's stay with it.
     ``transitions``: day pairs ``[P,2]``; the result also has ``transitions`` (``Engine.fit``), the
     best run's, as with ``day_stats``.
+    ``regions`` (4 / 8) and ``region_map_out`` (int32): the result also has ``regions`` /
+    ``region_means``, the best run's as with ``day_stats``; the region map as ``cluster_map_out``.
     ``gather_mappings``: with a multi-rank engine, the collective that lets the ranks agree on
     sklearn's "same clustering up to a permutation" test (see ``_is_same_clustering``); when it is
     missing the test is skipped on multi-rank engines (the inertia comparison alone decides)."""
@@ -206,7 +228,7 @@ def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_
         gather_mappings = torch_gather_mappings(eng)  # None unless torch.distributed spans the ranks
     single = int(n_init) == 1
     best = None
-    run_map = best_map = None
+    run_map = best_map = run_rmap = best_rmap = None
     if cluster_map_out is not None and not single:
         import torch
 
@@ -214,6 +236,11 @@ def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_
         tdt = torch.uint8 if np.dtype(cluster_map_dtype(k)) == np.uint8 else torch.uint16
         run_map = torch.empty(eng.raster_range[4], dtype=tdt, device=f"cuda:{eng.device}")
         best_map = torch.empty_like(run_map)
+    if region_map_out is not None and not single:
+        import torch
+
+        run_rmap = torch.empty(eng.raster_range[4], dtype=torch.int32, device=f"cuda:{eng.device}")
+        best_rmap = torch.empty_like(run_rmap)
     for _ in range(int(n_init)):
         if init_is_array:
             centers0 = init_arr
@@ -224,7 +251,8 @@ def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_
         r = eng.fit(centers0, max_iter=max_iter, tol=tol, want_labels=want_labels,
                     labels_out=labels_out if (single and want_labels) else None,
                     cluster_map_out=cluster_map_out if single else run_map, day_stats=day_stats,
-                    transitions=transitions)
+                    transitions=transitions, regions=regions,
+                    region_map_out=region_map_out if single else run_rmap)
         # sklearn/_kmeans.py:1534-1541: a run replaces the best one when its inertia is lower AND it
         # is not the same clustering up to a permutation.  The inertia is global, so every rank
         # takes the same branch and the (collective) permutation test pairs up.
@@ -238,11 +266,15 @@ def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_
                 best = dict(r, labels=r["labels"].copy())  # result buffers are reused by the next run
             if run_map is not None:
                 run_map, best_map = best_map, run_map
+            if run_rmap is not None:
+                run_rmap, best_rmap = best_rmap, run_rmap
     if labels_out is not None and want_labels and not single:
         labels_out[...] = best["labels"]
         best = dict(best, labels=labels_out)
     if best_map is not None:
         _copy_map_out(best_map, cluster_map_out)
+    if best_rmap is not None:
+        _copy_map_out(best_rmap, region_map_out)
     return best
 
 
@@ -266,7 +298,8 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
                          detrend=False, disparity_scale=None, ground_level=False, return_cloud=True,
                          device=0, devices=None, engine=None, stack_shape=None,
                          pix_begin=0, raster_layout=None, return_cluster_map=False,
-                         return_day_stats=False, return_transitions=False) -> FusionResult:
+                         return_day_stats=False, return_transitions=False, return_regions=False,
+                         region_connectivity=4, return_region_map=False) -> FusionResult:
     """Unproject a multi-day height-map stack into one XYZ cloud and cluster it (Lloyd).
 
     height_maps : float32 ``[D,H,W]`` (NaN = nodata), numpy or torch (CPU or CUDA); or int16
@@ -309,6 +342,19 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
         labelling pass writes (the map itself need not be returned).  A pre-sharded call needs
         ranks that together hold the whole stack; every rank receives the global counts.
         Out-of-range days raise ``ValueError`` before any GPU work.
+    return_regions : also return the connected regions of the cluster map -- maximal sets of
+        pixels of one day with the same label that are connected (``region_connectivity`` 4: edge
+        neighbours, as ``scipy.ndimage.label``; 8: edge and corner neighbours), numbered 1..R over
+        the whole stack in the raster order (day, y, x) of each region's first pixel: ``regions``,
+        int64 ``[R,7]`` rows (day, cluster, pixels, y_min, x_min, y_max, x_max; inclusive bounds),
+        and ``region_means``, float64 ``[R,3]``, the mean (x, y, z) of each region's points in the
+        clustered coordinates (computed like ``day_means``: bitwise the same on any number of
+        GPUs).  Labelled on the GPU from the cluster map; a pre-sharded call needs ranks that
+        together hold the whole stack, and every rank receives the whole table.
+    return_region_map : also return ``region_map``, int32, the region id of every pixel that
+        produced a point and 0 elsewhere; ``[D,H,W]``, or this rank's flat slice for a pre-sharded
+        call, like ``cluster_map``.  Implies ``return_regions``.  A connectivity other than 4 or 8
+        raises ``ValueError`` before any GPU work.
     Returns a FusionResult; ``fused_cloud`` is float32 ``[N,3]`` in napari (z,y,x) order.
     """
     from .group import DeviceGroup
@@ -316,6 +362,7 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
     pairs = None
     if return_transitions is not None and not (isinstance(return_transitions, (bool, np.bool_)) and not return_transitions):
         pairs = transition_pairs(return_transitions, _stack_days(height_maps, stack_shape, raster_layout))
+    conn = requested_connectivity(return_regions, region_connectivity, return_region_map)
     if devices is not None or isinstance(engine, DeviceGroup):
         if stack_shape is not None or pix_begin:
             raise ValueError("stack_shape / pix_begin describe a pre-sharded stack; a device group shards by itself")
@@ -324,7 +371,8 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
                               tol=tol, random_state=random_state, max_abs_height=max_abs_height, detrend=detrend,
                               disparity_scale=disparity_scale, ground_level=ground_level, return_cloud=return_cloud,
                               raster_layout=raster_layout, return_cluster_map=return_cluster_map,
-                              return_day_stats=return_day_stats, transitions=pairs)
+                              return_day_stats=return_day_stats, transitions=pairs, regions=conn,
+                              return_region_map=return_region_map)
     own = engine is None
     eng = engine or Engine(device)
     try:
@@ -349,16 +397,21 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
         if return_cluster_map:
             D, H, W, _, count = eng.raster_range
             cmap = np.empty((D, H, W) if stack_shape is None else (count,), dtype=cluster_map_dtype(n_clusters))
+        rmap = None
+        if return_region_map:
+            D, H, W, _, count = eng.raster_range
+            rmap = np.empty((D, H, W) if stack_shape is None else (count,), dtype=np.int32)
         r = _run_kmeans(eng, n_clusters=n_clusters, init=init, n_init=n_init, max_iter=max_iter,
                         tol=tol, random_state=random_state, cluster_map_out=cmap, day_stats=return_day_stats,
-                        transitions=pairs)
+                        transitions=pairs, regions=conn, region_map_out=rmap)
         eng.wait()
         return FusionResult(labels=r["labels"], centroids=r["centers"], fused_cloud=cloud,
                             n_iter=r["n_iter"], inertia=r["inertia"], n_points=n,
                             n_refined=r["n_refined"], n_relocations=r["n_relocations"],
                             height_norm=hn, extra=extra, cluster_map=cmap,
                             day_counts=r.get("day_counts"), day_means=r.get("day_means"),
-                            transitions=r.get("transitions"), transition_pairs=pairs)
+                            transitions=r.get("transitions"), transition_pairs=pairs,
+                            regions=r.get("regions"), region_means=r.get("region_means"), region_map=rmap)
     finally:
         if own:
             eng.close()
@@ -366,7 +419,7 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
 
 def _fuse_on_group(height_maps, valid_masks, *, group, devices, n_clusters, init, n_init, max_iter, tol,
                    random_state, return_cluster_map=False, return_day_stats=False, transitions=None,
-                   **unproject_kw) -> FusionResult:
+                   regions=None, return_region_map=False, **unproject_kw) -> FusionResult:
     """``fuse_multiday_kmeans`` on several devices of this process (``group.DeviceGroup``)."""
     import threading
 
@@ -391,22 +444,26 @@ def _fuse_on_group(height_maps, valid_masks, *, group, devices, n_clusters, init
                 return [g[0] for g in got], [g[1] for g in got]
             return gather
 
-        def run(eng, labels_out, cluster_map_out=None):
+        def run(eng, labels_out, cluster_map_out=None, region_map_out=None):
             r = eng.rank
             return _run_kmeans(eng, n_clusters=n_clusters, init=init, n_init=n_init, max_iter=max_iter, tol=tol,
                                random_state=states[r], labels_out=labels_out,
                                gather_mappings=gather_for(r) if grp.world > 1 else None,
-                               cluster_map_out=cluster_map_out, day_stats=return_day_stats, transitions=transitions)
+                               cluster_map_out=cluster_map_out, day_stats=return_day_stats, transitions=transitions,
+                               regions=regions, region_map_out=region_map_out)
 
         res, labels, cloud, hn, extra = grp.fuse(
             height_maps, valid_masks, run_kmeans=run,
-            cluster_map_dtype=cluster_map_dtype(n_clusters) if return_cluster_map else None, **unproject_kw)
+            cluster_map_dtype=cluster_map_dtype(n_clusters) if return_cluster_map else None,
+            region_map=return_region_map, **unproject_kw)
         return FusionResult(labels=labels, centroids=res["centers"], fused_cloud=cloud, n_iter=res["n_iter"],
                             inertia=res["inertia"], n_points=int(labels.shape[0]), n_refined=res["n_refined"],
                             n_relocations=res["n_relocations"], height_norm=hn, extra=extra,
                             cluster_map=extra.pop("cluster_map", None),
                             day_counts=res.get("day_counts"), day_means=res.get("day_means"),
-                            transitions=res.get("transitions"), transition_pairs=transitions)
+                            transitions=res.get("transitions"), transition_pairs=transitions,
+                            regions=res.get("regions"), region_means=res.get("region_means"),
+                            region_map=extra.pop("region_map", None))
     finally:
         if own:
             grp.close()
@@ -447,7 +504,8 @@ def to_layers(result: FusionResult, prefix: str = "Multi-day") -> List[Layer]:
 
     One Points layer with the fused cloud coloured by cluster (or by the reference's
     'height' property when it was computed) and one with the K centroids; when the result has a
-    ``cluster_map``, a third, Labels layer with it (0 = no point at that pixel).
+    ``cluster_map``, a Labels layer with it (0 = no point at that pixel), and when it has a
+    ``region_map``, a Labels layer with the region ids.
     """
     if result.fused_cloud is None:
         raise ValueError("result has no fused_cloud (return_cloud=False)")
@@ -479,6 +537,8 @@ def to_layers(result: FusionResult, prefix: str = "Multi-day") -> List[Layer]:
     ))
     if result.cluster_map is not None:
         layers.append((result.cluster_map, {"name": f"{prefix} Cluster Map", "opacity": 0.7}, "labels"))
+    if result.region_map is not None:
+        layers.append((result.region_map, {"name": f"{prefix} Regions", "opacity": 0.7}, "labels"))
     return layers
 
 

@@ -22,6 +22,7 @@
 #include "lloyd.cuh"
 #include "mirror.cuh"
 #include "nccl_shim.h"
+#include "regions.cuh"
 #include "seeding.cuh"
 #include "transitions.cuh"
 #include "unproject.cuh"
@@ -173,13 +174,27 @@ struct mdkm_handle {
   std::vector<int> bound_pairs;          // [n_pairs][2] days, copied when bound
   int64_t* bound_trans = nullptr;
   int bound_trans_kcap = 0;
-  int trans_cover = -1;                  // the ranks' pixel ranges cover the stack (1) or not (0); -1: not checked
-  DevBuf<unsigned char> trans_map;       // the map the final pass writes when none is bound; the whole stack with
-                                         // several ranks
   DevBuf<int> trans_pairs;
   DevBuf<unsigned long long> trans_bins;  // [n_pairs][(k+1)^2]
   unsigned char* trans_host = nullptr;    // pinned: their copy, handed to the caller after the sync
   size_t trans_host_cap = 0;
+  // the whole-stack cluster map that day transitions and regions read (take_stack_map)
+  int stack_cover = -1;                  // the ranks' pixel ranges cover the stack (1) or not (0); -1: not checked
+  DevBuf<unsigned char> stack_map;       // the map the final pass writes when none is bound; the whole stack with
+                                         // several ranks
+  // connected regions of the cluster map (mdkm_bind_regions) of the next fit / predict, and those
+  // of the last fit / predict that had them, kept on the device until the next unproject /
+  // set_points / fit or predict with regions
+  int bound_regions = 0;                 // connectivity 4 or 8; 0: not bound
+  int32_t* bound_region_map = nullptr;
+  int bound_region_map_mem = MDKM_MEM_HOST;
+  DevBuf<int> region_parent;             // [stack pixels] union-find parents
+  DevBuf<int> region_ids;                // [stack pixels] region map of the whole stack
+  DevBuf<unsigned long long> region_scan;  // look-back words of the numbering, then ticket + fault, then R
+  DevBuf<unsigned long long> region_acc;   // [R][4] (qx, qy, qz, count)
+  DevBuf<unsigned int> region_box;         // [R][5] first pixel, y_min, x_min, ~y_max, ~x_max
+  DevBuf<unsigned char> region_out;        // table int64 [R][7], then means float64 [R][3]
+  long long n_regions = -1;              // R of the last fit / predict with regions; -1: none
 
   // communicator
   ncclComm_t comm = nullptr;
@@ -932,6 +947,8 @@ struct MapOut {
   unsigned char* stack = nullptr;
   size_t stack_bytes = 0;
   void* dev_out = nullptr;
+  // day transitions / regions: the whole stack's map (device), once take_stack_map has set it up
+  const unsigned char* whole = nullptr;
 };
 
 // Per-(day, cluster) statistics taken by one fit / predict (mdkm_bind_day_stats): accumulated by
@@ -949,10 +966,16 @@ struct StatsOut {
 struct TransOut {
   int64_t* out = nullptr;
   int n_pairs = 0;
-  int k1 = 0;                          // states: k + 1
-  const unsigned char* map = nullptr;  // the whole stack's map (device)
-  int elem = 1;
-  bool reduce_map = false;             // several ranks: the bands of `map` are summed over the ranks first
+  int k1 = 0;  // states: k + 1
+};
+
+// Connected regions taken by one fit / predict (mdkm_bind_regions): labelled from the whole-stack
+// cluster map after the call's synchronisation; `map` (optional) receives this rank's range of
+// the region map.
+struct RegOut {
+  int conn = 0;  // 4 or 8; 0: not asked for
+  int32_t* map = nullptr;
+  int mem = MDKM_MEM_HOST;
 };
 
 // page-locked host buffer of at least `bytes` (the stages of results handed over after a sync)
@@ -1024,20 +1047,16 @@ int take_day_stats(mdkm_handle* h, int k, StatsOut& s) {
   return upload_day_offsets(h);
 }
 
-// Takes the binding of mdkm_bind_day_transitions (`out`, already consumed) for a call with k
-// clusters and its cluster map `m`: checks k against the bound capacity and, once per cloud, that
-// the ranks' pixel ranges cover the stack (one all-reduce); sizes the bins, uploads the pairs.
-// The map the pairs are binned from is the bound one (one rank) or one the final pass writes for
-// them: an internal map of the range when none is bound, and with several ranks a whole-stack
-// map of which every rank writes its band (a bound output then receives that band).
-int take_transitions(mdkm_handle* h, int k, int64_t* out, MapOut& m, TransOut& t) {
-  if (!out) return MDKM_OK;
-  const int kcap = h->bound_trans_kcap;
-  if (k > kcap) return fail(h, MDKM_ERR_INVALID, "k=%d exceeds the k_capacity %d of the bound day transitions", k, kcap);
-  if (k < 1 || k > kMaxK) return MDKM_OK;  // (rejected with the call's own message)
+// The whole-stack cluster map that day transitions and regions read, taken once per call for
+// both: checks, once per cloud, that the ranks' pixel ranges cover the stack (one all-reduce).
+// With one rank it is the call's map: the bound one, or an internal one the final pass writes
+// when none is bound.  With several ranks it is a whole-stack map of which every rank writes its
+// band (a bound device output then receives that band), merged by merge_stack_map.
+int take_stack_map(mdkm_handle* h, int k, MapOut& m) {
+  if (m.whole) return MDKM_OK;
   CU(cudaSetDevice(h->device));
   const long long HW = (long long)h->raster_H * h->raster_w, stack_px = (long long)h->stack_days * HW;
-  if (h->trans_cover < 0) {
+  if (h->stack_cover < 0) {
     long long px = h->raster_pix_count;
     if (h->n_ranks > 1) {
       OK(ensure(h, h->dscratch, 64));
@@ -1047,10 +1066,51 @@ int take_transitions(mdkm_handle* h, int k, int64_t* out, MapOut& m, TransOut& t
       OK(small_d2h(h, &px, d, 8));
       OK(sync_small(h));
     }
-    h->trans_cover = px == stack_px ? 1 : 0;
+    h->stack_cover = px == stack_px ? 1 : 0;
   }
-  if (!h->trans_cover)
-    return fail(h, MDKM_ERR_STATE, "day transitions need the pixel ranges of the ranks to cover the whole stack");
+  if (!h->stack_cover)
+    return fail(h, MDKM_ERR_STATE, "day transitions and regions need the pixel ranges of the ranks to cover the whole stack");
+  if (h->n_ranks == 1) {
+    if (!m.dev) {
+      m.elem = k <= 255 ? 1 : 2;
+      m.bytes = (size_t)h->raster_pix_count * m.elem;
+      OK(ensure(h, h->stack_map, std::max<size_t>(m.bytes, 1)));
+      m.dev = h->stack_map.p;
+      OK(upload_day_offsets(h));
+    }
+    m.whole = static_cast<const unsigned char*>(m.dev);
+    return MDKM_OK;
+  }
+  const int elem = m.dev ? m.elem : (k <= 255 ? 1 : 2);
+  const size_t stack_bytes = (size_t)stack_px * elem;
+  OK(ensure(h, h->stack_map, std::max<size_t>(stack_bytes, 1)));
+  if (m.dev && !m.host) m.dev_out = m.dev;
+  if (!m.dev) OK(upload_day_offsets(h));
+  m.dev = h->stack_map.p + (size_t)h->raster_pix_begin * elem;
+  m.elem = elem;
+  m.bytes = (size_t)h->raster_pix_count * elem;
+  m.stack = h->stack_map.p;
+  m.stack_bytes = stack_bytes;
+  m.whole = h->stack_map.p;
+  return MDKM_OK;
+}
+
+// Behind the final pass, on the stream: with several ranks the bands of the whole-stack map summed
+// over the ranks.  The bands are disjoint: their byte-wise sum is their union, for 16-bit maps too.
+int merge_stack_map(mdkm_handle* h, const MapOut& m) {
+  if (m.stack) OK(allreduce(h, m.stack, m.stack_bytes, kNcclUint8, kNcclSum));
+  return MDKM_OK;
+}
+
+// Takes the binding of mdkm_bind_day_transitions (`out`, already consumed) for a call with k
+// clusters and its cluster map `m`: checks k against the bound capacity, sets up the whole-stack
+// map, sizes the bins, uploads the pairs.
+int take_transitions(mdkm_handle* h, int k, int64_t* out, MapOut& m, TransOut& t) {
+  if (!out) return MDKM_OK;
+  const int kcap = h->bound_trans_kcap;
+  if (k > kcap) return fail(h, MDKM_ERR_INVALID, "k=%d exceeds the k_capacity %d of the bound day transitions", k, kcap);
+  if (k < 1 || k > kMaxK) return MDKM_OK;  // (rejected with the call's own message)
+  OK(take_stack_map(h, k, m));
   t.out = out;
   t.n_pairs = (int)(h->bound_pairs.size() / 2);
   t.k1 = k + 1;
@@ -1060,32 +1120,30 @@ int take_transitions(mdkm_handle* h, int k, int64_t* out, MapOut& m, TransOut& t
   CU(cudaMemcpyAsync(h->trans_pairs.p, h->bound_pairs.data(), h->bound_pairs.size() * 4, cudaMemcpyHostToDevice,
                      h->stream));
   OK(ensure_pinned(h, h->trans_host, h->trans_host_cap, words * 8));
-  if (h->n_ranks == 1) {
-    if (!m.dev) {
-      m.elem = k <= 255 ? 1 : 2;
-      m.bytes = (size_t)h->raster_pix_count * m.elem;
-      OK(ensure(h, h->trans_map, std::max<size_t>(m.bytes, 1)));
-      m.dev = h->trans_map.p;
-      OK(upload_day_offsets(h));
-    }
-    t.map = static_cast<const unsigned char*>(m.dev);
-    t.elem = m.elem;
+  return MDKM_OK;
+}
+
+// Consumes the binding of mdkm_bind_regions (whatever happens next).
+RegOut consume_regions(mdkm_handle* h) {
+  RegOut g;
+  g.conn = h->bound_regions;
+  g.map = h->bound_region_map;
+  g.mem = h->bound_region_map_mem;
+  h->bound_regions = 0;
+  h->bound_region_map = nullptr;
+  return g;
+}
+
+// Takes the regions `g` (consumed) for a call with k clusters and its cluster map `m`: sets up the
+// whole-stack map; the regions of an earlier call are dropped.
+int take_regions(mdkm_handle* h, int k, MapOut& m, RegOut& g) {
+  if (!g.conn) return MDKM_OK;
+  if (k < 1 || k > kMaxK) {  // (rejected with the call's own message)
+    g.conn = 0;
     return MDKM_OK;
   }
-  const int elem = m.dev ? m.elem : (k <= 255 ? 1 : 2);
-  const size_t stack_bytes = (size_t)stack_px * elem;
-  OK(ensure(h, h->trans_map, std::max<size_t>(stack_bytes, 1)));
-  if (m.dev && !m.host) m.dev_out = m.dev;
-  if (!m.dev) OK(upload_day_offsets(h));
-  m.dev = h->trans_map.p + (size_t)h->raster_pix_begin * elem;
-  m.elem = elem;
-  m.bytes = (size_t)h->raster_pix_count * elem;
-  m.stack = h->trans_map.p;
-  m.stack_bytes = stack_bytes;
-  t.map = h->trans_map.p;
-  t.elem = elem;
-  t.reduce_map = true;
-  return MDKM_OK;
+  h->n_regions = -1;
+  return take_stack_map(h, k, m);
 }
 
 typedef void (*TransKernel)(const TransParams);
@@ -1096,20 +1154,17 @@ TransKernel pick_trans_kernel(int mode) {
   return day_transitions_kernel<T, kTransGlobalBins>;
 }
 
-// Behind the final pass, on the stream: with several ranks the map's bands summed over the ranks,
-// then the bins of this rank's share of the pixels of every day, their sum over the ranks, the
-// copy to the pinned stage.  (Behind a final pass that returned early for a relocation this bins
-// a map of zeros; the pass after the relocation runs it again.)
-int run_transitions(mdkm_handle* h, const TransOut& t) {
+// Behind the final pass and merge_stack_map, on the stream: the bins of this rank's share of the
+// pixels of every day of the whole-stack map, their sum over the ranks, the copy to the pinned
+// stage.  (Behind a final pass that returned early for a relocation this bins a map of zeros; the
+// pass after the relocation runs it again.)
+int run_transitions(mdkm_handle* h, const TransOut& t, const MapOut& m) {
   if (!t.out) return MDKM_OK;
   const long long HW = (long long)h->raster_H * h->raster_w;
-  // the bands are disjoint: their byte-wise sum is their union, for 16-bit maps too
-  if (t.reduce_map)
-    OK(allreduce(h, const_cast<unsigned char*>(t.map), (size_t)h->stack_days * HW * t.elem, kNcclUint8, kNcclSum));
   const size_t nb = (size_t)t.k1 * t.k1, words = nb * t.n_pairs;
   CU(cudaMemsetAsync(h->trans_bins.p, 0, words * 8, h->stream));
   TransParams tp{};
-  tp.map = t.map;
+  tp.map = m.whole;
   tp.HW = HW;
   tp.q_begin = HW * h->rank / h->n_ranks;
   tp.q_end = HW * (h->rank + 1) / h->n_ranks;
@@ -1119,7 +1174,7 @@ int run_transitions(mdkm_handle* h, const TransOut& t) {
   tp.bins = h->trans_bins.p;
   // bins in shared memory when they do not cost a resident CTA (run-time occupancy query): a copy
   // per warp, else one per CTA; otherwise straight to the global bins
-  auto pick = [&](int mode) { return t.elem == 2 ? pick_trans_kernel<unsigned short>(mode) : pick_trans_kernel<unsigned char>(mode); };
+  auto pick = [&](int mode) { return m.elem == 2 ? pick_trans_kernel<unsigned short>(mode) : pick_trans_kernel<unsigned char>(mode); };
   int base = 0, optin = 0;
   CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&base, pick(kTransGlobalBins), kThreads, 0));
   CU(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
@@ -1180,6 +1235,96 @@ void deliver_day_stats(mdkm_handle* h, const StatsOut& s) {
   if (!s.counts) return;
   memcpy(s.counts, h->stats_host, (size_t)s.slots * 8);
   memcpy(s.means, h->stats_host + (size_t)s.slots * 8, (size_t)s.slots * 24);
+}
+
+// The regions `g` of the whole-stack map `m`, after the call's synchronisation (the map is final,
+// also after a relocation).  Every rank labels the whole stack: tile-local union-find, links
+// across the tile borders, ids of the roots, every pixel's id (regions.cuh); the caller's region
+// map receives this rank's range.  One synchronisation reads R, then this rank's points are
+// summed into per-region slots, the slots are reduced over the ranks (sums; minima of the
+// first pixel and the bounds) and the table and means are written on the device, where
+// mdkm_region_table finds them.
+int run_regions(mdkm_handle* h, const RegOut& g, const MapOut& m) {
+  if (!g.conn) return MDKM_OK;
+  const long long HW = (long long)h->raster_H * h->raster_w, n_px = (long long)h->stack_days * HW;
+  const bool in_place = g.map && g.mem == MDKM_MEM_DEVICE && h->n_ranks == 1;  // (one rank holds the whole stack)
+  OK(ensure(h, h->region_parent, (size_t)n_px));
+  if (!in_place) OK(ensure(h, h->region_ids, (size_t)n_px));
+  const long long n_chunks = (n_px + kRegChunk - 1) / kRegChunk;
+  OK(ensure(h, h->region_scan, (size_t)n_chunks + 2));
+  RegionParams rp{};
+  rp.map = m.whole;
+  rp.parent = h->region_parent.p;
+  rp.ids = in_place ? g.map : h->region_ids.p;
+  rp.n_px = n_px;
+  rp.HW = HW;
+  rp.H = h->raster_H;
+  rp.W = h->raster_w;
+  rp.tiles_x = (h->raster_w + kRegTile - 1) / kRegTile;
+  rp.tiles_y = (h->raster_H + kRegTile - 1) / kRegTile;
+  rp.n_tiles = (long long)h->stack_days * rp.tiles_x * rp.tiles_y;
+  rp.status = h->region_scan.p;
+  rp.ticket = reinterpret_cast<unsigned int*>(h->region_scan.p + n_chunks);
+  rp.n_regions = h->region_scan.p + n_chunks + 1;
+  const bool c8 = g.conn == 8, wide = m.elem == 2;
+  auto tile_fn = wide ? (c8 ? region_tile_kernel<unsigned short, true> : region_tile_kernel<unsigned short, false>)
+                      : (c8 ? region_tile_kernel<unsigned char, true> : region_tile_kernel<unsigned char, false>);
+  auto border_fn = wide ? (c8 ? region_border_kernel<unsigned short, true> : region_border_kernel<unsigned short, false>)
+                        : (c8 ? region_border_kernel<unsigned char, true> : region_border_kernel<unsigned char, false>);
+  tile_fn<<<(unsigned int)rp.n_tiles, kThreads, 0, h->stream>>>(rp);
+  border_fn<<<(unsigned int)((rp.n_tiles + kThreads / 32 - 1) / (kThreads / 32)), kThreads, 0, h->stream>>>(rp);
+  CU(cudaMemsetAsync(h->region_scan.p, 0, ((size_t)n_chunks + 2) * 8, h->stream));
+  region_number_kernel<<<(unsigned int)n_chunks, kThreads, 0, h->stream>>>(rp);
+  region_resolve_kernel<<<grid_for(h, (n_px + 1023) / 1024, resident_per_sm(h, region_resolve_kernel)), kThreads, 0,
+                          h->stream>>>(rp);
+  h->launches += 4;
+  CU(cudaGetLastError());
+  if (g.map && !in_place)
+    CU(cudaMemcpyAsync(g.map, rp.ids + h->raster_pix_begin, (size_t)h->raster_pix_count * 4,
+                       g.mem == MDKM_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, h->stream));
+  unsigned long long got[2] = {0, 0};  // ticket | fault << 32, R
+  OK(small_d2h(h, got, h->region_scan.p + n_chunks, 16));
+  OK(sync_small(h));
+  if (got[0] >> 32) return fail(h, MDKM_ERR_CUDA, "region numbering: the look-back over the chunks timed out");
+  const long long R = (long long)got[1];
+  if (R > 0) {
+    OK(ensure(h, h->region_acc, (size_t)R * 4));
+    OK(ensure(h, h->region_box, (size_t)R * 5));
+    OK(ensure(h, h->region_out, (size_t)R * 80));
+    CU(cudaMemsetAsync(h->region_acc.p, 0, (size_t)R * 32, h->stream));
+    CU(cudaMemsetAsync(h->region_box.p, 0xff, (size_t)R * 20, h->stream));
+    if (h->n > 0) {
+      RegionStatsParams sp{};
+      sp.pts = h->pts.p;
+      sp.n = h->n;
+      sp.seg = h->map_seg.p;
+      sp.nseg = (int)h->seg_off.size() - 1;
+      sp.pix0 = h->day0 * HW;
+      sp.HW = HW;
+      sp.W = h->raster_w;
+      sp.ids = rp.ids;
+      for (int d = 0; d < 3; ++d) {
+        sp.origin[d] = h->fr.origin[d];
+        sp.scale[d] = h->fr.scale[d];
+      }
+      sp.acc = h->region_acc.p;
+      sp.box = h->region_box.p;
+      const long long n_groups = (h->n + kGroup - 1) / kGroup;
+      region_stats_kernel<<<grid_for(h, (n_groups + 7) / 8, resident_per_sm(h, region_stats_kernel)), kThreads, 0,
+                            h->stream>>>(sp);
+      ++h->launches;
+    }
+    OK(allreduce(h, h->region_acc.p, (size_t)R * 4, kNcclInt64, kNcclSum));
+    OK(allreduce(h, h->region_box.p, (size_t)R * 5, kNcclUint32, kNcclMin));
+    long long* table = reinterpret_cast<long long*>(h->region_out.p);
+    region_finish_kernel<<<grid_for(h, (R + kThreads - 1) / kThreads, 4), kThreads, 0, h->stream>>>(
+        h->region_acc.p, h->region_box.p, R, m.whole, m.elem, HW, h->fr, table,
+        reinterpret_cast<double*>(table + R * 7));
+    ++h->launches;
+    CU(cudaGetLastError());
+  }
+  h->n_regions = R;
+  return MDKM_OK;
 }
 
 // The map's device->host copy (host outputs), on the compute stream behind the final pass.
@@ -1362,8 +1507,10 @@ void mdkm_destroy(mdkm_handle* h) {
   release(h->d_seg_off); release(h->sel_hist); release(h->sel_targets);
   release(h->map_stage); release(h->map_seg); release(h->stats_acc); release(h->stats_dev);
   if (h->stats_host) cudaFreeHost(h->stats_host);
-  release(h->trans_map); release(h->trans_pairs); release(h->trans_bins);
+  release(h->stack_map); release(h->trans_pairs); release(h->trans_bins);
   if (h->trans_host) cudaFreeHost(h->trans_host);
+  release(h->region_parent); release(h->region_ids); release(h->region_scan); release(h->region_acc);
+  release(h->region_box); release(h->region_out);
   release(h->kpp_closest); release(h->kpp_cell); release(h->kpp_blk); release(h->kpp_prefix);
   release(h->kpp_partials); release(h->kpp_rand); release(h->kpp_state);
   if (h->d_status) cudaFree(h->d_status);
@@ -1399,7 +1546,7 @@ int mdkm_comm_init(mdkm_handle* h, int n_ranks, int rank, const unsigned char id
   h->n_ranks = n_ranks;
   h->rank = rank;
   h->frame_ok = false;
-  h->trans_cover = -1;
+  h->stack_cover = -1;
   close_p2p(h);
   if (n_ranks == 1) return MDKM_OK;
   if (!id) return fail(h, MDKM_ERR_INVALID, "unique id required");
@@ -1568,7 +1715,10 @@ int mdkm_set_points(mdkm_handle* h, const float* xyz, int64_t n, int layout, int
   h->bound_map = nullptr;
   h->bound_counts = nullptr;
   h->bound_trans = nullptr;
-  h->trans_cover = -1;
+  h->stack_cover = -1;
+  h->bound_regions = 0;
+  h->bound_region_map = nullptr;
+  h->n_regions = -1;
   h->stack_days = 1;
   h->day0 = 0;
   h->runs_ok = false;
@@ -1657,6 +1807,49 @@ int mdkm_bind_day_transitions(mdkm_handle* h, const int32_t* pairs, int n_pairs,
   return MDKM_OK;
 }
 
+int mdkm_bind_regions(mdkm_handle* h, int connectivity, int32_t* map_out, int64_t capacity_pixels, int mem) {
+  if (!h) return MDKM_ERR_INVALID;
+  h->bound_regions = 0;
+  h->bound_region_map = nullptr;
+  if (!connectivity && !map_out) return MDKM_OK;
+  if (!h->have_points || h->raster_w <= 0)
+    return fail(h, MDKM_ERR_STATE, "regions need a resident cloud from mdkm_unproject");
+  if (connectivity != 4 && connectivity != 8)
+    return fail(h, MDKM_ERR_INVALID, "regions: connectivity must be 4 or 8, got %d", connectivity);
+  if ((long long)h->stack_days * h->raster_H * h->raster_w >= (1ll << 31))
+    return fail(h, MDKM_ERR_INVALID, "regions need a stack of fewer than 2^31 pixels");
+  if (h->raster_w >= (1 << 23) || h->raster_H >= (1 << 23))  // (the final pass writes the map they are labelled from)
+    return fail(h, MDKM_ERR_INVALID, "regions need rasters narrower and shorter than 2^23 pixels");
+  if (map_out && (capacity_pixels < h->raster_pix_count || (mem != MDKM_MEM_HOST && mem != MDKM_MEM_DEVICE)))
+    return fail(h, MDKM_ERR_INVALID, "region map: capacity %lld < %lld pixels, or bad memory kind",
+                (long long)capacity_pixels, h->raster_pix_count);
+  h->bound_regions = connectivity;
+  h->bound_region_map = map_out;
+  h->bound_region_map_mem = mem;
+  return MDKM_OK;
+}
+
+int mdkm_region_count(const mdkm_handle* h, int64_t* n_regions) {
+  if (!h || !n_regions) return MDKM_ERR_INVALID;
+  if (h->n_regions < 0) return fail(const_cast<mdkm_handle*>(h), MDKM_ERR_STATE, "no regions: no fit / predict with regions since the last unproject / set_points");
+  *n_regions = h->n_regions;
+  return MDKM_OK;
+}
+
+int mdkm_region_table(mdkm_handle* h, int64_t* table_out, double* means_out, int64_t capacity_regions) {
+  if (!h) return MDKM_ERR_INVALID;
+  if (h->n_regions < 0) return fail(h, MDKM_ERR_STATE, "no regions: no fit / predict with regions since the last unproject / set_points");
+  const long long R = h->n_regions;
+  if (capacity_regions < R) return fail(h, MDKM_ERR_INVALID, "region table: capacity %lld < %lld regions", (long long)capacity_regions, R);
+  if (R == 0) return MDKM_OK;
+  CU(cudaSetDevice(h->device));
+  if (table_out) CU(cudaMemcpyAsync(table_out, h->region_out.p, (size_t)R * 56, cudaMemcpyDeviceToHost, h->stream));
+  if (means_out)
+    CU(cudaMemcpyAsync(means_out, h->region_out.p + (size_t)R * 56, (size_t)R * 24, cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
+  return MDKM_OK;
+}
+
 int mdkm_bind_day_stats(mdkm_handle* h, int64_t* counts_out, double* means_out, int n_days, int k_capacity) {
   if (!h) return MDKM_ERR_INVALID;
   h->bound_counts = nullptr;
@@ -1690,7 +1883,10 @@ int mdkm_unproject(mdkm_handle* h, const void* hm, int hm_dtype, float hm_scale,
   h->bound_map = nullptr;  // (a cluster map describes the range it was bound for)
   h->bound_counts = nullptr;  // (and day statistics the stack)
   h->bound_trans = nullptr;
-  h->trans_cover = -1;
+  h->stack_cover = -1;
+  h->bound_regions = 0;  // (and regions the stack)
+  h->bound_region_map = nullptr;
+  h->n_regions = -1;
   if (D < 0 || H <= 0 || W <= 0 || pix_begin < 0 || pix_count < 0 ||
       pix_begin + pix_count > (int64_t)D * H * W || (pix_count > 0 && !hm))
     return fail(h, MDKM_ERR_INVALID, "bad stack geometry");
@@ -1976,10 +2172,12 @@ int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol
   TransOut trans;
   int64_t* trans_out = h->bound_trans;
   h->bound_trans = nullptr;
+  RegOut reg = consume_regions(h);
   const int map_rc = take_cluster_map(h, k, map);
   OK(take_day_stats(h, k, stats));
   OK(map_rc);
   OK(take_transitions(h, k, trans_out, map, trans));
+  OK(take_regions(h, k, map, reg));
   if (!init) return fail(h, MDKM_ERR_INVALID, "init centroids required");
   OK(check_centroids(h, k, init, "init"));
   if (max_iter < 1) return fail(h, MDKM_ERR_INVALID, "max_iter must be >= 1");
@@ -2105,7 +2303,8 @@ int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol
       prof_end(h, span);
     }
     OK(reduce_day_stats(h, stats));
-    OK(run_transitions(h, trans));
+    OK(merge_stack_map(h, map));
+    OK(run_transitions(h, trans, map));
     if (!one_rank) {
       OK(ensure(h, h->dscratch, (size_t)k * 3 + 16));
       read_table_kernel<<<(k + 255) / 256, 256, 0, h->stream>>>(h->table.p, k, kb.kpad, h->fr, h->dscratch.p);
@@ -2139,6 +2338,7 @@ int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol
 #endif
   if (fin.xchg_timeout == 2) return index_fault(h);
   if (fin.xchg_timeout) return fail(h, MDKM_ERR_NCCL, "a kernel-side wait timed out (peer exchange of the partial sums: a rank is missing; or the grid barrier)");
+  OK(run_regions(h, reg, map));
   deliver_day_stats(h, stats);
   deliver_transitions(h, trans);
   if (n_iter_out) *n_iter_out = fin.iter;
@@ -2218,10 +2418,12 @@ int mdkm_predict(mdkm_handle* h, int k, const double* centroids, int32_t* labels
   TransOut trans;
   int64_t* trans_out = h->bound_trans;
   h->bound_trans = nullptr;
+  RegOut reg = consume_regions(h);
   const int map_rc = take_cluster_map(h, k, map);
   OK(take_day_stats(h, k, stats));
   OK(map_rc);
   OK(take_transitions(h, k, trans_out, map, trans));
+  OK(take_regions(h, k, map, reg));
   if (!centroids) return fail(h, MDKM_ERR_INVALID, "centroids required");
   OK(check_centroids(h, k, centroids, "centroids"));
   CU(cudaSetDevice(h->device));
@@ -2244,13 +2446,15 @@ int mdkm_predict(mdkm_handle* h, int k, const double* centroids, int32_t* labels
   OK(run_final(h, kb, labels_dev, false, nullptr, nullptr, &map, &stats));
   if (h->n_ranks > 1) OK(allreduce(h, &h->d_status->inertia, 1, kNcclFloat64, kNcclSum));
   OK(reduce_day_stats(h, stats));
-  OK(run_transitions(h, trans));
+  OK(merge_stack_map(h, map));
+  OK(run_transitions(h, trans, map));
   OK(small_d2h(h, &h->h_status[0], h->d_status, sizeof(DevStatus), /*dst_is_pinned=*/true));
   if (labels_out && labels_mem != MDKM_MEM_DEVICE && h->n > 0)
     CU(cudaMemcpyAsync(labels_out, labels_dev, (size_t)h->n * 4, cudaMemcpyDeviceToHost, h->stream));
   OK(copy_cluster_map(h, map));
   OK(sync_small(h));
   if (h->h_status[0].xchg_timeout == 2) return index_fault(h);
+  OK(run_regions(h, reg, map));
   deliver_day_stats(h, stats);
   deliver_transitions(h, trans);
   if (inertia_out) *inertia_out = h->h_status[0].inertia;

@@ -13,7 +13,7 @@ typedef struct ncclComm* ncclComm_t;
 typedef struct { char internal[128]; } ncclUniqueId;
 typedef int ncclResult_t;
 // values from nccl.h (stable across 2.x)
-enum { kNcclUint8 = 1, kNcclInt64 = 4, kNcclUint64 = 5, kNcclFloat32 = 7, kNcclFloat64 = 8 };
+enum { kNcclUint8 = 1, kNcclUint32 = 3, kNcclInt64 = 4, kNcclUint64 = 5, kNcclFloat32 = 7, kNcclFloat64 = 8 };
 enum { kNcclSum = 0, kNcclMax = 2, kNcclMin = 3 };
 
 struct NcclApi {

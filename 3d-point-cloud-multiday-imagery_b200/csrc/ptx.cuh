@@ -152,6 +152,16 @@ __device__ __forceinline__ unsigned int ld_acquire_gpu_u32(const unsigned int* p
   return v;
 }
 
+// gpu-scope relaxed 32-bit accesses: union-find parents that other threads of the grid relink
+__device__ __forceinline__ unsigned int ld_relaxed_gpu_u32(const void* p) {
+  unsigned int v;
+  asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+  return v;
+}
+__device__ __forceinline__ void st_relaxed_gpu_u32(void* p, unsigned int v) {
+  asm volatile("st.relaxed.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+}
+
 // 8-byte (value, flag) packets: one store / one load each, so a reader never sees one without the other
 __device__ __forceinline__ void st_relaxed_sys_v2u32(void* p, unsigned int a, unsigned int b) {
   asm volatile("st.relaxed.sys.global.v2.u32 [%0], {%1, %2};" ::"l"(p), "r"(a), "r"(b) : "memory");

@@ -395,21 +395,52 @@ class Engine:
                                                         c_void_p(counts.ctypes.data), int(k)))
         return counts
 
-    def _bind_outputs(self, k, cluster_map_out, day_stats, transitions):
+    def _bind_regions(self, connectivity, out):
+        """Bind connected regions (``connectivity`` 4 or 8) and the optional int32 region map ``out``
+        (one element per pixel of the last unprojected range) to the next fit / predict.  -> the
+        map's memory kind (None without a map)."""
+        if connectivity not in (4, 8) or isinstance(connectivity, bool):
+            raise ValueError(f"regions must be 4 or 8 (the connectivity), got {connectivity!r}")
+        ptr, mem, cap = None, None, 0
+        if out is not None:
+            cap = self._raster[4] if self._raster is not None else (out.numel() if _is_torch(out) else np.size(out))
+            ptr, mem = _as_out_buffer(out, np.int32, cap, "region_map_out")
+        self._check(self._lib.mdkm_bind_regions(self._h, int(connectivity), c_void_p(ptr) if ptr else None, int(cap),
+                                                C.MEM_HOST if mem is None else mem))
+        if mem == C.MEM_DEVICE:
+            self._after_torch(out)  # earlier work on torch's stream may still use the buffer
+        return mem
+
+    def _region_table(self):
+        """The regions of the last fit / predict that had them -> (table int64 ``[R,7]``, means
+        float64 ``[R,3]``)."""
+        n = c_int64(0)
+        self._check(self._lib.mdkm_region_count(self._h, byref(n)))
+        table = np.empty((n.value, 7), dtype=np.int64)
+        means = np.empty((n.value, 3), dtype=np.float64)
+        self._check(self._lib.mdkm_region_table(self._h, c_void_p(table.ctypes.data), c_void_p(means.ctypes.data),
+                                                int(n.value)))
+        return table, means
+
+    def _bind_outputs(self, k, cluster_map_out, day_stats, transitions, regions=None, region_map_out=None):
         """Bind the optional outputs of the next fit / predict -> (map memory kind, (counts, means),
-        transitions), each None when not asked for.  When one binding is refused none is left
-        behind: the statistics and transition arrays live only in this call, and a binding that
-        outlived them would have the next fit / predict write into freed memory."""
+        transitions, region map memory kind), each None when not asked for.  When one binding is
+        refused none is left behind: the statistics and transition arrays live only in this call,
+        and a binding that outlived them would have the next fit / predict write into freed memory."""
+        if region_map_out is not None and regions is None:
+            raise ValueError("region_map_out needs regions=4 or regions=8")
         try:
             map_mem = self._bind_cluster_map(cluster_map_out) if cluster_map_out is not None else None
             stats = self._bind_day_stats(k) if day_stats else None
             trans = self._bind_day_transitions(transitions, k) if transitions is not None else None
+            reg_mem = self._bind_regions(regions, region_map_out) if regions is not None else None
         except BaseException:
             self._lib.mdkm_bind_cluster_map(self._h, None, 1, 0, C.MEM_HOST)
             self._lib.mdkm_bind_day_stats(self._h, None, None, 0, 0)
             self._lib.mdkm_bind_day_transitions(self._h, None, 0, None, 0)
+            self._lib.mdkm_bind_regions(self._h, 0, None, 0, C.MEM_HOST)
             raise
-        return map_mem, stats, trans
+        return map_mem, stats, trans, reg_mem
 
     @property
     def segment_offsets(self) -> np.ndarray:
@@ -435,7 +466,7 @@ class Engine:
 
     # -- k-means -------------------------------------------------------------------------
     def fit(self, init, max_iter=300, tol=1e-4, want_labels=True, labels_out=None, cluster_map_out=None,
-            day_stats=False, transitions=None):
+            day_stats=False, transitions=None, regions=None, region_map_out=None):
         """One Lloyd run from explicit centroids.  Returns dict(labels, centers, n_iter, inertia, ...).
 
         ``cluster_map_out``: optional uint8 (k <= 255) or uint16 array / tensor, host or CUDA, with
@@ -453,7 +484,17 @@ class Engine:
         day b of pair p, state = label + 1 where the pixel produced a point, 0 where it did not
         (the cluster map's value).  Binned on the GPU from the map the final pass writes; needs a
         cloud from ``unproject`` whose ranks together hold the whole stack, and with several ranks
-        every rank receives the counts of the whole stack."""
+        every rank receives the counts of the whole stack.
+
+        ``regions``: 4 or 8, the connectivity of the connected regions of the cluster map (maximal
+        connected sets of pixels of one day with the same label), numbered 1..R in the raster
+        order (day, y, x) of their first pixel.  The result also has ``regions``, int64 ``[R,7]``
+        rows (day, cluster, pixels, y_min, x_min, y_max, x_max), and ``region_means``, float64
+        ``[R,3]``, the mean (x, y, z) of each region's points in the clustered frame (computed like
+        ``day_means``).  ``region_map_out``: optional int32 array / tensor, host or CUDA, with one
+        element per pixel of the last ``unproject``'s range; it receives the region ids, 0 where a
+        pixel has no point.  Labelled on the GPU after the fit; same cover rule as
+        ``transitions``, and with several ranks every rank receives the whole stack's regions."""
         init = np.ascontiguousarray(init, dtype=np.float64)
         if init.ndim != 2 or init.shape[1] != 3:
             raise ValueError("init must be [K,3]")
@@ -471,12 +512,13 @@ class Engine:
         centers = np.empty((k, 3), dtype=np.float64)
         n_iter = c_int(0)
         inertia = c_double(0.0)
-        map_mem, stats, trans = self._bind_outputs(k, cluster_map_out, day_stats, transitions)
+        map_mem, stats, trans, reg_mem = self._bind_outputs(k, cluster_map_out, day_stats, transitions, regions,
+                                                            region_map_out)
         self._check(self._lib.mdkm_fit(
             self._h, int(k), init.ctypes.data_as(POINTER(c_double)), int(max_iter), float(tol),
             c_void_p(lab_ptr) if lab_ptr else None, lab_mem,
             centers.ctypes.data_as(POINTER(c_double)), byref(n_iter), byref(inertia)))
-        if lab_mem == C.MEM_DEVICE or map_mem == C.MEM_DEVICE:
+        if lab_mem == C.MEM_DEVICE or map_mem == C.MEM_DEVICE or reg_mem == C.MEM_DEVICE:
             self._before_torch()
         nref, nrel, tols = c_int64(0), c_int64(0), c_double(0)
         self._lib.mdkm_fit_stats(self._h, byref(nref), byref(nrel), byref(tols))
@@ -492,6 +534,8 @@ class Engine:
             out["day_counts"], out["day_means"] = stats
         if trans is not None:
             out["transitions"] = trans
+        if regions is not None:
+            out["regions"], out["region_means"] = self._region_table()
         return out
 
     def lloyd_step(self, centroids, want_labels=True):
@@ -510,27 +554,32 @@ class Engine:
         self._lib.mdkm_fit_stats(self._h, byref(nref), None, None)
         return labels, sums, counts, int(nref.value)
 
-    def predict(self, centroids, want_labels=True, cluster_map_out=None, day_stats=False, transitions=None):
+    def predict(self, centroids, want_labels=True, cluster_map_out=None, day_stats=False, transitions=None,
+                regions=None, region_map_out=None):
         """E-step only (KMeans.predict): returns (labels int32[N] or None, inertia).
         ``cluster_map_out``: as in ``fit``.  ``day_stats=True``: returns
         (labels, inertia, day_counts, day_means) instead, as in ``fit``.  ``transitions``: day
-        pairs as in ``fit``; their counts are appended to the returned tuple."""
+        pairs as in ``fit``; their counts are appended to the returned tuple.  ``regions`` /
+        ``region_map_out``: as in ``fit``; the table and the means are appended after that."""
         c = np.ascontiguousarray(centroids, dtype=np.float64)
         if c.ndim != 2 or c.shape[1] != 3:
             raise ValueError("centroids must be [K,3]")
         labels = self._result_buffer("labels", (self.n_points,), np.int32) if want_labels else None
         inertia = c_double(0.0)
-        map_mem, stats, trans = self._bind_outputs(c.shape[0], cluster_map_out, day_stats, transitions)
+        map_mem, stats, trans, reg_mem = self._bind_outputs(c.shape[0], cluster_map_out, day_stats, transitions,
+                                                            regions, region_map_out)
         self._check(self._lib.mdkm_predict(
             self._h, int(c.shape[0]), c.ctypes.data_as(POINTER(c_double)),
             c_void_p(labels.ctypes.data) if labels is not None else None, C.MEM_HOST, byref(inertia)))
-        if map_mem == C.MEM_DEVICE:
+        if map_mem == C.MEM_DEVICE or reg_mem == C.MEM_DEVICE:
             self._before_torch()
         out = (labels, float(inertia.value))
         if stats is not None:
             out += stats
         if trans is not None:
             out += (trans,)
+        if regions is not None:
+            out += self._region_table()
         return out
 
     def kmeans_plusplus(self, n_clusters: int, random_state):

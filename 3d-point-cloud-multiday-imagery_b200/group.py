@@ -90,14 +90,16 @@ class DeviceGroup:
 
     # -- the fused path -------------------------------------------------------------------
     def fuse(self, height_maps, valid_masks=None, *, run_kmeans: Callable, max_abs_height=144.0, detrend=False,
-             disparity_scale=None, ground_level=False, return_cloud=True, raster_layout=None, cluster_map_dtype=None):
+             disparity_scale=None, ground_level=False, return_cloud=True, raster_layout=None, cluster_map_dtype=None,
+             region_map=False):
         """Shard a HOST stack over the devices by row bands (whole days when ``detrend`` or
         ``ground_level`` need them), unproject, cluster, and assemble labels / cloud in the
         reference's point order.  ``run_kmeans(engine, labels_out) -> dict`` is ``api._run_kmeans``
         bound to the k-means arguments; it runs on every rank (the collectives inside pair up).
         ``cluster_map_dtype`` (uint8 / uint16): also build the ``[D,H,W]`` cluster map; every rank
         writes its row band of it in place (``run_kmeans(engine, labels_out, cluster_map_out)``)
-        and it is returned as ``extra["cluster_map"]``.
+        and it is returned as ``extra["cluster_map"]``.  ``region_map``: likewise the int32 ``[D,H,W]``
+        region map (``run_kmeans(..., region_map_out=band)``), returned as ``extra["region_map"]``.
         Returns ``(result dict of rank 0, labels, cloud or None, height_norm or None, extra)``."""
         hm = height_maps
         if type(hm).__module__.startswith("torch"):
@@ -138,16 +140,18 @@ class DeviceGroup:
         labels = np.empty(n_total, dtype=np.int32)
         cloud = np.empty((n_total, 3), dtype=np.float32) if return_cloud else None
         cmap = np.empty(D * H * W, dtype=cluster_map_dtype) if cluster_map_dtype is not None else None
+        rmap = np.empty(D * H * W, dtype=np.int32) if region_map else None
 
         def cluster(r):
             eng = self.engines[r]
             a, b = int(offs[r]), int(offs[r + 1])
             if cloud is not None and b > a:
                 eng.get_cloud(napari_order=True, out=cloud[a:b], wait=False)  # overlaps the Lloyd loop
+            kw = {} if rmap is None else {"region_map_out": rmap[spans[r][0]:spans[r][1]]}
             if cmap is not None:
-                res = run_kmeans(eng, labels[a:b], cmap[spans[r][0]:spans[r][1]])
+                res = run_kmeans(eng, labels[a:b], cmap[spans[r][0]:spans[r][1]], **kw)
             else:
-                res = run_kmeans(eng, labels[a:b])
+                res = run_kmeans(eng, labels[a:b], **kw)
             eng.wait()
             return res
 
@@ -169,6 +173,8 @@ class DeviceGroup:
         extra["segment_offsets"] = np.concatenate([[0], np.cumsum(day_counts)]).astype(np.int64)
         if cmap is not None:
             extra["cluster_map"] = cmap.reshape(D, H, W)
+        if rmap is not None:
+            extra["region_map"] = rmap.reshape(D, H, W)
         return results[0], labels, cloud, hn, extra
 
 

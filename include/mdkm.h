@@ -203,6 +203,47 @@ int mdkm_bind_day_stats(mdkm_handle* h, int64_t* counts_out, double* means_out, 
 int mdkm_bind_day_transitions(mdkm_handle* h, const int32_t* pairs, int n_pairs, int64_t* counts_out,
                               int k_capacity);
 
+/* Optional: have the NEXT mdkm_fit or mdkm_predict on this handle also find the connected regions
+ * of its cluster map.  A region is a maximal set of pixels of one day that all have the same
+ * non-zero map value (label + 1) and are connected: connectivity 4 (edge neighbours) or 8 (edge
+ * and corner neighbours).  Pixels without a point belong to no region; regions never span days.
+ * Regions are numbered 1..R over the whole stack in the raster order (day, y, x) of each region's
+ * first pixel, which does not depend on the schedule or the number of ranks.
+ * map_out (optional, int32, host or device memory per mem, room for capacity_pixels >= the
+ * pix_count of the last mdkm_unproject) receives the region map of that pixel range: the region
+ * id of every pixel that produced a point, 0 elsewhere.
+ * After the call, mdkm_region_count gives R and mdkm_region_table copies the table, int64
+ * [R][7] rows (day, cluster (0-based label), pixels (= its point count), y_min, x_min, y_max,
+ * x_max; inclusive bounds in pixel coordinates of the day), and the means, float64 [R][3], the
+ * mean (x, y, z) of the region's points in the frame that was clustered -- computed as the means
+ * of mdkm_bind_day_stats (int64 sums of fixed-point coordinates of the handle's frame, (sum_q /
+ * scale + count * origin) / count), with every coordinate rounded to its nearest grid point in
+ * FP64: bitwise the same on any number of ranks, within half a grid step of the exact mean even
+ * for a region of one point, exact on the grid.  The
+ * pixels of the regions of (day d, cluster j) add up to that day's count of cluster j.
+ * Where the numbers come from: after the call's synchronisation, when the map is final, a
+ * block-based union-find labels the whole-stack map on the device (tile-local union-find in
+ * shared memory, links across tile borders with atomicMin, ids by a scan of the roots); one more
+ * synchronisation reads R; a pass over the resident points sums each region's count, coordinates
+ * and bounds; with several ranks every rank labels the whole stack (the map is merged as for day
+ * transitions) and the sums are all-reduced.  Asking for regions changes no other result.
+ * connectivity == 0 with map_out == NULL clears the binding.  The binding is consumed by that one
+ * call, and dropped by mdkm_unproject / mdkm_set_points.  Errors: MDKM_ERR_STATE when the resident
+ * cloud did not come from mdkm_unproject; MDKM_ERR_INVALID for a connectivity other than 4 or 8,
+ * a stack of 2^31 pixels or more, H or W of 2^23 or more, a capacity below pix_count or a bad
+ * mem; from the mdkm_fit / mdkm_predict, before any work is enqueued, MDKM_ERR_STATE on every
+ * rank when the ranks' pixel ranges do not cover the whole stack (as for day transitions). */
+int mdkm_bind_regions(mdkm_handle* h, int connectivity, int32_t* map_out, int64_t capacity_pixels, int mem);
+
+/* The regions of the last mdkm_fit / mdkm_predict that had them bound, kept on the device until
+ * the next mdkm_unproject / mdkm_set_points or fit / predict with regions.  mdkm_region_count:
+ * their number R.  mdkm_region_table: copies the table (table_out, int64 [R][7]) and the means
+ * (means_out, float64 [R][3]) to host memory; either may be NULL.  Errors: MDKM_ERR_STATE when
+ * there are no regions (none computed since the last unproject / set_points);
+ * MDKM_ERR_INVALID from mdkm_region_table when capacity_regions < R. */
+int mdkm_region_count(const mdkm_handle* h, int64_t* n_regions);
+int mdkm_region_table(mdkm_handle* h, int64_t* table_out, double* means_out, int64_t capacity_regions);
+
 /* Load an already unprojected cloud (this rank's shard).  Replaces the `X` argument of the
  * reference's KMeans(...).fit_predict(X) call (members/jasraj/land_use_classification/
  * core.py:227-228) for d = 3. */
