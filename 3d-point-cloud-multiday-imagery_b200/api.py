@@ -30,6 +30,7 @@ LayerType = Literal["image", "labels", "points", "shapes"]
 Layer = Tuple[np.ndarray, Dict[str, Any], LayerType]  # interface.py:5-7
 
 MAX_ABS_HEIGHT = 144.0  # MAX_DISP / 2 (constants.py:54, plugin.py:151)
+MAX_REGION_OVERLAP_PAIRS = 8192  # day pairs of one call's region overlaps (mdkm_bind_region_overlaps)
 
 
 @dataclass
@@ -67,6 +68,12 @@ class FusionResult:
     regions: Optional[np.ndarray] = None
     region_means: Optional[np.ndarray] = None
     region_map: Optional[np.ndarray] = None
+    # region overlaps of day pairs (return_region_overlaps): one row per pair of regions (r of day a,
+    # s of day b) with a shared pixel -- int64 [M,6] (pair, region_a, region_b, pixels, y_first,
+    # x_first), sorted by pair, then by the first shared pixel -- and the pairs, int64 [P,2]; over
+    # the whole stack on every rank
+    region_overlaps: Optional[np.ndarray] = None
+    region_overlap_pairs: Optional[np.ndarray] = None
 
     # scikit-learn style aliases
     @property
@@ -140,14 +147,16 @@ def cluster_map_dtype(n_clusters: int):
     return np.uint8 if int(n_clusters) <= 255 else np.uint16
 
 
-def transition_pairs(spec, n_days: int) -> np.ndarray:
+def transition_pairs(spec, n_days: int, what: str = "transitions") -> np.ndarray:
     """The day pairs ``return_transitions`` asks for, as int64 ``[P,2]``: ``True`` -> the
     consecutive pairs ``(d, d+1)``; a sequence of ``(a, b)`` -> those pairs in that order (they
     may skip days, run backwards, repeat, or have ``a == b``).  Raises ``ValueError`` for a day
-    outside ``[0, n_days)`` or when there is no pair."""
+    outside ``[0, n_days)`` or when there is no pair.  ``what``: the output the pairs are for, as
+    the messages name it ("region overlaps" for ``return_region_overlaps``)."""
+    arg = "return_" + what.replace(" ", "_")
     if isinstance(spec, (bool, np.bool_)):
         if not spec:
-            raise ValueError("return_transitions=False asks for no pairs")
+            raise ValueError(f"{arg}=False asks for no pairs")
         d = np.arange(max(int(n_days) - 1, 0), dtype=np.int64)
         pairs = np.stack([d, d + 1], axis=1)
     else:
@@ -155,15 +164,20 @@ def transition_pairs(spec, n_days: int) -> np.ndarray:
         if pairs.size == 0:
             pairs = pairs.reshape(0, 2)
         if pairs.ndim != 2 or pairs.shape[1] != 2 or not (np.issubdtype(pairs.dtype, np.integer)):
-            raise ValueError("return_transitions must be True or a sequence of (day_a, day_b) integer pairs")
+            raise ValueError(f"{arg} must be True or a sequence of (day_a, day_b) integer pairs")
         pairs = pairs.astype(np.int64)
     if pairs.shape[0] == 0:
-        raise ValueError(f"no day pair to count transitions of (the stack has {n_days} day(s))")
+        raise ValueError(f"no day pair to count {what} of (the stack has {n_days} day(s))")
     bad = (pairs < 0) | (pairs >= n_days)
     if bad.any():
         p = int(np.argmax(bad.any(axis=1)))
-        raise ValueError(f"transition pair {p} = {tuple(int(v) for v in pairs[p])}: days must be in [0, {n_days})")
+        raise ValueError(f"{what[:-1]} pair {p} = {tuple(int(v) for v in pairs[p])}: days must be in [0, {n_days})")
     return pairs
+
+
+def _asks_for_pairs(spec) -> bool:
+    """Does a ``return_transitions`` / ``return_region_overlaps`` value ask for pairs (not None / False)?"""
+    return spec is not None and not (isinstance(spec, (bool, np.bool_)) and not spec)
 
 
 def requested_connectivity(return_regions, connectivity=4, return_region_map=False):
@@ -189,7 +203,7 @@ def _stack_days(height_maps, stack_shape, raster_layout) -> int:
 
 def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_state, want_labels=True,
                 labels_out=None, gather_mappings=None, cluster_map_out=None, day_stats=False, transitions=None,
-                regions=None, region_map_out=None):
+                regions=None, region_map_out=None, region_overlaps=None):
     """KMeans.fit driver (sklearn/_kmeans.py:1436-1563): init, n_init restarts, best inertia.
 
     ``labels_out``: optional int32 array that receives this rank's labels of the best run.
@@ -202,6 +216,8 @@ def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_
     best run's, as with ``day_stats``.
     ``regions`` (4 / 8) and ``region_map_out`` (int32): the result also has ``regions`` /
     ``region_means``, the best run's as with ``day_stats``; the region map as ``cluster_map_out``.
+    ``region_overlaps``: day pairs ``[P,2]`` (needs ``regions``); the result also has
+    ``region_overlaps`` (``Engine.fit``), the best run's, as with ``day_stats``.
     ``gather_mappings``: with a multi-rank engine, the collective that lets the ranks agree on
     sklearn's "same clustering up to a permutation" test (see ``_is_same_clustering``); when it is
     missing the test is skipped on multi-rank engines (the inertia comparison alone decides)."""
@@ -252,7 +268,7 @@ def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_
                     labels_out=labels_out if (single and want_labels) else None,
                     cluster_map_out=cluster_map_out if single else run_map, day_stats=day_stats,
                     transitions=transitions, regions=regions,
-                    region_map_out=region_map_out if single else run_rmap)
+                    region_map_out=region_map_out if single else run_rmap, region_overlaps=region_overlaps)
         # sklearn/_kmeans.py:1534-1541: a run replaces the best one when its inertia is lower AND it
         # is not the same clustering up to a permutation.  The inertia is global, so every rank
         # takes the same branch and the (collective) permutation test pairs up.
@@ -299,7 +315,8 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
                          device=0, devices=None, engine=None, stack_shape=None,
                          pix_begin=0, raster_layout=None, return_cluster_map=False,
                          return_day_stats=False, return_transitions=False, return_regions=False,
-                         region_connectivity=4, return_region_map=False) -> FusionResult:
+                         region_connectivity=4, return_region_map=False,
+                         return_region_overlaps=False) -> FusionResult:
     """Unproject a multi-day height-map stack into one XYZ cloud and cluster it (Lloyd).
 
     height_maps : float32 ``[D,H,W]`` (NaN = nodata), numpy or torch (CPU or CUDA); or int16
@@ -355,14 +372,30 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
         produced a point and 0 elsewhere; ``[D,H,W]``, or this rank's flat slice for a pre-sharded
         call, like ``cluster_map``.  Implies ``return_regions``.  A connectivity other than 4 or 8
         raises ``ValueError`` before any GPU work.
+    return_region_overlaps : ``True`` (the consecutive pairs ``(d, d+1)``) or a sequence of day
+        pairs ``(a, b)``, as for ``return_transitions``: also return ``region_overlaps``, int64
+        ``[M,6]`` rows (pair, region_a, region_b, pixels, y_first, x_first) -- one for every pair
+        of regions (r of day a, s of day b) that share at least one pixel, with the number of
+        shared pixels and the first shared pixel, sorted by pair and then by the raster order of
+        that pixel -- and ``region_overlap_pairs`` (int64 ``[P,2]``).  Region ids are those of
+        ``regions``; r and s may have different clusters.  Implies ``return_regions``.  Counted on
+        the GPU from the region map; every rank of a pre-sharded call receives the same rows.
+        Out-of-range days, or more than ``MAX_REGION_OVERLAP_PAIRS``
+        (8192) pairs, raise ``ValueError`` before any GPU work.
     Returns a FusionResult; ``fused_cloud`` is float32 ``[N,3]`` in napari (z,y,x) order.
     """
     from .group import DeviceGroup
 
-    pairs = None
-    if return_transitions is not None and not (isinstance(return_transitions, (bool, np.bool_)) and not return_transitions):
+    pairs = ov_pairs = None
+    if _asks_for_pairs(return_transitions):
         pairs = transition_pairs(return_transitions, _stack_days(height_maps, stack_shape, raster_layout))
-    conn = requested_connectivity(return_regions, region_connectivity, return_region_map)
+    if _asks_for_pairs(return_region_overlaps):
+        ov_pairs = transition_pairs(return_region_overlaps, _stack_days(height_maps, stack_shape, raster_layout),
+                                    "region overlaps")
+        if ov_pairs.shape[0] > MAX_REGION_OVERLAP_PAIRS:
+            raise ValueError(f"return_region_overlaps asks for {ov_pairs.shape[0]} pairs, at most "
+                             f"{MAX_REGION_OVERLAP_PAIRS} are allowed")
+    conn = requested_connectivity(return_regions or ov_pairs is not None, region_connectivity, return_region_map)
     if devices is not None or isinstance(engine, DeviceGroup):
         if stack_shape is not None or pix_begin:
             raise ValueError("stack_shape / pix_begin describe a pre-sharded stack; a device group shards by itself")
@@ -372,7 +405,7 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
                               disparity_scale=disparity_scale, ground_level=ground_level, return_cloud=return_cloud,
                               raster_layout=raster_layout, return_cluster_map=return_cluster_map,
                               return_day_stats=return_day_stats, transitions=pairs, regions=conn,
-                              return_region_map=return_region_map)
+                              return_region_map=return_region_map, region_overlaps=ov_pairs)
     own = engine is None
     eng = engine or Engine(device)
     try:
@@ -403,7 +436,7 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
             rmap = np.empty((D, H, W) if stack_shape is None else (count,), dtype=np.int32)
         r = _run_kmeans(eng, n_clusters=n_clusters, init=init, n_init=n_init, max_iter=max_iter,
                         tol=tol, random_state=random_state, cluster_map_out=cmap, day_stats=return_day_stats,
-                        transitions=pairs, regions=conn, region_map_out=rmap)
+                        transitions=pairs, regions=conn, region_map_out=rmap, region_overlaps=ov_pairs)
         eng.wait()
         return FusionResult(labels=r["labels"], centroids=r["centers"], fused_cloud=cloud,
                             n_iter=r["n_iter"], inertia=r["inertia"], n_points=n,
@@ -411,7 +444,8 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
                             height_norm=hn, extra=extra, cluster_map=cmap,
                             day_counts=r.get("day_counts"), day_means=r.get("day_means"),
                             transitions=r.get("transitions"), transition_pairs=pairs,
-                            regions=r.get("regions"), region_means=r.get("region_means"), region_map=rmap)
+                            regions=r.get("regions"), region_means=r.get("region_means"), region_map=rmap,
+                            region_overlaps=r.get("region_overlaps"), region_overlap_pairs=ov_pairs)
     finally:
         if own:
             eng.close()
@@ -419,7 +453,7 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
 
 def _fuse_on_group(height_maps, valid_masks, *, group, devices, n_clusters, init, n_init, max_iter, tol,
                    random_state, return_cluster_map=False, return_day_stats=False, transitions=None,
-                   regions=None, return_region_map=False, **unproject_kw) -> FusionResult:
+                   regions=None, return_region_map=False, region_overlaps=None, **unproject_kw) -> FusionResult:
     """``fuse_multiday_kmeans`` on several devices of this process (``group.DeviceGroup``)."""
     import threading
 
@@ -450,7 +484,7 @@ def _fuse_on_group(height_maps, valid_masks, *, group, devices, n_clusters, init
                                random_state=states[r], labels_out=labels_out,
                                gather_mappings=gather_for(r) if grp.world > 1 else None,
                                cluster_map_out=cluster_map_out, day_stats=return_day_stats, transitions=transitions,
-                               regions=regions, region_map_out=region_map_out)
+                               regions=regions, region_map_out=region_map_out, region_overlaps=region_overlaps)
 
         res, labels, cloud, hn, extra = grp.fuse(
             height_maps, valid_masks, run_kmeans=run,
@@ -463,7 +497,8 @@ def _fuse_on_group(height_maps, valid_masks, *, group, devices, n_clusters, init
                             day_counts=res.get("day_counts"), day_means=res.get("day_means"),
                             transitions=res.get("transitions"), transition_pairs=transitions,
                             regions=res.get("regions"), region_means=res.get("region_means"),
-                            region_map=extra.pop("region_map", None))
+                            region_map=extra.pop("region_map", None),
+                            region_overlaps=res.get("region_overlaps"), region_overlap_pairs=region_overlaps)
     finally:
         if own:
             grp.close()

@@ -22,6 +22,7 @@
 #include "lloyd.cuh"
 #include "mirror.cuh"
 #include "nccl_shim.h"
+#include "region_overlaps.cuh"
 #include "regions.cuh"
 #include "seeding.cuh"
 #include "transitions.cuh"
@@ -33,6 +34,7 @@ namespace {
 
 constexpr int kBatch = 10;                          // Lloyd iterations enqueued between status polls
 constexpr size_t kMappedBytes = 256 << 10;          // device-visible host buffer for small results
+constexpr int kMaxOvPairs = 8192;                   // day pairs of region overlaps (their bounds: one small copy)
 
 // copies `bytes` (a multiple of 4) from device memory into device-visible host memory
 __global__ void publish_kernel(void* dst_host, const void* src, int bytes) {
@@ -195,6 +197,16 @@ struct mdkm_handle {
   DevBuf<unsigned int> region_box;         // [R][5] first pixel, y_min, x_min, ~y_max, ~x_max
   DevBuf<unsigned char> region_out;        // table int64 [R][7], then means float64 [R][3]
   long long n_regions = -1;              // R of the last fit / predict with regions; -1: none
+  // region overlaps between days (mdkm_bind_region_overlaps) of the next fit / predict, and those
+  // of the last fit / predict that had them, with the lifecycle of the regions
+  std::vector<int> bound_ov_pairs;       // [n_pairs][2] days, copied when bound; empty: not bound
+  DevBuf<int> ov_pairs;
+  DevBuf<long long> ov_tab;              // [n_pairs + 1] slot offsets of the pairs' hash tables
+  DevBuf<unsigned long long> ov_slots;   // [slots][2] key, count | ~first << 32
+  DevBuf<unsigned int> ov_bits;          // first-pixel masks, then word offsets within the scan chunks
+  DevBuf<unsigned long long> ov_scan;    // look-back words, chunk offsets, ticket + fault, M, probe fault
+  DevBuf<long long> ov_rows;             // int64 [M][6]
+  long long n_overlaps = -1;             // M of the last fit / predict with overlaps; -1: none
 
   // communicator
   ncclComm_t comm = nullptr;
@@ -978,6 +990,14 @@ struct RegOut {
   int mem = MDKM_MEM_HOST;
 };
 
+// Region overlaps taken by one fit / predict (mdkm_bind_region_overlaps): counted from the
+// whole-stack region map that run_regions resolves; the rows stay on the device, where
+// mdkm_region_overlap_table finds them.
+struct OvOut {
+  std::vector<int> pairs;  // [n_pairs][2] days; empty: not asked for
+  int n_pairs() const { return (int)(pairs.size() / 2); }
+};
+
 // page-locked host buffer of at least `bytes` (the stages of results handed over after a sync)
 int ensure_pinned(mdkm_handle* h, unsigned char*& p, size_t& cap, size_t bytes) {
   if (cap >= bytes && p) return MDKM_OK;
@@ -1135,7 +1155,7 @@ RegOut consume_regions(mdkm_handle* h) {
 }
 
 // Takes the regions `g` (consumed) for a call with k clusters and its cluster map `m`: sets up the
-// whole-stack map; the regions of an earlier call are dropped.
+// whole-stack map; the regions (and region overlaps) of an earlier call are dropped.
 int take_regions(mdkm_handle* h, int k, MapOut& m, RegOut& g) {
   if (!g.conn) return MDKM_OK;
   if (k < 1 || k > kMaxK) {  // (rejected with the call's own message)
@@ -1143,7 +1163,27 @@ int take_regions(mdkm_handle* h, int k, MapOut& m, RegOut& g) {
     return MDKM_OK;
   }
   h->n_regions = -1;
+  h->n_overlaps = -1;
   return take_stack_map(h, k, m);
+}
+
+// Consumes the binding of mdkm_bind_region_overlaps (whatever happens next).
+OvOut consume_overlaps(mdkm_handle* h) {
+  OvOut o;
+  o.pairs.swap(h->bound_ov_pairs);
+  h->bound_ov_pairs.clear();
+  return o;
+}
+
+// Takes the region overlaps `o` (consumed) of a call whose regions are `g` (before take_regions):
+// they need the regions of the same call; uploads the pairs.
+int take_overlaps(mdkm_handle* h, const RegOut& g, const OvOut& o) {
+  if (o.pairs.empty()) return MDKM_OK;
+  if (!g.conn) return fail(h, MDKM_ERR_STATE, "region overlaps need regions bound for the same call (mdkm_bind_regions)");
+  CU(cudaSetDevice(h->device));
+  OK(ensure(h, h->ov_pairs, o.pairs.size()));
+  CU(cudaMemcpyAsync(h->ov_pairs.p, o.pairs.data(), o.pairs.size() * 4, cudaMemcpyHostToDevice, h->stream));
+  return MDKM_OK;
 }
 
 typedef void (*TransKernel)(const TransParams);
@@ -1237,21 +1277,44 @@ void deliver_day_stats(mdkm_handle* h, const StatsOut& s) {
   memcpy(s.means, h->stats_host + (size_t)s.slots * 8, (size_t)s.slots * 24);
 }
 
+int run_overlaps(mdkm_handle* h, const OvOut& o, const int* ids, const unsigned long long* bounds);
+
+// The pair-independent part of the overlap kernels' parameters.
+OverlapParams overlap_params(mdkm_handle* h, const int* ids, int n_pairs) {
+  OverlapParams op{};
+  op.ids = ids;
+  op.HW = (long long)h->raster_H * h->raster_w;
+  op.W = h->raster_w;
+  op.pairs = h->ov_pairs.p;
+  op.n_pairs = n_pairs;
+  op.wpp = (op.HW + 31) / 32;
+  return op;
+}
+
+// grid of the overlap passes that give a warp kOvSpan pixels of every pair (pairs along y)
+dim3 overlap_span_grid(long long HW, int n_pairs) {
+  const long long warps = (HW + kOvSpan - 1) / kOvSpan;
+  return dim3((unsigned int)((warps + kThreads / 32 - 1) / (kThreads / 32)), (unsigned int)std::min(n_pairs, 65535));
+}
+
 // The regions `g` of the whole-stack map `m`, after the call's synchronisation (the map is final,
 // also after a relocation).  Every rank labels the whole stack: tile-local union-find, links
 // across the tile borders, ids of the roots, every pixel's id (regions.cuh); the caller's region
-// map receives this rank's range.  One synchronisation reads R, then this rank's points are
+// map receives this rank's range.  One synchronisation reads R -- and, with region overlaps `o`,
+// the bounds of their pairs, counted right behind the ids -- then this rank's points are
 // summed into per-region slots, the slots are reduced over the ranks (sums; minima of the
 // first pixel and the bounds) and the table and means are written on the device, where
-// mdkm_region_table finds them.
-int run_regions(mdkm_handle* h, const RegOut& g, const MapOut& m) {
+// mdkm_region_table finds them.  The overlaps follow (run_overlaps).
+int run_regions(mdkm_handle* h, const RegOut& g, const MapOut& m, const OvOut& o) {
   if (!g.conn) return MDKM_OK;
   const long long HW = (long long)h->raster_H * h->raster_w, n_px = (long long)h->stack_days * HW;
   const bool in_place = g.map && g.mem == MDKM_MEM_DEVICE && h->n_ranks == 1;  // (one rank holds the whole stack)
   OK(ensure(h, h->region_parent, (size_t)n_px));
   if (!in_place) OK(ensure(h, h->region_ids, (size_t)n_px));
   const long long n_chunks = (n_px + kRegChunk - 1) / kRegChunk;
-  OK(ensure(h, h->region_scan, (size_t)n_chunks + 2));
+  const int n_pairs = o.n_pairs();
+  // look-back words of the numbering, ticket + fault, R, then the overlap bounds of the pairs
+  OK(ensure(h, h->region_scan, (size_t)n_chunks + 2 + n_pairs));
   RegionParams rp{};
   rp.map = m.whole;
   rp.parent = h->region_parent.p;
@@ -1273,17 +1336,23 @@ int run_regions(mdkm_handle* h, const RegOut& g, const MapOut& m) {
                         : (c8 ? region_border_kernel<unsigned char, true> : region_border_kernel<unsigned char, false>);
   tile_fn<<<(unsigned int)rp.n_tiles, kThreads, 0, h->stream>>>(rp);
   border_fn<<<(unsigned int)((rp.n_tiles + kThreads / 32 - 1) / (kThreads / 32)), kThreads, 0, h->stream>>>(rp);
-  CU(cudaMemsetAsync(h->region_scan.p, 0, ((size_t)n_chunks + 2) * 8, h->stream));
+  CU(cudaMemsetAsync(h->region_scan.p, 0, ((size_t)n_chunks + 2 + n_pairs) * 8, h->stream));
   region_number_kernel<<<(unsigned int)n_chunks, kThreads, 0, h->stream>>>(rp);
   region_resolve_kernel<<<grid_for(h, (n_px + 1023) / 1024, resident_per_sm(h, region_resolve_kernel)), kThreads, 0,
                           h->stream>>>(rp);
   h->launches += 4;
+  if (n_pairs) {
+    OverlapParams op = overlap_params(h, rp.ids, n_pairs);
+    op.bounds = h->region_scan.p + n_chunks + 2;
+    overlap_bound_kernel<<<overlap_span_grid(HW, n_pairs), kThreads, 0, h->stream>>>(op);
+    ++h->launches;
+  }
   CU(cudaGetLastError());
   if (g.map && !in_place)
     CU(cudaMemcpyAsync(g.map, rp.ids + h->raster_pix_begin, (size_t)h->raster_pix_count * 4,
                        g.mem == MDKM_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, h->stream));
-  unsigned long long got[2] = {0, 0};  // ticket | fault << 32, R
-  OK(small_d2h(h, got, h->region_scan.p + n_chunks, 16));
+  std::vector<unsigned long long> got(2 + (size_t)n_pairs, 0ull);  // ticket | fault << 32, R, the overlap bounds
+  OK(small_d2h(h, got.data(), h->region_scan.p + n_chunks, got.size() * 8));
   OK(sync_small(h));
   if (got[0] >> 32) return fail(h, MDKM_ERR_CUDA, "region numbering: the look-back over the chunks timed out");
   const long long R = (long long)got[1];
@@ -1324,6 +1393,68 @@ int run_regions(mdkm_handle* h, const RegOut& g, const MapOut& m) {
     CU(cudaGetLastError());
   }
   h->n_regions = R;
+  return run_overlaps(h, o, rp.ids, got.data() + 2);
+}
+
+// The region overlaps `o` of the region map `ids` (the whole stack, on every rank), behind the
+// region table on the stream, given the bounds of the pairs (region_overlaps.cuh): one hash table
+// per pair sized from its bound, the keys inserted, their first pixels marked, the masks scanned;
+// one synchronisation reads M, then the rows are written on the device, where
+// mdkm_region_overlap_table finds them.  Every rank builds the whole table on its own.
+int run_overlaps(mdkm_handle* h, const OvOut& o, const int* ids, const unsigned long long* bounds) {
+  const int n_pairs = o.n_pairs();
+  if (!n_pairs) return MDKM_OK;
+  std::vector<long long> tab((size_t)n_pairs + 1, 0);
+  long long max_cap = 0;
+  for (int q = 0; q < n_pairs; ++q) {
+    long long cap = 0;
+    if (bounds[q]) for (cap = 2; cap < 2 * (long long)bounds[q]; cap <<= 1) {}
+    tab[q + 1] = tab[q] + cap;
+    max_cap = std::max(max_cap, cap);
+  }
+  if (tab[n_pairs] == 0) {  // no pixel has ids on both days of any pair
+    h->n_overlaps = 0;
+    return MDKM_OK;
+  }
+  OverlapParams op = overlap_params(h, ids, n_pairs);
+  const long long n_words = (long long)n_pairs * op.wpp;
+  const long long n_chunks = (n_words + kOvChunkWords - 1) / kOvChunkWords, padded = n_chunks * kOvChunkWords;
+  OK(ensure(h, h->ov_tab, tab.size()));
+  OK(ensure(h, h->ov_slots, 2 * (size_t)tab[n_pairs]));
+  OK(ensure(h, h->ov_bits, 2 * (size_t)padded));
+  OK(ensure(h, h->ov_scan, 2 * (size_t)n_chunks + 3));
+  CU(cudaMemcpyAsync(h->ov_tab.p, tab.data(), tab.size() * 8, cudaMemcpyHostToDevice, h->stream));
+  CU(cudaMemsetAsync(h->ov_slots.p, 0, (size_t)tab[n_pairs] * 16, h->stream));
+  CU(cudaMemsetAsync(h->ov_bits.p, 0, (size_t)padded * 4, h->stream));
+  CU(cudaMemsetAsync(h->ov_scan.p, 0, (2 * (size_t)n_chunks + 3) * 8, h->stream));
+  op.tab = h->ov_tab.p;
+  op.slots = h->ov_slots.p;
+  op.bits = h->ov_bits.p;
+  op.word_rel = h->ov_bits.p + padded;
+  op.status = h->ov_scan.p;
+  op.chunk_base = h->ov_scan.p + n_chunks;
+  op.ticket = reinterpret_cast<unsigned int*>(h->ov_scan.p + 2 * n_chunks);
+  op.total = h->ov_scan.p + 2 * n_chunks + 1;
+  op.probe_fault = reinterpret_cast<unsigned int*>(h->ov_scan.p + 2 * n_chunks + 2);
+  const dim3 slot_grid((unsigned int)grid_for(h, (max_cap + kThreads - 1) / kThreads, 4),
+                       (unsigned int)std::min(n_pairs, 65535));
+  overlap_insert_kernel<<<overlap_span_grid(op.HW, n_pairs), kThreads, 0, h->stream>>>(op);
+  overlap_mark_kernel<<<slot_grid, kThreads, 0, h->stream>>>(op);
+  overlap_scan_kernel<<<(unsigned int)n_chunks, kThreads, 0, h->stream>>>(op, n_chunks);
+  h->launches += 3;
+  CU(cudaGetLastError());
+  unsigned long long got[3] = {0, 0, 0};  // ticket | fault << 32, M, probe fault
+  OK(small_d2h(h, got, op.ticket, 24));
+  OK(sync_small(h));
+  if (got[0] >> 32) return fail(h, MDKM_ERR_CUDA, "region overlaps: the look-back over the chunks timed out");
+  if (got[2]) return fail(h, MDKM_ERR_CUDA, "region overlaps: a hash table had no free slot");
+  const long long M = (long long)got[1];
+  OK(ensure(h, h->ov_rows, (size_t)M * 6));
+  op.rows = h->ov_rows.p;
+  overlap_emit_kernel<<<slot_grid, kThreads, 0, h->stream>>>(op);
+  ++h->launches;
+  CU(cudaGetLastError());
+  h->n_overlaps = M;
   return MDKM_OK;
 }
 
@@ -1511,6 +1642,8 @@ void mdkm_destroy(mdkm_handle* h) {
   if (h->trans_host) cudaFreeHost(h->trans_host);
   release(h->region_parent); release(h->region_ids); release(h->region_scan); release(h->region_acc);
   release(h->region_box); release(h->region_out);
+  release(h->ov_pairs); release(h->ov_tab); release(h->ov_slots); release(h->ov_bits); release(h->ov_scan);
+  release(h->ov_rows);
   release(h->kpp_closest); release(h->kpp_cell); release(h->kpp_blk); release(h->kpp_prefix);
   release(h->kpp_partials); release(h->kpp_rand); release(h->kpp_state);
   if (h->d_status) cudaFree(h->d_status);
@@ -1719,6 +1852,8 @@ int mdkm_set_points(mdkm_handle* h, const float* xyz, int64_t n, int layout, int
   h->bound_regions = 0;
   h->bound_region_map = nullptr;
   h->n_regions = -1;
+  h->bound_ov_pairs.clear();
+  h->n_overlaps = -1;
   h->stack_days = 1;
   h->day0 = 0;
   h->runs_ok = false;
@@ -1850,6 +1985,43 @@ int mdkm_region_table(mdkm_handle* h, int64_t* table_out, double* means_out, int
   return MDKM_OK;
 }
 
+int mdkm_bind_region_overlaps(mdkm_handle* h, const int32_t* pairs, int n_pairs) {
+  if (!h) return MDKM_ERR_INVALID;
+  h->bound_ov_pairs.clear();
+  if (!pairs) return MDKM_OK;
+  if (!h->have_points || h->raster_w <= 0)
+    return fail(h, MDKM_ERR_STATE, "region overlaps need a resident cloud from mdkm_unproject");
+  if (n_pairs < 1 || n_pairs > kMaxOvPairs)
+    return fail(h, MDKM_ERR_INVALID, "region overlaps need 1 <= n_pairs <= %d, got %d", kMaxOvPairs, n_pairs);
+  for (int i = 0; i < 2 * n_pairs; ++i)
+    if (pairs[i] < 0 || pairs[i] >= h->stack_days)
+      return fail(h, MDKM_ERR_INVALID, "region overlap pair %d: day %d is not in [0, %d)", i / 2, (int)pairs[i],
+                  h->stack_days);
+  h->bound_ov_pairs.assign(pairs, pairs + 2 * (size_t)n_pairs);
+  return MDKM_OK;
+}
+
+int mdkm_region_overlap_count(const mdkm_handle* h, int64_t* n_rows) {
+  if (!h || !n_rows) return MDKM_ERR_INVALID;
+  if (h->n_overlaps < 0)
+    return fail(const_cast<mdkm_handle*>(h), MDKM_ERR_STATE, "no region overlaps: no fit / predict with region overlaps since the last unproject / set_points or fit / predict with regions");
+  *n_rows = h->n_overlaps;
+  return MDKM_OK;
+}
+
+int mdkm_region_overlap_table(mdkm_handle* h, int64_t* table_out, int64_t capacity_rows) {
+  if (!h) return MDKM_ERR_INVALID;
+  if (h->n_overlaps < 0)
+    return fail(h, MDKM_ERR_STATE, "no region overlaps: no fit / predict with region overlaps since the last unproject / set_points or fit / predict with regions");
+  const long long M = h->n_overlaps;
+  if (capacity_rows < M) return fail(h, MDKM_ERR_INVALID, "region overlap table: capacity %lld < %lld rows", (long long)capacity_rows, M);
+  if (M == 0 || !table_out) return MDKM_OK;
+  CU(cudaSetDevice(h->device));
+  CU(cudaMemcpyAsync(table_out, h->ov_rows.p, (size_t)M * 48, cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
+  return MDKM_OK;
+}
+
 int mdkm_bind_day_stats(mdkm_handle* h, int64_t* counts_out, double* means_out, int n_days, int k_capacity) {
   if (!h) return MDKM_ERR_INVALID;
   h->bound_counts = nullptr;
@@ -1887,6 +2059,8 @@ int mdkm_unproject(mdkm_handle* h, const void* hm, int hm_dtype, float hm_scale,
   h->bound_regions = 0;  // (and regions the stack)
   h->bound_region_map = nullptr;
   h->n_regions = -1;
+  h->bound_ov_pairs.clear();
+  h->n_overlaps = -1;
   if (D < 0 || H <= 0 || W <= 0 || pix_begin < 0 || pix_count < 0 ||
       pix_begin + pix_count > (int64_t)D * H * W || (pix_count > 0 && !hm))
     return fail(h, MDKM_ERR_INVALID, "bad stack geometry");
@@ -2173,10 +2347,12 @@ int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol
   int64_t* trans_out = h->bound_trans;
   h->bound_trans = nullptr;
   RegOut reg = consume_regions(h);
+  OvOut ov = consume_overlaps(h);
   const int map_rc = take_cluster_map(h, k, map);
   OK(take_day_stats(h, k, stats));
   OK(map_rc);
   OK(take_transitions(h, k, trans_out, map, trans));
+  OK(take_overlaps(h, reg, ov));
   OK(take_regions(h, k, map, reg));
   if (!init) return fail(h, MDKM_ERR_INVALID, "init centroids required");
   OK(check_centroids(h, k, init, "init"));
@@ -2338,7 +2514,7 @@ int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol
 #endif
   if (fin.xchg_timeout == 2) return index_fault(h);
   if (fin.xchg_timeout) return fail(h, MDKM_ERR_NCCL, "a kernel-side wait timed out (peer exchange of the partial sums: a rank is missing; or the grid barrier)");
-  OK(run_regions(h, reg, map));
+  OK(run_regions(h, reg, map, ov));
   deliver_day_stats(h, stats);
   deliver_transitions(h, trans);
   if (n_iter_out) *n_iter_out = fin.iter;
@@ -2419,10 +2595,12 @@ int mdkm_predict(mdkm_handle* h, int k, const double* centroids, int32_t* labels
   int64_t* trans_out = h->bound_trans;
   h->bound_trans = nullptr;
   RegOut reg = consume_regions(h);
+  OvOut ov = consume_overlaps(h);
   const int map_rc = take_cluster_map(h, k, map);
   OK(take_day_stats(h, k, stats));
   OK(map_rc);
   OK(take_transitions(h, k, trans_out, map, trans));
+  OK(take_overlaps(h, reg, ov));
   OK(take_regions(h, k, map, reg));
   if (!centroids) return fail(h, MDKM_ERR_INVALID, "centroids required");
   OK(check_centroids(h, k, centroids, "centroids"));
@@ -2454,7 +2632,7 @@ int mdkm_predict(mdkm_handle* h, int k, const double* centroids, int32_t* labels
   OK(copy_cluster_map(h, map));
   OK(sync_small(h));
   if (h->h_status[0].xchg_timeout == 2) return index_fault(h);
-  OK(run_regions(h, reg, map));
+  OK(run_regions(h, reg, map, ov));
   deliver_day_stats(h, stats);
   deliver_transitions(h, trans);
   if (inertia_out) *inertia_out = h->h_status[0].inertia;

@@ -422,23 +422,44 @@ class Engine:
                                                 int(n.value)))
         return table, means
 
-    def _bind_outputs(self, k, cluster_map_out, day_stats, transitions, regions=None, region_map_out=None):
+    def _bind_region_overlaps(self, pairs):
+        """Bind the day pairs ``pairs`` (``[P,2]`` global days) of region overlaps to the next fit /
+        predict."""
+        pr = np.ascontiguousarray(np.clip(np.asarray(pairs, dtype=np.int64).reshape(-1, 2), -1, 2**31 - 1),
+                                  dtype=np.int32)
+        self._check(self._lib.mdkm_bind_region_overlaps(self._h, c_void_p(pr.ctypes.data), int(pr.shape[0])))
+
+    def _region_overlap_table(self):
+        """The region overlaps of the last fit / predict that had them -> int64 ``[M,6]``."""
+        n = c_int64(0)
+        self._check(self._lib.mdkm_region_overlap_count(self._h, byref(n)))
+        rows = np.empty((n.value, 6), dtype=np.int64)
+        self._check(self._lib.mdkm_region_overlap_table(self._h, c_void_p(rows.ctypes.data), int(n.value)))
+        return rows
+
+    def _bind_outputs(self, k, cluster_map_out, day_stats, transitions, regions=None, region_map_out=None,
+                      region_overlaps=None):
         """Bind the optional outputs of the next fit / predict -> (map memory kind, (counts, means),
         transitions, region map memory kind), each None when not asked for.  When one binding is
         refused none is left behind: the statistics and transition arrays live only in this call,
         and a binding that outlived them would have the next fit / predict write into freed memory."""
         if region_map_out is not None and regions is None:
             raise ValueError("region_map_out needs regions=4 or regions=8")
+        if region_overlaps is not None and regions is None:
+            raise ValueError("region_overlaps needs regions=4 or regions=8")
         try:
             map_mem = self._bind_cluster_map(cluster_map_out) if cluster_map_out is not None else None
             stats = self._bind_day_stats(k) if day_stats else None
             trans = self._bind_day_transitions(transitions, k) if transitions is not None else None
             reg_mem = self._bind_regions(regions, region_map_out) if regions is not None else None
+            if region_overlaps is not None:
+                self._bind_region_overlaps(region_overlaps)
         except BaseException:
             self._lib.mdkm_bind_cluster_map(self._h, None, 1, 0, C.MEM_HOST)
             self._lib.mdkm_bind_day_stats(self._h, None, None, 0, 0)
             self._lib.mdkm_bind_day_transitions(self._h, None, 0, None, 0)
             self._lib.mdkm_bind_regions(self._h, 0, None, 0, C.MEM_HOST)
+            self._lib.mdkm_bind_region_overlaps(self._h, None, 0)
             raise
         return map_mem, stats, trans, reg_mem
 
@@ -466,7 +487,7 @@ class Engine:
 
     # -- k-means -------------------------------------------------------------------------
     def fit(self, init, max_iter=300, tol=1e-4, want_labels=True, labels_out=None, cluster_map_out=None,
-            day_stats=False, transitions=None, regions=None, region_map_out=None):
+            day_stats=False, transitions=None, regions=None, region_map_out=None, region_overlaps=None):
         """One Lloyd run from explicit centroids.  Returns dict(labels, centers, n_iter, inertia, ...).
 
         ``cluster_map_out``: optional uint8 (k <= 255) or uint16 array / tensor, host or CUDA, with
@@ -494,7 +515,15 @@ class Engine:
         ``day_means``).  ``region_map_out``: optional int32 array / tensor, host or CUDA, with one
         element per pixel of the last ``unproject``'s range; it receives the region ids, 0 where a
         pixel has no point.  Labelled on the GPU after the fit; same cover rule as
-        ``transitions``, and with several ranks every rank receives the whole stack's regions."""
+        ``transitions``, and with several ranks every rank receives the whole stack's regions.
+
+        ``region_overlaps``: day pairs ``[P,2]`` (global days; needs ``regions``, else
+        ``ValueError`` before any GPU work); the result also has ``region_overlaps``, int64
+        ``[M,6]`` rows (pair, region_a, region_b, pixels, y_first, x_first): one for every pair of
+        regions (r of day a, s of day b) that share at least one pixel, with the number of shared
+        pixels and the first shared pixel, sorted by pair and then by that pixel's raster order.
+        Counted on the GPU from the region map; with several ranks every rank builds the same
+        rows."""
         init = np.ascontiguousarray(init, dtype=np.float64)
         if init.ndim != 2 or init.shape[1] != 3:
             raise ValueError("init must be [K,3]")
@@ -513,7 +542,7 @@ class Engine:
         n_iter = c_int(0)
         inertia = c_double(0.0)
         map_mem, stats, trans, reg_mem = self._bind_outputs(k, cluster_map_out, day_stats, transitions, regions,
-                                                            region_map_out)
+                                                            region_map_out, region_overlaps)
         self._check(self._lib.mdkm_fit(
             self._h, int(k), init.ctypes.data_as(POINTER(c_double)), int(max_iter), float(tol),
             c_void_p(lab_ptr) if lab_ptr else None, lab_mem,
@@ -536,6 +565,8 @@ class Engine:
             out["transitions"] = trans
         if regions is not None:
             out["regions"], out["region_means"] = self._region_table()
+        if region_overlaps is not None:
+            out["region_overlaps"] = self._region_overlap_table()
         return out
 
     def lloyd_step(self, centroids, want_labels=True):
@@ -555,19 +586,20 @@ class Engine:
         return labels, sums, counts, int(nref.value)
 
     def predict(self, centroids, want_labels=True, cluster_map_out=None, day_stats=False, transitions=None,
-                regions=None, region_map_out=None):
+                regions=None, region_map_out=None, region_overlaps=None):
         """E-step only (KMeans.predict): returns (labels int32[N] or None, inertia).
         ``cluster_map_out``: as in ``fit``.  ``day_stats=True``: returns
         (labels, inertia, day_counts, day_means) instead, as in ``fit``.  ``transitions``: day
         pairs as in ``fit``; their counts are appended to the returned tuple.  ``regions`` /
-        ``region_map_out``: as in ``fit``; the table and the means are appended after that."""
+        ``region_map_out``: as in ``fit``; the table and the means are appended after that.
+        ``region_overlaps``: as in ``fit``; the rows are appended last."""
         c = np.ascontiguousarray(centroids, dtype=np.float64)
         if c.ndim != 2 or c.shape[1] != 3:
             raise ValueError("centroids must be [K,3]")
         labels = self._result_buffer("labels", (self.n_points,), np.int32) if want_labels else None
         inertia = c_double(0.0)
         map_mem, stats, trans, reg_mem = self._bind_outputs(c.shape[0], cluster_map_out, day_stats, transitions,
-                                                            regions, region_map_out)
+                                                            regions, region_map_out, region_overlaps)
         self._check(self._lib.mdkm_predict(
             self._h, int(c.shape[0]), c.ctypes.data_as(POINTER(c_double)),
             c_void_p(labels.ctypes.data) if labels is not None else None, C.MEM_HOST, byref(inertia)))
@@ -580,6 +612,8 @@ class Engine:
             out += (trans,)
         if regions is not None:
             out += self._region_table()
+        if region_overlaps is not None:
+            out += (self._region_overlap_table(),)
         return out
 
     def kmeans_plusplus(self, n_clusters: int, random_state):

@@ -244,6 +244,49 @@ int mdkm_bind_regions(mdkm_handle* h, int connectivity, int32_t* map_out, int64_
 int mdkm_region_count(const mdkm_handle* h, int64_t* n_regions);
 int mdkm_region_table(mdkm_handle* h, int64_t* table_out, double* means_out, int64_t capacity_regions);
 
+/* Optional: have the NEXT mdkm_fit or mdkm_predict on this handle, which must also have regions
+ * bound (mdkm_bind_regions), return the overlaps of the regions of pairs of days: which object of
+ * day a became which object of day b.  For pair p = (a, b), pairs[2p] = a and pairs[2p+1] = b
+ * (global days of the stack; any order, repeats and a == b allowed; copied by this call), there is
+ * one row for every pair of regions (r of day a, s of day b) such that at least one pixel (y, x)
+ * lies in r on day a and in s on day b; r and s may have different clusters.
+ * After the call, mdkm_region_overlap_count gives the number of rows M and
+ * mdkm_region_overlap_table copies them, int64 [M][6]: pair, region_a, region_b, pixels (shared
+ * pixels), y_first, x_first (the first shared pixel in raster order).  Rows are sorted by pair,
+ * then by the raster order of their first shared pixel -- the rule that numbers the regions -- so
+ * they do not depend on the schedule or the number of ranks.  For a == b the rows are (r, r,
+ * pixels of r, first pixel of r) for every region of day a, in id order; the rows of (b, a) are
+ * those of (a, b) with columns 1 and 2 swapped, in the same order; summed by (cluster of r,
+ * cluster of s) the pixels are the transition counts of the pair without row and column 0.
+ * Where the numbers come from: behind the region ids, a pass counts for every pair the pixels
+ * where both ids are non-zero and the (id_a, id_b) key differs from the left neighbour's or x ==
+ * 0, an upper bound on the pair's rows, read by the synchronisation that reads R (no extra one).
+ * Each pair gets an open-addressing hash table of 16-byte slots (the smallest power of two >= 2 x
+ * its bound); equal keys are combined in the warp, and their leaders add the pixels and lower the
+ * first pixel with atomics.  Every occupied slot sets the bit of its first pixel in an H*W-bit mask
+ * per pair, a popcount scan of the masks gives each slot its row, and one more synchronisation
+ * reads M.  Memory: 16 B x table capacity (<= 64 B per pixel and pair) plus 8 B per 32 pixels and
+ * pair (mask and scan offsets), plus 48 B per row; the worst case, where every pixel is a row, is
+ * a one-pixel checkerboard against its one-pixel shift (about 112 B per pixel and pair).  A failed
+ * allocation returns MDKM_ERR_OOM.  With several ranks every rank builds the whole table from its
+ * whole-stack region map: no collective, the same bits on every rank, and every rank pays the
+ * whole cost.  Asking for overlaps changes no other result of the call.
+ * pairs == NULL clears the binding.  The binding is consumed by that one call, and dropped by
+ * mdkm_unproject / mdkm_set_points.  Errors: MDKM_ERR_STATE when the resident cloud did not come
+ * from mdkm_unproject; MDKM_ERR_INVALID when n_pairs < 1 or n_pairs > 8192, or a day is outside
+ * [0, D); from the mdkm_fit / mdkm_predict, before any work is enqueued, MDKM_ERR_STATE when no
+ * regions are bound for that call. */
+int mdkm_bind_region_overlaps(mdkm_handle* h, const int32_t* pairs, int n_pairs);
+
+/* The region overlaps of the last mdkm_fit / mdkm_predict that had them bound, kept on the device
+ * until the next mdkm_unproject / mdkm_set_points or fit / predict with regions (a later call with
+ * regions but without overlaps drops them).  mdkm_region_overlap_count: their number M.
+ * mdkm_region_overlap_table: copies the rows (table_out, int64 [M][6]) to host memory.  Errors:
+ * MDKM_ERR_STATE when there are none (none computed since the last unproject / set_points);
+ * MDKM_ERR_INVALID from mdkm_region_overlap_table when capacity_rows < M. */
+int mdkm_region_overlap_count(const mdkm_handle* h, int64_t* n_rows);
+int mdkm_region_overlap_table(mdkm_handle* h, int64_t* table_out, int64_t capacity_rows);
+
 /* Load an already unprojected cloud (this rank's shard).  Replaces the `X` argument of the
  * reference's KMeans(...).fit_predict(X) call (members/jasraj/land_use_classification/
  * core.py:227-228) for d = 3. */
