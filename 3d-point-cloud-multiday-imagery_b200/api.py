@@ -24,7 +24,7 @@ from typing import Any, Dict, List, Literal, Optional, Tuple
 
 import numpy as np
 
-from .engine import Engine
+from .engine import Engine, check_min_iou
 
 LayerType = Literal["image", "labels", "points", "shapes"]
 Layer = Tuple[np.ndarray, Dict[str, Any], LayerType]  # interface.py:5-7
@@ -74,6 +74,14 @@ class FusionResult:
     # the whole stack on every rank
     region_overlaps: Optional[np.ndarray] = None
     region_overlap_pairs: Optional[np.ndarray] = None
+    # object tracks (return_tracks): regions of consecutive days linked by IoU >= track_min_iou and
+    # the same cluster, numbered 1..T by their smallest region id -- int64 [T,7] (cluster,
+    # first_day, last_day, regions, pixels, first_region, branched) and the track of every region,
+    # int32 [R] (region r at index r - 1), over the whole stack on every rank; track_map
+    # (return_track_map): int32 track id per pixel, 0 where no point, shaped like region_map
+    tracks: Optional[np.ndarray] = None
+    region_tracks: Optional[np.ndarray] = None
+    track_map: Optional[np.ndarray] = None
 
     # scikit-learn style aliases
     @property
@@ -191,6 +199,15 @@ def requested_connectivity(return_regions, connectivity=4, return_region_map=Fal
     return int(connectivity)
 
 
+def requested_min_iou(return_tracks, min_iou=0.5, return_track_map=False):
+    """The min_iou ``return_tracks`` / ``return_track_map`` ask for: None (no tracks) or a float in
+    (0, 1].  The track map implies the tracks.  Raises ``ValueError`` for a value that is not a
+    real number in (0, 1] (NaN and bools included)."""
+    if not (return_tracks or return_track_map):
+        return None
+    return check_min_iou(min_iou, "track_min_iou")
+
+
 def _stack_days(height_maps, stack_shape, raster_layout) -> int:
     """D of the stack ``fuse_multiday_kmeans`` is given (before anything reaches the GPU)."""
     if stack_shape is not None:
@@ -203,7 +220,7 @@ def _stack_days(height_maps, stack_shape, raster_layout) -> int:
 
 def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_state, want_labels=True,
                 labels_out=None, gather_mappings=None, cluster_map_out=None, day_stats=False, transitions=None,
-                regions=None, region_map_out=None, region_overlaps=None):
+                regions=None, region_map_out=None, region_overlaps=None, tracks=None, track_map_out=None):
     """KMeans.fit driver (sklearn/_kmeans.py:1436-1563): init, n_init restarts, best inertia.
 
     ``labels_out``: optional int32 array that receives this rank's labels of the best run.
@@ -218,6 +235,9 @@ def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_
     ``region_means``, the best run's as with ``day_stats``; the region map as ``cluster_map_out``.
     ``region_overlaps``: day pairs ``[P,2]`` (needs ``regions``); the result also has
     ``region_overlaps`` (``Engine.fit``), the best run's, as with ``day_stats``.
+    ``tracks`` (min_iou; needs ``regions``) and ``track_map_out`` (int32): the result also has
+    ``tracks`` / ``region_tracks``, the best run's as with ``day_stats``; the track map as
+    ``cluster_map_out``.
     ``gather_mappings``: with a multi-rank engine, the collective that lets the ranks agree on
     sklearn's "same clustering up to a permutation" test (see ``_is_same_clustering``); when it is
     missing the test is skipped on multi-rank engines (the inertia comparison alone decides)."""
@@ -244,7 +264,7 @@ def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_
         gather_mappings = torch_gather_mappings(eng)  # None unless torch.distributed spans the ranks
     single = int(n_init) == 1
     best = None
-    run_map = best_map = run_rmap = best_rmap = None
+    run_map = best_map = run_rmap = best_rmap = run_tmap = best_tmap = None
     if cluster_map_out is not None and not single:
         import torch
 
@@ -257,6 +277,11 @@ def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_
 
         run_rmap = torch.empty(eng.raster_range[4], dtype=torch.int32, device=f"cuda:{eng.device}")
         best_rmap = torch.empty_like(run_rmap)
+    if track_map_out is not None and not single:
+        import torch
+
+        run_tmap = torch.empty(eng.raster_range[4], dtype=torch.int32, device=f"cuda:{eng.device}")
+        best_tmap = torch.empty_like(run_tmap)
     for _ in range(int(n_init)):
         if init_is_array:
             centers0 = init_arr
@@ -268,7 +293,8 @@ def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_
                     labels_out=labels_out if (single and want_labels) else None,
                     cluster_map_out=cluster_map_out if single else run_map, day_stats=day_stats,
                     transitions=transitions, regions=regions,
-                    region_map_out=region_map_out if single else run_rmap, region_overlaps=region_overlaps)
+                    region_map_out=region_map_out if single else run_rmap, region_overlaps=region_overlaps,
+                    tracks=tracks, track_map_out=track_map_out if single else run_tmap)
         # sklearn/_kmeans.py:1534-1541: a run replaces the best one when its inertia is lower AND it
         # is not the same clustering up to a permutation.  The inertia is global, so every rank
         # takes the same branch and the (collective) permutation test pairs up.
@@ -284,6 +310,8 @@ def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_
                 run_map, best_map = best_map, run_map
             if run_rmap is not None:
                 run_rmap, best_rmap = best_rmap, run_rmap
+            if run_tmap is not None:
+                run_tmap, best_tmap = best_tmap, run_tmap
     if labels_out is not None and want_labels and not single:
         labels_out[...] = best["labels"]
         best = dict(best, labels=labels_out)
@@ -291,6 +319,8 @@ def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_
         _copy_map_out(best_map, cluster_map_out)
     if best_rmap is not None:
         _copy_map_out(best_rmap, region_map_out)
+    if best_tmap is not None:
+        _copy_map_out(best_tmap, track_map_out)
     return best
 
 
@@ -316,7 +346,8 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
                          pix_begin=0, raster_layout=None, return_cluster_map=False,
                          return_day_stats=False, return_transitions=False, return_regions=False,
                          region_connectivity=4, return_region_map=False,
-                         return_region_overlaps=False) -> FusionResult:
+                         return_region_overlaps=False, return_tracks=False, track_min_iou=0.5,
+                         return_track_map=False) -> FusionResult:
     """Unproject a multi-day height-map stack into one XYZ cloud and cluster it (Lloyd).
 
     height_maps : float32 ``[D,H,W]`` (NaN = nodata), numpy or torch (CPU or CUDA); or int16
@@ -382,6 +413,23 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
         the GPU from the region map; every rank of a pre-sharded call receives the same rows.
         Out-of-range days, or more than ``MAX_REGION_OVERLAP_PAIRS``
         (8192) pairs, raise ``ValueError`` before any GPU work.
+    return_tracks : also return object tracks -- which region is the same object over the stack.
+        Region r of day d and region s of day d+1 are linked when they have the same cluster and
+        share at least one pixel with ``shared / (pixels_r + pixels_s - shared) >= track_min_iou``
+        (FP64); a track is a connected component of the links (a region without links is a track
+        of its own), numbered 1..T in the order of its smallest region id, and does not bridge a
+        day without the object.  ``tracks``, int64 ``[T,7]`` rows (cluster, first_day, last_day,
+        regions, pixels, first_region, branched: 1 when a region of the track has two or more
+        links to one neighbouring day), and ``region_tracks``, int32 ``[R]`` (the track of region r
+        at index r - 1).  With ``track_min_iou > 0.5`` every track is a chain with one region per
+        day over ``[first_day, last_day]``: two regions of day d+1 cannot both overlap more than
+        half of one region of day d.  Implies ``return_regions``; built on the GPU, with no map
+        copy to the host, and every rank of a pre-sharded call receives the same tracks.
+    track_min_iou : the IoU a link needs, a real number in (0, 1] (default 0.5); anything else,
+        NaN and bools included, raises ``ValueError`` before any GPU work.
+    return_track_map : also return ``track_map``, int32, the track id of every pixel that produced
+        a point and 0 elsewhere (a napari Labels layer in which an object keeps its colour across
+        days); shaped like ``region_map``.  Implies ``return_tracks``.
     Returns a FusionResult; ``fused_cloud`` is float32 ``[N,3]`` in napari (z,y,x) order.
     """
     from .group import DeviceGroup
@@ -395,7 +443,9 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
         if ov_pairs.shape[0] > MAX_REGION_OVERLAP_PAIRS:
             raise ValueError(f"return_region_overlaps asks for {ov_pairs.shape[0]} pairs, at most "
                              f"{MAX_REGION_OVERLAP_PAIRS} are allowed")
-    conn = requested_connectivity(return_regions or ov_pairs is not None, region_connectivity, return_region_map)
+    min_iou = requested_min_iou(return_tracks, track_min_iou, return_track_map)
+    conn = requested_connectivity(return_regions or ov_pairs is not None or min_iou is not None, region_connectivity,
+                                  return_region_map)
     if devices is not None or isinstance(engine, DeviceGroup):
         if stack_shape is not None or pix_begin:
             raise ValueError("stack_shape / pix_begin describe a pre-sharded stack; a device group shards by itself")
@@ -405,7 +455,8 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
                               disparity_scale=disparity_scale, ground_level=ground_level, return_cloud=return_cloud,
                               raster_layout=raster_layout, return_cluster_map=return_cluster_map,
                               return_day_stats=return_day_stats, transitions=pairs, regions=conn,
-                              return_region_map=return_region_map, region_overlaps=ov_pairs)
+                              return_region_map=return_region_map, region_overlaps=ov_pairs, tracks=min_iou,
+                              return_track_map=return_track_map)
     own = engine is None
     eng = engine or Engine(device)
     try:
@@ -434,9 +485,14 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
         if return_region_map:
             D, H, W, _, count = eng.raster_range
             rmap = np.empty((D, H, W) if stack_shape is None else (count,), dtype=np.int32)
+        tmap = None
+        if return_track_map:
+            D, H, W, _, count = eng.raster_range
+            tmap = np.empty((D, H, W) if stack_shape is None else (count,), dtype=np.int32)
         r = _run_kmeans(eng, n_clusters=n_clusters, init=init, n_init=n_init, max_iter=max_iter,
                         tol=tol, random_state=random_state, cluster_map_out=cmap, day_stats=return_day_stats,
-                        transitions=pairs, regions=conn, region_map_out=rmap, region_overlaps=ov_pairs)
+                        transitions=pairs, regions=conn, region_map_out=rmap, region_overlaps=ov_pairs,
+                        tracks=min_iou, track_map_out=tmap)
         eng.wait()
         return FusionResult(labels=r["labels"], centroids=r["centers"], fused_cloud=cloud,
                             n_iter=r["n_iter"], inertia=r["inertia"], n_points=n,
@@ -445,7 +501,8 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
                             day_counts=r.get("day_counts"), day_means=r.get("day_means"),
                             transitions=r.get("transitions"), transition_pairs=pairs,
                             regions=r.get("regions"), region_means=r.get("region_means"), region_map=rmap,
-                            region_overlaps=r.get("region_overlaps"), region_overlap_pairs=ov_pairs)
+                            region_overlaps=r.get("region_overlaps"), region_overlap_pairs=ov_pairs,
+                            tracks=r.get("tracks"), region_tracks=r.get("region_tracks"), track_map=tmap)
     finally:
         if own:
             eng.close()
@@ -453,7 +510,8 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
 
 def _fuse_on_group(height_maps, valid_masks, *, group, devices, n_clusters, init, n_init, max_iter, tol,
                    random_state, return_cluster_map=False, return_day_stats=False, transitions=None,
-                   regions=None, return_region_map=False, region_overlaps=None, **unproject_kw) -> FusionResult:
+                   regions=None, return_region_map=False, region_overlaps=None, tracks=None, return_track_map=False,
+                   **unproject_kw) -> FusionResult:
     """``fuse_multiday_kmeans`` on several devices of this process (``group.DeviceGroup``)."""
     import threading
 
@@ -478,18 +536,19 @@ def _fuse_on_group(height_maps, valid_masks, *, group, devices, n_clusters, init
                 return [g[0] for g in got], [g[1] for g in got]
             return gather
 
-        def run(eng, labels_out, cluster_map_out=None, region_map_out=None):
+        def run(eng, labels_out, cluster_map_out=None, region_map_out=None, track_map_out=None):
             r = eng.rank
             return _run_kmeans(eng, n_clusters=n_clusters, init=init, n_init=n_init, max_iter=max_iter, tol=tol,
                                random_state=states[r], labels_out=labels_out,
                                gather_mappings=gather_for(r) if grp.world > 1 else None,
                                cluster_map_out=cluster_map_out, day_stats=return_day_stats, transitions=transitions,
-                               regions=regions, region_map_out=region_map_out, region_overlaps=region_overlaps)
+                               regions=regions, region_map_out=region_map_out, region_overlaps=region_overlaps,
+                               tracks=tracks, track_map_out=track_map_out)
 
         res, labels, cloud, hn, extra = grp.fuse(
             height_maps, valid_masks, run_kmeans=run,
             cluster_map_dtype=cluster_map_dtype(n_clusters) if return_cluster_map else None,
-            region_map=return_region_map, **unproject_kw)
+            region_map=return_region_map, track_map=return_track_map, **unproject_kw)
         return FusionResult(labels=labels, centroids=res["centers"], fused_cloud=cloud, n_iter=res["n_iter"],
                             inertia=res["inertia"], n_points=int(labels.shape[0]), n_refined=res["n_refined"],
                             n_relocations=res["n_relocations"], height_norm=hn, extra=extra,
@@ -498,7 +557,9 @@ def _fuse_on_group(height_maps, valid_masks, *, group, devices, n_clusters, init
                             transitions=res.get("transitions"), transition_pairs=transitions,
                             regions=res.get("regions"), region_means=res.get("region_means"),
                             region_map=extra.pop("region_map", None),
-                            region_overlaps=res.get("region_overlaps"), region_overlap_pairs=region_overlaps)
+                            region_overlaps=res.get("region_overlaps"), region_overlap_pairs=region_overlaps,
+                            tracks=res.get("tracks"), region_tracks=res.get("region_tracks"),
+                            track_map=extra.pop("track_map", None))
     finally:
         if own:
             grp.close()
@@ -540,7 +601,8 @@ def to_layers(result: FusionResult, prefix: str = "Multi-day") -> List[Layer]:
     One Points layer with the fused cloud coloured by cluster (or by the reference's
     'height' property when it was computed) and one with the K centroids; when the result has a
     ``cluster_map``, a Labels layer with it (0 = no point at that pixel), and when it has a
-    ``region_map``, a Labels layer with the region ids.
+    ``region_map``, a Labels layer with the region ids, and when it has a ``track_map``, a Labels
+    layer with the track ids (one object keeps its colour from day to day).
     """
     if result.fused_cloud is None:
         raise ValueError("result has no fused_cloud (return_cloud=False)")
@@ -574,6 +636,8 @@ def to_layers(result: FusionResult, prefix: str = "Multi-day") -> List[Layer]:
         layers.append((result.cluster_map, {"name": f"{prefix} Cluster Map", "opacity": 0.7}, "labels"))
     if result.region_map is not None:
         layers.append((result.region_map, {"name": f"{prefix} Regions", "opacity": 0.7}, "labels"))
+    if result.track_map is not None:
+        layers.append((result.track_map, {"name": f"{prefix} Tracks", "opacity": 0.7}, "labels"))
     return layers
 
 

@@ -25,6 +25,7 @@
 #include "region_overlaps.cuh"
 #include "regions.cuh"
 #include "seeding.cuh"
+#include "tracks.cuh"
 #include "transitions.cuh"
 #include "unproject.cuh"
 
@@ -35,6 +36,9 @@ namespace {
 constexpr int kBatch = 10;                          // Lloyd iterations enqueued between status polls
 constexpr size_t kMappedBytes = 256 << 10;          // device-visible host buffer for small results
 constexpr int kMaxOvPairs = 8192;                   // day pairs of region overlaps (their bounds: one small copy)
+constexpr int kMaxTrackDays = 16384;                // days of a stack with tracks: their D - 1 consecutive pairs are
+                                                    // counted with the caller's, and all the bounds share that copy
+static_assert((2 + kMaxOvPairs + kMaxTrackDays) * 8 <= kMappedBytes, "overlap bounds exceed the small result buffer");
 
 // copies `bytes` (a multiple of 4) from device memory into device-visible host memory
 __global__ void publish_kernel(void* dst_host, const void* src, int bytes) {
@@ -207,6 +211,19 @@ struct mdkm_handle {
   DevBuf<unsigned long long> ov_scan;    // look-back words, chunk offsets, ticket + fault, M, probe fault
   DevBuf<long long> ov_rows;             // int64 [M][6]
   long long n_overlaps = -1;             // M of the last fit / predict with overlaps; -1: none
+  // object tracks (mdkm_bind_tracks) of the next fit / predict, and those of the last fit / predict
+  // that had them, with the lifecycle of the regions
+  double bound_track_iou = 0.0;          // min_iou; 0: not bound
+  int32_t* bound_track_map = nullptr;
+  int bound_track_map_mem = MDKM_MEM_HOST;
+  DevBuf<int> track_link_day;            // [counted pairs] d of the counted pair (d, d+1), else -1
+  DevBuf<int> track_parent;              // [R] union-find parents (region index)
+  DevBuf<unsigned int> track_links;      // [2R] links forward, then backward
+  DevBuf<int> track_ids;                 // [R] track of each region (region_tracks)
+  DevBuf<unsigned long long> track_scan; // look-back words of the numbering, ticket + fault, T, caller's M
+  DevBuf<long long> track_tab;           // int64 [R][7]: the first T rows are the track table
+  DevBuf<int> track_stage;               // a host track map is written here, then copied
+  long long n_tracks = -1;               // T of the last fit / predict with tracks; -1: none
 
   // communicator
   ncclComm_t comm = nullptr;
@@ -998,6 +1015,17 @@ struct OvOut {
   int n_pairs() const { return (int)(pairs.size() / 2); }
 };
 
+// Object tracks taken by one fit / predict (mdkm_bind_tracks): linked from the overlap rows of the
+// consecutive pairs, which are counted behind the caller's own pairs; `map` (optional) receives
+// this rank's range of the track map.
+struct TrackOut {
+  double iou = 0.0;             // min_iou; 0: not asked for
+  int32_t* map = nullptr;
+  int mem = MDKM_MEM_HOST;
+  int n_user = 0;               // the caller's overlap pairs, which come first
+  std::vector<int> link_day;    // [counted pairs] d of the counted pair (d, d+1), else -1
+};
+
 // page-locked host buffer of at least `bytes` (the stages of results handed over after a sync)
 int ensure_pinned(mdkm_handle* h, unsigned char*& p, size_t& cap, size_t bytes) {
   if (cap >= bytes && p) return MDKM_OK;
@@ -1164,6 +1192,7 @@ int take_regions(mdkm_handle* h, int k, MapOut& m, RegOut& g) {
   }
   h->n_regions = -1;
   h->n_overlaps = -1;
+  h->n_tracks = -1;
   return take_stack_map(h, k, m);
 }
 
@@ -1183,6 +1212,46 @@ int take_overlaps(mdkm_handle* h, const RegOut& g, const OvOut& o) {
   CU(cudaSetDevice(h->device));
   OK(ensure(h, h->ov_pairs, o.pairs.size()));
   CU(cudaMemcpyAsync(h->ov_pairs.p, o.pairs.data(), o.pairs.size() * 4, cudaMemcpyHostToDevice, h->stream));
+  return MDKM_OK;
+}
+
+// Consumes the binding of mdkm_bind_tracks (whatever happens next).
+TrackOut consume_tracks(mdkm_handle* h) {
+  TrackOut t;
+  t.iou = h->bound_track_iou;
+  t.map = h->bound_track_map;
+  t.mem = h->bound_track_map_mem;
+  h->bound_track_iou = 0.0;
+  h->bound_track_map = nullptr;
+  return t;
+}
+
+// Takes the tracks `t` (consumed) of a call whose regions are `g` and overlaps `o` (before
+// take_overlaps): they need the regions of the same call.  The consecutive pairs (d, d+1) that
+// the caller did not ask for are counted after the caller's pairs, whose rows stay a prefix; the
+// link pass finds the counted pair of every d through link_day.
+int take_tracks(mdkm_handle* h, const RegOut& g, OvOut& o, TrackOut& t) {
+  if (!t.iou) return MDKM_OK;
+  if (!g.conn) return fail(h, MDKM_ERR_STATE, "tracks need regions bound for the same call (mdkm_bind_regions)");
+  const int D = h->stack_days;
+  t.n_user = o.n_pairs();
+  std::vector<int> pair_of(std::max(D - 1, 0), -1);
+  for (int q = 0; q < t.n_user; ++q) {
+    const int a = o.pairs[2 * q], b = o.pairs[2 * q + 1];
+    if (b == a + 1 && pair_of[a] < 0) pair_of[a] = q;
+  }
+  for (int d = 0; d + 1 < D; ++d) {
+    if (pair_of[d] >= 0) continue;
+    pair_of[d] = o.n_pairs();
+    o.pairs.push_back(d);
+    o.pairs.push_back(d + 1);
+  }
+  t.link_day.assign(std::max(o.n_pairs(), 1), -1);
+  for (int d = 0; d + 1 < D; ++d) t.link_day[pair_of[d]] = d;
+  CU(cudaSetDevice(h->device));
+  OK(ensure(h, h->track_link_day, t.link_day.size()));
+  CU(cudaMemcpyAsync(h->track_link_day.p, t.link_day.data(), t.link_day.size() * 4, cudaMemcpyHostToDevice,
+                     h->stream));
   return MDKM_OK;
 }
 
@@ -1278,6 +1347,7 @@ void deliver_day_stats(mdkm_handle* h, const StatsOut& s) {
 }
 
 int run_overlaps(mdkm_handle* h, const OvOut& o, const int* ids, const unsigned long long* bounds);
+int run_tracks(mdkm_handle* h, const TrackOut& t, const OvOut& o, const int* ids);
 
 // The pair-independent part of the overlap kernels' parameters.
 OverlapParams overlap_params(mdkm_handle* h, const int* ids, int n_pairs) {
@@ -1304,8 +1374,8 @@ dim3 overlap_span_grid(long long HW, int n_pairs) {
 // the bounds of their pairs, counted right behind the ids -- then this rank's points are
 // summed into per-region slots, the slots are reduced over the ranks (sums; minima of the
 // first pixel and the bounds) and the table and means are written on the device, where
-// mdkm_region_table finds them.  The overlaps follow (run_overlaps).
-int run_regions(mdkm_handle* h, const RegOut& g, const MapOut& m, const OvOut& o) {
+// mdkm_region_table finds them.  The overlaps follow (run_overlaps), then the tracks (run_tracks).
+int run_regions(mdkm_handle* h, const RegOut& g, const MapOut& m, const OvOut& o, const TrackOut& t) {
   if (!g.conn) return MDKM_OK;
   const long long HW = (long long)h->raster_H * h->raster_w, n_px = (long long)h->stack_days * HW;
   const bool in_place = g.map && g.mem == MDKM_MEM_DEVICE && h->n_ranks == 1;  // (one rank holds the whole stack)
@@ -1393,7 +1463,8 @@ int run_regions(mdkm_handle* h, const RegOut& g, const MapOut& m, const OvOut& o
     CU(cudaGetLastError());
   }
   h->n_regions = R;
-  return run_overlaps(h, o, rp.ids, got.data() + 2);
+  OK(run_overlaps(h, o, rp.ids, got.data() + 2));
+  return run_tracks(h, t, o, rp.ids);
 }
 
 // The region overlaps `o` of the region map `ids` (the whole stack, on every rank), behind the
@@ -1455,6 +1526,77 @@ int run_overlaps(mdkm_handle* h, const OvOut& o, const int* ids, const unsigned 
   ++h->launches;
   CU(cudaGetLastError());
   h->n_overlaps = M;
+  return MDKM_OK;
+}
+
+// The tracks `t` of the R regions of the last run_regions, behind the overlap rows of the
+// counted pairs `o` on the stream (tracks.cuh): links, the numbering passes of the regions on the
+// R parents, the table into R zeroed rows, this rank's range of the track map from the region
+// map `ids` (the whole stack).  One synchronisation reads T and the number of the caller's rows,
+// which becomes the count mdkm_region_overlap_count reports.  Every rank builds the same tracks.
+int run_tracks(mdkm_handle* h, const TrackOut& t, const OvOut& o, const int* ids) {
+  if (!t.iou) return MDKM_OK;
+  const long long R = h->n_regions, M = o.n_pairs() ? h->n_overlaps : 0;
+  const long long n_chunks = (R + kRegChunk - 1) / kRegChunk;
+  OK(ensure(h, h->track_parent, (size_t)R));
+  OK(ensure(h, h->track_links, 2 * (size_t)R));
+  OK(ensure(h, h->track_ids, (size_t)R));
+  OK(ensure(h, h->track_tab, 7 * (size_t)R));
+  OK(ensure(h, h->track_scan, (size_t)n_chunks + 3));  // look-back words, ticket + fault, T, caller's M
+  CU(cudaMemsetAsync(h->track_scan.p, 0, ((size_t)n_chunks + 3) * 8, h->stream));
+  CU(cudaMemsetAsync(h->track_tab.p, 0, (size_t)R * 56, h->stream));
+  TrackParams tp{};
+  tp.rows = h->ov_rows.p;
+  tp.n_rows = M;
+  tp.link_day = h->track_link_day.p;
+  tp.n_user = t.n_user;
+  tp.user_rows = h->track_scan.p + n_chunks + 2;
+  tp.regions = reinterpret_cast<const long long*>(h->region_out.p);
+  tp.n_regions = R;
+  tp.min_iou = t.iou;
+  tp.parent = h->track_parent.p;
+  tp.links = h->track_links.p;
+  tp.tracks = h->track_ids.p;
+  tp.table = h->track_tab.p;
+  if (R > 0) {
+    RegionParams np{};
+    np.parent = h->track_parent.p;
+    np.ids = h->track_ids.p;
+    np.n_px = R;
+    np.status = h->track_scan.p;
+    np.ticket = reinterpret_cast<unsigned int*>(h->track_scan.p + n_chunks);
+    np.n_regions = h->track_scan.p + n_chunks + 1;
+    const int per_region = grid_for(h, (R + kThreads - 1) / kThreads, resident_per_sm(h, track_table_kernel));
+    track_init_kernel<<<per_region, kThreads, 0, h->stream>>>(tp);
+    if (M > 0)
+      track_link_kernel<<<grid_for(h, (M + kThreads - 1) / kThreads, resident_per_sm(h, track_link_kernel)), kThreads, 0,
+                          h->stream>>>(tp);
+    region_number_kernel<<<(unsigned int)n_chunks, kThreads, 0, h->stream>>>(np);
+    region_resolve_kernel<<<grid_for(h, (R + 1023) / 1024, resident_per_sm(h, region_resolve_kernel)), kThreads, 0,
+                            h->stream>>>(np);
+    track_table_kernel<<<per_region, kThreads, 0, h->stream>>>(tp);
+    h->launches += M > 0 ? 5 : 4;
+  }
+  const long long n = h->raster_pix_count;
+  if (t.map && n > 0) {
+    int* out = t.map;
+    if (t.mem != MDKM_MEM_DEVICE) {
+      OK(ensure(h, h->track_stage, (size_t)n));
+      out = h->track_stage.p;
+    }
+    track_map_kernel<<<grid_for(h, (n / 4 + kThreads) / kThreads, resident_per_sm(h, track_map_kernel)), kThreads, 0,
+                       h->stream>>>(ids + h->raster_pix_begin, h->track_ids.p, out, n);
+    ++h->launches;
+    if (t.mem != MDKM_MEM_DEVICE)
+      CU(cudaMemcpyAsync(t.map, out, (size_t)n * 4, cudaMemcpyDeviceToHost, h->stream));
+  }
+  CU(cudaGetLastError());
+  unsigned long long got[3] = {0, 0, 0};  // ticket | fault << 32, T, the caller's rows
+  OK(small_d2h(h, got, h->track_scan.p + n_chunks, 24));
+  OK(sync_small(h));
+  if (got[0] >> 32) return fail(h, MDKM_ERR_CUDA, "track numbering: the look-back over the chunks timed out");
+  h->n_tracks = (long long)got[1];
+  h->n_overlaps = t.n_user ? (long long)got[2] : -1;
   return MDKM_OK;
 }
 
@@ -1644,6 +1786,8 @@ void mdkm_destroy(mdkm_handle* h) {
   release(h->region_box); release(h->region_out);
   release(h->ov_pairs); release(h->ov_tab); release(h->ov_slots); release(h->ov_bits); release(h->ov_scan);
   release(h->ov_rows);
+  release(h->track_link_day); release(h->track_parent); release(h->track_links); release(h->track_ids);
+  release(h->track_scan); release(h->track_tab); release(h->track_stage);
   release(h->kpp_closest); release(h->kpp_cell); release(h->kpp_blk); release(h->kpp_prefix);
   release(h->kpp_partials); release(h->kpp_rand); release(h->kpp_state);
   if (h->d_status) cudaFree(h->d_status);
@@ -1854,6 +1998,9 @@ int mdkm_set_points(mdkm_handle* h, const float* xyz, int64_t n, int layout, int
   h->n_regions = -1;
   h->bound_ov_pairs.clear();
   h->n_overlaps = -1;
+  h->bound_track_iou = 0.0;
+  h->bound_track_map = nullptr;
+  h->n_tracks = -1;
   h->stack_days = 1;
   h->day0 = 0;
   h->runs_ok = false;
@@ -2022,6 +2169,53 @@ int mdkm_region_overlap_table(mdkm_handle* h, int64_t* table_out, int64_t capaci
   return MDKM_OK;
 }
 
+int mdkm_bind_tracks(mdkm_handle* h, double min_iou, int32_t* map_out, int64_t capacity_pixels, int mem) {
+  if (!h) return MDKM_ERR_INVALID;
+  h->bound_track_iou = 0.0;
+  h->bound_track_map = nullptr;
+  if (min_iou == 0.0 && !map_out) return MDKM_OK;
+  if (!h->have_points || h->raster_w <= 0)
+    return fail(h, MDKM_ERR_STATE, "tracks need a resident cloud from mdkm_unproject");
+  if (!(min_iou > 0.0 && min_iou <= 1.0))
+    return fail(h, MDKM_ERR_INVALID, "tracks: min_iou must be in (0, 1], got %g", min_iou);
+  if (h->stack_days > kMaxTrackDays)
+    return fail(h, MDKM_ERR_INVALID, "tracks need a stack of at most %d days, got %d", kMaxTrackDays, h->stack_days);
+  if (map_out && (capacity_pixels < h->raster_pix_count || (mem != MDKM_MEM_HOST && mem != MDKM_MEM_DEVICE)))
+    return fail(h, MDKM_ERR_INVALID, "track map: capacity %lld < %lld pixels, or bad memory kind",
+                (long long)capacity_pixels, h->raster_pix_count);
+  h->bound_track_iou = min_iou;
+  h->bound_track_map = map_out;
+  h->bound_track_map_mem = mem;
+  return MDKM_OK;
+}
+
+int mdkm_track_count(const mdkm_handle* h, int64_t* n_tracks) {
+  if (!h || !n_tracks) return MDKM_ERR_INVALID;
+  if (h->n_tracks < 0)
+    return fail(const_cast<mdkm_handle*>(h), MDKM_ERR_STATE, "no tracks: no fit / predict with tracks since the last unproject / set_points or fit / predict with regions");
+  *n_tracks = h->n_tracks;
+  return MDKM_OK;
+}
+
+int mdkm_track_table(mdkm_handle* h, int64_t* table_out, int32_t* region_tracks_out, int64_t capacity_tracks,
+                     int64_t capacity_regions) {
+  if (!h) return MDKM_ERR_INVALID;
+  if (h->n_tracks < 0)
+    return fail(h, MDKM_ERR_STATE, "no tracks: no fit / predict with tracks since the last unproject / set_points or fit / predict with regions");
+  const long long T = h->n_tracks, R = h->n_regions;
+  if (table_out && capacity_tracks < T)
+    return fail(h, MDKM_ERR_INVALID, "track table: capacity %lld < %lld tracks", (long long)capacity_tracks, T);
+  if (region_tracks_out && capacity_regions < R)
+    return fail(h, MDKM_ERR_INVALID, "region tracks: capacity %lld < %lld regions", (long long)capacity_regions, R);
+  if (R == 0) return MDKM_OK;
+  CU(cudaSetDevice(h->device));
+  if (table_out) CU(cudaMemcpyAsync(table_out, h->track_tab.p, (size_t)T * 56, cudaMemcpyDeviceToHost, h->stream));
+  if (region_tracks_out)
+    CU(cudaMemcpyAsync(region_tracks_out, h->track_ids.p, (size_t)R * 4, cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
+  return MDKM_OK;
+}
+
 int mdkm_bind_day_stats(mdkm_handle* h, int64_t* counts_out, double* means_out, int n_days, int k_capacity) {
   if (!h) return MDKM_ERR_INVALID;
   h->bound_counts = nullptr;
@@ -2061,6 +2255,9 @@ int mdkm_unproject(mdkm_handle* h, const void* hm, int hm_dtype, float hm_scale,
   h->n_regions = -1;
   h->bound_ov_pairs.clear();
   h->n_overlaps = -1;
+  h->bound_track_iou = 0.0;
+  h->bound_track_map = nullptr;
+  h->n_tracks = -1;
   if (D < 0 || H <= 0 || W <= 0 || pix_begin < 0 || pix_count < 0 ||
       pix_begin + pix_count > (int64_t)D * H * W || (pix_count > 0 && !hm))
     return fail(h, MDKM_ERR_INVALID, "bad stack geometry");
@@ -2348,10 +2545,12 @@ int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol
   h->bound_trans = nullptr;
   RegOut reg = consume_regions(h);
   OvOut ov = consume_overlaps(h);
+  TrackOut trk = consume_tracks(h);
   const int map_rc = take_cluster_map(h, k, map);
   OK(take_day_stats(h, k, stats));
   OK(map_rc);
   OK(take_transitions(h, k, trans_out, map, trans));
+  OK(take_tracks(h, reg, ov, trk));
   OK(take_overlaps(h, reg, ov));
   OK(take_regions(h, k, map, reg));
   if (!init) return fail(h, MDKM_ERR_INVALID, "init centroids required");
@@ -2514,7 +2713,7 @@ int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol
 #endif
   if (fin.xchg_timeout == 2) return index_fault(h);
   if (fin.xchg_timeout) return fail(h, MDKM_ERR_NCCL, "a kernel-side wait timed out (peer exchange of the partial sums: a rank is missing; or the grid barrier)");
-  OK(run_regions(h, reg, map, ov));
+  OK(run_regions(h, reg, map, ov, trk));
   deliver_day_stats(h, stats);
   deliver_transitions(h, trans);
   if (n_iter_out) *n_iter_out = fin.iter;
@@ -2596,10 +2795,12 @@ int mdkm_predict(mdkm_handle* h, int k, const double* centroids, int32_t* labels
   h->bound_trans = nullptr;
   RegOut reg = consume_regions(h);
   OvOut ov = consume_overlaps(h);
+  TrackOut trk = consume_tracks(h);
   const int map_rc = take_cluster_map(h, k, map);
   OK(take_day_stats(h, k, stats));
   OK(map_rc);
   OK(take_transitions(h, k, trans_out, map, trans));
+  OK(take_tracks(h, reg, ov, trk));
   OK(take_overlaps(h, reg, ov));
   OK(take_regions(h, k, map, reg));
   if (!centroids) return fail(h, MDKM_ERR_INVALID, "centroids required");
@@ -2632,7 +2833,7 @@ int mdkm_predict(mdkm_handle* h, int k, const double* centroids, int32_t* labels
   OK(copy_cluster_map(h, map));
   OK(sync_small(h));
   if (h->h_status[0].xchg_timeout == 2) return index_fault(h);
-  OK(run_regions(h, reg, map, ov));
+  OK(run_regions(h, reg, map, ov, trk));
   deliver_day_stats(h, stats);
   deliver_transitions(h, trans);
   if (inertia_out) *inertia_out = h->h_status[0].inertia;

@@ -41,6 +41,17 @@ def _as_buffer(a, dtype=None):
     return arr.ctypes.data, C.MEM_HOST, arr, arr.shape, arr.dtype
 
 
+def check_min_iou(value, what="tracks"):
+    """``value`` as the float min_iou of object tracks: a real number in (0, 1] (not a bool, not
+    NaN).  Raises ``ValueError`` otherwise."""
+    if isinstance(value, (bool, np.bool_)) or not isinstance(value, (int, float, np.integer, np.floating)):
+        raise ValueError(f"{what} must be a real number in (0, 1], got {value!r}")
+    v = float(value)
+    if not (0.0 < v <= 1.0):
+        raise ValueError(f"{what} must be a real number in (0, 1], got {value!r}")
+    return v
+
+
 def _as_out_buffer(a, dtype, n_elems, what):
     """-> (pointer:int, mem_kind) of a caller-supplied OUTPUT array.  The library writes through
     the raw pointer, so anything that would make numpy / torch hand over a temporary copy (wrong
@@ -437,16 +448,48 @@ class Engine:
         self._check(self._lib.mdkm_region_overlap_table(self._h, c_void_p(rows.ctypes.data), int(n.value)))
         return rows
 
+    def _bind_tracks(self, min_iou, out):
+        """Bind object tracks (``min_iou`` in (0, 1]) and the optional int32 track map ``out`` (one
+        element per pixel of the last unprojected range) to the next fit / predict.  -> the map's
+        memory kind (None without a map)."""
+        iou = check_min_iou(min_iou)
+        ptr, mem, cap = None, None, 0
+        if out is not None:
+            cap = self._raster[4] if self._raster is not None else (out.numel() if _is_torch(out) else np.size(out))
+            ptr, mem = _as_out_buffer(out, np.int32, cap, "track_map_out")
+        self._check(self._lib.mdkm_bind_tracks(self._h, iou, c_void_p(ptr) if ptr else None, int(cap),
+                                               C.MEM_HOST if mem is None else mem))
+        if mem == C.MEM_DEVICE:
+            self._after_torch(out)  # earlier work on torch's stream may still use the buffer
+        return mem
+
+    def _track_table(self):
+        """The tracks of the last fit / predict that had them -> (table int64 ``[T,7]``, region
+        tracks int32 ``[R]``)."""
+        n, r = c_int64(0), c_int64(0)
+        self._check(self._lib.mdkm_track_count(self._h, byref(n)))
+        self._check(self._lib.mdkm_region_count(self._h, byref(r)))
+        table = np.empty((n.value, 7), dtype=np.int64)
+        region_tracks = np.empty(r.value, dtype=np.int32)
+        self._check(self._lib.mdkm_track_table(self._h, c_void_p(table.ctypes.data),
+                                               c_void_p(region_tracks.ctypes.data), int(n.value), int(r.value)))
+        return table, region_tracks
+
     def _bind_outputs(self, k, cluster_map_out, day_stats, transitions, regions=None, region_map_out=None,
-                      region_overlaps=None):
+                      region_overlaps=None, tracks=None, track_map_out=None):
         """Bind the optional outputs of the next fit / predict -> (map memory kind, (counts, means),
-        transitions, region map memory kind), each None when not asked for.  When one binding is
-        refused none is left behind: the statistics and transition arrays live only in this call,
-        and a binding that outlived them would have the next fit / predict write into freed memory."""
+        transitions, region map memory kind, track map memory kind), each None when not asked for.
+        When one binding is refused none is left behind: the statistics and transition arrays live
+        only in this call, and a binding that outlived them would have the next fit / predict write
+        into freed memory."""
         if region_map_out is not None and regions is None:
             raise ValueError("region_map_out needs regions=4 or regions=8")
         if region_overlaps is not None and regions is None:
             raise ValueError("region_overlaps needs regions=4 or regions=8")
+        if tracks is not None and regions is None:
+            raise ValueError("tracks needs regions=4 or regions=8")
+        if track_map_out is not None and tracks is None:
+            raise ValueError("track_map_out needs tracks=min_iou")
         try:
             map_mem = self._bind_cluster_map(cluster_map_out) if cluster_map_out is not None else None
             stats = self._bind_day_stats(k) if day_stats else None
@@ -454,14 +497,16 @@ class Engine:
             reg_mem = self._bind_regions(regions, region_map_out) if regions is not None else None
             if region_overlaps is not None:
                 self._bind_region_overlaps(region_overlaps)
+            trk_mem = self._bind_tracks(tracks, track_map_out) if tracks is not None else None
         except BaseException:
             self._lib.mdkm_bind_cluster_map(self._h, None, 1, 0, C.MEM_HOST)
             self._lib.mdkm_bind_day_stats(self._h, None, None, 0, 0)
             self._lib.mdkm_bind_day_transitions(self._h, None, 0, None, 0)
             self._lib.mdkm_bind_regions(self._h, 0, None, 0, C.MEM_HOST)
             self._lib.mdkm_bind_region_overlaps(self._h, None, 0)
+            self._lib.mdkm_bind_tracks(self._h, 0.0, None, 0, C.MEM_HOST)
             raise
-        return map_mem, stats, trans, reg_mem
+        return map_mem, stats, trans, reg_mem, trk_mem
 
     @property
     def segment_offsets(self) -> np.ndarray:
@@ -487,7 +532,8 @@ class Engine:
 
     # -- k-means -------------------------------------------------------------------------
     def fit(self, init, max_iter=300, tol=1e-4, want_labels=True, labels_out=None, cluster_map_out=None,
-            day_stats=False, transitions=None, regions=None, region_map_out=None, region_overlaps=None):
+            day_stats=False, transitions=None, regions=None, region_map_out=None, region_overlaps=None,
+            tracks=None, track_map_out=None):
         """One Lloyd run from explicit centroids.  Returns dict(labels, centers, n_iter, inertia, ...).
 
         ``cluster_map_out``: optional uint8 (k <= 255) or uint16 array / tensor, host or CUDA, with
@@ -523,7 +569,20 @@ class Engine:
         regions (r of day a, s of day b) that share at least one pixel, with the number of shared
         pixels and the first shared pixel, sorted by pair and then by that pixel's raster order.
         Counted on the GPU from the region map; with several ranks every rank builds the same
-        rows."""
+        rows.
+
+        ``tracks``: min_iou, a real number in (0, 1] (needs ``regions``, else ``ValueError`` before
+        any GPU work): object tracks over the stack.  Region r of day d and region s of day d+1 are
+        linked when they have the same cluster and share at least one pixel with
+        ``shared / (pixels_r + pixels_s - shared) >= min_iou`` (FP64); a track is a connected
+        component of the links, numbered 1..T in the order of its smallest region id.  With
+        ``min_iou > 0.5`` every track is a chain with one region per day over its days.  The result
+        also has ``tracks``, int64 ``[T,7]`` rows (cluster, first_day, last_day, regions, pixels,
+        first_region, branched), and ``region_tracks``, int32 ``[R]``, the track of region r at
+        index r - 1.  ``track_map_out``: optional int32 array / tensor, host or CUDA, like
+        ``region_map_out``; it receives the track id of every pixel, 0 where no point.  Built on
+        the GPU from the region map and the overlaps of consecutive days; the caller's own
+        ``region_overlaps`` stay as they are without tracks."""
         init = np.ascontiguousarray(init, dtype=np.float64)
         if init.ndim != 2 or init.shape[1] != 3:
             raise ValueError("init must be [K,3]")
@@ -541,13 +600,14 @@ class Engine:
         centers = np.empty((k, 3), dtype=np.float64)
         n_iter = c_int(0)
         inertia = c_double(0.0)
-        map_mem, stats, trans, reg_mem = self._bind_outputs(k, cluster_map_out, day_stats, transitions, regions,
-                                                            region_map_out, region_overlaps)
+        map_mem, stats, trans, reg_mem, trk_mem = self._bind_outputs(k, cluster_map_out, day_stats, transitions,
+                                                                     regions, region_map_out, region_overlaps,
+                                                                     tracks, track_map_out)
         self._check(self._lib.mdkm_fit(
             self._h, int(k), init.ctypes.data_as(POINTER(c_double)), int(max_iter), float(tol),
             c_void_p(lab_ptr) if lab_ptr else None, lab_mem,
             centers.ctypes.data_as(POINTER(c_double)), byref(n_iter), byref(inertia)))
-        if lab_mem == C.MEM_DEVICE or map_mem == C.MEM_DEVICE or reg_mem == C.MEM_DEVICE:
+        if C.MEM_DEVICE in (lab_mem, map_mem, reg_mem, trk_mem):
             self._before_torch()
         nref, nrel, tols = c_int64(0), c_int64(0), c_double(0)
         self._lib.mdkm_fit_stats(self._h, byref(nref), byref(nrel), byref(tols))
@@ -567,6 +627,8 @@ class Engine:
             out["regions"], out["region_means"] = self._region_table()
         if region_overlaps is not None:
             out["region_overlaps"] = self._region_overlap_table()
+        if tracks is not None:
+            out["tracks"], out["region_tracks"] = self._track_table()
         return out
 
     def lloyd_step(self, centroids, want_labels=True):
@@ -586,24 +648,26 @@ class Engine:
         return labels, sums, counts, int(nref.value)
 
     def predict(self, centroids, want_labels=True, cluster_map_out=None, day_stats=False, transitions=None,
-                regions=None, region_map_out=None, region_overlaps=None):
+                regions=None, region_map_out=None, region_overlaps=None, tracks=None, track_map_out=None):
         """E-step only (KMeans.predict): returns (labels int32[N] or None, inertia).
         ``cluster_map_out``: as in ``fit``.  ``day_stats=True``: returns
         (labels, inertia, day_counts, day_means) instead, as in ``fit``.  ``transitions``: day
         pairs as in ``fit``; their counts are appended to the returned tuple.  ``regions`` /
         ``region_map_out``: as in ``fit``; the table and the means are appended after that.
-        ``region_overlaps``: as in ``fit``; the rows are appended last."""
+        ``region_overlaps``: as in ``fit``; the rows are appended after that.  ``tracks`` /
+        ``track_map_out``: as in ``fit``; the track table and the region tracks are appended last."""
         c = np.ascontiguousarray(centroids, dtype=np.float64)
         if c.ndim != 2 or c.shape[1] != 3:
             raise ValueError("centroids must be [K,3]")
         labels = self._result_buffer("labels", (self.n_points,), np.int32) if want_labels else None
         inertia = c_double(0.0)
-        map_mem, stats, trans, reg_mem = self._bind_outputs(c.shape[0], cluster_map_out, day_stats, transitions,
-                                                            regions, region_map_out, region_overlaps)
+        map_mem, stats, trans, reg_mem, trk_mem = self._bind_outputs(c.shape[0], cluster_map_out, day_stats,
+                                                                     transitions, regions, region_map_out,
+                                                                     region_overlaps, tracks, track_map_out)
         self._check(self._lib.mdkm_predict(
             self._h, int(c.shape[0]), c.ctypes.data_as(POINTER(c_double)),
             c_void_p(labels.ctypes.data) if labels is not None else None, C.MEM_HOST, byref(inertia)))
-        if map_mem == C.MEM_DEVICE or reg_mem == C.MEM_DEVICE:
+        if C.MEM_DEVICE in (map_mem, reg_mem, trk_mem):
             self._before_torch()
         out = (labels, float(inertia.value))
         if stats is not None:
@@ -614,6 +678,8 @@ class Engine:
             out += self._region_table()
         if region_overlaps is not None:
             out += (self._region_overlap_table(),)
+        if tracks is not None:
+            out += self._track_table()
         return out
 
     def kmeans_plusplus(self, n_clusters: int, random_state):

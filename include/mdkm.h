@@ -287,6 +287,64 @@ int mdkm_bind_region_overlaps(mdkm_handle* h, const int32_t* pairs, int n_pairs)
 int mdkm_region_overlap_count(const mdkm_handle* h, int64_t* n_rows);
 int mdkm_region_overlap_table(mdkm_handle* h, int64_t* table_out, int64_t capacity_rows);
 
+/* Optional: have the NEXT mdkm_fit or mdkm_predict on this handle, which must also have regions
+ * bound (mdkm_bind_regions), return object tracks: which region is the same object over the whole
+ * stack.  Region r of day d and region s of day d+1 (consecutive global days) are linked when
+ * cluster(r) == cluster(s) and they share at least one pixel with
+ *   (double)shared / (double)(pixels_r + pixels_s - shared) >= min_iou
+ * in FP64 (the counts are exact integers below 2^31 and the division is correctly rounded, so a
+ * numpy restatement gives the same bits; pixels are column 2 of the region table).  A track is a
+ * connected component of the graph whose nodes are the regions and whose edges are the links; a
+ * region without links is a track of its own, so T <= R and every region is in exactly one
+ * track.  Tracks do not bridge a gap: a day on which the object has no region ends its track.
+ * Tracks are numbered 1..T in the order of their smallest region id, so the numbering does not
+ * depend on the schedule or the number of ranks, and all regions of a track have one cluster.
+ * Chains: with min_iou > 0.5 every region has at most one link forward and one back, so every
+ * track is a chain with one region per day over [first_day, last_day].  If r linked to two
+ * disjoint regions s1, s2 of day d+1, each IoU > 1/2 would force shared_i > pixels_r / 2, and
+ * shared_1 + shared_2 > pixels_r is impossible; the FP64 rounding keeps this, because 0.5 is
+ * representable and rounding is monotone, so a rounded quotient >= min_iou > 0.5 means an exact
+ * quotient > 0.5.  With min_iou <= 0.5, splits and merges join tracks.
+ * After the call, mdkm_track_count gives T and mdkm_track_table copies the track table, int64
+ * [T][7]: cluster, first_day, last_day, regions (the number of regions in the track), pixels (the
+ * sum of its regions' pixels), first_region (its smallest region id), branched (1 when some
+ * region of the track has two or more links to the next day or to the previous day, else 0) --
+ * and the region tracks, int32 [R]: the track id of region r at index r - 1.
+ * map_out (optional, int32, capacity_pixels >= the pix_count of the last mdkm_unproject; host or
+ * device memory as `mem` says) receives the track id of every pixel of this rank's range that
+ * produced a point, 0 elsewhere: the region map with every id replaced by its track's.  A device
+ * map is written in place; a host map is written into a device stage of 4 B per pixel and copied.
+ * Where the numbers come from: the overlaps of the consecutive pairs (d, d+1) are counted with
+ * those of mdkm_bind_region_overlaps (the caller's pairs first, then the consecutive pairs the
+ * caller did not ask for; the caller's rows and their count are the same as without tracks), one
+ * thread per row of a consecutive pair applies the rule and joins the two regions in a union-find
+ * on the R regions (integer atomics: the root is the smallest region id), the numbering passes of
+ * the regions give the roots their ids and every region its root's, and one pass over the regions
+ * fills the table with integer atomics; then the map pass.  One more synchronisation reads T.
+ * Memory: 72 B per region (parents, links, ids, table slots), the overlaps of the consecutive pairs
+ * (see mdkm_bind_region_overlaps), and 4 B per pixel of the range for a host map.  With several
+ * ranks every rank builds the same tracks from its whole-stack region map, with no collective.
+ * Asking for tracks changes no other result of the call.
+ * min_iou == 0 with map_out == NULL clears the binding.  The binding is consumed by that one call,
+ * and dropped by mdkm_unproject / mdkm_set_points.  Errors: MDKM_ERR_STATE when the resident cloud
+ * did not come from mdkm_unproject; MDKM_ERR_INVALID when min_iou is not in (0, 1] (NaN included),
+ * the stack has more than 16384 days, capacity_pixels < pix_count, or `mem` is neither
+ * MDKM_MEM_HOST nor MDKM_MEM_DEVICE; from the mdkm_fit / mdkm_predict, before any work is
+ * enqueued, MDKM_ERR_STATE when no regions are bound for that call. */
+int mdkm_bind_tracks(mdkm_handle* h, double min_iou, int32_t* map_out, int64_t capacity_pixels, int mem);
+
+/* The tracks of the last mdkm_fit / mdkm_predict that had them bound, kept on the device until
+ * the next mdkm_unproject / mdkm_set_points or fit / predict with regions (a later call with
+ * regions but without tracks drops them).  mdkm_track_count: their number T.  mdkm_track_table:
+ * copies the track table (table_out, int64 [T][7]) and the region tracks (region_tracks_out, int32
+ * [R]) to host memory; either may be NULL.  Errors: MDKM_ERR_STATE when there are none (none
+ * computed since the last unproject / set_points); MDKM_ERR_INVALID from mdkm_track_table when
+ * table_out is given and capacity_tracks < T, or region_tracks_out is given and capacity_regions
+ * < R. */
+int mdkm_track_count(const mdkm_handle* h, int64_t* n_tracks);
+int mdkm_track_table(mdkm_handle* h, int64_t* table_out, int32_t* region_tracks_out, int64_t capacity_tracks,
+                     int64_t capacity_regions);
+
 /* Load an already unprojected cloud (this rank's shard).  Replaces the `X` argument of the
  * reference's KMeans(...).fit_predict(X) call (members/jasraj/land_use_classification/
  * core.py:227-228) for d = 3. */
