@@ -155,6 +155,15 @@ def cluster_map_dtype(n_clusters: int):
     return np.uint8 if int(n_clusters) <= 255 else np.uint16
 
 
+# The pixel-map outputs of ``Engine.fit``; the FusionResult field of each is its name without "_out".
+PIXEL_MAP_OUTPUTS = ("cluster_map_out", "region_map_out", "track_map_out")
+
+
+def _pixel_map_dtype(kw, n_clusters):
+    """Element type of the pixel map output ``kw``: labels + 1 for the cluster map, int32 ids otherwise."""
+    return cluster_map_dtype(n_clusters) if kw == "cluster_map_out" else np.int32
+
+
 def transition_pairs(spec, n_days: int, what: str = "transitions") -> np.ndarray:
     """The day pairs ``return_transitions`` asks for, as int64 ``[P,2]``: ``True`` -> the
     consecutive pairs ``(d, d+1)``; a sequence of ``(a, b)`` -> those pairs in that order (they
@@ -219,25 +228,15 @@ def _stack_days(height_maps, stack_shape, raster_layout) -> int:
 
 
 def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_state, want_labels=True,
-                labels_out=None, gather_mappings=None, cluster_map_out=None, day_stats=False, transitions=None,
-                regions=None, region_map_out=None, region_overlaps=None, tracks=None, track_map_out=None):
+                labels_out=None, gather_mappings=None, **outputs):
     """KMeans.fit driver (sklearn/_kmeans.py:1436-1563): init, n_init restarts, best inertia.
 
     ``labels_out``: optional int32 array that receives this rank's labels of the best run.
-    ``cluster_map_out``: optional uint8 / uint16 array that receives the best run's cluster map
-    (``Engine.fit``).  With restarts every run writes its map into a device scratch tensor; the
-    best one is kept by swapping and copied out once at the end.
-    ``day_stats``: the result also has ``day_counts`` / ``day_means`` (``Engine.fit``) -- every run
-    returns fresh arrays, so the best run's stay with it.
-    ``transitions``: day pairs ``[P,2]``; the result also has ``transitions`` (``Engine.fit``), the
-    best run's, as with ``day_stats``.
-    ``regions`` (4 / 8) and ``region_map_out`` (int32): the result also has ``regions`` /
-    ``region_means``, the best run's as with ``day_stats``; the region map as ``cluster_map_out``.
-    ``region_overlaps``: day pairs ``[P,2]`` (needs ``regions``); the result also has
-    ``region_overlaps`` (``Engine.fit``), the best run's, as with ``day_stats``.
-    ``tracks`` (min_iou; needs ``regions``) and ``track_map_out`` (int32): the result also has
-    ``tracks`` / ``region_tracks``, the best run's as with ``day_stats``; the track map as
-    ``cluster_map_out``.
+    ``outputs``: the optional outputs of ``Engine.fit`` (``cluster_map_out``, ``day_stats``,
+    ``transitions``, ``regions``, ...); the result has the best run's -- every run returns fresh
+    arrays, so the best run's stay with it.  With restarts every run writes its pixel maps
+    (``PIXEL_MAP_OUTPUTS``) into device scratch tensors; the best run's are kept by swapping and
+    copied out once at the end.
     ``gather_mappings``: with a multi-rank engine, the collective that lets the ranks agree on
     sklearn's "same clustering up to a permutation" test (see ``_is_same_clustering``); when it is
     missing the test is skipped on multi-rank engines (the inertia comparison alone decides)."""
@@ -264,24 +263,15 @@ def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_
         gather_mappings = torch_gather_mappings(eng)  # None unless torch.distributed spans the ranks
     single = int(n_init) == 1
     best = None
-    run_map = best_map = run_rmap = best_rmap = run_tmap = best_tmap = None
-    if cluster_map_out is not None and not single:
-        import torch
+    scratch = {}  # pixel-map keyword -> [this run's map, the best run's map]
+    for kw in PIXEL_MAP_OUTPUTS:
+        if outputs.get(kw) is not None and not single:
+            import torch
 
-        # (a copy of the best map per improvement would cost a device->host transfer each time)
-        tdt = torch.uint8 if np.dtype(cluster_map_dtype(k)) == np.uint8 else torch.uint16
-        run_map = torch.empty(eng.raster_range[4], dtype=tdt, device=f"cuda:{eng.device}")
-        best_map = torch.empty_like(run_map)
-    if region_map_out is not None and not single:
-        import torch
-
-        run_rmap = torch.empty(eng.raster_range[4], dtype=torch.int32, device=f"cuda:{eng.device}")
-        best_rmap = torch.empty_like(run_rmap)
-    if track_map_out is not None and not single:
-        import torch
-
-        run_tmap = torch.empty(eng.raster_range[4], dtype=torch.int32, device=f"cuda:{eng.device}")
-        best_tmap = torch.empty_like(run_tmap)
+            # (a copy of the best map per improvement would cost a device->host transfer each time)
+            tdt = getattr(torch, np.dtype(_pixel_map_dtype(kw, k)).name)
+            run_map = torch.empty(eng.raster_range[4], dtype=tdt, device=f"cuda:{eng.device}")
+            scratch[kw] = [run_map, torch.empty_like(run_map)]
     for _ in range(int(n_init)):
         if init_is_array:
             centers0 = init_arr
@@ -291,10 +281,7 @@ def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_
             centers0, _ = eng.kmeans_plusplus(k, rs)
         r = eng.fit(centers0, max_iter=max_iter, tol=tol, want_labels=want_labels,
                     labels_out=labels_out if (single and want_labels) else None,
-                    cluster_map_out=cluster_map_out if single else run_map, day_stats=day_stats,
-                    transitions=transitions, regions=regions,
-                    region_map_out=region_map_out if single else run_rmap, region_overlaps=region_overlaps,
-                    tracks=tracks, track_map_out=track_map_out if single else run_tmap)
+                    **dict(outputs, **{kw: maps[0] for kw, maps in scratch.items()}))
         # sklearn/_kmeans.py:1534-1541: a run replaces the best one when its inertia is lower AND it
         # is not the same clustering up to a permutation.  The inertia is global, so every rank
         # takes the same branch and the (collective) permutation test pairs up.
@@ -306,21 +293,13 @@ def _run_kmeans(eng: Engine, *, n_clusters, init, n_init, max_iter, tol, random_
             best = r
             if not single and r["labels"] is not None:
                 best = dict(r, labels=r["labels"].copy())  # result buffers are reused by the next run
-            if run_map is not None:
-                run_map, best_map = best_map, run_map
-            if run_rmap is not None:
-                run_rmap, best_rmap = best_rmap, run_rmap
-            if run_tmap is not None:
-                run_tmap, best_tmap = best_tmap, run_tmap
+            for maps in scratch.values():
+                maps.reverse()  # this run's map becomes the best one
     if labels_out is not None and want_labels and not single:
         labels_out[...] = best["labels"]
         best = dict(best, labels=labels_out)
-    if best_map is not None:
-        _copy_map_out(best_map, cluster_map_out)
-    if best_rmap is not None:
-        _copy_map_out(best_rmap, region_map_out)
-    if best_tmap is not None:
-        _copy_map_out(best_tmap, track_map_out)
+    for kw, (_, best_map) in scratch.items():
+        _copy_map_out(best_map, outputs[kw])
     return best
 
 
@@ -446,6 +425,10 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
     min_iou = requested_min_iou(return_tracks, track_min_iou, return_track_map)
     conn = requested_connectivity(return_regions or ov_pairs is not None or min_iou is not None, region_connectivity,
                                   return_region_map)
+    outputs = {"day_stats": return_day_stats, "transitions": pairs, "regions": conn, "region_overlaps": ov_pairs,
+               "tracks": min_iou}
+    wanted = (return_cluster_map, return_region_map, return_track_map)
+    maps = [kw for kw, want in zip(PIXEL_MAP_OUTPUTS, wanted) if want]
     if devices is not None or isinstance(engine, DeviceGroup):
         if stack_shape is not None or pix_begin:
             raise ValueError("stack_shape / pix_begin describe a pre-sharded stack; a device group shards by itself")
@@ -453,10 +436,7 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
                               devices=devices, n_clusters=n_clusters, init=init, n_init=n_init, max_iter=max_iter,
                               tol=tol, random_state=random_state, max_abs_height=max_abs_height, detrend=detrend,
                               disparity_scale=disparity_scale, ground_level=ground_level, return_cloud=return_cloud,
-                              raster_layout=raster_layout, return_cluster_map=return_cluster_map,
-                              return_day_stats=return_day_stats, transitions=pairs, regions=conn,
-                              return_region_map=return_region_map, region_overlaps=ov_pairs, tracks=min_iou,
-                              return_track_map=return_track_map)
+                              raster_layout=raster_layout, outputs=outputs, maps=maps)
     own = engine is None
     eng = engine or Engine(device)
     try:
@@ -477,42 +457,39 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
         # otherwise its device->host copy is issued now and overlaps the Lloyd loop
         if return_cloud and cloud is None:
             cloud = eng.get_cloud(napari_order=True, wait=False)
-        cmap = None
-        if return_cluster_map:
+        for kw in maps:
             D, H, W, _, count = eng.raster_range
-            cmap = np.empty((D, H, W) if stack_shape is None else (count,), dtype=cluster_map_dtype(n_clusters))
-        rmap = None
-        if return_region_map:
-            D, H, W, _, count = eng.raster_range
-            rmap = np.empty((D, H, W) if stack_shape is None else (count,), dtype=np.int32)
-        tmap = None
-        if return_track_map:
-            D, H, W, _, count = eng.raster_range
-            tmap = np.empty((D, H, W) if stack_shape is None else (count,), dtype=np.int32)
+            shape = (D, H, W) if stack_shape is None else (count,)
+            outputs[kw] = np.empty(shape, dtype=_pixel_map_dtype(kw, n_clusters))
         r = _run_kmeans(eng, n_clusters=n_clusters, init=init, n_init=n_init, max_iter=max_iter,
-                        tol=tol, random_state=random_state, cluster_map_out=cmap, day_stats=return_day_stats,
-                        transitions=pairs, regions=conn, region_map_out=rmap, region_overlaps=ov_pairs,
-                        tracks=min_iou, track_map_out=tmap)
+                        tol=tol, random_state=random_state, **outputs)
         eng.wait()
-        return FusionResult(labels=r["labels"], centroids=r["centers"], fused_cloud=cloud,
-                            n_iter=r["n_iter"], inertia=r["inertia"], n_points=n,
-                            n_refined=r["n_refined"], n_relocations=r["n_relocations"],
-                            height_norm=hn, extra=extra, cluster_map=cmap,
-                            day_counts=r.get("day_counts"), day_means=r.get("day_means"),
-                            transitions=r.get("transitions"), transition_pairs=pairs,
-                            regions=r.get("regions"), region_means=r.get("region_means"), region_map=rmap,
-                            region_overlaps=r.get("region_overlaps"), region_overlap_pairs=ov_pairs,
-                            tracks=r.get("tracks"), region_tracks=r.get("region_tracks"), track_map=tmap)
+        return _fusion_result(r, outputs, {kw: outputs[kw] for kw in maps}, labels=r["labels"], fused_cloud=cloud,
+                              n_points=n, height_norm=hn, extra=extra)
     finally:
         if own:
             eng.close()
 
 
+def _fusion_result(r, outputs, maps, **fields) -> FusionResult:
+    """The FusionResult of the k-means result ``r`` of a call with the ``Engine.fit`` keywords
+    ``outputs`` and the pixel maps ``maps`` (keyword -> array).  ``fields``: labels, fused_cloud,
+    n_points, height_norm and extra."""
+    return FusionResult(centroids=r["centers"], n_iter=r["n_iter"], inertia=r["inertia"], n_refined=r["n_refined"],
+                        n_relocations=r["n_relocations"],
+                        day_counts=r.get("day_counts"), day_means=r.get("day_means"),
+                        transitions=r.get("transitions"), transition_pairs=outputs["transitions"],
+                        regions=r.get("regions"), region_means=r.get("region_means"),
+                        region_overlaps=r.get("region_overlaps"), region_overlap_pairs=outputs["region_overlaps"],
+                        tracks=r.get("tracks"), region_tracks=r.get("region_tracks"),
+                        **{kw.removesuffix("_out"): m for kw, m in maps.items()}, **fields)
+
+
 def _fuse_on_group(height_maps, valid_masks, *, group, devices, n_clusters, init, n_init, max_iter, tol,
-                   random_state, return_cluster_map=False, return_day_stats=False, transitions=None,
-                   regions=None, return_region_map=False, region_overlaps=None, tracks=None, return_track_map=False,
-                   **unproject_kw) -> FusionResult:
-    """``fuse_multiday_kmeans`` on several devices of this process (``group.DeviceGroup``)."""
+                   random_state, outputs, maps, **unproject_kw) -> FusionResult:
+    """``fuse_multiday_kmeans`` on several devices of this process (``group.DeviceGroup``):
+    ``outputs`` are the ``Engine.fit`` keywords of every rank, ``maps`` the keywords of the pixel
+    maps to build."""
     import threading
 
     from .group import DeviceGroup, clone_random_state
@@ -536,30 +513,17 @@ def _fuse_on_group(height_maps, valid_masks, *, group, devices, n_clusters, init
                 return [g[0] for g in got], [g[1] for g in got]
             return gather
 
-        def run(eng, labels_out, cluster_map_out=None, region_map_out=None, track_map_out=None):
+        def run(eng, labels_out, **map_bands):
             r = eng.rank
             return _run_kmeans(eng, n_clusters=n_clusters, init=init, n_init=n_init, max_iter=max_iter, tol=tol,
                                random_state=states[r], labels_out=labels_out,
-                               gather_mappings=gather_for(r) if grp.world > 1 else None,
-                               cluster_map_out=cluster_map_out, day_stats=return_day_stats, transitions=transitions,
-                               regions=regions, region_map_out=region_map_out, region_overlaps=region_overlaps,
-                               tracks=tracks, track_map_out=track_map_out)
+                               gather_mappings=gather_for(r) if grp.world > 1 else None, **outputs, **map_bands)
 
-        res, labels, cloud, hn, extra = grp.fuse(
-            height_maps, valid_masks, run_kmeans=run,
-            cluster_map_dtype=cluster_map_dtype(n_clusters) if return_cluster_map else None,
-            region_map=return_region_map, track_map=return_track_map, **unproject_kw)
-        return FusionResult(labels=labels, centroids=res["centers"], fused_cloud=cloud, n_iter=res["n_iter"],
-                            inertia=res["inertia"], n_points=int(labels.shape[0]), n_refined=res["n_refined"],
-                            n_relocations=res["n_relocations"], height_norm=hn, extra=extra,
-                            cluster_map=extra.pop("cluster_map", None),
-                            day_counts=res.get("day_counts"), day_means=res.get("day_means"),
-                            transitions=res.get("transitions"), transition_pairs=transitions,
-                            regions=res.get("regions"), region_means=res.get("region_means"),
-                            region_map=extra.pop("region_map", None),
-                            region_overlaps=res.get("region_overlaps"), region_overlap_pairs=region_overlaps,
-                            tracks=res.get("tracks"), region_tracks=res.get("region_tracks"),
-                            track_map=extra.pop("track_map", None))
+        res, labels, cloud, hn, extra = grp.fuse(height_maps, valid_masks, run_kmeans=run,
+                                                 maps={kw: _pixel_map_dtype(kw, n_clusters) for kw in maps},
+                                                 **unproject_kw)
+        return _fusion_result(res, outputs, {kw: extra.pop(kw.removesuffix("_out")) for kw in maps}, labels=labels,
+                              fused_cloud=cloud, n_points=int(labels.shape[0]), height_norm=hn, extra=extra)
     finally:
         if own:
             grp.close()

@@ -13,6 +13,7 @@
 #include <cstdlib>
 #include <string>
 #include <map>
+#include <utility>
 #include <vector>
 
 #include "../../include/mdkm.h"
@@ -52,6 +53,33 @@ template <typename T>
 struct DevBuf {
   T* p = nullptr;
   size_t cap = 0;  // elements
+};
+
+// The outputs bound for the next fit / predict.  Each mdkm_bind_* call clears and sets its own
+// part; the next fit / predict moves the whole struct out (take_outputs), so every binding is
+// consumed by that call whatever happens.
+struct OutputBindings {
+  // cluster map (mdkm_bind_cluster_map)
+  void* map = nullptr;
+  int map_elem = 0, map_mem = MDKM_MEM_HOST;
+  // per-(day, cluster) statistics (mdkm_bind_day_stats)
+  int64_t* counts = nullptr;
+  double* means = nullptr;
+  int stats_kcap = 0;
+  // day-pair transition counts (mdkm_bind_day_transitions)
+  std::vector<int> pairs;  // [n_pairs][2] days, copied when bound
+  int64_t* trans = nullptr;
+  int trans_kcap = 0;
+  // connected regions (mdkm_bind_regions)
+  int regions = 0;  // connectivity 4 or 8; 0: not bound
+  int32_t* region_map = nullptr;
+  int region_map_mem = MDKM_MEM_HOST;
+  // region overlaps (mdkm_bind_region_overlaps)
+  std::vector<int> ov_pairs;  // [n_pairs][2] days, copied when bound; empty: not bound
+  // object tracks (mdkm_bind_tracks)
+  double track_iou = 0.0;  // min_iou; 0: not bound
+  int32_t* track_map = nullptr;
+  int track_map_mem = MDKM_MEM_HOST;
 };
 
 }  // namespace
@@ -159,27 +187,20 @@ struct mdkm_handle {
   float* bound_cloud_out = nullptr;  // mdkm_bind_cloud_output
   long long bound_cloud_cap = 0;
   int bound_cloud_napari = 1;
+  OutputBindings bound;              // the outputs of the next fit / predict
   // cluster map (mdkm_bind_cluster_map) over the pixel range of the last mdkm_unproject
   long long raster_pix_begin = 0, raster_pix_count = 0;
   int raster_H = 0;                  // (the width is raster_w)
-  void* bound_map = nullptr;
-  int bound_map_elem = 0, bound_map_mem = MDKM_MEM_HOST;
   DevBuf<unsigned char> map_stage;   // host outputs are written here, then copied
   DevBuf<long long> map_seg;         // the days' point offsets (d_seg_off may hold merged segments)
   // per-(day, cluster) statistics (mdkm_bind_day_stats) of the next fit / predict
   int stack_days = 0;                // days of the stack of the last mdkm_unproject (1 after mdkm_set_points)
   long long day0 = 0;                // global day of the resident cloud's first segment
-  int64_t* bound_counts = nullptr;
-  double* bound_means = nullptr;
-  int bound_stats_kcap = 0;
   DevBuf<unsigned long long> stats_acc;  // [days * k * 4] (qx, qy, qz, count) per slot
   DevBuf<unsigned char> stats_dev;       // counts, then means, converted on the device
   unsigned char* stats_host = nullptr;   // pinned: their copy, handed to the caller after the sync
   size_t stats_host_cap = 0;
   // day-pair transition counts (mdkm_bind_day_transitions) of the next fit / predict
-  std::vector<int> bound_pairs;          // [n_pairs][2] days, copied when bound
-  int64_t* bound_trans = nullptr;
-  int bound_trans_kcap = 0;
   DevBuf<int> trans_pairs;
   DevBuf<unsigned long long> trans_bins;  // [n_pairs][(k+1)^2]
   unsigned char* trans_host = nullptr;    // pinned: their copy, handed to the caller after the sync
@@ -191,9 +212,6 @@ struct mdkm_handle {
   // connected regions of the cluster map (mdkm_bind_regions) of the next fit / predict, and those
   // of the last fit / predict that had them, kept on the device until the next unproject /
   // set_points / fit or predict with regions
-  int bound_regions = 0;                 // connectivity 4 or 8; 0: not bound
-  int32_t* bound_region_map = nullptr;
-  int bound_region_map_mem = MDKM_MEM_HOST;
   DevBuf<int> region_parent;             // [stack pixels] union-find parents
   DevBuf<int> region_ids;                // [stack pixels] region map of the whole stack
   DevBuf<unsigned long long> region_scan;  // look-back words of the numbering, then ticket + fault, then R
@@ -203,7 +221,6 @@ struct mdkm_handle {
   long long n_regions = -1;              // R of the last fit / predict with regions; -1: none
   // region overlaps between days (mdkm_bind_region_overlaps) of the next fit / predict, and those
   // of the last fit / predict that had them, with the lifecycle of the regions
-  std::vector<int> bound_ov_pairs;       // [n_pairs][2] days, copied when bound; empty: not bound
   DevBuf<int> ov_pairs;
   DevBuf<long long> ov_tab;              // [n_pairs + 1] slot offsets of the pairs' hash tables
   DevBuf<unsigned long long> ov_slots;   // [slots][2] key, count | ~first << 32
@@ -213,9 +230,6 @@ struct mdkm_handle {
   long long n_overlaps = -1;             // M of the last fit / predict with overlaps; -1: none
   // object tracks (mdkm_bind_tracks) of the next fit / predict, and those of the last fit / predict
   // that had them, with the lifecycle of the regions
-  double bound_track_iou = 0.0;          // min_iou; 0: not bound
-  int32_t* bound_track_map = nullptr;
-  int bound_track_map_mem = MDKM_MEM_HOST;
   DevBuf<int> track_link_day;            // [counted pairs] d of the counted pair (d, d+1), else -1
   DevBuf<int> track_parent;              // [R] union-find parents (region index)
   DevBuf<unsigned int> track_links;      // [2R] links forward, then backward
@@ -1026,6 +1040,16 @@ struct TrackOut {
   std::vector<int> link_day;    // [counted pairs] d of the counted pair (d, d+1), else -1
 };
 
+// The optional outputs taken by one fit / predict (take_outputs).
+struct CallOutputs {
+  MapOut map;
+  StatsOut stats;
+  TransOut trans;
+  RegOut reg;
+  OvOut ov;
+  TrackOut trk;
+};
+
 // page-locked host buffer of at least `bytes` (the stages of results handed over after a sync)
 int ensure_pinned(mdkm_handle* h, unsigned char*& p, size_t& cap, size_t bytes) {
   if (cap >= bytes && p) return MDKM_OK;
@@ -1052,12 +1076,11 @@ int upload_day_offsets(mdkm_handle* h) {
   return MDKM_OK;
 }
 
-// Consumes the binding of mdkm_bind_cluster_map (whatever happens) for a call with k clusters:
-// checks that k fits the element type, stages host outputs, uploads the days' point offsets.
-int take_cluster_map(mdkm_handle* h, int k, MapOut& m) {
-  void* out = h->bound_map;
-  const int elem = h->bound_map_elem, mem = h->bound_map_mem;
-  h->bound_map = nullptr;
+// Takes the cluster map of the bindings `b` for a call with k clusters: checks that k fits the
+// element type, stages host outputs, uploads the days' point offsets.
+int take_cluster_map(mdkm_handle* h, int k, const OutputBindings& b, MapOut& m) {
+  void* out = b.map;
+  const int elem = b.map_elem, mem = b.map_mem;
   if (!out) return MDKM_OK;
   if (k > (elem == 1 ? 255 : 65535))
     return fail(h, MDKM_ERR_INVALID, "k=%d labels do not fit a cluster map of %d-byte elements", k, elem);
@@ -1074,14 +1097,12 @@ int take_cluster_map(mdkm_handle* h, int k, MapOut& m) {
   return upload_day_offsets(h);
 }
 
-// Consumes the binding of mdkm_bind_day_stats (whatever happens) for a call with k clusters:
-// checks k against the bound capacity, sizes the accumulators, uploads the days' point offsets.
-int take_day_stats(mdkm_handle* h, int k, StatsOut& s) {
-  int64_t* counts = h->bound_counts;
-  double* means = h->bound_means;
-  const int kcap = h->bound_stats_kcap;
-  h->bound_counts = nullptr;
-  h->bound_means = nullptr;
+// Takes the day statistics of the bindings `b` for a call with k clusters: checks k against the
+// bound capacity, sizes the accumulators, uploads the days' point offsets.
+int take_day_stats(mdkm_handle* h, int k, const OutputBindings& b, StatsOut& s) {
+  int64_t* counts = b.counts;
+  double* means = b.means;
+  const int kcap = b.stats_kcap;
   if (!counts) return MDKM_OK;
   if (k > kcap) return fail(h, MDKM_ERR_INVALID, "k=%d exceeds the k_capacity %d of the bound day statistics", k, kcap);
   if (k < 1 || k > kMaxK) return MDKM_OK;  // (rejected with the call's own message)
@@ -1150,62 +1171,47 @@ int merge_stack_map(mdkm_handle* h, const MapOut& m) {
   return MDKM_OK;
 }
 
-// Takes the binding of mdkm_bind_day_transitions (`out`, already consumed) for a call with k
-// clusters and its cluster map `m`: checks k against the bound capacity, sets up the whole-stack
-// map, sizes the bins, uploads the pairs.
-int take_transitions(mdkm_handle* h, int k, int64_t* out, MapOut& m, TransOut& t) {
-  if (!out) return MDKM_OK;
-  const int kcap = h->bound_trans_kcap;
+// Takes the day transitions of the bindings `b` for a call with k clusters and its cluster map
+// `m`: checks k against the bound capacity, sets up the whole-stack map, sizes the bins, uploads
+// the pairs.
+int take_transitions(mdkm_handle* h, int k, const OutputBindings& b, MapOut& m, TransOut& t) {
+  if (!b.trans) return MDKM_OK;
+  const int kcap = b.trans_kcap;
   if (k > kcap) return fail(h, MDKM_ERR_INVALID, "k=%d exceeds the k_capacity %d of the bound day transitions", k, kcap);
   if (k < 1 || k > kMaxK) return MDKM_OK;  // (rejected with the call's own message)
   OK(take_stack_map(h, k, m));
-  t.out = out;
-  t.n_pairs = (int)(h->bound_pairs.size() / 2);
+  t.out = b.trans;
+  t.n_pairs = (int)(b.pairs.size() / 2);
   t.k1 = k + 1;
   const size_t words = (size_t)t.n_pairs * t.k1 * t.k1;
   OK(ensure(h, h->trans_bins, words));
-  OK(ensure(h, h->trans_pairs, h->bound_pairs.size()));
-  CU(cudaMemcpyAsync(h->trans_pairs.p, h->bound_pairs.data(), h->bound_pairs.size() * 4, cudaMemcpyHostToDevice,
-                     h->stream));
+  OK(ensure(h, h->trans_pairs, b.pairs.size()));
+  CU(cudaMemcpyAsync(h->trans_pairs.p, b.pairs.data(), b.pairs.size() * 4, cudaMemcpyHostToDevice, h->stream));
   OK(ensure_pinned(h, h->trans_host, h->trans_host_cap, words * 8));
   return MDKM_OK;
 }
 
-// Consumes the binding of mdkm_bind_regions (whatever happens next).
-RegOut consume_regions(mdkm_handle* h) {
-  RegOut g;
-  g.conn = h->bound_regions;
-  g.map = h->bound_region_map;
-  g.mem = h->bound_region_map_mem;
-  h->bound_regions = 0;
-  h->bound_region_map = nullptr;
-  return g;
+// The regions, region overlaps and tracks of an earlier call are dropped.
+void drop_results(mdkm_handle* h) {
+  h->n_regions = -1;
+  h->n_overlaps = -1;
+  h->n_tracks = -1;
 }
 
-// Takes the regions `g` (consumed) for a call with k clusters and its cluster map `m`: sets up the
-// whole-stack map; the regions (and region overlaps) of an earlier call are dropped.
+// Takes the regions `g` for a call with k clusters and its cluster map `m`: sets up the
+// whole-stack map; the results of an earlier call are dropped.
 int take_regions(mdkm_handle* h, int k, MapOut& m, RegOut& g) {
   if (!g.conn) return MDKM_OK;
   if (k < 1 || k > kMaxK) {  // (rejected with the call's own message)
     g.conn = 0;
     return MDKM_OK;
   }
-  h->n_regions = -1;
-  h->n_overlaps = -1;
-  h->n_tracks = -1;
+  drop_results(h);
   return take_stack_map(h, k, m);
 }
 
-// Consumes the binding of mdkm_bind_region_overlaps (whatever happens next).
-OvOut consume_overlaps(mdkm_handle* h) {
-  OvOut o;
-  o.pairs.swap(h->bound_ov_pairs);
-  h->bound_ov_pairs.clear();
-  return o;
-}
-
-// Takes the region overlaps `o` (consumed) of a call whose regions are `g` (before take_regions):
-// they need the regions of the same call; uploads the pairs.
+// Takes the region overlaps `o` of a call whose regions are `g` (before take_regions): they need
+// the regions of the same call; uploads the pairs.
 int take_overlaps(mdkm_handle* h, const RegOut& g, const OvOut& o) {
   if (o.pairs.empty()) return MDKM_OK;
   if (!g.conn) return fail(h, MDKM_ERR_STATE, "region overlaps need regions bound for the same call (mdkm_bind_regions)");
@@ -1215,21 +1221,10 @@ int take_overlaps(mdkm_handle* h, const RegOut& g, const OvOut& o) {
   return MDKM_OK;
 }
 
-// Consumes the binding of mdkm_bind_tracks (whatever happens next).
-TrackOut consume_tracks(mdkm_handle* h) {
-  TrackOut t;
-  t.iou = h->bound_track_iou;
-  t.map = h->bound_track_map;
-  t.mem = h->bound_track_map_mem;
-  h->bound_track_iou = 0.0;
-  h->bound_track_map = nullptr;
-  return t;
-}
-
-// Takes the tracks `t` (consumed) of a call whose regions are `g` and overlaps `o` (before
-// take_overlaps): they need the regions of the same call.  The consecutive pairs (d, d+1) that
-// the caller did not ask for are counted after the caller's pairs, whose rows stay a prefix; the
-// link pass finds the counted pair of every d through link_day.
+// Takes the tracks `t` of a call whose regions are `g` and overlaps `o` (before take_overlaps):
+// they need the regions of the same call.  The consecutive pairs (d, d+1) that the caller did not
+// ask for are counted after the caller's pairs, whose rows stay a prefix; the link pass finds the
+// counted pair of every d through link_day.
 int take_tracks(mdkm_handle* h, const RegOut& g, OvOut& o, TrackOut& t) {
   if (!t.iou) return MDKM_OK;
   if (!g.conn) return fail(h, MDKM_ERR_STATE, "tracks need regions bound for the same call (mdkm_bind_regions)");
@@ -1597,6 +1592,41 @@ int run_tracks(mdkm_handle* h, const TrackOut& t, const OvOut& o, const int* ids
   if (got[0] >> 32) return fail(h, MDKM_ERR_CUDA, "track numbering: the look-back over the chunks timed out");
   h->n_tracks = (long long)got[1];
   h->n_overlaps = t.n_user ? (long long)got[2] : -1;
+  return MDKM_OK;
+}
+
+// Takes the outputs bound for a call with k clusters into `o`.  The bindings are moved out of the
+// handle first, so the call consumes every one of them whatever happens.  When several checks
+// fail the first in this order is reported, except that the cluster map's comes after the day
+// statistics'.
+int take_outputs(mdkm_handle* h, int k, CallOutputs& o) {
+  OutputBindings b = std::exchange(h->bound, OutputBindings{});
+  o.reg = {b.regions, b.region_map, b.region_map_mem};
+  o.ov.pairs = std::move(b.ov_pairs);
+  o.trk = {b.track_iou, b.track_map, b.track_map_mem};
+  const int map_rc = take_cluster_map(h, k, b, o.map);
+  OK(take_day_stats(h, k, b, o.stats));
+  OK(map_rc);
+  OK(take_transitions(h, k, b, o.map, o.trans));
+  OK(take_tracks(h, o.reg, o.ov, o.trk));
+  OK(take_overlaps(h, o.reg, o.ov));
+  return take_regions(h, k, o.map, o.reg);
+}
+
+// Behind the final pass, on the stream: the day statistics, the whole-stack map and the day
+// transitions of `o`.
+int reduce_outputs(mdkm_handle* h, const CallOutputs& o) {
+  OK(reduce_day_stats(h, o.stats));
+  OK(merge_stack_map(h, o.map));
+  return run_transitions(h, o.trans, o.map);
+}
+
+// After the call's synchronisation: the regions of `o` with their overlaps and tracks, then the
+// day statistics and transitions handed to the caller.
+int deliver_outputs(mdkm_handle* h, const CallOutputs& o) {
+  OK(run_regions(h, o.reg, o.map, o.ov, o.trk));
+  deliver_day_stats(h, o.stats);
+  deliver_transitions(h, o.trans);
   return MDKM_OK;
 }
 
@@ -1989,18 +2019,9 @@ int mdkm_set_points(mdkm_handle* h, const float* xyz, int64_t n, int layout, int
   h->seg_off.assign({0, (long long)n});
   h->seg_whole = true;
   h->raster_w = 0;
-  h->bound_map = nullptr;
-  h->bound_counts = nullptr;
-  h->bound_trans = nullptr;
+  h->bound = {};
   h->stack_cover = -1;
-  h->bound_regions = 0;
-  h->bound_region_map = nullptr;
-  h->n_regions = -1;
-  h->bound_ov_pairs.clear();
-  h->n_overlaps = -1;
-  h->bound_track_iou = 0.0;
-  h->bound_track_map = nullptr;
-  h->n_tracks = -1;
+  drop_results(h);
   h->stack_days = 1;
   h->day0 = 0;
   h->runs_ok = false;
@@ -2053,7 +2074,7 @@ int mdkm_bind_cloud_output(mdkm_handle* h, float* out_host, int64_t capacity_poi
 
 int mdkm_bind_cluster_map(mdkm_handle* h, void* out, int elem_bytes, int64_t capacity_pixels, int mem) {
   if (!h) return MDKM_ERR_INVALID;
-  h->bound_map = nullptr;
+  h->bound.map = nullptr;
   if (!out) return MDKM_OK;
   if (!h->have_points || h->raster_w <= 0)
     return fail(h, MDKM_ERR_STATE, "a cluster map needs a resident cloud from mdkm_unproject");
@@ -2063,15 +2084,15 @@ int mdkm_bind_cluster_map(mdkm_handle* h, void* out, int elem_bytes, int64_t cap
   if (capacity_pixels < h->raster_pix_count)
     return fail(h, MDKM_ERR_INVALID, "cluster map holds %lld pixels, the range has %lld", (long long)capacity_pixels,
                 h->raster_pix_count);
-  h->bound_map = out;
-  h->bound_map_elem = elem_bytes;
-  h->bound_map_mem = mem;
+  h->bound.map = out;
+  h->bound.map_elem = elem_bytes;
+  h->bound.map_mem = mem;
   return MDKM_OK;
 }
 
 int mdkm_bind_day_transitions(mdkm_handle* h, const int32_t* pairs, int n_pairs, int64_t* counts_out, int k_capacity) {
   if (!h) return MDKM_ERR_INVALID;
-  h->bound_trans = nullptr;
+  h->bound.trans = nullptr;
   if (!counts_out) return MDKM_OK;
   if (!h->have_points || h->raster_w <= 0)
     return fail(h, MDKM_ERR_STATE, "day transitions need a resident cloud from mdkm_unproject");
@@ -2083,16 +2104,16 @@ int mdkm_bind_day_transitions(mdkm_handle* h, const int32_t* pairs, int n_pairs,
   for (int i = 0; i < 2 * n_pairs; ++i)
     if (pairs[i] < 0 || pairs[i] >= h->stack_days)
       return fail(h, MDKM_ERR_INVALID, "pair %d: day %d is not in [0, %d)", i / 2, (int)pairs[i], h->stack_days);
-  h->bound_pairs.assign(pairs, pairs + 2 * (size_t)n_pairs);
-  h->bound_trans = counts_out;
-  h->bound_trans_kcap = k_capacity;
+  h->bound.pairs.assign(pairs, pairs + 2 * (size_t)n_pairs);
+  h->bound.trans = counts_out;
+  h->bound.trans_kcap = k_capacity;
   return MDKM_OK;
 }
 
 int mdkm_bind_regions(mdkm_handle* h, int connectivity, int32_t* map_out, int64_t capacity_pixels, int mem) {
   if (!h) return MDKM_ERR_INVALID;
-  h->bound_regions = 0;
-  h->bound_region_map = nullptr;
+  h->bound.regions = 0;
+  h->bound.region_map = nullptr;
   if (!connectivity && !map_out) return MDKM_OK;
   if (!h->have_points || h->raster_w <= 0)
     return fail(h, MDKM_ERR_STATE, "regions need a resident cloud from mdkm_unproject");
@@ -2105,9 +2126,9 @@ int mdkm_bind_regions(mdkm_handle* h, int connectivity, int32_t* map_out, int64_
   if (map_out && (capacity_pixels < h->raster_pix_count || (mem != MDKM_MEM_HOST && mem != MDKM_MEM_DEVICE)))
     return fail(h, MDKM_ERR_INVALID, "region map: capacity %lld < %lld pixels, or bad memory kind",
                 (long long)capacity_pixels, h->raster_pix_count);
-  h->bound_regions = connectivity;
-  h->bound_region_map = map_out;
-  h->bound_region_map_mem = mem;
+  h->bound.regions = connectivity;
+  h->bound.region_map = map_out;
+  h->bound.region_map_mem = mem;
   return MDKM_OK;
 }
 
@@ -2134,7 +2155,7 @@ int mdkm_region_table(mdkm_handle* h, int64_t* table_out, double* means_out, int
 
 int mdkm_bind_region_overlaps(mdkm_handle* h, const int32_t* pairs, int n_pairs) {
   if (!h) return MDKM_ERR_INVALID;
-  h->bound_ov_pairs.clear();
+  h->bound.ov_pairs.clear();
   if (!pairs) return MDKM_OK;
   if (!h->have_points || h->raster_w <= 0)
     return fail(h, MDKM_ERR_STATE, "region overlaps need a resident cloud from mdkm_unproject");
@@ -2144,7 +2165,7 @@ int mdkm_bind_region_overlaps(mdkm_handle* h, const int32_t* pairs, int n_pairs)
     if (pairs[i] < 0 || pairs[i] >= h->stack_days)
       return fail(h, MDKM_ERR_INVALID, "region overlap pair %d: day %d is not in [0, %d)", i / 2, (int)pairs[i],
                   h->stack_days);
-  h->bound_ov_pairs.assign(pairs, pairs + 2 * (size_t)n_pairs);
+  h->bound.ov_pairs.assign(pairs, pairs + 2 * (size_t)n_pairs);
   return MDKM_OK;
 }
 
@@ -2171,8 +2192,8 @@ int mdkm_region_overlap_table(mdkm_handle* h, int64_t* table_out, int64_t capaci
 
 int mdkm_bind_tracks(mdkm_handle* h, double min_iou, int32_t* map_out, int64_t capacity_pixels, int mem) {
   if (!h) return MDKM_ERR_INVALID;
-  h->bound_track_iou = 0.0;
-  h->bound_track_map = nullptr;
+  h->bound.track_iou = 0.0;
+  h->bound.track_map = nullptr;
   if (min_iou == 0.0 && !map_out) return MDKM_OK;
   if (!h->have_points || h->raster_w <= 0)
     return fail(h, MDKM_ERR_STATE, "tracks need a resident cloud from mdkm_unproject");
@@ -2183,9 +2204,9 @@ int mdkm_bind_tracks(mdkm_handle* h, double min_iou, int32_t* map_out, int64_t c
   if (map_out && (capacity_pixels < h->raster_pix_count || (mem != MDKM_MEM_HOST && mem != MDKM_MEM_DEVICE)))
     return fail(h, MDKM_ERR_INVALID, "track map: capacity %lld < %lld pixels, or bad memory kind",
                 (long long)capacity_pixels, h->raster_pix_count);
-  h->bound_track_iou = min_iou;
-  h->bound_track_map = map_out;
-  h->bound_track_map_mem = mem;
+  h->bound.track_iou = min_iou;
+  h->bound.track_map = map_out;
+  h->bound.track_map_mem = mem;
   return MDKM_OK;
 }
 
@@ -2218,8 +2239,8 @@ int mdkm_track_table(mdkm_handle* h, int64_t* table_out, int32_t* region_tracks_
 
 int mdkm_bind_day_stats(mdkm_handle* h, int64_t* counts_out, double* means_out, int n_days, int k_capacity) {
   if (!h) return MDKM_ERR_INVALID;
-  h->bound_counts = nullptr;
-  h->bound_means = nullptr;
+  h->bound.counts = nullptr;
+  h->bound.means = nullptr;
   if (!counts_out) return MDKM_OK;
   if (!h->have_points) return fail(h, MDKM_ERR_STATE, "day statistics need a resident cloud");
   if (!means_out) return fail(h, MDKM_ERR_INVALID, "day statistics need a means array");
@@ -2227,9 +2248,9 @@ int mdkm_bind_day_stats(mdkm_handle* h, int64_t* counts_out, double* means_out, 
     return fail(h, MDKM_ERR_INVALID, "n_days=%d, the resident cloud's stack has %d days", n_days, h->stack_days);
   if (k_capacity < 1 || (long long)n_days * k_capacity >= (1ll << 29))  // (slot indices are int32 on the device)
     return fail(h, MDKM_ERR_INVALID, "k_capacity must be >= 1 and n_days * k_capacity < 2^29");
-  h->bound_counts = counts_out;
-  h->bound_means = means_out;
-  h->bound_stats_kcap = k_capacity;
+  h->bound.counts = counts_out;
+  h->bound.means = means_out;
+  h->bound.stats_kcap = k_capacity;
   return MDKM_OK;
 }
 
@@ -2246,18 +2267,9 @@ int mdkm_unproject(mdkm_handle* h, const void* hm, int hm_dtype, float hm_scale,
   const int cloud_napari = h->bound_cloud_napari;
   h->bound_cloud_out = nullptr;
   h->bound_cloud_cap = 0;
-  h->bound_map = nullptr;  // (a cluster map describes the range it was bound for)
-  h->bound_counts = nullptr;  // (and day statistics the stack)
-  h->bound_trans = nullptr;
+  h->bound = {};  // (the outputs describe the range and the stack they were bound for)
   h->stack_cover = -1;
-  h->bound_regions = 0;  // (and regions the stack)
-  h->bound_region_map = nullptr;
-  h->n_regions = -1;
-  h->bound_ov_pairs.clear();
-  h->n_overlaps = -1;
-  h->bound_track_iou = 0.0;
-  h->bound_track_map = nullptr;
-  h->n_tracks = -1;
+  drop_results(h);
   if (D < 0 || H <= 0 || W <= 0 || pix_begin < 0 || pix_count < 0 ||
       pix_begin + pix_count > (int64_t)D * H * W || (pix_count > 0 && !hm))
     return fail(h, MDKM_ERR_INVALID, "bad stack geometry");
@@ -2538,21 +2550,8 @@ int mdkm_wait(mdkm_handle* h) {
 int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol, int32_t* labels_out,
              int labels_mem, double* centroids_out, int* n_iter_out, double* inertia_out) {
   if (!h) return MDKM_ERR_INVALID;
-  MapOut map;
-  StatsOut stats;
-  TransOut trans;
-  int64_t* trans_out = h->bound_trans;
-  h->bound_trans = nullptr;
-  RegOut reg = consume_regions(h);
-  OvOut ov = consume_overlaps(h);
-  TrackOut trk = consume_tracks(h);
-  const int map_rc = take_cluster_map(h, k, map);
-  OK(take_day_stats(h, k, stats));
-  OK(map_rc);
-  OK(take_transitions(h, k, trans_out, map, trans));
-  OK(take_tracks(h, reg, ov, trk));
-  OK(take_overlaps(h, reg, ov));
-  OK(take_regions(h, k, map, reg));
+  CallOutputs outs;
+  OK(take_outputs(h, k, outs));
   if (!init) return fail(h, MDKM_ERR_INVALID, "init centroids required");
   OK(check_centroids(h, k, init, "init"));
   if (max_iter < 1) return fail(h, MDKM_ERR_INVALID, "max_iter must be >= 1");
@@ -2674,12 +2673,10 @@ int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol
       const int span = prof_begin(h, MDKM_PHASE_FINAL, h->n);
       // (a pause leaves the map alone: the pass after the relocation writes it)
       OK(run_final(h, kb, labels_dev, /*skip_paused=*/true, centroids_host, one_rank ? &h->h_status[0] : nullptr,
-                   &map, &stats));
+                   &outs.map, &outs.stats));
       prof_end(h, span);
     }
-    OK(reduce_day_stats(h, stats));
-    OK(merge_stack_map(h, map));
-    OK(run_transitions(h, trans, map));
+    OK(reduce_outputs(h, outs));
     if (!one_rank) {
       OK(ensure(h, h->dscratch, (size_t)k * 3 + 16));
       read_table_kernel<<<(k + 255) / 256, 256, 0, h->stream>>>(h->table.p, k, kb.kpad, h->fr, h->dscratch.p);
@@ -2691,7 +2688,7 @@ int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol
     }
     if (labels_out && labels_mem != MDKM_MEM_DEVICE && h->n > 0)
       CU(cudaMemcpyAsync(labels_out, labels_dev, (size_t)h->n * 4, cudaMemcpyDeviceToHost, h->stream));
-    OK(copy_cluster_map(h, map));
+    OK(copy_cluster_map(h, outs.map));
     OK(sync_small(h));
     if (h->h_status[0].paused && !h->h_status[0].done && !h->h_status[0].xchg_timeout) {
       // an update of the last batch, or the settle kernel, found an empty cluster: relocate, go on
@@ -2713,9 +2710,7 @@ int mdkm_fit(mdkm_handle* h, int k, const double* init, int max_iter, double tol
 #endif
   if (fin.xchg_timeout == 2) return index_fault(h);
   if (fin.xchg_timeout) return fail(h, MDKM_ERR_NCCL, "a kernel-side wait timed out (peer exchange of the partial sums: a rank is missing; or the grid barrier)");
-  OK(run_regions(h, reg, map, ov, trk));
-  deliver_day_stats(h, stats);
-  deliver_transitions(h, trans);
+  OK(deliver_outputs(h, outs));
   if (n_iter_out) *n_iter_out = fin.iter;
   if (inertia_out) *inertia_out = fin.inertia;
   h->stat_refined = (long long)fin.n_refined;
@@ -2788,21 +2783,8 @@ int mdkm_lloyd_step(mdkm_handle* h, int k, const double* centroids, int32_t* lab
 int mdkm_predict(mdkm_handle* h, int k, const double* centroids, int32_t* labels_out, int labels_mem,
                  double* inertia_out) {
   if (!h) return MDKM_ERR_INVALID;
-  MapOut map;
-  StatsOut stats;
-  TransOut trans;
-  int64_t* trans_out = h->bound_trans;
-  h->bound_trans = nullptr;
-  RegOut reg = consume_regions(h);
-  OvOut ov = consume_overlaps(h);
-  TrackOut trk = consume_tracks(h);
-  const int map_rc = take_cluster_map(h, k, map);
-  OK(take_day_stats(h, k, stats));
-  OK(map_rc);
-  OK(take_transitions(h, k, trans_out, map, trans));
-  OK(take_tracks(h, reg, ov, trk));
-  OK(take_overlaps(h, reg, ov));
-  OK(take_regions(h, k, map, reg));
+  CallOutputs outs;
+  OK(take_outputs(h, k, outs));
   if (!centroids) return fail(h, MDKM_ERR_INVALID, "centroids required");
   OK(check_centroids(h, k, centroids, "centroids"));
   CU(cudaSetDevice(h->device));
@@ -2822,20 +2804,16 @@ int mdkm_predict(mdkm_handle* h, int k, const double* centroids, int32_t* labels
       labels_dev = h->labels32.p;
     }
   }
-  OK(run_final(h, kb, labels_dev, false, nullptr, nullptr, &map, &stats));
+  OK(run_final(h, kb, labels_dev, false, nullptr, nullptr, &outs.map, &outs.stats));
   if (h->n_ranks > 1) OK(allreduce(h, &h->d_status->inertia, 1, kNcclFloat64, kNcclSum));
-  OK(reduce_day_stats(h, stats));
-  OK(merge_stack_map(h, map));
-  OK(run_transitions(h, trans, map));
+  OK(reduce_outputs(h, outs));
   OK(small_d2h(h, &h->h_status[0], h->d_status, sizeof(DevStatus), /*dst_is_pinned=*/true));
   if (labels_out && labels_mem != MDKM_MEM_DEVICE && h->n > 0)
     CU(cudaMemcpyAsync(labels_out, labels_dev, (size_t)h->n * 4, cudaMemcpyDeviceToHost, h->stream));
-  OK(copy_cluster_map(h, map));
+  OK(copy_cluster_map(h, outs.map));
   OK(sync_small(h));
   if (h->h_status[0].xchg_timeout == 2) return index_fault(h);
-  OK(run_regions(h, reg, map, ov, trk));
-  deliver_day_stats(h, stats);
-  deliver_transitions(h, trans);
+  OK(deliver_outputs(h, outs));
   if (inertia_out) *inertia_out = h->h_status[0].inertia;
   h->stat_refined = (long long)h->h_status[0].n_refined;
   h->stat_reloc = 0;

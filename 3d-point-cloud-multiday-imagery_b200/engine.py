@@ -84,6 +84,12 @@ def _as_out_buffer(a, dtype, n_elems, what):
     return a.ctypes.data, C.MEM_HOST
 
 
+def _day_pairs(pairs) -> np.ndarray:
+    """Day pairs ``[P,2]`` as int32, clipped so that the library refuses out-of-range days."""
+    return np.ascontiguousarray(np.clip(np.asarray(pairs, dtype=np.int64).reshape(-1, 2), -1, 2**31 - 1),
+                                dtype=np.int32)
+
+
 class Engine:
     """Owns one ``mdkm_handle``.  Use as a context manager or call ``close()``."""
 
@@ -370,15 +376,23 @@ class Engine:
         cloud came from ``set_points`` (or there is none)."""
         return self._raster
 
+    def _pixel_map(self, out, dtype, what):
+        """-> (pointer, memory kind, capacity) of the caller's pixel map ``out`` (one element per pixel
+        of the last unprojected range), or (None, host, 0) without one."""
+        if out is None:
+            return None, C.MEM_HOST, 0
+        cap = self._raster[4] if self._raster is not None else (out.numel() if _is_torch(out) else np.size(out))
+        ptr, mem = _as_out_buffer(out, dtype, cap, what)
+        if mem == C.MEM_DEVICE:
+            self._after_torch(out)  # earlier work on torch's stream may still use the buffer
+        return ptr, mem, cap
+
     def _bind_cluster_map(self, out):
         """Bind ``out`` (uint8 / uint16, one element per pixel of the last unprojected range) as the
         cluster map of the next fit / predict.  -> its memory kind."""
-        n_pix = self._raster[4] if self._raster is not None else (out.numel() if _is_torch(out) else np.size(out))
-        ptr, mem = _as_out_buffer(out, (np.uint8, np.uint16), n_pix, "cluster_map_out")
+        ptr, mem, n_pix = self._pixel_map(out, (np.uint8, np.uint16), "cluster_map_out")
         elem = out.element_size() if _is_torch(out) else out.itemsize
         self._check(self._lib.mdkm_bind_cluster_map(self._h, c_void_p(ptr), int(elem), int(n_pix), mem))
-        if mem == C.MEM_DEVICE:
-            self._after_torch(out)  # earlier work on torch's stream may still use the buffer
         return mem
 
     @property
@@ -400,7 +414,7 @@ class Engine:
     def _bind_day_transitions(self, pairs, k):
         """Bind the day pairs ``pairs`` (``[P,2]`` global days) and a fresh int64 ``[P,k+1,k+1]``
         array to the next fit / predict.  -> the array."""
-        pr = np.clip(np.asarray(pairs, dtype=np.int64).reshape(-1, 2), -1, 2**31 - 1).astype(np.int32)
+        pr = _day_pairs(pairs)
         counts = np.empty((pr.shape[0], k + 1, k + 1), dtype=np.int64)
         self._check(self._lib.mdkm_bind_day_transitions(self._h, c_void_p(pr.ctypes.data), int(pr.shape[0]),
                                                         c_void_p(counts.ctypes.data), int(k)))
@@ -409,17 +423,11 @@ class Engine:
     def _bind_regions(self, connectivity, out):
         """Bind connected regions (``connectivity`` 4 or 8) and the optional int32 region map ``out``
         (one element per pixel of the last unprojected range) to the next fit / predict.  -> the
-        map's memory kind (None without a map)."""
+        map's memory kind (host without a map)."""
         if connectivity not in (4, 8) or isinstance(connectivity, bool):
             raise ValueError(f"regions must be 4 or 8 (the connectivity), got {connectivity!r}")
-        ptr, mem, cap = None, None, 0
-        if out is not None:
-            cap = self._raster[4] if self._raster is not None else (out.numel() if _is_torch(out) else np.size(out))
-            ptr, mem = _as_out_buffer(out, np.int32, cap, "region_map_out")
-        self._check(self._lib.mdkm_bind_regions(self._h, int(connectivity), c_void_p(ptr) if ptr else None, int(cap),
-                                                C.MEM_HOST if mem is None else mem))
-        if mem == C.MEM_DEVICE:
-            self._after_torch(out)  # earlier work on torch's stream may still use the buffer
+        ptr, mem, cap = self._pixel_map(out, np.int32, "region_map_out")
+        self._check(self._lib.mdkm_bind_regions(self._h, int(connectivity), c_void_p(ptr), int(cap), mem))
         return mem
 
     def _region_table(self):
@@ -436,8 +444,7 @@ class Engine:
     def _bind_region_overlaps(self, pairs):
         """Bind the day pairs ``pairs`` (``[P,2]`` global days) of region overlaps to the next fit /
         predict."""
-        pr = np.ascontiguousarray(np.clip(np.asarray(pairs, dtype=np.int64).reshape(-1, 2), -1, 2**31 - 1),
-                                  dtype=np.int32)
+        pr = _day_pairs(pairs)
         self._check(self._lib.mdkm_bind_region_overlaps(self._h, c_void_p(pr.ctypes.data), int(pr.shape[0])))
 
     def _region_overlap_table(self):
@@ -451,16 +458,10 @@ class Engine:
     def _bind_tracks(self, min_iou, out):
         """Bind object tracks (``min_iou`` in (0, 1]) and the optional int32 track map ``out`` (one
         element per pixel of the last unprojected range) to the next fit / predict.  -> the map's
-        memory kind (None without a map)."""
+        memory kind (host without a map)."""
         iou = check_min_iou(min_iou)
-        ptr, mem, cap = None, None, 0
-        if out is not None:
-            cap = self._raster[4] if self._raster is not None else (out.numel() if _is_torch(out) else np.size(out))
-            ptr, mem = _as_out_buffer(out, np.int32, cap, "track_map_out")
-        self._check(self._lib.mdkm_bind_tracks(self._h, iou, c_void_p(ptr) if ptr else None, int(cap),
-                                               C.MEM_HOST if mem is None else mem))
-        if mem == C.MEM_DEVICE:
-            self._after_torch(out)  # earlier work on torch's stream may still use the buffer
+        ptr, mem, cap = self._pixel_map(out, np.int32, "track_map_out")
+        self._check(self._lib.mdkm_bind_tracks(self._h, iou, c_void_p(ptr), int(cap), mem))
         return mem
 
     def _track_table(self):
@@ -475,13 +476,13 @@ class Engine:
                                                c_void_p(region_tracks.ctypes.data), int(n.value), int(r.value)))
         return table, region_tracks
 
-    def _bind_outputs(self, k, cluster_map_out, day_stats, transitions, regions=None, region_map_out=None,
-                      region_overlaps=None, tracks=None, track_map_out=None):
-        """Bind the optional outputs of the next fit / predict -> (map memory kind, (counts, means),
-        transitions, region map memory kind, track map memory kind), each None when not asked for.
-        When one binding is refused none is left behind: the statistics and transition arrays live
-        only in this call, and a binding that outlived them would have the next fit / predict write
-        into freed memory."""
+    def _bind_outputs(self, k, cluster_map_out=None, day_stats=False, transitions=None, regions=None,
+                      region_map_out=None, region_overlaps=None, tracks=None, track_map_out=None):
+        """Bind the optional outputs of the next fit / predict (the keywords of ``fit``) -> (whether
+        a pixel map is device memory, (counts, means) or None, transitions or None).  When one
+        binding is refused none is left behind: the statistics and transition arrays live only in
+        this call, and a binding that outlived them would have the next fit / predict write into
+        freed memory."""
         if region_map_out is not None and regions is None:
             raise ValueError("region_map_out needs regions=4 or regions=8")
         if region_overlaps is not None and regions is None:
@@ -506,7 +507,23 @@ class Engine:
             self._lib.mdkm_bind_region_overlaps(self._h, None, 0)
             self._lib.mdkm_bind_tracks(self._h, 0.0, None, 0, C.MEM_HOST)
             raise
-        return map_mem, stats, trans, reg_mem, trk_mem
+        return C.MEM_DEVICE in (map_mem, reg_mem, trk_mem), stats, trans
+
+    def _read_outputs(self, stats, trans, regions, region_overlaps, tracks) -> dict:
+        """The optional results of the last fit / predict that were asked for, in ``predict``'s order:
+        day_counts, day_means, transitions, regions, region_means, region_overlaps, tracks, region_tracks."""
+        out = {}
+        if stats is not None:
+            out["day_counts"], out["day_means"] = stats
+        if trans is not None:
+            out["transitions"] = trans
+        if regions is not None:
+            out["regions"], out["region_means"] = self._region_table()
+        if region_overlaps is not None:
+            out["region_overlaps"] = self._region_overlap_table()
+        if tracks is not None:
+            out["tracks"], out["region_tracks"] = self._track_table()
+        return out
 
     @property
     def segment_offsets(self) -> np.ndarray:
@@ -600,14 +617,14 @@ class Engine:
         centers = np.empty((k, 3), dtype=np.float64)
         n_iter = c_int(0)
         inertia = c_double(0.0)
-        map_mem, stats, trans, reg_mem, trk_mem = self._bind_outputs(k, cluster_map_out, day_stats, transitions,
-                                                                     regions, region_map_out, region_overlaps,
-                                                                     tracks, track_map_out)
+        dev_maps, stats, trans = self._bind_outputs(
+            k, cluster_map_out=cluster_map_out, day_stats=day_stats, transitions=transitions, regions=regions,
+            region_map_out=region_map_out, region_overlaps=region_overlaps, tracks=tracks, track_map_out=track_map_out)
         self._check(self._lib.mdkm_fit(
             self._h, int(k), init.ctypes.data_as(POINTER(c_double)), int(max_iter), float(tol),
             c_void_p(lab_ptr) if lab_ptr else None, lab_mem,
             centers.ctypes.data_as(POINTER(c_double)), byref(n_iter), byref(inertia)))
-        if C.MEM_DEVICE in (lab_mem, map_mem, reg_mem, trk_mem):
+        if lab_mem == C.MEM_DEVICE or dev_maps:
             self._before_torch()
         nref, nrel, tols = c_int64(0), c_int64(0), c_double(0)
         self._lib.mdkm_fit_stats(self._h, byref(nref), byref(nrel), byref(tols))
@@ -619,16 +636,7 @@ class Engine:
             "n_relocations": int(nrel.value), "tol_scaled": float(tols.value),
             "worklist_groups": int(work.value), "groups": int(groups.value),
         }
-        if stats is not None:
-            out["day_counts"], out["day_means"] = stats
-        if trans is not None:
-            out["transitions"] = trans
-        if regions is not None:
-            out["regions"], out["region_means"] = self._region_table()
-        if region_overlaps is not None:
-            out["region_overlaps"] = self._region_overlap_table()
-        if tracks is not None:
-            out["tracks"], out["region_tracks"] = self._track_table()
+        out.update(self._read_outputs(stats, trans, regions, region_overlaps, tracks))
         return out
 
     def lloyd_step(self, centroids, want_labels=True):
@@ -661,26 +669,16 @@ class Engine:
             raise ValueError("centroids must be [K,3]")
         labels = self._result_buffer("labels", (self.n_points,), np.int32) if want_labels else None
         inertia = c_double(0.0)
-        map_mem, stats, trans, reg_mem, trk_mem = self._bind_outputs(c.shape[0], cluster_map_out, day_stats,
-                                                                     transitions, regions, region_map_out,
-                                                                     region_overlaps, tracks, track_map_out)
+        dev_maps, stats, trans = self._bind_outputs(
+            c.shape[0], cluster_map_out=cluster_map_out, day_stats=day_stats, transitions=transitions, regions=regions,
+            region_map_out=region_map_out, region_overlaps=region_overlaps, tracks=tracks, track_map_out=track_map_out)
         self._check(self._lib.mdkm_predict(
             self._h, int(c.shape[0]), c.ctypes.data_as(POINTER(c_double)),
             c_void_p(labels.ctypes.data) if labels is not None else None, C.MEM_HOST, byref(inertia)))
-        if C.MEM_DEVICE in (map_mem, reg_mem, trk_mem):
+        if dev_maps:
             self._before_torch()
-        out = (labels, float(inertia.value))
-        if stats is not None:
-            out += stats
-        if trans is not None:
-            out += (trans,)
-        if regions is not None:
-            out += self._region_table()
-        if region_overlaps is not None:
-            out += (self._region_overlap_table(),)
-        if tracks is not None:
-            out += self._track_table()
-        return out
+        results = self._read_outputs(stats, trans, regions, region_overlaps, tracks)
+        return (labels, float(inertia.value)) + tuple(results.values())
 
     def kmeans_plusplus(self, n_clusters: int, random_state):
         """k-means++ seeding (sklearn/_kmeans.py:180-278); RNG draws come from ``random_state``

@@ -90,18 +90,15 @@ class DeviceGroup:
 
     # -- the fused path -------------------------------------------------------------------
     def fuse(self, height_maps, valid_masks=None, *, run_kmeans: Callable, max_abs_height=144.0, detrend=False,
-             disparity_scale=None, ground_level=False, return_cloud=True, raster_layout=None, cluster_map_dtype=None,
-             region_map=False, track_map=False):
+             disparity_scale=None, ground_level=False, return_cloud=True, raster_layout=None, maps=None):
         """Shard a HOST stack over the devices by row bands (whole days when ``detrend`` or
         ``ground_level`` need them), unproject, cluster, and assemble labels / cloud in the
         reference's point order.  ``run_kmeans(engine, labels_out) -> dict`` is ``api._run_kmeans``
         bound to the k-means arguments; it runs on every rank (the collectives inside pair up).
-        ``cluster_map_dtype`` (uint8 / uint16): also build the ``[D,H,W]`` cluster map; every rank
-        writes its row band of it in place (``run_kmeans(engine, labels_out, cluster_map_out)``)
-        and it is returned as ``extra["cluster_map"]``.  ``region_map``: likewise the int32 ``[D,H,W]``
-        region map (``run_kmeans(..., region_map_out=band)``), returned as ``extra["region_map"]``,
-        and ``track_map``: the int32 ``[D,H,W]`` track map (``track_map_out=band``), returned as
-        ``extra["track_map"]``.
+        ``maps`` (``{keyword: dtype}``, e.g. ``{"cluster_map_out": np.uint8}``): also build these
+        ``[D,H,W]`` pixel maps; every rank writes its row band of each in place
+        (``run_kmeans(engine, labels_out, cluster_map_out=band, ...)``), and each is returned as
+        ``extra`` under its keyword without "_out" (``extra["cluster_map"]``).
         Returns ``(result dict of rank 0, labels, cloud or None, height_norm or None, extra)``."""
         hm = height_maps
         if type(hm).__module__.startswith("torch"):
@@ -141,22 +138,14 @@ class DeviceGroup:
         n_total = int(offs[-1])
         labels = np.empty(n_total, dtype=np.int32)
         cloud = np.empty((n_total, 3), dtype=np.float32) if return_cloud else None
-        cmap = np.empty(D * H * W, dtype=cluster_map_dtype) if cluster_map_dtype is not None else None
-        rmap = np.empty(D * H * W, dtype=np.int32) if region_map else None
-        tmap = np.empty(D * H * W, dtype=np.int32) if track_map else None
+        whole = {kw: np.empty(D * H * W, dtype=dtype) for kw, dtype in (maps or {}).items()}
 
         def cluster(r):
             eng = self.engines[r]
             a, b = int(offs[r]), int(offs[r + 1])
             if cloud is not None and b > a:
                 eng.get_cloud(napari_order=True, out=cloud[a:b], wait=False)  # overlaps the Lloyd loop
-            kw = {} if rmap is None else {"region_map_out": rmap[spans[r][0]:spans[r][1]]}
-            if tmap is not None:
-                kw["track_map_out"] = tmap[spans[r][0]:spans[r][1]]
-            if cmap is not None:
-                res = run_kmeans(eng, labels[a:b], cmap[spans[r][0]:spans[r][1]], **kw)
-            else:
-                res = run_kmeans(eng, labels[a:b], **kw)
+            res = run_kmeans(eng, labels[a:b], **{kw: m[spans[r][0]:spans[r][1]] for kw, m in whole.items()})
             eng.wait()
             return res
 
@@ -176,12 +165,8 @@ class DeviceGroup:
                 seg = np.diff(ups[r][1])
                 day_counts[d_first:d_first + seg.shape[0]] += seg
         extra["segment_offsets"] = np.concatenate([[0], np.cumsum(day_counts)]).astype(np.int64)
-        if cmap is not None:
-            extra["cluster_map"] = cmap.reshape(D, H, W)
-        if rmap is not None:
-            extra["region_map"] = rmap.reshape(D, H, W)
-        if tmap is not None:
-            extra["track_map"] = tmap.reshape(D, H, W)
+        for kw, m in whole.items():
+            extra[kw.removesuffix("_out")] = m.reshape(D, H, W)
         return results[0], labels, cloud, hn, extra
 
 
