@@ -68,6 +68,9 @@ SIGNATURES = {
     "mdkm_bind_tracks": (c_int, [c_void_p, c_double, c_void_p, c_int64, c_int]),
     "mdkm_track_count": (c_int, [c_void_p, POINTER(c_int64)]),
     "mdkm_track_table": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64]),
+    "mdkm_bind_region_adjacency": (c_int, [c_void_p, c_int]),
+    "mdkm_region_adjacency_count": (c_int, [c_void_p, POINTER(c_int64)]),
+    "mdkm_region_adjacency_table": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64]),
     "mdkm_set_points": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_int]),
     "mdkm_num_points": (c_int64, [c_void_p]),
     "mdkm_num_points_global": (c_int64, [c_void_p]),

@@ -82,6 +82,12 @@ class FusionResult:
     tracks: Optional[np.ndarray] = None
     region_tracks: Optional[np.ndarray] = None
     track_map: Optional[np.ndarray] = None
+    # region adjacency within a day (return_region_adjacency): one row per pair of regions a < b of
+    # one day that share an edge -- int64 [M,6] (day, region_a, region_b, edges, y_first, x_first),
+    # sorted by their first edge -- and per region int64 [R,4] (perimeter, region_edges,
+    # background_edges, border_edges); over the whole stack on every rank
+    region_adjacency: Optional[np.ndarray] = None
+    region_boundaries: Optional[np.ndarray] = None
 
     # scikit-learn style aliases
     @property
@@ -326,7 +332,7 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
                          return_day_stats=False, return_transitions=False, return_regions=False,
                          region_connectivity=4, return_region_map=False,
                          return_region_overlaps=False, return_tracks=False, track_min_iou=0.5,
-                         return_track_map=False) -> FusionResult:
+                         return_track_map=False, return_region_adjacency=False) -> FusionResult:
     """Unproject a multi-day height-map stack into one XYZ cloud and cluster it (Lloyd).
 
     height_maps : float32 ``[D,H,W]`` (NaN = nodata), numpy or torch (CPU or CUDA); or int16
@@ -392,6 +398,18 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
         the GPU from the region map; every rank of a pre-sharded call receives the same rows.
         Out-of-range days, or more than ``MAX_REGION_OVERLAP_PAIRS``
         (8192) pairs, raise ``ValueError`` before any GPU work.
+    return_region_adjacency : also return which regions of one day touch and each region's
+        perimeter.  ``region_adjacency``, int64 ``[M,6]`` rows (day, region_a, region_b, edges,
+        y_first, x_first): one for every pair of regions a < b of one day joined by at least one
+        edge between 4-neighbouring pixels, with the number of such edges (the length of their
+        shared border) and the upper or left pixel of their first edge, sorted by that edge (index
+        ``2 (y W + x) + direction`` within the day, direction 0 to the right, 1 downwards).
+        Regions that touch only at a corner have no row.  ``region_boundaries``, int64 ``[R,4]``
+        (perimeter, region_edges, background_edges, border_edges; region r at index r - 1): the
+        sides of a region's pixels facing another region, a pixel without a point and the raster
+        edge, and their sum (``4 pixels = perimeter + 2 x inner edges``).  Implies
+        ``return_regions``; counted on the GPU from the region map, and every rank of a
+        pre-sharded call receives the same rows.
     return_tracks : also return object tracks -- which region is the same object over the stack.
         Region r of day d and region s of day d+1 are linked when they have the same cluster and
         share at least one pixel with ``shared / (pixels_r + pixels_s - shared) >= track_min_iou``
@@ -423,10 +441,10 @@ def fuse_multiday_kmeans(height_maps, valid_masks=None, *, n_clusters=8, init="k
             raise ValueError(f"return_region_overlaps asks for {ov_pairs.shape[0]} pairs, at most "
                              f"{MAX_REGION_OVERLAP_PAIRS} are allowed")
     min_iou = requested_min_iou(return_tracks, track_min_iou, return_track_map)
-    conn = requested_connectivity(return_regions or ov_pairs is not None or min_iou is not None, region_connectivity,
-                                  return_region_map)
+    conn = requested_connectivity(return_regions or ov_pairs is not None or min_iou is not None
+                                  or return_region_adjacency, region_connectivity, return_region_map)
     outputs = {"day_stats": return_day_stats, "transitions": pairs, "regions": conn, "region_overlaps": ov_pairs,
-               "tracks": min_iou}
+               "tracks": min_iou, "region_adjacency": bool(return_region_adjacency)}
     wanted = (return_cluster_map, return_region_map, return_track_map)
     maps = [kw for kw, want in zip(PIXEL_MAP_OUTPUTS, wanted) if want]
     if devices is not None or isinstance(engine, DeviceGroup):
@@ -482,6 +500,7 @@ def _fusion_result(r, outputs, maps, **fields) -> FusionResult:
                         regions=r.get("regions"), region_means=r.get("region_means"),
                         region_overlaps=r.get("region_overlaps"), region_overlap_pairs=outputs["region_overlaps"],
                         tracks=r.get("tracks"), region_tracks=r.get("region_tracks"),
+                        region_adjacency=r.get("region_adjacency"), region_boundaries=r.get("region_boundaries"),
                         **{kw.removesuffix("_out"): m for kw, m in maps.items()}, **fields)
 
 

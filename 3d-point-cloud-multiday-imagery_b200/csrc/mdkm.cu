@@ -23,6 +23,7 @@
 #include "lloyd.cuh"
 #include "mirror.cuh"
 #include "nccl_shim.h"
+#include "region_adjacency.cuh"
 #include "region_overlaps.cuh"
 #include "regions.cuh"
 #include "seeding.cuh"
@@ -80,6 +81,8 @@ struct OutputBindings {
   double track_iou = 0.0;  // min_iou; 0: not bound
   int32_t* track_map = nullptr;
   int track_map_mem = MDKM_MEM_HOST;
+  // region adjacency (mdkm_bind_region_adjacency)
+  bool adjacency = false;
 };
 
 }  // namespace
@@ -238,6 +241,17 @@ struct mdkm_handle {
   DevBuf<long long> track_tab;           // int64 [R][7]: the first T rows are the track table
   DevBuf<int> track_stage;               // a host track map is written here, then copied
   long long n_tracks = -1;               // T of the last fit / predict with tracks; -1: none
+  // region adjacency within a day (mdkm_bind_region_adjacency) of the next fit / predict, and that
+  // of the last fit / predict that had it, with the lifecycle of the regions
+  DevBuf<long long> adj_tab;             // [D + 1] slot offsets of the days' hash tables
+  DevBuf<unsigned long long> adj_slots;  // [slots][2] key, count | ~first edge << 32
+  DevBuf<unsigned int> adj_bits;         // first-edge masks, then word offsets within the scan chunks
+  DevBuf<unsigned long long> adj_scan;   // look-back words, chunk offsets, ticket + fault, M, probe fault
+  DevBuf<long long> adj_rows;            // int64 [M][6]
+  DevBuf<unsigned long long> adj_sides;  // int64 [R][4] region boundaries
+  unsigned char* adj_bounds = nullptr;   // pinned: the days' bounds, read with R
+  size_t adj_bounds_cap = 0;
+  long long n_adjacency = -1;            // M of the last fit / predict with adjacency; -1: none
 
   // communicator
   ncclComm_t comm = nullptr;
@@ -1048,6 +1062,7 @@ struct CallOutputs {
   RegOut reg;
   OvOut ov;
   TrackOut trk;
+  bool adj = false;  // region adjacency (mdkm_bind_region_adjacency)
 };
 
 // page-locked host buffer of at least `bytes` (the stages of results handed over after a sync)
@@ -1191,11 +1206,12 @@ int take_transitions(mdkm_handle* h, int k, const OutputBindings& b, MapOut& m, 
   return MDKM_OK;
 }
 
-// The regions, region overlaps and tracks of an earlier call are dropped.
+// The regions, region overlaps, tracks and region adjacency of an earlier call are dropped.
 void drop_results(mdkm_handle* h) {
   h->n_regions = -1;
   h->n_overlaps = -1;
   h->n_tracks = -1;
+  h->n_adjacency = -1;
 }
 
 // Takes the regions `g` for a call with k clusters and its cluster map `m`: sets up the
@@ -1248,6 +1264,15 @@ int take_tracks(mdkm_handle* h, const RegOut& g, OvOut& o, TrackOut& t) {
   CU(cudaMemcpyAsync(h->track_link_day.p, t.link_day.data(), t.link_day.size() * 4, cudaMemcpyHostToDevice,
                      h->stream));
   return MDKM_OK;
+}
+
+// Takes the region adjacency of a call whose regions are `g` (before take_regions): it needs the
+// regions of the same call; sizes the pinned stage of the days' bounds.
+int take_adjacency(mdkm_handle* h, const RegOut& g, bool adj) {
+  if (!adj) return MDKM_OK;
+  if (!g.conn) return fail(h, MDKM_ERR_STATE, "region adjacency needs regions bound for the same call (mdkm_bind_regions)");
+  CU(cudaSetDevice(h->device));
+  return ensure_pinned(h, h->adj_bounds, h->adj_bounds_cap, (size_t)h->stack_days * 8);
 }
 
 typedef void (*TransKernel)(const TransParams);
@@ -1343,6 +1368,7 @@ void deliver_day_stats(mdkm_handle* h, const StatsOut& s) {
 
 int run_overlaps(mdkm_handle* h, const OvOut& o, const int* ids, const unsigned long long* bounds);
 int run_tracks(mdkm_handle* h, const TrackOut& t, const OvOut& o, const int* ids);
+int run_adjacency(mdkm_handle* h, bool adj, const int* ids, const unsigned long long* bounds);
 
 // The pair-independent part of the overlap kernels' parameters.
 OverlapParams overlap_params(mdkm_handle* h, const int* ids, int n_pairs) {
@@ -1365,21 +1391,23 @@ dim3 overlap_span_grid(long long HW, int n_pairs) {
 // The regions `g` of the whole-stack map `m`, after the call's synchronisation (the map is final,
 // also after a relocation).  Every rank labels the whole stack: tile-local union-find, links
 // across the tile borders, ids of the roots, every pixel's id (regions.cuh); the caller's region
-// map receives this rank's range.  One synchronisation reads R -- and, with region overlaps `o`,
-// the bounds of their pairs, counted right behind the ids -- then this rank's points are
-// summed into per-region slots, the slots are reduced over the ranks (sums; minima of the
-// first pixel and the bounds) and the table and means are written on the device, where
-// mdkm_region_table finds them.  The overlaps follow (run_overlaps), then the tracks (run_tracks).
-int run_regions(mdkm_handle* h, const RegOut& g, const MapOut& m, const OvOut& o, const TrackOut& t) {
+// map receives this rank's range.  One synchronisation reads R -- and, with region overlaps `o` or
+// adjacency `adj`, the bounds of their pairs or days, counted right behind the ids -- then this
+// rank's points are summed into per-region slots, the slots are reduced over the ranks (sums;
+// minima of the first pixel and the bounds) and the table and means are written on the device,
+// where mdkm_region_table finds them.  The overlaps follow (run_overlaps), then the tracks (run_tracks),
+// then the adjacency (run_adjacency).
+int run_regions(mdkm_handle* h, const RegOut& g, const MapOut& m, const OvOut& o, const TrackOut& t, bool adj) {
   if (!g.conn) return MDKM_OK;
   const long long HW = (long long)h->raster_H * h->raster_w, n_px = (long long)h->stack_days * HW;
   const bool in_place = g.map && g.mem == MDKM_MEM_DEVICE && h->n_ranks == 1;  // (one rank holds the whole stack)
   OK(ensure(h, h->region_parent, (size_t)n_px));
   if (!in_place) OK(ensure(h, h->region_ids, (size_t)n_px));
   const long long n_chunks = (n_px + kRegChunk - 1) / kRegChunk;
-  const int n_pairs = o.n_pairs();
-  // look-back words of the numbering, ticket + fault, R, then the overlap bounds of the pairs
-  OK(ensure(h, h->region_scan, (size_t)n_chunks + 2 + n_pairs));
+  const int n_pairs = o.n_pairs(), n_adj = adj ? h->stack_days : 0;
+  // look-back words of the numbering, ticket + fault, R, the overlap bounds of the pairs, then the
+  // adjacency bounds of the days
+  OK(ensure(h, h->region_scan, (size_t)n_chunks + 2 + n_pairs + n_adj));
   RegionParams rp{};
   rp.map = m.whole;
   rp.parent = h->region_parent.p;
@@ -1401,7 +1429,7 @@ int run_regions(mdkm_handle* h, const RegOut& g, const MapOut& m, const OvOut& o
                         : (c8 ? region_border_kernel<unsigned char, true> : region_border_kernel<unsigned char, false>);
   tile_fn<<<(unsigned int)rp.n_tiles, kThreads, 0, h->stream>>>(rp);
   border_fn<<<(unsigned int)((rp.n_tiles + kThreads / 32 - 1) / (kThreads / 32)), kThreads, 0, h->stream>>>(rp);
-  CU(cudaMemsetAsync(h->region_scan.p, 0, ((size_t)n_chunks + 2 + n_pairs) * 8, h->stream));
+  CU(cudaMemsetAsync(h->region_scan.p, 0, ((size_t)n_chunks + 2 + n_pairs + n_adj) * 8, h->stream));
   region_number_kernel<<<(unsigned int)n_chunks, kThreads, 0, h->stream>>>(rp);
   region_resolve_kernel<<<grid_for(h, (n_px + 1023) / 1024, resident_per_sm(h, region_resolve_kernel)), kThreads, 0,
                           h->stream>>>(rp);
@@ -1411,6 +1439,15 @@ int run_regions(mdkm_handle* h, const RegOut& g, const MapOut& m, const OvOut& o
     op.bounds = h->region_scan.p + n_chunks + 2;
     overlap_bound_kernel<<<overlap_span_grid(HW, n_pairs), kThreads, 0, h->stream>>>(op);
     ++h->launches;
+  }
+  unsigned long long* adj_bounds = reinterpret_cast<unsigned long long*>(h->adj_bounds);
+  if (n_adj) {
+    AdjacencyParams ap{};
+    ap.ov = overlap_params(h, rp.ids, n_adj);
+    ap.ov.bounds = h->region_scan.p + n_chunks + 2 + n_pairs;
+    adjacency_bound_kernel<<<overlap_span_grid(HW, n_adj), kThreads, 0, h->stream>>>(ap);
+    ++h->launches;
+    OK(small_d2h(h, adj_bounds, ap.ov.bounds, (size_t)n_adj * 8, /*dst_is_pinned=*/true));
   }
   CU(cudaGetLastError());
   if (g.map && !in_place)
@@ -1459,7 +1496,8 @@ int run_regions(mdkm_handle* h, const RegOut& g, const MapOut& m, const OvOut& o
   }
   h->n_regions = R;
   OK(run_overlaps(h, o, rp.ids, got.data() + 2));
-  return run_tracks(h, t, o, rp.ids);
+  OK(run_tracks(h, t, o, rp.ids));
+  return run_adjacency(h, adj, rp.ids, adj_bounds);
 }
 
 // The region overlaps `o` of the region map `ids` (the whole stack, on every rank), behind the
@@ -1595,6 +1633,86 @@ int run_tracks(mdkm_handle* h, const TrackOut& t, const OvOut& o, const int* ids
   return MDKM_OK;
 }
 
+// The region adjacency of the R regions of the last run_regions in the region map `ids` (the
+// whole stack, on every rank), given the bounds of the days (region_adjacency.cuh): one hash table
+// per day sized from its bound, the keys inserted while the sides towards pixels without a point
+// and the raster border are summed, their first edges marked and the masks scanned (the overlap
+// passes, a day in place of a pair); one synchronisation reads M, then the rows are written and
+// the boundaries finished on the device, where mdkm_region_adjacency_table finds them.  Every rank
+// builds the whole table on its own.
+int run_adjacency(mdkm_handle* h, bool adj, const int* ids, const unsigned long long* bounds) {
+  if (!adj) return MDKM_OK;
+  const int D = h->stack_days;
+  const long long R = h->n_regions;
+  h->n_adjacency = 0;
+  if (R == 0) return MDKM_OK;
+  std::vector<long long> tab((size_t)D + 1, 0);
+  long long max_cap = 0;
+  for (int d = 0; d < D; ++d) {
+    long long cap = 0;
+    if (bounds[d]) for (cap = 2; cap < 2 * (long long)bounds[d]; cap <<= 1) {}
+    tab[d + 1] = tab[d] + cap;
+    max_cap = std::max(max_cap, cap);
+  }
+  AdjacencyParams ap{};
+  ap.ov = overlap_params(h, ids, D);
+  ap.ov.wpp = (2 * ap.ov.HW + 31) / 32;
+  const long long n_words = (long long)D * ap.ov.wpp;
+  const long long n_chunks = (n_words + kOvChunkWords - 1) / kOvChunkWords, padded = n_chunks * kOvChunkWords;
+  const bool keyed = tab[D] > 0;  // some day has an edge between two regions
+  OK(ensure(h, h->adj_tab, tab.size()));
+  OK(ensure(h, h->adj_sides, 4 * (size_t)R));
+  if (keyed) {
+    OK(ensure(h, h->adj_slots, 2 * (size_t)tab[D]));
+    OK(ensure(h, h->adj_bits, 2 * (size_t)padded));
+    OK(ensure(h, h->adj_scan, 2 * (size_t)n_chunks + 3));
+  }
+  CU(cudaMemcpyAsync(h->adj_tab.p, tab.data(), tab.size() * 8, cudaMemcpyHostToDevice, h->stream));
+  CU(cudaMemsetAsync(h->adj_sides.p, 0, (size_t)R * 32, h->stream));
+  ap.ov.tab = h->adj_tab.p;
+  ap.sides = h->adj_sides.p;
+  ap.n_regions = R;
+  if (keyed) {
+    CU(cudaMemsetAsync(h->adj_slots.p, 0, (size_t)tab[D] * 16, h->stream));
+    CU(cudaMemsetAsync(h->adj_bits.p, 0, (size_t)padded * 4, h->stream));
+    CU(cudaMemsetAsync(h->adj_scan.p, 0, (2 * (size_t)n_chunks + 3) * 8, h->stream));
+    ap.ov.slots = h->adj_slots.p;
+    ap.ov.bits = h->adj_bits.p;
+    ap.ov.word_rel = h->adj_bits.p + padded;
+    ap.ov.status = h->adj_scan.p;
+    ap.ov.chunk_base = h->adj_scan.p + n_chunks;
+    ap.ov.ticket = reinterpret_cast<unsigned int*>(h->adj_scan.p + 2 * n_chunks);
+    ap.ov.total = h->adj_scan.p + 2 * n_chunks + 1;
+    ap.ov.probe_fault = reinterpret_cast<unsigned int*>(h->adj_scan.p + 2 * n_chunks + 2);
+  }
+  const dim3 slot_grid((unsigned int)grid_for(h, (max_cap + kThreads - 1) / kThreads, 4),
+                       (unsigned int)std::min(D, 65535));
+  const int per_region = grid_for(h, (R + kThreads - 1) / kThreads, 4);
+  adjacency_insert_kernel<<<overlap_span_grid(ap.ov.HW, D), kThreads, 0, h->stream>>>(ap);
+  ++h->launches;
+  if (keyed) {
+    overlap_mark_kernel<<<slot_grid, kThreads, 0, h->stream>>>(ap.ov);
+    overlap_scan_kernel<<<(unsigned int)n_chunks, kThreads, 0, h->stream>>>(ap.ov, n_chunks);
+    h->launches += 2;
+    CU(cudaGetLastError());
+    unsigned long long got[3] = {0, 0, 0};  // ticket | fault << 32, M, probe fault
+    OK(small_d2h(h, got, ap.ov.ticket, 24));
+    OK(sync_small(h));
+    if (got[0] >> 32) return fail(h, MDKM_ERR_CUDA, "region adjacency: the look-back over the chunks timed out");
+    if (got[2]) return fail(h, MDKM_ERR_CUDA, "region adjacency: a hash table had no free slot");
+    const long long M = (long long)got[1];
+    OK(ensure(h, h->adj_rows, (size_t)M * 6));
+    ap.ov.rows = h->adj_rows.p;
+    adjacency_emit_kernel<<<slot_grid, kThreads, 0, h->stream>>>(ap);
+    ++h->launches;
+    h->n_adjacency = M;
+  }
+  adjacency_finish_kernel<<<per_region, kThreads, 0, h->stream>>>(ap);
+  ++h->launches;
+  CU(cudaGetLastError());
+  return MDKM_OK;
+}
+
 // Takes the outputs bound for a call with k clusters into `o`.  The bindings are moved out of the
 // handle first, so the call consumes every one of them whatever happens.  When several checks
 // fail the first in this order is reported, except that the cluster map's comes after the day
@@ -1604,12 +1722,14 @@ int take_outputs(mdkm_handle* h, int k, CallOutputs& o) {
   o.reg = {b.regions, b.region_map, b.region_map_mem};
   o.ov.pairs = std::move(b.ov_pairs);
   o.trk = {b.track_iou, b.track_map, b.track_map_mem};
+  o.adj = b.adjacency;
   const int map_rc = take_cluster_map(h, k, b, o.map);
   OK(take_day_stats(h, k, b, o.stats));
   OK(map_rc);
   OK(take_transitions(h, k, b, o.map, o.trans));
   OK(take_tracks(h, o.reg, o.ov, o.trk));
   OK(take_overlaps(h, o.reg, o.ov));
+  OK(take_adjacency(h, o.reg, o.adj));
   return take_regions(h, k, o.map, o.reg);
 }
 
@@ -1621,10 +1741,10 @@ int reduce_outputs(mdkm_handle* h, const CallOutputs& o) {
   return run_transitions(h, o.trans, o.map);
 }
 
-// After the call's synchronisation: the regions of `o` with their overlaps and tracks, then the
-// day statistics and transitions handed to the caller.
+// After the call's synchronisation: the regions of `o` with their overlaps, tracks and adjacency,
+// then the day statistics and transitions handed to the caller.
 int deliver_outputs(mdkm_handle* h, const CallOutputs& o) {
-  OK(run_regions(h, o.reg, o.map, o.ov, o.trk));
+  OK(run_regions(h, o.reg, o.map, o.ov, o.trk, o.adj));
   deliver_day_stats(h, o.stats);
   deliver_transitions(h, o.trans);
   return MDKM_OK;
@@ -1818,6 +1938,9 @@ void mdkm_destroy(mdkm_handle* h) {
   release(h->ov_rows);
   release(h->track_link_day); release(h->track_parent); release(h->track_links); release(h->track_ids);
   release(h->track_scan); release(h->track_tab); release(h->track_stage);
+  release(h->adj_tab); release(h->adj_slots); release(h->adj_bits); release(h->adj_scan); release(h->adj_rows);
+  release(h->adj_sides);
+  if (h->adj_bounds) cudaFreeHost(h->adj_bounds);
   release(h->kpp_closest); release(h->kpp_cell); release(h->kpp_blk); release(h->kpp_prefix);
   release(h->kpp_partials); release(h->kpp_rand); release(h->kpp_state);
   if (h->d_status) cudaFree(h->d_status);
@@ -2233,6 +2356,42 @@ int mdkm_track_table(mdkm_handle* h, int64_t* table_out, int32_t* region_tracks_
   if (table_out) CU(cudaMemcpyAsync(table_out, h->track_tab.p, (size_t)T * 56, cudaMemcpyDeviceToHost, h->stream));
   if (region_tracks_out)
     CU(cudaMemcpyAsync(region_tracks_out, h->track_ids.p, (size_t)R * 4, cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
+  return MDKM_OK;
+}
+
+int mdkm_bind_region_adjacency(mdkm_handle* h, int on) {
+  if (!h) return MDKM_ERR_INVALID;
+  h->bound.adjacency = false;
+  if (!on) return MDKM_OK;
+  if (!h->have_points || h->raster_w <= 0)
+    return fail(h, MDKM_ERR_STATE, "region adjacency needs a resident cloud from mdkm_unproject");
+  h->bound.adjacency = true;
+  return MDKM_OK;
+}
+
+int mdkm_region_adjacency_count(const mdkm_handle* h, int64_t* n_rows) {
+  if (!h || !n_rows) return MDKM_ERR_INVALID;
+  if (h->n_adjacency < 0)
+    return fail(const_cast<mdkm_handle*>(h), MDKM_ERR_STATE, "no region adjacency: no fit / predict with region adjacency since the last unproject / set_points or fit / predict with regions");
+  *n_rows = h->n_adjacency;
+  return MDKM_OK;
+}
+
+int mdkm_region_adjacency_table(mdkm_handle* h, int64_t* rows_out, int64_t* boundaries_out, int64_t capacity_rows,
+                                int64_t capacity_regions) {
+  if (!h) return MDKM_ERR_INVALID;
+  if (h->n_adjacency < 0)
+    return fail(h, MDKM_ERR_STATE, "no region adjacency: no fit / predict with region adjacency since the last unproject / set_points or fit / predict with regions");
+  const long long M = h->n_adjacency, R = h->n_regions;
+  if (rows_out && capacity_rows < M)
+    return fail(h, MDKM_ERR_INVALID, "region adjacency table: capacity %lld < %lld rows", (long long)capacity_rows, M);
+  if (boundaries_out && capacity_regions < R)
+    return fail(h, MDKM_ERR_INVALID, "region boundaries: capacity %lld < %lld regions", (long long)capacity_regions, R);
+  CU(cudaSetDevice(h->device));
+  if (rows_out && M) CU(cudaMemcpyAsync(rows_out, h->adj_rows.p, (size_t)M * 48, cudaMemcpyDeviceToHost, h->stream));
+  if (boundaries_out && R)
+    CU(cudaMemcpyAsync(boundaries_out, h->adj_sides.p, (size_t)R * 32, cudaMemcpyDeviceToHost, h->stream));
   CU(cudaStreamSynchronize(h->stream));
   return MDKM_OK;
 }

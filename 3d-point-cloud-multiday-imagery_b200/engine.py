@@ -476,8 +476,21 @@ class Engine:
                                                c_void_p(region_tracks.ctypes.data), int(n.value), int(r.value)))
         return table, region_tracks
 
+    def _region_adjacency_table(self):
+        """The region adjacency of the last fit / predict that had it -> (rows int64 ``[M,6]``,
+        region boundaries int64 ``[R,4]``)."""
+        n, r = c_int64(0), c_int64(0)
+        self._check(self._lib.mdkm_region_adjacency_count(self._h, byref(n)))
+        self._check(self._lib.mdkm_region_count(self._h, byref(r)))
+        rows = np.empty((n.value, 6), dtype=np.int64)
+        boundaries = np.empty((r.value, 4), dtype=np.int64)
+        self._check(self._lib.mdkm_region_adjacency_table(self._h, c_void_p(rows.ctypes.data),
+                                                          c_void_p(boundaries.ctypes.data), int(n.value), int(r.value)))
+        return rows, boundaries
+
     def _bind_outputs(self, k, cluster_map_out=None, day_stats=False, transitions=None, regions=None,
-                      region_map_out=None, region_overlaps=None, tracks=None, track_map_out=None):
+                      region_map_out=None, region_overlaps=None, tracks=None, track_map_out=None,
+                      region_adjacency=False):
         """Bind the optional outputs of the next fit / predict (the keywords of ``fit``) -> (whether
         a pixel map is device memory, (counts, means) or None, transitions or None).  When one
         binding is refused none is left behind: the statistics and transition arrays live only in
@@ -491,6 +504,8 @@ class Engine:
             raise ValueError("tracks needs regions=4 or regions=8")
         if track_map_out is not None and tracks is None:
             raise ValueError("track_map_out needs tracks=min_iou")
+        if region_adjacency and regions is None:
+            raise ValueError("region_adjacency needs regions=4 or regions=8")
         try:
             map_mem = self._bind_cluster_map(cluster_map_out) if cluster_map_out is not None else None
             stats = self._bind_day_stats(k) if day_stats else None
@@ -499,6 +514,8 @@ class Engine:
             if region_overlaps is not None:
                 self._bind_region_overlaps(region_overlaps)
             trk_mem = self._bind_tracks(tracks, track_map_out) if tracks is not None else None
+            if region_adjacency:
+                self._check(self._lib.mdkm_bind_region_adjacency(self._h, 1))
         except BaseException:
             self._lib.mdkm_bind_cluster_map(self._h, None, 1, 0, C.MEM_HOST)
             self._lib.mdkm_bind_day_stats(self._h, None, None, 0, 0)
@@ -506,12 +523,14 @@ class Engine:
             self._lib.mdkm_bind_regions(self._h, 0, None, 0, C.MEM_HOST)
             self._lib.mdkm_bind_region_overlaps(self._h, None, 0)
             self._lib.mdkm_bind_tracks(self._h, 0.0, None, 0, C.MEM_HOST)
+            self._lib.mdkm_bind_region_adjacency(self._h, 0)
             raise
         return C.MEM_DEVICE in (map_mem, reg_mem, trk_mem), stats, trans
 
-    def _read_outputs(self, stats, trans, regions, region_overlaps, tracks) -> dict:
+    def _read_outputs(self, stats, trans, regions, region_overlaps, tracks, region_adjacency=False) -> dict:
         """The optional results of the last fit / predict that were asked for, in ``predict``'s order:
-        day_counts, day_means, transitions, regions, region_means, region_overlaps, tracks, region_tracks."""
+        day_counts, day_means, transitions, regions, region_means, region_overlaps, tracks, region_tracks,
+        region_adjacency, region_boundaries."""
         out = {}
         if stats is not None:
             out["day_counts"], out["day_means"] = stats
@@ -523,6 +542,8 @@ class Engine:
             out["region_overlaps"] = self._region_overlap_table()
         if tracks is not None:
             out["tracks"], out["region_tracks"] = self._track_table()
+        if region_adjacency:
+            out["region_adjacency"], out["region_boundaries"] = self._region_adjacency_table()
         return out
 
     @property
@@ -550,7 +571,7 @@ class Engine:
     # -- k-means -------------------------------------------------------------------------
     def fit(self, init, max_iter=300, tol=1e-4, want_labels=True, labels_out=None, cluster_map_out=None,
             day_stats=False, transitions=None, regions=None, region_map_out=None, region_overlaps=None,
-            tracks=None, track_map_out=None):
+            tracks=None, track_map_out=None, region_adjacency=False):
         """One Lloyd run from explicit centroids.  Returns dict(labels, centers, n_iter, inertia, ...).
 
         ``cluster_map_out``: optional uint8 (k <= 255) or uint16 array / tensor, host or CUDA, with
@@ -599,7 +620,18 @@ class Engine:
         index r - 1.  ``track_map_out``: optional int32 array / tensor, host or CUDA, like
         ``region_map_out``; it receives the track id of every pixel, 0 where no point.  Built on
         the GPU from the region map and the overlaps of consecutive days; the caller's own
-        ``region_overlaps`` stay as they are without tracks."""
+        ``region_overlaps`` stay as they are without tracks.
+
+        ``region_adjacency=True`` (needs ``regions``, else ``ValueError`` before any GPU work): the
+        result also has ``region_adjacency``, int64 ``[M,6]`` rows (day, region_a, region_b, edges,
+        y_first, x_first): one for every pair of regions a < b of one day joined by at least one
+        edge between 4-neighbouring pixels, with the number of such edges (their shared border) and
+        the upper or left pixel of their first edge, sorted by that edge (index 2 (y W + x) +
+        direction, 0 to the right and 1 downwards, within the day).  Corner contacts have no row.
+        And ``region_boundaries``, int64 ``[R,4]`` (perimeter, region_edges, background_edges,
+        border_edges) of region r at index r - 1: the sides of its pixels facing another region,
+        a pixel without a point and the raster edge, and their sum.  Counted on the GPU from the
+        region map; with several ranks every rank builds the same rows."""
         init = np.ascontiguousarray(init, dtype=np.float64)
         if init.ndim != 2 or init.shape[1] != 3:
             raise ValueError("init must be [K,3]")
@@ -619,7 +651,8 @@ class Engine:
         inertia = c_double(0.0)
         dev_maps, stats, trans = self._bind_outputs(
             k, cluster_map_out=cluster_map_out, day_stats=day_stats, transitions=transitions, regions=regions,
-            region_map_out=region_map_out, region_overlaps=region_overlaps, tracks=tracks, track_map_out=track_map_out)
+            region_map_out=region_map_out, region_overlaps=region_overlaps, tracks=tracks, track_map_out=track_map_out,
+            region_adjacency=region_adjacency)
         self._check(self._lib.mdkm_fit(
             self._h, int(k), init.ctypes.data_as(POINTER(c_double)), int(max_iter), float(tol),
             c_void_p(lab_ptr) if lab_ptr else None, lab_mem,
@@ -636,7 +669,7 @@ class Engine:
             "n_relocations": int(nrel.value), "tol_scaled": float(tols.value),
             "worklist_groups": int(work.value), "groups": int(groups.value),
         }
-        out.update(self._read_outputs(stats, trans, regions, region_overlaps, tracks))
+        out.update(self._read_outputs(stats, trans, regions, region_overlaps, tracks, region_adjacency))
         return out
 
     def lloyd_step(self, centroids, want_labels=True):
@@ -656,14 +689,17 @@ class Engine:
         return labels, sums, counts, int(nref.value)
 
     def predict(self, centroids, want_labels=True, cluster_map_out=None, day_stats=False, transitions=None,
-                regions=None, region_map_out=None, region_overlaps=None, tracks=None, track_map_out=None):
+                regions=None, region_map_out=None, region_overlaps=None, tracks=None, track_map_out=None,
+                region_adjacency=False):
         """E-step only (KMeans.predict): returns (labels int32[N] or None, inertia).
         ``cluster_map_out``: as in ``fit``.  ``day_stats=True``: returns
         (labels, inertia, day_counts, day_means) instead, as in ``fit``.  ``transitions``: day
         pairs as in ``fit``; their counts are appended to the returned tuple.  ``regions`` /
         ``region_map_out``: as in ``fit``; the table and the means are appended after that.
         ``region_overlaps``: as in ``fit``; the rows are appended after that.  ``tracks`` /
-        ``track_map_out``: as in ``fit``; the track table and the region tracks are appended last."""
+        ``track_map_out``: as in ``fit``; the track table and the region tracks are appended after
+        that.  ``region_adjacency``: as in ``fit``; the rows and the region boundaries are appended
+        last."""
         c = np.ascontiguousarray(centroids, dtype=np.float64)
         if c.ndim != 2 or c.shape[1] != 3:
             raise ValueError("centroids must be [K,3]")
@@ -671,13 +707,14 @@ class Engine:
         inertia = c_double(0.0)
         dev_maps, stats, trans = self._bind_outputs(
             c.shape[0], cluster_map_out=cluster_map_out, day_stats=day_stats, transitions=transitions, regions=regions,
-            region_map_out=region_map_out, region_overlaps=region_overlaps, tracks=tracks, track_map_out=track_map_out)
+            region_map_out=region_map_out, region_overlaps=region_overlaps, tracks=tracks, track_map_out=track_map_out,
+            region_adjacency=region_adjacency)
         self._check(self._lib.mdkm_predict(
             self._h, int(c.shape[0]), c.ctypes.data_as(POINTER(c_double)),
             c_void_p(labels.ctypes.data) if labels is not None else None, C.MEM_HOST, byref(inertia)))
         if dev_maps:
             self._before_torch()
-        results = self._read_outputs(stats, trans, regions, region_overlaps, tracks)
+        results = self._read_outputs(stats, trans, regions, region_overlaps, tracks, region_adjacency)
         return (labels, float(inertia.value)) + tuple(results.values())
 
     def kmeans_plusplus(self, n_clusters: int, random_state):

@@ -345,6 +345,59 @@ int mdkm_track_count(const mdkm_handle* h, int64_t* n_tracks);
 int mdkm_track_table(mdkm_handle* h, int64_t* table_out, int32_t* region_tracks_out, int64_t capacity_tracks,
                      int64_t capacity_regions);
 
+/* Optional: have the NEXT mdkm_fit or mdkm_predict on this handle, which must also have regions
+ * bound (mdkm_bind_regions), return the adjacency of the regions within each day: which objects of
+ * one day touch, along how long a border, and each region's perimeter.  An edge joins two
+ * 4-neighbouring pixels of one day: direction 0 joins (y, x) and (y, x+1), direction 1 joins (y, x)
+ * and (y+1, x); its index within the day is e = 2 (y W + x) + direction, and edges are ordered by
+ * (day, e).  After the call, mdkm_region_adjacency_count gives the number of rows M and
+ * mdkm_region_adjacency_table copies them, int64 [M][6]: day, region_a, region_b, edges, y_first,
+ * x_first -- one row for every unordered pair of distinct regions r = region_a < s = region_b
+ * joined by at least one edge, with the number of edges between them (their shared border in pixel
+ * edges) and the upper or left pixel of their first edge.  Rows are sorted by that first edge;
+ * every edge belongs to at most one row, so the order is total and does not depend on the schedule
+ * or the number of ranks.  Regions that touch only at a corner have no row, under either
+ * connectivity; regions that share an edge have different clusters.  It also copies the region
+ * boundaries, int64 [R][4], row r - 1 for region r: perimeter (the sides of the region's pixels
+ * whose other side is not in the region), region_edges (sides facing another region: the sum of
+ * `edges` over the rows of r), background_edges (sides facing a pixel of the same day without a
+ * point) and border_edges (sides on the edge of the H x W grid); perimeter = region_edges +
+ * background_edges + border_edges, and 4 pixels = perimeter + 2 x (edges inside the region).
+ * Where the numbers come from: behind the region ids, a pass counts for every day the run starts
+ * along each image row of the horizontal key (id[p], id[p+1]) and of the vertical key (id[p],
+ * id[p+W]) of two different non-zero ids, an upper bound on the day's rows, read by the
+ * synchronisation that reads R (no extra one).  Each day gets an open-addressing hash table of
+ * 16-byte slots keyed min << 32 | max (the smallest power of two >= 2 x its bound); equal keys are
+ * combined in the warp, and their leaders add the edges and lower the first edge with atomics; the
+ * same pass adds every pixel's background and border sides to its region, summed per warp.  Every
+ * occupied slot sets the bit of its first edge in a 2 H W-bit mask per day, the popcount scan of
+ * the region overlaps gives each slot its row, and one more synchronisation reads M; the rows are
+ * then written and each row's edges added to both regions' region_edges.  Memory: 16 B x table
+ * capacity (<= 128 B per pixel) plus 8 B per 16 pixels (mask and scan offsets), 48 B per row and
+ * 32 B per region; the worst case, where every edge is a row of its own, is a one-pixel
+ * checkerboard (2 rows per pixel: 96 B of rows and 64 to 128 B of table per pixel).  A failed
+ * allocation returns MDKM_ERR_OOM.
+ * With several ranks every rank builds the whole table from its whole-stack region map: no
+ * collective, the same bits on every rank, and every rank pays the whole cost.  Asking for
+ * adjacency changes no other result of the call.
+ * on == 0 clears the binding.  The binding is consumed by that one call, and dropped by
+ * mdkm_unproject / mdkm_set_points.  Errors: MDKM_ERR_STATE when the resident cloud did not come
+ * from mdkm_unproject; from the mdkm_fit / mdkm_predict, before any work is enqueued,
+ * MDKM_ERR_STATE when no regions are bound for that call. */
+int mdkm_bind_region_adjacency(mdkm_handle* h, int on);
+
+/* The region adjacency of the last mdkm_fit / mdkm_predict that had it bound, kept on the device
+ * until the next mdkm_unproject / mdkm_set_points or fit / predict with regions (a later call with
+ * regions but without adjacency drops it).  mdkm_region_adjacency_count: the number of rows M.
+ * mdkm_region_adjacency_table: copies the rows (rows_out, int64 [M][6]) and the region boundaries
+ * (boundaries_out, int64 [R][4]) to host memory; either may be NULL.  Errors: MDKM_ERR_STATE when
+ * there is none (none computed since the last unproject / set_points); MDKM_ERR_INVALID from
+ * mdkm_region_adjacency_table when rows_out is given and capacity_rows < M, or boundaries_out is
+ * given and capacity_regions < R. */
+int mdkm_region_adjacency_count(const mdkm_handle* h, int64_t* n_rows);
+int mdkm_region_adjacency_table(mdkm_handle* h, int64_t* rows_out, int64_t* boundaries_out, int64_t capacity_rows,
+                                int64_t capacity_regions);
+
 /* Load an already unprojected cloud (this rank's shard).  Replaces the `X` argument of the
  * reference's KMeans(...).fit_predict(X) call (members/jasraj/land_use_classification/
  * core.py:227-228) for d = 3. */
